@@ -11,7 +11,11 @@ tail kernel over NVLink peer memory (reduce-scatter, prior + Adagrad on the owne
 VAEB_DP_P2P=0: ncclAllReduce + replicated Adagrad).  Total work per step is fixed => "scaling": "strong".
 
   value  device-resident: the rank's rows already in HBM (several minibatches, > L2 in total, visited in turn),
-         K updates enqueued back to back, CUDA events on the launch stream, max over ranks.
+         K updates enqueued back to back, CUDA events on the launch stream, max over ranks.  The K timed updates
+         start from the same state in every run (seeded data and parameters, W warm-up updates, Philox noise):
+         --dump-outputs DIR writes what the last of them left for the caller -- its bound (bound.npy) and the
+         parameters and Adagrad accumulators it wrote (param_<name>.npy, ada_<name>.npy; float32, 6.5 MB) -- so
+         that two builds can be compared output for output.
   e2e    the reference-facing call with HOST inputs: every step copies ITS minibatch share from pinned host memory
          (H2D) and reads ITS bound back (D2H); streaming form (vaeb_update_host_async + vaeb_collect).
          e2e.sync_call: the synchronous call; e2e.u8_host: the same streaming call fed uint8 pixels (a quarter of the
@@ -129,6 +133,27 @@ def make_problem(seed=15485863):
     return synthetic_mnist(N_TRAIN, seed=seed)
 
 
+def reset_state(m, params, ada):
+    """Puts back everything an update reads besides the data: parameters, Adagrad accumulators and the Philox step
+    counter (0 after construction), so that what follows does not depend on how many updates ran before."""
+    from vaeb_b200 import _lib
+    m.set_params(params)
+    m._set_buffer(_lib.BUF_ADA, ada)
+    _lib.check(m._lib.vaeb_set_step_counter(m._h, 0))
+
+
+def dump_outputs(out_dir, m, bounds):
+    """The last timed update as its caller sees it: the bound it returned and the parameters and Adagrad
+    accumulators it left on the device, as out_dir/<name>.npy (float32)."""
+    from vaeb_b200 import _lib
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"bound": np.asarray(bounds[-1:], np.float32)}
+    for p, v, a in zip(m.params, m.get_params(), m._get_buffer(_lib.BUF_ADA)):
+        arrays["param_" + p.name], arrays["ada_" + p.name] = v, a
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------
 # reference arm / cpu baseline: the oracle port on the host cores
 # ------------------------------------------------------------------------------------------
@@ -210,7 +235,7 @@ def run_own(args):
 
     import vaeb_b200
     from vaeb_b200.data import synthetic_mnist, synthetic_frey
-    from vaeb_b200 import distributed as vd
+    from vaeb_b200 import _lib, distributed as vd
     stream = torch.cuda.current_stream()
     peaks = measured_peaks()
 
@@ -246,6 +271,7 @@ def run_own(args):
     m3.set_stream(stream.cuda_stream)
     if world > 1:
         vd.attach_data_parallel(m3)
+    params0, ada0 = m3.get_params(), m3._get_buffer(_lib.BUF_ADA)
 
     def order3(n, start=0):
         return (np.arange(start, start + n) % nb3).astype(np.int32)
@@ -273,6 +299,12 @@ def run_own(args):
             break
         prev_ms = cur_ms
     probe_ms_per_step = cur_ms / n_probe
+    # the ramp ran as many updates as the clocks needed: start again from the initial state and replay the fixed
+    # warm-up, so that the timed updates compute the same thing in every run
+    barrier()
+    reset_state(m3, params0, ada0)
+    barrier()
+    m3.update_many(order3(max(W, 3)))
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     order_k = order3(K, 1)
     barrier()
@@ -288,6 +320,8 @@ def run_own(args):
     clocks.__exit__(None, None, None)
     clocks_summary = clocks.summary(*window)
     value = K * MG / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, m3, elbos)
 
     # ---- e2e: every step copies its minibatch share H2D from pinned host memory and reads its bound back D2H ----
     pinned = torch.empty((per * nb3, D), dtype=torch.float32, pin_memory=True)
@@ -540,7 +574,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-also", action="store_true", help="skip the side measurements (c1, c2, c4, c5, Adagrad)")
     ap.add_argument("--precision", default=C3_PREC, choices=["fp32", "bf16x3", "bf16"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the bound, parameters and Adagrad accumulators of the last timed update as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "own":
+        ap.error("--dump-outputs writes the outputs of --impl own")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,9 +1,11 @@
 """Generates tests/golden/*.npz.  Run in the build container (needs /root/reference):
     python tests/golden/make_golden.py
 
-frey_z2_trained.npz  -- the trained fp32 Frey weights the reference ships in
+frey_z2_trained_{encoder,decoder}.npz
+                     -- the trained fp32 Frey weights the reference ships in
                         reconstruction_res/continuous_2.mdl (12 tensors, reference order),
-                        extracted with the restricted unpickler (vaeb_b200/io.py).
+                        extracted with the restricted unpickler (vaeb_b200/io.py); W3-W5, b3-b5
+                        in the first file, W1, W2, W6, b1, b2, b6 in the second.
 golden_frey_z2.npz   -- oracle (fp64) outputs for those weights on seeded synthetic
                         Frey-shaped rows with seeded eps: per-row bound, SGVB, gradient
                         fingerprints, parameters after one Adagrad step, IS estimates.
@@ -54,8 +56,11 @@ def main():
     # ---- trained Frey weights -------------------------------------------------------
     header, params = io.read_mdl(os.path.join(REF, "reconstruction_res", "continuous_2.mdl"))
     assert header["continuous"] and header["n_latent"] == 2 and header["n_hidden_units"] == 200
-    np.savez_compressed(os.path.join(HERE, "frey_z2_trained.npz"),
-                        **{n: p for n, p in zip(O.param_names(True), params)})
+    named = dict(zip(O.param_names(True), params))
+    enc = ("W3", "W4", "W5", "b3", "b4", "b5")          # two halves, so that neither file exceeds 1 MB
+    np.savez_compressed(os.path.join(HERE, "frey_z2_trained_encoder.npz"), **{n: named[n] for n in enc})
+    np.savez_compressed(os.path.join(HERE, "frey_z2_trained_decoder.npz"),
+                        **{n: p for n, p in named.items() if n not in enc})
     x = O.synthetic_frey(300)
     g = {"x_seed": np.int64(15485863)}
     for est in ("LB", "LA"):

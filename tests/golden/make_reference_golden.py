@@ -220,13 +220,13 @@ def main():
     from vaeb_b200 import io
     _, trained = io.read_mdl(os.path.join(REF, "reconstruction_res", "continuous_2.mdl"))
     x = cont_x(300, 560)
-    g = {}
+    g = {"x": x.astype(np.float32)}                 # the rows of both estimators, stored once (keeps the file < 1 MB)
     for est, generic in (("LB", False), ("LA", True)):
         r = run_vaeb_case(V, th, x, True, 200, 2, 100, 1, 0.01, generic, order=[1, 0], n_valid=300,
                           params0=[np.asarray(p, np.float64) for p in trained])
         for k, v in r.items():
-            if k.startswith("init_"):
-                continue                            # = tests/golden/frey_z2_trained.npz
+            if k.startswith("init_") or k == "x":
+                continue                            # init_ = tests/golden/frey_z2_trained_{encoder,decoder}.npz
             if k.startswith(("final_W", "ada_W")) and v.size > 2000:
                 v = fingerprint(v)
                 k = "fp_" + k

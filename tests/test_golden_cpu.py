@@ -103,13 +103,12 @@ def test_restricted_unpickler_never_imports_foreign_classes(tmp_path):
     from vaeb_b200 import io
 
     f = str(tmp_path / "evil.mdl")
+    marker = tmp_path / "pwned"
     with open(f, "wb") as fh:
-        fh.write(b"cos\nsystem\n(S'echo pwned > /tmp/vaeb_pwned'\ntR.")
-    if os.path.exists("/tmp/vaeb_pwned"):
-        os.remove("/tmp/vaeb_pwned")
+        fh.write(b"cos\nsystem\n(S'echo pwned > " + str(marker).encode() + b"'\ntR.")
     with pytest.raises(Exception):
         io.read_mdl(f)
-    assert not os.path.exists("/tmp/vaeb_pwned")
+    assert not marker.exists()
 
 
 def test_trace_layout(tmp_path):

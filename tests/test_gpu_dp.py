@@ -26,7 +26,7 @@ def _free_port():
 def test_dp_step_matches_oracle_over_nccl(tmp_path, world, p2p):
     import torch
     if torch.cuda.device_count() < world:
-        pytest.skip("needs %d GPUs (run under `gpurun --gpus %d`)" % (world, world))
+        pytest.skip("needs %d GPUs" % world)
     out = tmp_path / "dp.json"
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(world),
            "--master-addr", "127.0.0.1", "--master-port", str(_free_port()),

@@ -12,7 +12,9 @@ def load_golden(name):
 
 
 def frey_trained_params():
-    z = load_golden("frey_z2_trained.npz")
+    # stored in two halves so that neither file exceeds 1 MB
+    z = load_golden("frey_z2_trained_encoder.npz")
+    z.update(load_golden("frey_z2_trained_decoder.npz"))
     return [z[n] for n in O.param_names(True)]
 
 
