@@ -1,6 +1,6 @@
 """Worker of tests/test_gpu_c3_paths.py: three large-batch updates (bf16x3 or bf16) with whatever launch structure the
-environment selects (VAEB_TC_CHAIN / VAEB_TC_PAIR / VAEB_TC_WGRAD_MERGE / VAEB_TC_TAIL are read once per process);
-bounds, parameters and Adagrad accumulators go to an .npz."""
+environment selects (VAEB_TC_TAIL is read once per process); bounds, parameters, Adagrad accumulators and the launch
+count go to an .npz."""
 import os
 import sys
 

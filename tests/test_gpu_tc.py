@@ -112,27 +112,3 @@ def test_is_logpx_tensor_core_philox_sharding_invariance():
     np.testing.assert_allclose(whole, ref, rtol=1e-2)
     m.close(); m32.close()
 
-
-def test_is_logpx_cta_pair_form_matches_oracle(tmp_path):
-    """The cta_group::2 form of the importance-sampling kernel (VAEB_IS_PAIR=1; measured slower than the single-CTA form
-    and therefore off by default, DESIGN 4.4) stays correct: same estimates as the oracle at the bf16 tier.  The switch is
-    read once per process, hence the subprocess."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = str(tmp_path / "pair.npz")
-    code = (
-        "import sys, numpy as np\n"
-        "sys.path.insert(0, %r)\n"
-        "from tests.test_gpu_tc import _is_case\n"
-        "lp, lw, ref_lp, ref_lw = _is_case(784, 500, 20, 4, 256, 11, 0.08)\n"      # 4 points x 2 tiles: pairs
-        "lpg, lwg, ref_lpg, ref_lwg = _is_case(560, 200, 2, 2, 384, 12, 0.08, continuous=True)\n"
-        "np.savez(%r, lp=lp, lw=lw, ref_lp=ref_lp, ref_lw=ref_lw, lpg=lpg, ref_lpg=ref_lpg)\n" % (root, out))
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300, cwd=root,
-                       env=dict(os.environ, VAEB_IS_PAIR="1"))
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    d = np.load(out)
-    np.testing.assert_allclose(d["lw"], d["ref_lw"], rtol=1e-2, atol=1e-2)
-    np.testing.assert_allclose(d["lp"], d["ref_lp"], rtol=1e-2, atol=1e-2)
-    np.testing.assert_allclose(d["lpg"], d["ref_lpg"], rtol=1e-2, atol=1e-2)

@@ -291,30 +291,16 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
   TcState& t = h->tc;
   int x_row_off = 0, bn = 64, bna = 64;   // UMMA N of the weight-gradient / of the activation layers
   int bnd = 64;                           // ... of dec2 (D wide: more column tiles per row block than the H-wide layers)
-  int bnt = 0;                            // ... of the thin layers dec1 / dgrad h_e when they differ (persistent, narrow tiles)
-  bool chain = false, chain_pair = false;
   const void *x_mirror_hi = nullptr, *x_mirror_lo = nullptr;
   if (tcp) {
     VAEB_TRY(tc_ensure(h, rows, R));
     bn = R >= 1024 ? 128 : 64;
     bna = tc_act_bn(rows, std::min(H, D));
-    static const int env_bn = getenv("VAEB_TC_BN") ? atoi(getenv("VAEB_TC_BN")) : 0;     // measurement switch
-    if (env_bn == 64 || env_bn == 128 || env_bn == 256) bna = env_bn;
-    // the activation chain as ONE launch (tc_chain.cu, VAEB_TC_CHAIN=1): large-batch training steps of the Bernoulli model.
-    // In its CTA-pair form (cta_group::2) a CTA stages half of a 256-wide B tile: the maps carry 128-wide boxes.
-    static const int env_chain = getenv("VAEB_TC_CHAIN") ? atoi(getenv("VAEB_TC_CHAIN")) : -1;   // measurement switches
-    static const int env_pair = getenv("VAEB_TC_PAIR") ? atoi(getenv("VAEB_TC_PAIR")) : -1;
-    chain = want_grads && !h->cont && L == 1 && latent_large_batch(rows, H, Z, L) && 4 * ((2 * Z + 63) / 64) <= Z &&
-            env_chain > 0;      // measured: not faster than the seven layer launches at any size (DESIGN 4.3b) -> opt-in
-    chain_pair = chain && (env_pair >= 0 ? env_pair != 0 : rows >= 4096);
-    if (chain_pair) bna = 128;
     bnd = bna;
     // few row blocks (the data-parallel split): one tile per CTA, and a layer should fill most of the SMs in ONE wave --
     // 64-wide tiles for the H-wide layers when 128-wide ones give fewer than 96 CTAs (2048 rows: 64 -> 128 CTAs, enc1
     // 14.5 -> 12.2 us, dgrad 15.6 -> 13.1), dec2 keeps 128 (7 column tiles per row block: 112 CTAs)
-    static const int env_thin = getenv("VAEB_TC_THIN_BN") ? atoi(getenv("VAEB_TC_THIN_BN")) : 0;    // measurement switch
-    if (bna == 256 && !chain && (env_thin == 64 || env_thin == 128)) bnt = env_thin;
-    if (bna == 128 && env_bn == 0 && !chain) {
+    if (bna == 128) {
       const int rb = (rows + 127) / 128;
       if (rb * ((H + 127) / 128) < 96) bna = 64;
       if (rb * (((h->cont ? 2 * D : D) + 127) / 128) < 96) bnd = 64;
@@ -345,9 +331,9 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
       rows_data = rows;
     }
     x_mirror_hi = b.xh; x_mirror_lo = t.ns == 2 ? b.xl : nullptr;
-    if (t.key_rows != rows || t.key_R != R || t.key_data != rows_data || t.key_bn != (bna * 1024 + bn) * 1024 + bnd + bnt / 64 || t.key_x != b.xh) {
-      VAEB_TRY(tc_build_maps(&t.maps, b, (int)rows_data, R, rows, D, H, bna, Z, bn, bnd, h->cont ? 2 * D : D, bnt));
-      t.key_rows = rows; t.key_R = R; t.key_data = rows_data; t.key_bn = (bna * 1024 + bn) * 1024 + bnd + bnt / 64; t.key_x = b.xh;
+    if (t.key_rows != rows || t.key_R != R || t.key_data != rows_data || t.key_bn != (bna * 1024 + bn) * 1024 + bnd || t.key_x != b.xh) {
+      VAEB_TRY(tc_build_maps(&t.maps, b, (int)rows_data, R, rows, D, H, bna, Z, bn, bnd, h->cont ? 2 * D : D));
+      t.key_rows = rows; t.key_R = R; t.key_data = rows_data; t.key_bn = (bna * 1024 + bn) * 1024 + bnd; t.key_x = b.xh;
     }
     if (want_grads && b.heh && b.zh && b.d1h && b.ddh && latent_large_batch(rows, H, Z, L) && t.weights_ready &&
         theta == h->d_params) {
@@ -365,75 +351,9 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
   // large-batch training on the tensor-core path: the thin weight gradients also run on tcgen05 (their operands'
   // bf16 mirrors come from the kernels that produce h_e, z, da1 and [dmu|dls])
   const bool tcl = tcp && want_grads && tb.heh && tb.zh && tb.d1h && tb.ddh && latent_large_batch(rows, H, Z, L);
-  // large batch: the split-K slices of the four weight-gradient GEMMs stay in their scratch regions and ONE launch
-  // after the last GEMM sums them all (4 launches less per update)
+  // large batch: the four weight-gradient GEMMs are one launch after the last dgrad; their split-K slices stay in
+  // their scratch regions, and one launch after it (or the tail kernel) sums them all
   TcReduceJobs reduce_jobs;
-  TcReduceJobs* defer = tcl ? &reduce_jobs : nullptr;
-  const size_t wg_region = tcp ? tc_wgrad_scratch_elems(D, H) : 0;
-  // the four weight-gradient GEMMs are one launch after the last dgrad (VAEB_TC_WGRAD_MERGE=0: four launches)
-  const bool merged_wgrad = tcl && tc_wgrad_merged_supported(rows);
-  if (merged_wgrad && t.n_sm == 0) VAEB_CUDA(cudaDeviceGetAttribute(&t.n_sm, cudaDevAttrMultiProcessorCount, h->cfg.device));
-#define WGRAD_ALL_CALL                                                                                                  \
-  tc_wgrad_all(st, lc, t.maps, t.ns, bn, R, rows, D, H, Z, x_row_off, T_(h, grads, l.iW2), T_(h, grads, l.ib2),        \
-               T_(h, grads, l.iW1), T_(h, grads, l.ib1), T_(h, grads, l.iW4), T_(h, grads, l.ib4), T_(h, grads, l.iW5), \
-               T_(h, grads, l.ib5), T_(h, grads, l.iW3), T_(h, grads, l.ib3), tb.wg_scratch, wg_region, defer, t.n_sm,    \
-               h->cont ? T_(h, grads, l.iW6) : nullptr, h->cont ? T_(h, grads, l.ib6) : nullptr)
-  // ---- large-batch training step: the seven activation layers are ONE persistent launch (tc_chain.cu) ----------
-  if (tcl && chain) {
-    const int cbn = chain_pair ? 256 : bna;
-    if (t.n_sm == 0) VAEB_CUDA(cudaDeviceGetAttribute(&t.n_sm, cudaDevAttrMultiProcessorCount, h->cfg.device));
-    const int need = tc_chain_ready_elems(rows);
-    if (need > t.chain_ready_cap) {
-      VAEB_CUDA(cudaStreamSynchronize(st));
-      if (t.chain_ready) VAEB_CUDA(cudaFree(t.chain_ready));
-      t.chain_ready = nullptr;
-      VAEB_CUDA(cudaMalloc((void**)&t.chain_ready, (size_t)need * sizeof(unsigned int)));
-      t.chain_ready_cap = need;
-      t.chain_key_rows = -1;
-    }
-    if (t.chain_key_rows != rows || t.chain_key_bn != cbn + (chain_pair ? 1 : 0)) {
-      VAEB_CUDA(cudaMemsetAsync(t.chain_ready, 0, (size_t)t.chain_ready_cap * sizeof(unsigned int), st));
-      t.chain_epoch = 0;
-      t.chain_key_rows = rows; t.chain_key_bn = cbn + (chain_pair ? 1 : 0);
-    }
-    int n_aux = 0;
-    TcBuffers cb = tb;
-    PH("activation chain enc1..dgrad h_e [tcgen05, one launch]", 6 * dr * dD * dH + 12 * dr * dH * dZ,
-       2.0 * t.ns * (2 * dr * dD + 6 * dr * dH + 3 * dD * dH) + 60 * dr * dZ,
-       tc_chain_step(st, lc, t.maps, t.ns, cbn, rows, D, H, Z, la, x_row_off, T_(h, theta, l.ib3), T_(h, theta, l.ib4),
-                     T_(h, theta, l.ib5), T_(h, theta, l.ib1), T_(h, theta, l.ib2), src, w / (float)L, w, s.mu, s.ls, s.eps,
-                     s.z, s.dmu, s.dls, s.dz, &n_aux, s.partial, &tiles, cb, x_mirror_hi, x_mirror_lo, t.chain_ready,
-                     ++t.chain_epoch, t.n_sm, chain_pair ? 1 : 0));
-    if (tail) {
-      tail->partial = s.partial; tail->n_tiles = tiles; tail->aux_part = s.dz; tail->n_aux = n_aux; tail->row_aux = nullptr;
-      tail->rows = rows;
-    } else {
-      VAEB_LAUNCH(launch_row_partials_sum(st, lc, s.dz, n_aux, rows, s.row_aux));
-      PH("bound (per row + total)", 0, 4 * (dR * tiles + 2 * dr),
-         launch_finalize(st, lc, s.partial, tiles, s.row_aux, rows, L, s.per_row, bo.base_out, bo.mult, bo.tprior,
-                         bo.n_tprior, bo.div, bo.scalar_out, h->d_counter, s.dec_aux));
-    }
-    if (merged_wgrad) {
-      PH("wgrad W2,W1,W4|W5,W3 (+ biases) [tcgen05, one launch]", 4 * dR * dH * dD + 2 * dR * dZ * dH + 4 * dr * dH * dZ,
-         2.0 * t.ns * (2 * dR * dH + 2 * dR * dD) + 8 * dH * dD, WGRAD_ALL_CALL);
-    } else {
-    PH("wgrad W2,b2 [tcgen05]", 2 * dR * dH * dD, 2.0 * t.ns * (dR * dH + dR * dD) + 4 * dH * dD,
-       tc_wgrad2(st, lc, t.maps, t.ns, bn, R, H, D, T_(h, grads, l.iW2), T_(h, grads, l.ib2), tb.wg_scratch, defer));
-    PH("wgrad W1,b1 [tcgen05]", 2 * dR * dZ * dH, 2.0 * t.ns * (dR * 32 + dR * dH) + 4 * dZ * dH,
-       tc_wgrad1(st, lc, t.maps, t.ns, bn, R, Z, H, T_(h, grads, l.iW1), T_(h, grads, l.ib1), tb.wg_scratch + wg_region,
-                 defer));
-    PH("wgrad W4,b4,W5,b5 [tcgen05]", 4 * dr * dH * dZ, 2.0 * t.ns * (dr * dH + dr * 64) + 8 * dZ * dH,
-       tc_wgrad45(st, lc, t.maps, t.ns, rows, H, Z, T_(h, grads, l.iW4), T_(h, grads, l.ib4), T_(h, grads, l.iW5),
-                  T_(h, grads, l.ib5), tb.wg_scratch + 2 * wg_region, defer));
-    PH("wgrad W3,b3 [tcgen05]", 2 * dr * dD * dH, 2.0 * t.ns * (dr * dD + dr * dH) + 4 * dD * dH,
-       tc_wgrad3(st, lc, t.maps, t.ns, bn, rows, D, H, x_row_off, T_(h, grads, l.iW3), T_(h, grads, l.ib3),
-                 tb.wg_scratch + 3 * wg_region, defer));
-    }
-    if (tail) tail->jobs = reduce_jobs;
-    else if (reduce_jobs.n > 0)
-      PH("sum of the split-K weight-gradient slices (one launch)", 0, 0, tc_wgrad_reduce_all(st, lc, reduce_jobs));
-    return VAEB_OK;
-  }
   // encoder hidden layer, VAEB.py:246
   if (tcp)
     PH("enc1 x.W3+tanh [tcgen05]", 2 * dr * dD * dH, 2.0 * t.ns * (dr * dD + dD * dH) + 4 * dr * dH,
@@ -461,7 +381,7 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
     if (aux_to_tail) n_aux_tail = n_aux;
     else VAEB_LAUNCH(launch_row_partials_sum(st, lc, s.partial, n_aux, rows, s.row_aux));
     PH("dec1 tanh(z.W1+b1) [tcgen05]", 2 * dR * dZ * dH, 2.0 * t.ns * (dR * 32 + dZ * dH) + 4 * dR * dH + 2.0 * t.ns * dR * dH,
-       tc_dec1(st, lc, t.maps, t.ns, bnt ? 1000 + bnt : bna, R, Z, H, T_(h, theta, l.ib1), nullptr, tb.hdh, tb.hdl, tb.ldh));
+       tc_dec1(st, lc, t.maps, t.ns, bna, R, Z, H, T_(h, theta, l.ib1), nullptr, tb.hdh, tb.hdl, tb.ldh));
   } else
   PH("latent fwd (enc2,reparam,KL,dec1)", 4 * dr * dH * dZ + 2 * dR * dZ * dH,
      4 * (dr * dH + 3 * dH * dZ + 2 * dr * dZ + 2 * dR * dZ + dR * dH),
@@ -499,10 +419,10 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
   }
   // backward (T.grad, VAEB.py:397); formulas in SURVEY.md 8a
   if (tcp) {
-    if (!merged_wgrad)
+    if (!tcl)
       PH("wgrad W2,b2 [tcgen05]", 2 * dR * dH * dD, 2.0 * t.ns * (dR * dH + dR * dD) + 4 * dH * dD,
          tc_wgrad2(st, lc, t.maps, t.ns, bn, R, H, h->cont ? 2 * D : D, T_(h, grads, l.iW2), T_(h, grads, l.ib2), tb.wg_scratch,
-                   defer, h->cont ? T_(h, grads, l.iW6) : nullptr, h->cont ? T_(h, grads, l.ib6) : nullptr));
+                   h->cont ? T_(h, grads, l.iW6) : nullptr, h->cont ? T_(h, grads, l.ib6) : nullptr));
     PH("dgrad h_d (.W2^T)*(1-h^2) [tcgen05]", 2 * dR * dH * dD * c, 2.0 * t.ns * c * (dR * dD + dH * dD) + 8 * dR * dH,
        tc_dgrad_hd(st, lc, t.maps, t.ns, bna, R, h->cont ? 2 * D : D, H, tcl ? nullptr : s.h_d, tcl ? nullptr : s.da1,
                    tcl ? tb.d1h : nullptr, tcl ? tb.d1l : nullptr, tb.ldh, tb.hdh, tb.hdl));
@@ -535,31 +455,25 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
                        bo.scalar_out, tcl ? tb.ddh : nullptr, tcl ? tb.ddl : nullptr, tb.ldq, h->hidden_act));
   if (tcl) {
     PH("dgrad h_e ([dmu|dls].W45^T)*(1-h^2) [tcgen05]", 4 * dr * dH * dZ, 2.0 * t.ns * (dr * 64 + 2 * dZ * dH) + 8 * dr * dH,
-       tc_dgrad_he(st, lc, t.maps, t.ns, bnt ? 1000 + bnt : bna, rows, Z, H, nullptr, nullptr, tb.da3h, tb.da3l, tb.ldh, tb.heh, tb.hel));
-    if (merged_wgrad) {
-      PH("wgrad W2,W1,W4|W5,W3 (+ biases) [tcgen05, one launch]", 4 * dR * dH * dD + 2 * dR * dZ * dH + 4 * dr * dH * dZ,
-         2.0 * t.ns * (2 * dR * dH + 2 * dR * dD) + 8 * dH * dD, WGRAD_ALL_CALL);
-    } else {
-    PH("wgrad W1,b1 [tcgen05]", 2 * dR * dZ * dH, 2.0 * t.ns * (dR * 32 + dR * dH) + 4 * dZ * dH,
-       tc_wgrad1(st, lc, t.maps, t.ns, bn, R, Z, H, T_(h, grads, l.iW1), T_(h, grads, l.ib1), tb.wg_scratch + wg_region,
-                 defer));
-    PH("wgrad W4,b4,W5,b5 [tcgen05]", 4 * dr * dH * dZ, 2.0 * t.ns * (dr * dH + dr * 64) + 8 * dZ * dH,
-       tc_wgrad45(st, lc, t.maps, t.ns, rows, H, Z, T_(h, grads, l.iW4), T_(h, grads, l.ib4), T_(h, grads, l.iW5),
-                  T_(h, grads, l.ib5), tb.wg_scratch + 2 * wg_region, defer));
-    }
+       tc_dgrad_he(st, lc, t.maps, t.ns, bna, rows, Z, H, nullptr, nullptr, tb.da3h, tb.da3l, tb.ldh, tb.heh, tb.hel));
+    if (t.n_sm == 0) VAEB_CUDA(cudaDeviceGetAttribute(&t.n_sm, cudaDevAttrMultiProcessorCount, h->cfg.device));
+    PH("wgrad W2,W1,W4|W5,W3 (+ biases) [tcgen05, one launch]", 4 * dR * dH * dD + 2 * dR * dZ * dH + 4 * dr * dH * dZ,
+       2.0 * t.ns * (2 * dR * dH + 2 * dR * dD) + 8 * dH * dD,
+       tc_wgrad_all(st, lc, t.maps, t.ns, bn, R, rows, D, H, Z, x_row_off, T_(h, grads, l.iW2), T_(h, grads, l.ib2),
+                    T_(h, grads, l.iW1), T_(h, grads, l.ib1), T_(h, grads, l.iW4), T_(h, grads, l.ib4), T_(h, grads, l.iW5),
+                    T_(h, grads, l.ib5), T_(h, grads, l.iW3), T_(h, grads, l.ib3), tb.wg_scratch,
+                    tc_wgrad_scratch_elems(D, H), &reduce_jobs, t.n_sm, h->cont ? T_(h, grads, l.iW6) : nullptr,
+                    h->cont ? T_(h, grads, l.ib6) : nullptr));
   } else
   PH("wgrad W1,b1,W4,b4,W5,b5", 2 * dR * dZ * dH + 4 * dr * dH * dZ,
      4 * (dR * dZ + dR * dH + dr * dH + 2 * dr * dZ + 3 * dH * dZ),
      launch_small_wgrad(st, lc, s.z, s.da1, R, s.h_e, s.dmu, s.dls, rows, H, Z, T_(h, grads, l.iW1),
                         T_(h, grads, l.ib1), T_(h, grads, l.iW4), T_(h, grads, l.ib4), T_(h, grads, l.iW5),
                         T_(h, grads, l.ib5), s.wg_scratch));
-  if (tcp && merged_wgrad) {
-    // (launched above, with the other weight gradients)
-  } else if (tcp)
+  if (tcp && !tcl)
     PH("wgrad W3,b3 [tcgen05]", 2 * dr * dD * dH, 2.0 * t.ns * (dr * dD + dr * dH) + 4 * dD * dH,
-       tc_wgrad3(st, lc, t.maps, t.ns, bn, rows, D, H, x_row_off, T_(h, grads, l.iW3), T_(h, grads, l.ib3),
-                 tcl ? tb.wg_scratch + 3 * wg_region : tb.wg_scratch, defer));
-  else {
+       tc_wgrad3(st, lc, t.maps, t.ns, bn, rows, D, H, x_row_off, T_(h, grads, l.iW3), T_(h, grads, l.ib3), tb.wg_scratch));
+  else if (!tcp) {
     // deeper encoders: da3 is the gradient at the pre-activation of the LAST hidden layer; for k = depth .. 2 the layer's
     // weight gradient is h_{k-1}^T . da_k and da_{k-1} = (da_k . W3_k^T) * f'(h_{k-1})
     float* dcur = s.da3;
@@ -894,7 +808,6 @@ int vaeb_destroy(vaeb_handle* h) {
   cudaSetDevice(h->cfg.device);
   cudaStreamSynchronize(h->stream);
   p2p_release(h);
-  if (h->tc.chain_ready) cudaFree(h->tc.chain_ready);
   if (h->tc.tail_bar) cudaFree(h->tc.tail_bar);
   if (h->comm && h->nccl.CommDestroy) h->nccl.CommDestroy(h->comm);
   free_ws(h->ws);

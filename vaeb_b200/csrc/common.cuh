@@ -81,9 +81,6 @@ struct TcState {
   int64_t cap_data = 0, cap_stage = 0, cap_R = 0, cap_rows = 0;
   TcMaps maps;
   int64_t key_rows = -1, key_R = -1, key_data = -1; int key_bn = 0; const void* key_x = nullptr;
-  // the activation chain as one launch (tc_chain.cu): arrival counters, launches since they were zeroed
-  unsigned int* chain_ready = nullptr; int chain_ready_cap = 0; unsigned int chain_epoch = 0;
-  int64_t chain_key_rows = -1; int chain_key_bn = 0;
   int n_sm = 0;
   // the fused tail of an update (tc_tail.cu)
   bool weights_ready = false;              // the weight mirrors hold the CURRENT parameters (written by the tail)
@@ -116,8 +113,6 @@ struct IsTcState {
   float* bias26 = nullptr;                           // Gaussian decoder: b2 / b6 interleaved like the output columns
   alignas(64) unsigned char map_w1[128];             // CUtensorMap over w1t, boxes of 64 rows (one pass)
   alignas(64) unsigned char map_full[128];           // CUtensorMap over w2t, boxes of `tail_cols` rows (one output chunk)
-  alignas(64) unsigned char map_half[128];           // ... boxes of tail_cols / 2 rows, map_w1_half: 32 rows (CTA-pair form)
-  alignas(64) unsigned char map_w1_half[128];
   int n_sm = 0, n_chunks = 0, tail_cols = 0;         // tail_cols = chunk width NC (multiple of 16)
   void* partial = nullptr; int64_t partial_cap = 0;  // per-tile (max, sum exp)
   // pipelined host input of vaeb_is_logpx: the next chunk of points is copied on `copy` while this one is sampled

@@ -61,7 +61,6 @@ struct Params {
   const float* mu; const float* ls;             // [n_points, Z]
   const float* b2;                              // [D] output biases (Gaussian: b2 / b6 interleaved)
   int cont, Dx;                                 // Gaussian decoder; pixels per point (D = 2 Dx columns then)
-  int ld16;                                     // 16 accumulator columns per TMEM read (default; VAEB_IS_LD16=0: 8, pipelined)
   const float* eps_inj;                         // [n_points, L, Z] or nullptr
   uint64_t seed; int64_t row_offset;
   float2* partial;                              // [n_points * tiles_per_point] (max, sum exp)
@@ -192,51 +191,6 @@ __device__ __forceinline__ uint64_t mk64(uint32_t lo, uint32_t hi) {
 }
 constexpr uint32_t DESC_HI = (1024u >> 4) | (1u << 14) | (2u << 29);   // SBO = 1024 B, version 1, SWIZZLE_128B
 
-// ---- CTA pair (cta_group::2): the W2^T stream is what bounds this kernel (every 128-sample tile re-reads the whole
-// 0.8 MB matrix from L2: 7.6-7.8 TB/s of L2 -> shared-memory traffic over the chip).  Two CTAs of a cluster work on
-// adjacent tiles with ONE UMMA of M = 256: each stages its own A tile and HALF of every B box (80 of the 160 W2^T rows of
-// a chunk, 32 of the 64 W1^T rows of a pass), so the stream per SM halves.  The even CTA issues every MMA; TMA loads of
-// both CTAs complete on its `b_full`; its commits are multicast to the barriers of both; producers and epilogue warps of
-// the odd CTA arrive on the even CTA's barriers.
-constexpr uint32_t PEER_MASK = 0xFEFFFFFFu;      // shared::cluster address of the same offset in the even CTA of the pair
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-template <bool PAIR>
-__device__ __forceinline__ void umma(uint32_t d, uint64_t a, uint64_t b, uint32_t idesc, uint32_t accumulate) {
-  if constexpr (PAIR) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d), "l"(a), "l"(b), "r"(idesc), "r"(accumulate)
-        : "memory");
-  } else {
-    tc::umma_bf16(d, a, b, idesc, accumulate);
-  }
-}
-template <bool PAIR>
-__device__ __forceinline__ void commit(uint32_t addr) {
-  if constexpr (PAIR)
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(addr), "h"((uint16_t)3) : "memory");
-  else
-    commit_to(addr);
-}
-// arrive on the barrier the MMA thread waits on: the even CTA's copy in the pair form
-template <bool PAIR>
-__device__ __forceinline__ void arrive_mma(uint64_t* bar) {
-  if constexpr (PAIR)
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(tc::smem_u32(bar) & PEER_MASK) : "memory");
-  else
-    tc::mbar_arrive(bar);
-}
-
 // The order in which one CTA consumes ring stages, shared by the TMA and the MMA thread.  A "pass" is the
 // hidden-layer GEMM [z|1].W1^T for 64 hidden units of a tile (-> one k block of its A tile); a "w2" item is one
 // k block of one output chunk.  The passes of tile i+1 are interleaved with the LAST output chunk of tile i:
@@ -286,9 +240,7 @@ struct BarAddrs {
   uint32_t b_full, b_empty, z_full, z_empty, mini_full, mini_empty, a_ready, a_free, acc_full, acc_empty;
 };
 
-template <bool PAIR>
 struct TmaIssuer {
-  uint32_t rank = 0;             // PAIR: which half of every B box this CTA stages
   const CUtensorMap* map_w2; const CUtensorMap* map_w1;
   BarAddrs bar;
   uint32_t ring;                 // shared address of the ring
@@ -302,21 +254,11 @@ struct TmaIssuer {
     if (turn == me) {
       const uint32_t full = bar.b_full + 8u * stage;
       bar_wait(bar.b_empty + 8u * stage, parity ^ 1u);
-      if constexpr (PAIR) {
-        // `bytes` = this CTA's half; both halves complete on the even CTA's barrier, which expects their sum
-        if (rank == 0)
-          asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full), "r"(2u * bytes) : "memory");
-        asm volatile(
-            "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-            ::"r"(ring + stage * (uint32_t)B_STAGE), "l"(m), "r"(full & PEER_MASK), "r"(c0), "r"(c1)
-            : "memory");
-      } else {
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full), "r"(bytes) : "memory");
-        asm volatile(
-            "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-            ::"r"(ring + stage * (uint32_t)B_STAGE), "l"(m), "r"(full), "r"(c0), "r"(c1)
-            : "memory");
-      }
+      asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full), "r"(bytes) : "memory");
+      asm volatile(
+          "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+          ::"r"(ring + stage * (uint32_t)B_STAGE), "l"(m), "r"(full), "r"(c0), "r"(c1)
+          : "memory");
     }
     turn ^= 1u;
     if (++stage == STAGES) { stage = 0; parity ^= 1u; }
@@ -325,18 +267,11 @@ struct TmaIssuer {
   __device__ __forceinline__ void chunk_end() {}
   template <bool FIRST>
   __device__ __forceinline__ bool chunk_static(uint32_t, int) { return false; }
-  __device__ __forceinline__ void pass(uint32_t, int j) {
-    if constexpr (PAIR) load(map_w1, (uint32_t)(MINI_N / 2) * 128u, 0, j * MINI_N + (int)rank * (MINI_N / 2));
-    else load(map_w1, (uint32_t)MINI_N * 128u, 0, j * MINI_N);
-  }
+  __device__ __forceinline__ void pass(uint32_t, int j) { load(map_w1, (uint32_t)MINI_N * 128u, 0, j * MINI_N); }
   template <bool FIRST, bool LAST>
-  __device__ __forceinline__ void w2(uint32_t, int c, int kb) {
-    if constexpr (PAIR) load(map_w2, w2_bytes / 2u, kb * BK, c * NC + (int)rank * (NC / 2));
-    else load(map_w2, w2_bytes, kb * BK, c * NC);
-  }
+  __device__ __forceinline__ void w2(uint32_t, int c, int kb) { load(map_w2, w2_bytes, kb * BK, c * NC); }
 };
 
-template <bool PAIR>
 struct MmaIssuer {
   BarAddrs bar;
   uint32_t tmem_base, a_lo0, b_lo0, z_lo0, idesc, idesc_mini;
@@ -350,7 +285,7 @@ struct MmaIssuer {
     d_acc = tmem_base + buf * ACC_STRIDE;
   }
   __device__ __forceinline__ void chunk_end() {
-    commit<PAIR>(bar.acc_full + 8u * (acc_it & 1u));
+    commit_to(bar.acc_full + 8u * (acc_it & 1u));
     ++acc_it;
   }
   __device__ __forceinline__ void pass(uint32_t tseq, int j) {
@@ -362,10 +297,10 @@ struct MmaIssuer {
     const uint32_t d = tmem_base + MINI_COL0 + mb * MINI_N;
     const uint32_t b_lo = b_lo0 + stage * (uint32_t)(B_STAGE >> 4);
     for (int k = 0; k < zk; ++k)
-      umma<PAIR>(d, mk64(z_lo0 + 2u * k, DESC_HI), mk64(b_lo + 2u * k, DESC_HI), idesc_mini, k ? 1u : 0u);
-    commit<PAIR>(bar.b_empty + 8u * stage);
-    commit<PAIR>(bar.mini_full + 8u * mb);
-    if (j == KB - 1) commit<PAIR>(bar.z_empty);
+      tc::umma_bf16(d, mk64(z_lo0 + 2u * k, DESC_HI), mk64(b_lo + 2u * k, DESC_HI), idesc_mini, k ? 1u : 0u);
+    commit_to(bar.b_empty + 8u * stage);
+    commit_to(bar.mini_full + 8u * mb);
+    if (j == KB - 1) commit_to(bar.z_empty);
     advance();
     ++mini_it;
   }
@@ -384,8 +319,8 @@ struct MmaIssuer {
       const uint32_t b_lo = b_lo0 + st * (uint32_t)(B_STAGE >> 4);
 #pragma unroll
       for (int k = 0; k < BK / 16; ++k)
-        umma<PAIR>(d_acc, mk64(a_lo + 2u * k, DESC_HI), mk64(b_lo + 2u * k, DESC_HI), idesc, (kb | k) != 0 ? 1u : 0u);
-      commit<PAIR>(bar.b_empty + 8u * st);
+        tc::umma_bf16(d_acc, mk64(a_lo + 2u * k, DESC_HI), mk64(b_lo + 2u * k, DESC_HI), idesc, (kb | k) != 0 ? 1u : 0u);
+      commit_to(bar.b_empty + 8u * st);
     }
     stage = (uint32_t)((S0 + 8) % STAGES);
     parity ^= (uint32_t)(((S0 + 8) / STAGES) & 1);
@@ -411,16 +346,15 @@ struct MmaIssuer {
     const uint32_t b_lo = b_lo0 + stage * (uint32_t)(B_STAGE >> 4);
 #pragma unroll
     for (int k = 0; k < BK / 16; ++k)
-      umma<PAIR>(d_acc, mk64(a_lo + 2u * k, DESC_HI), mk64(b_lo + 2u * k, DESC_HI), idesc, (kb | k) != 0 ? 1u : 0u);
-    commit<PAIR>(bar.b_empty + 8u * stage);
-    if (LAST) commit<PAIR>(bar.a_free + 8u * kb);
+      tc::umma_bf16(d_acc, mk64(a_lo + 2u * k, DESC_HI), mk64(b_lo + 2u * k, DESC_HI), idesc, (kb | k) != 0 ? 1u : 0u);
+    commit_to(bar.b_empty + 8u * stage);
+    if (LAST) commit_to(bar.a_free + 8u * kb);
     advance();
   }
 };
 
 // Roles (640 threads): warp 0 TMA, warp 1 MMA issuer, warp 2 TMEM allocator, warps 4-11 producers
 // (z generation + TMEM -> tanh -> bf16 A tile conversion), warps 12-19 epilogue.
-template <bool PAIR>
 __global__ void __launch_bounds__(THREADS, 1)
 is_tc_kernel(const __grid_constant__ CUtensorMap map_w2, const __grid_constant__ CUtensorMap map_w1, const Params p) {
   extern __shared__ uint8_t smem_raw[];
@@ -451,23 +385,14 @@ is_tc_kernel(const __grid_constant__ CUtensorMap map_w2, const __grid_constant__
     tc::tma_prefetch_desc(&map_w2);
     tc::tma_prefetch_desc(&map_w1);
     for (int s = 0; s < STAGES; ++s) { tc::mbar_init(&b_full[s], 1); tc::mbar_init(&b_empty[s], 1); }
-    constexpr int NC2 = PAIR ? 2 : 1;            // PAIR: the barriers the MMA thread waits on count the warps of both CTAs
-    tc::mbar_init(z_full, NC2 * PROD_WARPS);
+    tc::mbar_init(z_full, PROD_WARPS);
     tc::mbar_init(z_empty, 1);
-    for (int b = 0; b < MINI_BUFS; ++b) { tc::mbar_init(&mini_full[b], 1); tc::mbar_init(&mini_empty[b], NC2 * PROD_WARPS); }
-    for (int j = 0; j < KB_MAX; ++j) { tc::mbar_init(&a_ready[j], NC2 * PROD_WARPS); tc::mbar_init(&a_free[j], 1); }
-    for (int b = 0; b < 2; ++b) { tc::mbar_init(&acc_full[b], 1); tc::mbar_init(&acc_empty[b], NC2 * EPI_WARPS); }
+    for (int b = 0; b < MINI_BUFS; ++b) { tc::mbar_init(&mini_full[b], 1); tc::mbar_init(&mini_empty[b], PROD_WARPS); }
+    for (int j = 0; j < KB_MAX; ++j) { tc::mbar_init(&a_ready[j], PROD_WARPS); tc::mbar_init(&a_free[j], 1); }
+    for (int b = 0; b < 2; ++b) { tc::mbar_init(&acc_full[b], 1); tc::mbar_init(&acc_empty[b], EPI_WARPS); }
     tc::fence_barrier_init();
   }
-  if (PAIR) cluster_sync_all();                  // the peer's barriers exist before anything is sent to them
-  if (warp == 2) {
-    if constexpr (PAIR) {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tc::smem_u32(tmem_slot)), "r"((uint32_t)TMEM_COLS) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    } else {
-      tc::tmem_alloc(tmem_slot, TMEM_COLS);
-    }
-  }
+  if (warp == 2) tc::tmem_alloc(tmem_slot, TMEM_COLS);
   // columns past D: a = -30 (the W2^T rows are zero-filled), x - 1/2 = -1/2: a (x - 1/2) - |a|/2 = 15 - 15 and
   // ln(1 + e^-30) ~ 1e-13, so padding contributes nothing (no per-element bounds test)
   for (int i = threadIdx.x; i < DMAX; i += THREADS) {
@@ -492,8 +417,7 @@ is_tc_kernel(const __grid_constant__ CUtensorMap map_w2, const __grid_constant__
   if (warp == 0 || warp == 3) {
     // ===== TMA: W1^T boxes of the passes and W2^T boxes of the sweep, in walk_items order (alternate items) =====
     if (elect_one()) {
-      TmaIssuer<PAIR> r;
-      r.rank = PAIR ? cluster_ctarank() : 0u;
+      TmaIssuer r;
       r.me = warp == 0 ? 0u : 1u;
       r.map_w2 = &map_w2; r.map_w1 = &map_w1; r.bar = ba;
       r.ring = tc::smem_u32(smem + Smem::B);
@@ -502,17 +426,17 @@ is_tc_kernel(const __grid_constant__ CUtensorMap map_w2, const __grid_constant__
     }
     __syncwarp();
   } else if (warp == 1) {
-    // ===== MMA issuer: ONE elected lane runs the whole loop (PAIR: of the even CTA) =====
-    if ((!PAIR || cluster_ctarank() == 0) && elect_one()) {
-      MmaIssuer<PAIR> r;
+    // ===== MMA issuer: ONE elected lane runs the whole loop =====
+    if (elect_one()) {
+      MmaIssuer r;
       r.bar = ba;
       r.tmem_base = tmem_base;
-      // (shared addresses of a cluster launch carry the CTA rank above bit 17: the descriptor field takes 14 bits)
+      // (the descriptor's address field takes 14 bits of the shared address >> 4)
       r.a_lo0 = ((tc::smem_u32(smem + Smem::A) & 0x3FFFFu) >> 4) | (1u << 16);       // LBO field = 1 (unused for SW128 K-major)
       r.b_lo0 = ((tc::smem_u32(smem + Smem::B) & 0x3FFFFu) >> 4) | (1u << 16);
       r.z_lo0 = ((tc::smem_u32(smem + Smem::ZB) & 0x3FFFFu) >> 4) | (1u << 16);
-      r.idesc = tc::make_idesc_bf16(PAIR ? 2 * BM : BM, p.NC, 0, 0);
-      r.idesc_mini = tc::make_idesc_bf16(PAIR ? 2 * BM : BM, MINI_N, 0, 0);
+      r.idesc = tc::make_idesc_bf16(BM, p.NC, 0, 0);
+      r.idesc_mini = tc::make_idesc_bf16(BM, MINI_N, 0, 0);
       r.KB = p.KB; r.zk = p.zk;
       walk_items(p, n_tiles, r);
     }
@@ -565,7 +489,7 @@ is_tc_kernel(const __grid_constant__ CUtensorMap map_w2, const __grid_constant__
         aux_s[(ti % 3) * BM + pt] = a;
       }
       __syncwarp();
-      if (lane == 0) arrive_mma<PAIR>(z_full);
+      if (lane == 0) tc::mbar_arrive(z_full);
     };
 
     uint32_t tile_it = 0, mini_it = 0;
@@ -596,7 +520,7 @@ is_tc_kernel(const __grid_constant__ CUtensorMap map_w2, const __grid_constant__
         tc::fence_proxy_async();                               // generic-proxy writes -> visible to the MMA
         tc::tc_fence_before();
         __syncwarp();
-        if (lane == 0) { arrive_mma<PAIR>(&mini_empty[mb]); arrive_mma<PAIR>(&a_ready[j]); }
+        if (lane == 0) { tc::mbar_arrive(&mini_empty[mb]); tc::mbar_arrive(&a_ready[j]); }
       }
       // --- z of the NEXT tile while this tile's output sweep runs
       const int tn = t + gridDim.x;
@@ -629,7 +553,7 @@ is_tc_kernel(const __grid_constant__ CUtensorMap map_w2, const __grid_constant__
         const uint32_t taddr = tmem_base + buf * ACC_STRIDE + (uint32_t)c_lo + ((uint32_t)(q * 32) << 16);
         const uint32_t col4 = (uint32_t)(c * p.NC + c_lo) * 4u;
         const uint32_t ba = bb_addr + col4, xa = xh_addr + col4;
-        // this warp's half of the chunk, 8 columns per TMEM load; the next load is in flight while the
+        // this warp's slice of the chunk; Gaussian decoder: 8 columns per TMEM load, the next load in flight while the
         // current 8 columns are folded
         float va[8], vb[8];
         tmem_ld8(taddr, va);
@@ -644,7 +568,7 @@ is_tc_kernel(const __grid_constant__ CUtensorMap map_w2, const __grid_constant__
               fold8g(vb, ba + 32u * (i + 1), xa + 32u * (i + 1), accg);
             }
           }
-        } else if (p.ld16) {
+        } else {
           // fewer, larger TMEM reads: a tcgen05.ld round trip is several times slower while MMAs accumulate into the other
           // buffer (DESIGN 4.3b), and a warp makes five of them per chunk with 8-column reads
           tc::tmem_ld_wait();
@@ -662,20 +586,10 @@ is_tc_kernel(const __grid_constant__ CUtensorMap map_w2, const __grid_constant__
               fold8(vb, ba + 32u * i, xa + 32u * i, fk, acc);
             }
           }
-        } else
-        for (int i = 0; i < n8; i += 2) {
-          tc::tmem_ld_wait();
-          if (i + 1 < n8) tmem_ld8(taddr + 8u * (i + 1), vb);
-          fold8(va, ba + 32u * i, xa + 32u * i, fk, acc);
-          if (i + 1 < n8) {
-            tc::tmem_ld_wait();
-            if (i + 2 < n8) tmem_ld8(taddr + 8u * (i + 2), va);
-            fold8(vb, ba + 32u * (i + 1), xa + 32u * (i + 1), fk, acc);
-          }
         }
         tc::tc_fence_before();
         __syncwarp();
-        if (lane == 0) arrive_mma<PAIR>(&acc_empty[buf]);
+        if (lane == 0) tc::mbar_arrive(&acc_empty[buf]);
       }
       float rs0, rs1;
       upk2(acc, rs0, rs1);
@@ -710,13 +624,7 @@ is_tc_kernel(const __grid_constant__ CUtensorMap map_w2, const __grid_constant__
   }
   tc::tc_fence_before();
   __syncthreads();
-  if (PAIR) cluster_sync_all();                  // the even CTA's MMAs read the odd CTA's shared memory: leave together
-  if (warp == 2) {
-    if constexpr (PAIR)
-      asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)TMEM_COLS) : "memory");
-    else
-      tc::tmem_dealloc(tmem_base, TMEM_COLS);
-  }
+  if (warp == 2) tc::tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
 // log p^(x_i) = log sum_t S_t exp(M_t - M) + M - log L   over the tiles of point i
@@ -784,9 +692,7 @@ int is_tc_run(vaeb_handle* h, const float* d_x, const float* d_mu, const float* 
     if (h->cont) VAEB_CUDA(cudaMalloc((void**)&s.bias26, (size_t)D * sizeof(float)));
     VAEB_CUDA(cudaMemset(s.w1t, 0, (size_t)(KB_MAX * 64) * 64 * 2));
     VAEB_TRY(vaeb_make_tmap_bf16((CUtensorMap*)s.map_w1, s.w1t, (uint64_t)(KB_MAX * 64), 64, 64, MINI_N));
-    VAEB_TRY(vaeb_make_tmap_bf16((CUtensorMap*)s.map_w1_half, s.w1t, (uint64_t)(KB_MAX * 64), 64, 64, MINI_N / 2));
-    VAEB_CUDA(cudaFuncSetAttribute(is_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem::TOTAL));
-    VAEB_CUDA(cudaFuncSetAttribute(is_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem::TOTAL));
+    VAEB_CUDA(cudaFuncSetAttribute(is_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem::TOTAL));
     VAEB_CUDA(cudaDeviceGetAttribute(&s.n_sm, cudaDevAttrMultiProcessorCount, h->cfg.device));
     // output chunks: as few as fit NC_MAX accumulator columns, equal width (a multiple of 32): 784 -> 5 x 160
     const int n_chunks = (D + NC_MAX - 1) / NC_MAX;
@@ -794,8 +700,6 @@ int is_tc_run(vaeb_handle* h, const float* d_x, const float* d_mu, const float* 
     s.n_chunks = n_chunks; s.tail_cols = nc;
     VAEB_TRY(vaeb_make_tmap_bf16((CUtensorMap*)s.map_full, s.w2t, (uint64_t)D, (uint64_t)KP, (uint64_t)(KP + W2T_PAD),
                                  (uint32_t)nc));
-    VAEB_TRY(vaeb_make_tmap_bf16((CUtensorMap*)s.map_half, s.w2t, (uint64_t)D, (uint64_t)KP, (uint64_t)(KP + W2T_PAD),
-                                 (uint32_t)(nc / 2)));
   }
   // the weights may have changed since the last call: refresh the bf16 transpose (0.8 MB)
   {
@@ -827,34 +731,11 @@ int is_tc_run(vaeb_handle* h, const float* d_x, const float* d_mu, const float* 
   p.x = d_x; p.mu = d_mu; p.ls = d_ls;
   p.b2 = h->cont ? s.bias26 : h->d_params + l.off[l.ib2];
   p.cont = h->cont ? 1 : 0; p.Dx = Dx;
-  { static const int ld16 = getenv("VAEB_IS_LD16") ? atoi(getenv("VAEB_IS_LD16")) : 1; p.ld16 = ld16; }   // 42.25 -> 41.5 ms (10k x 5000)
   p.eps_inj = d_eps; p.seed = h->cfg.seed; p.row_offset = row_offset;
   p.partial = (float2*)s.partial; p.logw_out = d_logw;
   int grid = (int)std::min<int64_t>(n_tiles, s.n_sm);
   { const char* e = getenv("VAEB_IS_GRID"); if (e) grid = std::min(grid, atoi(e)); }
-  // CTA-pair form (cta_group::2: half of the W2^T stream per SM) whenever the tiles pair up: an even number of them on an
-  // even grid gives both CTAs of a pair the same number of tiles; half a chunk must be whole 8-row swizzle atoms
-  // MEASURED SLOWER (10k x 5000: 58.3 vs 41.6 ms): every producer / epilogue hand-shake with the MMA thread becomes a
-  // cross-CTA arrival, and a tile has ~50 of them -- the kernel is bound by those latencies, not by the W2^T bytes.  Off by
-  // default; VAEB_IS_PAIR=1 selects it (tests/test_gpu_tc.py runs it in a subprocess).
-  static const int env_pair = getenv("VAEB_IS_PAIR") ? atoi(getenv("VAEB_IS_PAIR")) : 0;
-  const bool pair = env_pair != 0 && (n_tiles % 2) == 0 && grid >= 2 && (s.tail_cols % 32) == 0;
-  if (pair) {
-    grid &= ~1;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(THREADS);
-    cfg.dynamicSmemBytes = Smem::TOTAL;
-    cfg.stream = st;
-    cudaLaunchAttribute attr{};
-    attr.id = cudaLaunchAttributeClusterDimension;
-    attr.val.clusterDim.x = 2; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
-    cfg.attrs = &attr;
-    cfg.numAttrs = 1;
-    VAEB_CUDA(cudaLaunchKernelEx(&cfg, is_tc_kernel<true>, *(const CUtensorMap*)s.map_half, *(const CUtensorMap*)s.map_w1_half, p));
-  } else {
-    is_tc_kernel<false><<<grid, THREADS, Smem::TOTAL, st>>>(*(const CUtensorMap*)s.map_full, *(const CUtensorMap*)s.map_w1, p);
-  }
+  is_tc_kernel<<<grid, THREADS, Smem::TOTAL, st>>>(*(const CUtensorMap*)s.map_full, *(const CUtensorMap*)s.map_w1, p);
   ++h->launches;
   VAEB_CUDA(cudaGetLastError());
   is_tc_finish_kernel<<<(n + 127) / 128, 128, 0, st>>>((const float2*)s.partial, n, tpp, L, d_logp);

@@ -204,10 +204,9 @@ thread_local bool g_pdl = false;   // set and read within one forward_backward c
 // producer runs ahead into the next tile while the last k blocks of this one are still being contracted.  BN up to
 // 256 (2 x 256 TMEM columns): a 128 x 256 tile re-reads A half as often as two 128 x 128 tiles -- these layers are
 // bound by L2 -> shared-memory operand traffic (K <= 784: 64 flop per operand byte at 128 x 128).
-template <int BN, int NS, int MT>
+template <int BN, int NS>
 struct PersistSmem {
-  static constexpr int A1_BYTES = BM * BK * 2;              // one 128-row block of A
-  static constexpr int A_BYTES = MT * A1_BYTES;
+  static constexpr int A_BYTES = BM * BK * 2;               // one 128-row block of A
   static constexpr int B_BYTES = BN * BK * 2;
   static constexpr int STAGE_BYTES = NS * (A_BYTES + B_BYTES);
   static constexpr int BUDGET = 208 * 1024;
@@ -248,15 +247,12 @@ struct TileSeq {
   }
 };
 
-// MT = 2: a CTA tile is 256 x BN -- two 128-row blocks of A share every B stage (two MMAs per k step into two
-// accumulators that fill TMEM, so the epilogue of a tile overlaps only the operand loads of the next one).  ncu on
-// the MT = 1 kernels: tensor pipe 25 % active, L2 slices 25 %, 6.8 TB/s of L2 -> shared-memory fill (46 GB/s per SM,
-// the same rate the IS kernel streams W2^T at): the fill rate bounds these layers, and MT = 2 moves 36 % fewer bytes
-// per flop -- yet it measured slower (see dispatch_layer).
-template <int BN, bool B_MN, int NS, class Epi, int MT>
+// ncu: tensor pipe 25 % active, L2 slices 25 %, 6.8 TB/s of L2 -> shared-memory fill (46 GB/s per SM, the same rate the
+// IS kernel streams W2^T at): the fill rate bounds these layers.
+template <int BN, bool B_MN, int NS, class Epi>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 tc_layer_persistent_kernel(const __grid_constant__ LayerMaps maps, Epi epi, int M, int N, int K, int a_row_off) {
-  using S = PersistSmem<BN, NS, MT>;
+  using S = PersistSmem<BN, NS>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   uint64_t* full = (uint64_t*)(smem + S::STAGES * S::STAGE_BYTES);
@@ -267,14 +263,12 @@ tc_layer_persistent_kernel(const __grid_constant__ LayerMaps maps, Epi epi, int 
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int nkb = (K + BK - 1) / BK;
-  constexpr int TILE_M = MT * BM;
-  const int tiles_n = (N + BN - 1) / BN, tiles_m = (M + TILE_M - 1) / TILE_M;
-  // a last column tile at most a quarter wide is a "sliver" (see TileSeq); MT = 2 keeps the plain order
-  const bool sliver = MT == 1 && tile_sliver(N, BN, tiles_n);
-  const TileSeq seq(tiles_m, tiles_n, sliver, (int)gridDim.x, (int)blockIdx.x);
+  const int tiles_n = (N + BN - 1) / BN, tiles_m = (M + BM - 1) / BM;
+  // a last column tile at most a quarter wide is a "sliver" (see TileSeq)
+  const TileSeq seq(tiles_m, tiles_n, tile_sliver(N, BN, tiles_n), (int)gridDim.x, (int)blockIdx.x);
   constexpr uint32_t ACC_COLS = BN <= 32 ? 32 : (BN <= 64 ? 64 : (BN <= 128 ? 128 : 256));
-  constexpr uint32_t NBUF = (512u / (MT * ACC_COLS)) >= 2u ? 2u : 1u;      // accumulator sets in TMEM
-  constexpr uint32_t TMEM_COLS = NBUF * MT * ACC_COLS;
+  constexpr uint32_t NBUF = 2;                          // accumulator sets in TMEM
+  constexpr uint32_t TMEM_COLS = NBUF * ACC_COLS;
   static_assert(TMEM_COLS <= 512 && (TMEM_COLS & (TMEM_COLS - 1)) == 0, "TMEM allocation");
 
   if (warp == 0 && lane == 0) {
@@ -297,7 +291,7 @@ tc_layer_persistent_kernel(const __grid_constant__ LayerMaps maps, Epi epi, int 
     uint32_t it = 0;                                   // k blocks issued so far (ring position across tiles)
     int tm, tn;
     for (int lt = 0; seq.get(lt, tm, tn); ++lt) {
-      const int m0 = tm * TILE_M, n0 = tn * BN;
+      const int m0 = tm * BM, n0 = tn * BN;
       for (int kb = 0; kb < nkb; ++kb, ++it) {
         const int s = it % S::STAGES;
         tc::mbar_wait(&empty[s], ((it / S::STAGES) & 1) ^ 1);
@@ -309,9 +303,7 @@ tc_layer_persistent_kernel(const __grid_constant__ LayerMaps maps, Epi epi, int 
           uint8_t* b = base + NS * S::A_BYTES + sp * S::B_BYTES;
           const CUtensorMap* ta = sp ? &maps.a_lo : &maps.a_hi;
           const CUtensorMap* tb = sp ? &maps.b_lo : &maps.b_hi;
-#pragma unroll
-          for (int mt = 0; mt < MT; ++mt)
-            tc::tma_load_2d(a + mt * S::A1_BYTES, ta, &full[s], kb * BK, a_row_off + m0 + mt * BM);
+          tc::tma_load_2d(a, ta, &full[s], kb * BK, a_row_off + m0);
           if (B_MN) {
             tc::tma_load_3d(b, tb, &full[s], 0, kb * BK, n0 / 64);      // one box: BN/64 column groups
           } else {
@@ -331,7 +323,7 @@ tc_layer_persistent_kernel(const __grid_constant__ LayerMaps maps, Epi epi, int 
       const uint32_t idesc = tc::make_idesc_bf16(BM, n_live >= BN ? BN : ((n_live + 15) & ~15), 0, B_MN ? 1 : 0);
       tc::mbar_wait(&tmem_empty[buf], (use & 1) ^ 1);           // the epilogue drained this accumulator set
       tc::tc_fence_after();
-      const uint32_t acc = tmem_base + buf * (MT * ACC_COLS);
+      const uint32_t acc = tmem_base + buf * ACC_COLS;
       for (int kb = 0; kb < nkb; ++kb, ++it) {
         const int s = it % S::STAGES;
         tc::mbar_wait(&full[s], (it / S::STAGES) & 1);
@@ -342,15 +334,12 @@ tc_layer_persistent_kernel(const __grid_constant__ LayerMaps maps, Epi epi, int 
         for (int k = 0; k < BK / 16; ++k) {
           const uint64_t dbh = B_MN ? tc::desc_mnmajor(b, k, 8192u) : tc::desc_kmajor(b, k);
           const uint64_t dbl = NS == 2 ? (B_MN ? tc::desc_mnmajor(b + S::B_BYTES, k, 8192u) : tc::desc_kmajor(b + S::B_BYTES, k)) : 0;
-#pragma unroll
-          for (int mt = 0; mt < MT; ++mt) {
-            const uint64_t dah = tc::desc_kmajor(a + mt * S::A1_BYTES, k);
-            tc::umma_bf16(acc + mt * ACC_COLS, dah, dbh, idesc, (kb | k) != 0 ? 1u : 0u);
-            if (NS == 2) {
-              const uint64_t dal = tc::desc_kmajor(a + S::A_BYTES + mt * S::A1_BYTES, k);
-              tc::umma_bf16(acc + mt * ACC_COLS, dah, dbl, idesc, 1u);
-              tc::umma_bf16(acc + mt * ACC_COLS, dal, dbh, idesc, 1u);
-            }
+          const uint64_t dah = tc::desc_kmajor(a, k);
+          tc::umma_bf16(acc, dah, dbh, idesc, (kb | k) != 0 ? 1u : 0u);
+          if (NS == 2) {
+            const uint64_t dal = tc::desc_kmajor(a + S::A_BYTES, k);
+            tc::umma_bf16(acc, dah, dbl, idesc, 1u);
+            tc::umma_bf16(acc, dal, dbh, idesc, 1u);
           }
         }
         tc::umma_commit(&empty[s]);
@@ -366,69 +355,60 @@ tc_layer_persistent_kernel(const __grid_constant__ LayerMaps maps, Epi epi, int 
     for (; seq.get((int)lt, tm, tn); ++lt) {
       const int n0 = tn * BN;
       const uint32_t buf = lt % NBUF, use = lt / NBUF;
-#pragma unroll 1
-      for (int mt = 0; mt < MT; ++mt) {
-        const int row = tm * TILE_M + mt * BM + q * 32 + lane;
-        const bool ok = row < M;
-        epi.begin();
-        const uint32_t acc = tmem_base + buf * (MT * ACC_COLS) + mt * ACC_COLS + ((uint32_t)(q * 32) << 16);
-        // the global operand of chunk i+1 (one 32-byte sector of a bf16 mirror) is requested before chunk i is finished:
-        // 4 warps per scheduler, each a serial chain TMEM read -> global operand -> math -> store, cannot hide that
-        // latency otherwise (ncu: 22 % of the samples on the first use of the load)
-        constexpr int NCH = SLICE / 16;
-        // chunks of this warp's column slice that hold live columns (a sliver tile: at most one warp group has any)
-        int live = (N - n0 - cs * SLICE + 15) >> 4;
-        live = live < 0 ? 0 : (live > NCH ? NCH : live);
-        if (live == 0) {                                      // nothing to read: hand the accumulators straight back
-          if (mt == 0) tc::mbar_wait(&tmem_full[buf], use & 1);
-          if (mt == MT - 1) {
+      const int row = tm * BM + q * 32 + lane;
+      const bool ok = row < M;
+      epi.begin();
+      const uint32_t acc = tmem_base + buf * ACC_COLS + ((uint32_t)(q * 32) << 16);
+      // the global operand of chunk i+1 (one 32-byte sector of a bf16 mirror) is requested before chunk i is finished:
+      // 4 warps per scheduler, each a serial chain TMEM read -> global operand -> math -> store, cannot hide that
+      // latency otherwise (ncu: 22 % of the samples on the first use of the load)
+      constexpr int NCH = SLICE / 16;
+      // chunks of this warp's column slice that hold live columns (a sliver tile: at most one warp group has any)
+      int live = (N - n0 - cs * SLICE + 15) >> 4;
+      live = live < 0 ? 0 : (live > NCH ? NCH : live);
+      if (live == 0) {                                      // nothing to read: hand the accumulators straight back
+        tc::mbar_wait(&tmem_full[buf], use & 1);
+        __syncwarp();
+        if (lane == 0) tc::mbar_arrive(&tmem_empty[buf]);
+      } else if constexpr (Epi::PREFETCH) {
+        uint32_t pw[2][8];
+        bool ph[2];
+        ph[0] = (n0 + cs * SLICE < N) && epi.preload(row, ok, n0 + cs * SLICE, N, pw[0]);
+        tc::mbar_wait(&tmem_full[buf], use & 1);            // the first request overlaps the wait for the accumulator
+        tc::tc_fence_after();
+#pragma unroll
+        for (int i = 0; i < NCH; ++i) {
+          if (i >= live) break;
+          const int c = cs * SLICE + 16 * i;
+          if (i + 1 < NCH) ph[(i + 1) & 1] = (n0 + c + 16 < N) && epi.preload(row, ok, n0 + c + 16, N, pw[(i + 1) & 1]);
+          float v[16];
+          tc::tmem_ld16(acc + (uint32_t)c, v);
+          tc::tmem_ld_wait();
+          if (i == live - 1) {                              // last read of this warp: hand the accumulators back early
+            tc::tc_fence_before();
             __syncwarp();
             if (lane == 0) tc::mbar_arrive(&tmem_empty[buf]);
           }
-        } else if constexpr (Epi::PREFETCH) {
-          uint32_t pw[2][8];
-          bool ph[2];
-          ph[0] = (n0 + cs * SLICE < N) && epi.preload(row, ok, n0 + cs * SLICE, N, pw[0]);
-          if (mt == 0) {                                      // the first request overlaps the wait for the accumulator
-            tc::mbar_wait(&tmem_full[buf], use & 1);
-            tc::tc_fence_after();
-          }
-#pragma unroll
-          for (int i = 0; i < NCH; ++i) {
-            if (i >= live) break;
-            const int c = cs * SLICE + 16 * i;
-            if (i + 1 < NCH) ph[(i + 1) & 1] = (n0 + c + 16 < N) && epi.preload(row, ok, n0 + c + 16, N, pw[(i + 1) & 1]);
-            float v[16];
-            tc::tmem_ld16(acc + (uint32_t)c, v);
-            tc::tmem_ld_wait();
-            if (mt == MT - 1 && i == live - 1) {              // last read of this warp: hand the accumulators back early
-              tc::tc_fence_before();
-              __syncwarp();
-              if (lane == 0) tc::mbar_arrive(&tmem_empty[buf]);
-            }
-            if (n0 + c < N) epi.chunk(row, ok, n0 + c, N, v, ph[i & 1] ? pw[i & 1] : nullptr);
-          }
-        } else {
-          if (mt == 0) {
-            tc::mbar_wait(&tmem_full[buf], use & 1);
-            tc::tc_fence_after();
-          }
-#pragma unroll 1
-          for (int i = 0; i < live; ++i) {
-            const int c = cs * SLICE + 16 * i;
-            float v[16];
-            tc::tmem_ld16(acc + (uint32_t)c, v);
-            tc::tmem_ld_wait();
-            if (mt == MT - 1 && i == live - 1) {
-              tc::tc_fence_before();
-              __syncwarp();
-              if (lane == 0) tc::mbar_arrive(&tmem_empty[buf]);
-            }
-            epi.chunk(row, ok, n0 + c, N, v);
-          }
+          if (n0 + c < N) epi.chunk(row, ok, n0 + c, N, v, ph[i & 1] ? pw[i & 1] : nullptr);
         }
-        epi.end(row, ok, tn * (EPI_WARPS / 4) + cs, tiles_n * (EPI_WARPS / 4));
+      } else {
+        tc::mbar_wait(&tmem_full[buf], use & 1);
+        tc::tc_fence_after();
+#pragma unroll 1
+        for (int i = 0; i < live; ++i) {
+          const int c = cs * SLICE + 16 * i;
+          float v[16];
+          tc::tmem_ld16(acc + (uint32_t)c, v);
+          tc::tmem_ld_wait();
+          if (i == live - 1) {
+            tc::tc_fence_before();
+            __syncwarp();
+            if (lane == 0) tc::mbar_arrive(&tmem_empty[buf]);
+          }
+          epi.chunk(row, ok, n0 + c, N, v);
+        }
       }
+      epi.end(row, ok, tn * (EPI_WARPS / 4) + cs, tiles_n * (EPI_WARPS / 4));
     }
   }
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
@@ -437,22 +417,18 @@ tc_layer_persistent_kernel(const __grid_constant__ LayerMaps maps, Epi epi, int 
   if (warp == 2) tc::tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
-int g_persist = -1;     // -1: by size; 0 / 1: forced (VAEB_TC_PERSIST, measurement switch)
-
-int g_persist_mt = -1;  // -1: by size; 1 / 2: forced (VAEB_TC_MT, measurement switch)
-
-template <int BN, bool B_MN, int NS, class Epi, int MT>
+template <int BN, bool B_MN, int NS, class Epi>
 cudaError_t launch_layer_persistent(cudaStream_t st, const LayerMaps& maps, const Epi& epi, int M, int N, int K,
                                     int a_row_off) {
-  using S = PersistSmem<BN, NS, MT>;
-  auto kfn = tc_layer_persistent_kernel<BN, B_MN, NS, Epi, MT>;
+  using S = PersistSmem<BN, NS>;
+  auto kfn = tc_layer_persistent_kernel<BN, B_MN, NS, Epi>;
   static bool attr_done = false;   // per instantiation
   if (!attr_done) {
     cudaError_t e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, S::TOTAL);
     if (e != cudaSuccess) return e;
     attr_done = true;
   }
-  const int tiles = ((N + BN - 1) / BN) * ((M + MT * BM - 1) / (MT * BM));
+  const int tiles = ((N + BN - 1) / BN) * ((M + BM - 1) / BM);
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(tiles < 148 ? tiles : 148);
   cfg.blockDim = dim3(TC_THREADS);
@@ -472,8 +448,6 @@ cudaError_t launch_layer_persistent(cudaStream_t st, const LayerMaps& maps, cons
 
 // the persistent form pays off from about one 128 x 256 tile per SM (4096 rows: 145 vs 142 us, bf16x3 190 vs 169 us)
 inline bool use_persistent(int M, int N, int bn) {
-  if (g_persist == -1) { const char* e = getenv("VAEB_TC_PERSIST"); g_persist = e ? (e[0] != '0' ? 1 : 0) : 2; }
-  if (g_persist != 2) return g_persist == 1;
   return ((N + bn - 1) / bn) * ((M + BM - 1) / BM) >= 120;   // 8192 rows x 500: 128 tiles (measured: 196 -> 170 us per update)
 }
 
@@ -510,26 +484,11 @@ template <bool A_MN, bool B_MN, class Epi>
 cudaError_t dispatch_layer(cudaStream_t st, int ns, int bn, const LayerMaps& maps, const Epi& epi, int M, int N, int K,
                            int a_row_off, int splits = 1) {
   if constexpr (!A_MN) {
-    // the persistent form with narrower tiles (thin layers of large batches: pure epilogue, so small tiles only even out
-    // the last wave -- 256 tiles of 256 columns on 148 SMs are two rounds, 1024 tiles of 64 columns are 1.75)
-    if (bn == 1064) {
-      if (ns == 2) return launch_layer_persistent<64, B_MN, 2, Epi, 1>(st, maps, epi, M, N, K, a_row_off);
-      return launch_layer_persistent<64, B_MN, 1, Epi, 1>(st, maps, epi, M, N, K, a_row_off);
-    }
-    if (bn == 1128) {
-      if (ns == 2) return launch_layer_persistent<128, B_MN, 2, Epi, 1>(st, maps, epi, M, N, K, a_row_off);
-      return launch_layer_persistent<128, B_MN, 1, Epi, 1>(st, maps, epi, M, N, K, a_row_off);
-    }
     if (bn == 256) {                   // tc_act_bn chose the persistent form
-      // (32 accumulator columns per TMEM read, the chain kernel's default, measured slower here: the Bernoulli epilogue
-      // loses its operand prefetch, dec2 57.5 -> 62.6 us, and the tanh / dgrad epilogues gain nothing)
-      if (ns == 2) return launch_layer_persistent<256, B_MN, 2, Epi, 1>(st, maps, epi, M, N, K, a_row_off);
-      // 256 x 256 tiles (VAEB_TC_MT=2): measured SLOWER at 16384 rows (275 vs 263 us per update; enc1 25.2 vs 23.2,
-      // dec2 44.1 vs 38.1 us) -- one wave of 128 tiles with the epilogue of both accumulators serialised behind the
-      // MMAs loses more than the halved operand traffic gains.  Kept as a measurement switch.
-      if (g_persist_mt == -1) { const char* e = getenv("VAEB_TC_MT"); g_persist_mt = e ? atoi(e) : 0; }
-      if (g_persist_mt == 2) return launch_layer_persistent<256, B_MN, 1, Epi, 2>(st, maps, epi, M, N, K, a_row_off);
-      return launch_layer_persistent<256, B_MN, 1, Epi, 1>(st, maps, epi, M, N, K, a_row_off);
+      // (32 accumulator columns per TMEM read measured slower here: the Bernoulli epilogue loses its operand prefetch,
+      // dec2 57.5 -> 62.6 us, and the tanh / dgrad epilogues gain nothing)
+      if (ns == 2) return launch_layer_persistent<256, B_MN, 2, Epi>(st, maps, epi, M, N, K, a_row_off);
+      return launch_layer_persistent<256, B_MN, 1, Epi>(st, maps, epi, M, N, K, a_row_off);
     }
   }
   if (ns == 2) {
@@ -607,9 +566,8 @@ bool add_reduce_job(TcReduceJobs* jobs, const TcReduceJob& j) {
   return true;
 }
 
-// `defer` != nullptr: the slices stay in `scratch` (a region of its own) and their reduction is appended to the list
 cudaError_t tc_wgrad_generic(cudaStream_t st, int64_t* launches, const LayerMaps& maps, int ns, int bn, int Kred,
-                             int Hreal, int N, int a_row_off, float* gW, float* gb, float* scratch, TcReduceJobs* defer,
+                             int Hreal, int N, int a_row_off, float* gW, float* gb, float* scratch,
                              float* gW6 = nullptr, float* gb6 = nullptr) {
   int splits = scratch ? tc_wgrad_splits(Hreal + 1, N, Kred, bn, ns) : 1;
   const size_t stride = (size_t)(Hreal + 1) * N;
@@ -622,18 +580,15 @@ cudaError_t tc_wgrad_generic(cudaStream_t st, int64_t* launches, const LayerMaps
     ++*launches;
     cudaError_t e = dispatch_layer<true, true>(st, ns, bn, maps, epi, Hreal + 1, N, Kred, a_row_off, splits);
     if (e != cudaSuccess) return e;
-    const TcReduceJob job{scratch, splits, stride, (Hreal + 1) * N, 0, gW, gb, gW6, gb6, 2, Hreal, N / 2};
-    if (defer && add_reduce_job(defer, job)) return cudaSuccess;
     TcReduceJobs one;
-    one.job[0] = job; one.n = 1;
+    one.job[0] = TcReduceJob{scratch, splits, stride, (Hreal + 1) * N, 0, gW, gb, gW6, gb6, 2, Hreal, N / 2};
+    one.n = 1;
     return reduce_all_impl(st, launches, one);
   }
   EpiWgradTc epi{gW, gb, Hreal, N, splits > 1 ? scratch : nullptr, stride};
   ++*launches;
   cudaError_t e = dispatch_layer<true, true>(st, ns, bn, maps, epi, Hreal + 1, N, Kred, a_row_off, splits);
   if (e != cudaSuccess || splits == 1) return e;
-  if (defer && add_reduce_job(defer, TcReduceJob{scratch, splits, stride, Hreal * N, N, gW, gb, nullptr, nullptr, 0, 0, 0}))
-    return cudaSuccess;
   const int tot = (int)stride;
   wgrad_split_reduce_kernel<<<(tot + 255) / 256, 256, 0, st>>>(scratch, splits, stride, Hreal * N, N, gW, gb);
   ++*launches;
@@ -825,9 +780,8 @@ static int make_pair_mn(CUtensorMap* hi, CUtensorMap* lo, const void* bh, const 
 
 // bn: UMMA N of the activation layers (tc_act_bn); bn_w: of the weight-gradient GEMMs
 int tc_build_maps(TcMaps* m, const TcBuffers& b, int rows_data, int R, int rows, int D, int H, int bn, int Z, int bn_w,
-                  int bn_d, int Dd, int bn_thin) {
+                  int bn_d, int Dd) {
   const uint32_t gd = (uint32_t)(bn_d > 0 ? bn_d : bn) / 64;
-  const uint32_t gt = (uint32_t)(bn_thin > 0 ? bn_thin : bn) / 64;      // dec1, dgrad h_e (K <= 64: pure epilogue)
   if (Dd <= 0) Dd = D;      // width of the decoder output layer: D, or 2 D for the interleaved Gaussian head
   const uint32_t ga = BM / 64, gb = (uint32_t)bn / 64, gw = (uint32_t)bn_w / 64;
   const uint32_t kw = b.w3l ? BK : 2 * BK;      // contraction rows per box of the weight-gradient operands (stage_k)
@@ -856,13 +810,10 @@ int tc_build_maps(TcMaps* m, const TcBuffers& b, int rows_data, int R, int rows,
     LayerMaps* w1 = reinterpret_cast<LayerMaps*>(m->wgrad1);
     VAEB_TRY(make_pair_mn(&w1->a_hi, &w1->a_lo, b.zh, b.zl, R, Z + 1, b.ldz, ga, kw));
     VAEB_TRY(make_pair_mn(&w1->b_hi, &w1->b_lo, b.d1h, b.d1l, R, H, b.ldh, gw, kw));
-    // wgrad W4|W5: A = h_e mirror [rows, H+1] MN-major (ones column -> gb4|gb5), B = [dmu|dls] mirror [rows, 2Z]
-    LayerMaps* w45 = reinterpret_cast<LayerMaps*>(m->wgrad45);
-    VAEB_TRY(make_pair_mn(&w45->a_hi, &w45->a_lo, b.heh, b.hel, rows, H + 1, b.ldh, ga, kw));
-    VAEB_TRY(make_pair_mn(&w45->b_hi, &w45->b_lo, b.ddh, b.ddl, rows, 2 * Z, b.ldq, 1, kw));
-    // the same GEMM inside the merged weight-gradient launch: B boxes as wide as the other jobs' (columns >= 2Z: zeros)
+    // wgrad W4|W5: A = h_e mirror [rows, H+1] MN-major (ones column -> gb4|gb5), B = [dmu|dls] mirror [rows, 2Z] with
+    // boxes as wide as the other weight-gradient jobs' (columns >= 2Z: zeros)
     LayerMaps* w45w = reinterpret_cast<LayerMaps*>(m->wgrad45w);
-    *w45w = *w45;
+    VAEB_TRY(make_pair_mn(&w45w->a_hi, &w45w->a_lo, b.heh, b.hel, rows, H + 1, b.ldh, ga, kw));
     VAEB_TRY(make_pair_mn(&w45w->b_hi, &w45w->b_lo, b.ddh, b.ddl, rows, 2 * Z, b.ldq, gw, kw));
     // enc2: A = h_e mirror [rows, H] K-major, B = interleaved heads mirror [H, 2Z] MN-major
     LayerMaps* e2 = reinterpret_cast<LayerMaps*>(m->enc2);
@@ -871,7 +822,7 @@ int tc_build_maps(TcMaps* m, const TcBuffers& b, int rows_data, int R, int rows,
     // dec1: A = z mirror [R, Z] K-major (the ones column at Z stays out of the map), B = W1 mirror [Z, H] MN-major
     LayerMaps* d1 = reinterpret_cast<LayerMaps*>(m->dec1);
     VAEB_TRY(make_pair(&d1->a_hi, &d1->a_lo, b.zh, b.zl, R, Z, b.ldz, BM));
-    VAEB_TRY(make_pair_mn(&d1->b_hi, &d1->b_lo, b.w1h, b.w1l, Z, H, b.ldh, gt));
+    VAEB_TRY(make_pair_mn(&d1->b_hi, &d1->b_lo, b.w1h, b.w1l, Z, H, b.ldh, gb));
     // dz: A = da1 mirror [R, H] K-major, B = W1 mirror [Z, H] K-major (N = Z rows)
     LayerMaps* dzm = reinterpret_cast<LayerMaps*>(m->dz);
     VAEB_TRY(make_pair(&dzm->a_hi, &dzm->a_lo, b.d1h, b.d1l, R, H, b.ldh, BM));
@@ -879,7 +830,7 @@ int tc_build_maps(TcMaps* m, const TcBuffers& b, int rows_data, int R, int rows,
     // dgrad h_e: A = [dmu|dls] mirror [rows, 2Z] K-major, B = [W4^T;W5^T] mirror [2Z, H] MN-major
     LayerMaps* dh = reinterpret_cast<LayerMaps*>(m->dhe);
     VAEB_TRY(make_pair(&dh->a_hi, &dh->a_lo, b.ddh, b.ddl, rows, 2 * Z, b.ldq, BM));
-    VAEB_TRY(make_pair_mn(&dh->b_hi, &dh->b_lo, b.w45h, b.w45l, 2 * Z, H, b.ldh, gt));
+    VAEB_TRY(make_pair_mn(&dh->b_hi, &dh->b_lo, b.w45h, b.w45l, 2 * Z, H, b.ldh, gb));
   }
   return VAEB_OK;
 }
@@ -976,44 +927,6 @@ cudaError_t tc_dgrad_he(cudaStream_t st, int64_t* launches, const TcMaps& m, int
   return dispatch_layer<false, true>(st, ns, bn, *reinterpret_cast<const LayerMaps*>(m.dhe), epi, rows, H, 2 * Z, 0);
 }
 
-cudaError_t tc_wgrad1(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int bn, int R, int Z, int H,
-                      float* gW1, float* gb1, float* scratch, TcReduceJobs* defer) {
-  return tc_wgrad_generic(st, launches, *reinterpret_cast<const LayerMaps*>(m.wgrad1), ns, bn, R, Z, H, 0, gW1, gb1,
-                          scratch, defer);
-}
-
-// scratch slices hold [(H+1) x 2Z]: column c < Z belongs to W4 / b4, c >= Z to W5 / b5
-__global__ void __launch_bounds__(256)
-wgrad45_reduce_kernel(const float* __restrict__ scratch, int splits, size_t stride, int H, int Z, float* __restrict__ gW4,
-                      float* __restrict__ gb4, float* __restrict__ gW5, float* __restrict__ gb5) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= (H + 1) * 2 * Z) return;
-  float a = 0.f;
-  for (int z = 0; z < splits; ++z) a += scratch[(size_t)z * stride + i];
-  const int k = i / (2 * Z), c = i - k * 2 * Z;
-  float* gW = c < Z ? gW4 : gW5;
-  float* gb = c < Z ? gb4 : gb5;
-  const int j = c < Z ? c : c - Z;
-  if (k < H) gW[(size_t)k * Z + j] = a; else gb[j] = a;
-}
-
-cudaError_t tc_wgrad45(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int rows, int H, int Z, float* gW4,
-                       float* gb4, float* gW5, float* gb5, float* scratch, TcReduceJobs* defer) {
-  const int N = 2 * Z;
-  const int splits = tc_wgrad_splits(H + 1, N, rows, 64, ns);
-  const size_t stride = (size_t)(H + 1) * N;
-  EpiWgradTc epi{nullptr, nullptr, H, N, scratch, stride};      // always through scratch: the reduce also de-interleaves
-  ++*launches;
-  cudaError_t e = dispatch_layer<true, true>(st, ns, 64, *reinterpret_cast<const LayerMaps*>(m.wgrad45), epi, H + 1, N, rows,
-                                             0, splits);
-  if (e != cudaSuccess) return e;
-  if (defer && add_reduce_job(defer, TcReduceJob{scratch, splits, stride, (H + 1) * N, 0, gW4, gb4, gW5, gb5, 1, H, Z}))
-    return cudaSuccess;
-  wgrad45_reduce_kernel<<<((H + 1) * N + 255) / 256, 256, 0, st>>>(scratch, splits, stride, H, Z, gW4, gb4, gW5, gb5);
-  ++*launches;
-  return cudaGetLastError();
-}
-
 size_t tc_wgrad_scratch_elems(int D, int H) {
   (void)D; (void)H;
   return (size_t)148 * BM * 128;          // splits * Mo * No <= (148 / tiles) * tiles * 128 * 128
@@ -1021,24 +934,19 @@ size_t tc_wgrad_scratch_elems(int D, int H) {
 
 // gW6 != nullptr (Gaussian decoder): D is the width of the interleaved head (2 x pixels); the reduction de-interleaves
 cudaError_t tc_wgrad2(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int bn, int R, int H, int D,
-                      float* gW2, float* gb2, float* scratch, TcReduceJobs* defer, float* gW6, float* gb6) {
+                      float* gW2, float* gb2, float* scratch, float* gW6, float* gb6) {
   return tc_wgrad_generic(st, launches, *reinterpret_cast<const LayerMaps*>(m.wgrad2), ns, bn, R, H, D, 0, gW2, gb2,
-                          scratch, defer, gW6, gb6);
+                          scratch, gW6, gb6);
 }
 
 cudaError_t tc_wgrad3(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int bn, int rows, int D, int H,
-                      int x_row_off, float* gW3, float* gb3, float* scratch, TcReduceJobs* defer) {
+                      int x_row_off, float* gW3, float* gb3, float* scratch) {
   return tc_wgrad_generic(st, launches, *reinterpret_cast<const LayerMaps*>(m.wgrad3), ns, bn, rows, D, H, x_row_off, gW3,
-                          gb3, scratch, defer);
+                          gb3, scratch);
 }
 
 // ---- every weight gradient of the step in one launch ------------------------------------------------------------
-bool tc_wgrad_merged_supported(int rows) {
-  static const int env = getenv("VAEB_TC_WGRAD_MERGE") ? atoi(getenv("VAEB_TC_WGRAD_MERGE")) : -1;   // measurement switch
-  if (env >= 0) return env != 0;
-  (void)rows;
-  return true;      // measured faster at every size (16384 rows bf16x3: 354.7 -> 339.6 us per update, bf16 222 -> 203)
-}
+// (measured faster than four launches at every size: 16384 rows bf16x3 354.7 -> 339.6 us per update, bf16 222 -> 203)
 
 cudaError_t tc_wgrad_all(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int bn, int R, int rows, int D, int H,
                          int Z, int x_row_off, float* gW2, float* gb2, float* gW1, float* gb1, float* gW4, float* gb4,

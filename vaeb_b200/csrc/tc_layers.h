@@ -32,8 +32,8 @@ struct TcMaps {
   alignas(64) unsigned char wgrad2[TC_LAYER_MAPS_BYTES];
   alignas(64) unsigned char wgrad3[TC_LAYER_MAPS_BYTES];
   alignas(64) unsigned char wgrad1[TC_LAYER_MAPS_BYTES];    // gW1|gb1 = [z|1]^T . da1
-  alignas(64) unsigned char wgrad45[TC_LAYER_MAPS_BYTES];   // gW4|gW5 (+ bias row) = [h_e|1]^T . [dmu|dls]
-  alignas(64) unsigned char wgrad45w[TC_LAYER_MAPS_BYTES];  // the same with B boxes as wide as the other weight gradients'
+  alignas(64) unsigned char wgrad45w[TC_LAYER_MAPS_BYTES];  // gW4|gW5 (+ bias row) = [h_e|1]^T . [dmu|dls], B boxes as wide
+                                                            // as the other weight gradients'
   alignas(64) unsigned char dhe[TC_LAYER_MAPS_BYTES];       // da3 = ([dmu|dls] . [W4^T;W5^T]) * (1 - h_e^2)
   alignas(64) unsigned char dz[TC_LAYER_MAPS_BYTES];        // dz = da1 . W1^T (+ dmu, dls in the epilogue)
   alignas(64) unsigned char enc2[TC_LAYER_MAPS_BYTES];      // (mu, ls) = h_e . [W4|W5] (+ reparameterisation in the epilogue)
@@ -49,7 +49,7 @@ int tc_act_bn(int rows, int n_min);
 // bn: UMMA N of the H-wide activation layers (enc1, dec1, both dgrads); bn_d (0: = bn): of dec2 (D wide)
 // Dd (0: = D): width of the decoder output layer -- 2 D for the Gaussian head's interleaved columns [W2|W6]'
 int tc_build_maps(TcMaps* m, const TcBuffers& b, int rows_data, int R, int rows, int D, int H, int bn, int Z, int bn_w,
-                  int bn_d = 0, int Dd = 0, int bn_thin = 0);   // bn_thin (0: = bn): tile width of dec1 / dgrad h_e
+                  int bn_d = 0, int Dd = 0);
 // Gaussian decoder (VAEB.py:257-258, 306-307): a|lv = h_d.[W2|W6]' + b, log-density and both deltas in the epilogue
 cudaError_t tc_dec2_gaussian(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int bn, int R, int H, int D,
                              const float* b2, const float* b6, const float* x, int x_div, int x_mod, float scale, void* da_hi,
@@ -69,7 +69,6 @@ cudaError_t tc_dec2_bernoulli(cudaStream_t st, int64_t* launches, const TcMaps& 
 cudaError_t tc_dgrad_hd(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int bn, int R, int D, int H,
                         const float* h_d, float* da1, void* d1_hi, void* d1_lo, int ldm, const void* h_hi = nullptr,
                         const void* h_lo = nullptr);   // h_d == nullptr: h is read from its mirror; da1 == nullptr: mirror only
-// thin weight gradients of the latent layers on tcgen05 (large batch): split-K over the rows, fixed-order reduction
 // Deferred reduction of split-K slices: the weight-gradient GEMMs of a step append their job, one launch sums all
 constexpr int TC_MAX_REDUCE_JOBS = 4;
 struct TcReduceJob {
@@ -78,8 +77,6 @@ struct TcReduceJob {
 };
 struct TcReduceJobs { TcReduceJob job[TC_MAX_REDUCE_JOBS]; int n = 0; };
 cudaError_t tc_wgrad_reduce_all(cudaStream_t st, int64_t* launches, const TcReduceJobs& jobs);
-cudaError_t tc_wgrad1(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int bn, int R, int Z, int H,
-                      float* gW1, float* gb1, float* scratch, TcReduceJobs* defer = nullptr);
 // all per-step weight mirrors / transposes of the large-batch path in one launch (W3, W2, [W4^T;W5^T] incl. its fp32
 // copy w45t, the interleaved heads, W1)
 cudaError_t tc_prepare_weights(cudaStream_t st, int64_t* launches, const float* W3, const float* W2, const float* W4,
@@ -104,31 +101,15 @@ cudaError_t tc_dz_dprep(cudaStream_t st, int64_t* launches, const TcMaps& m, int
 cudaError_t tc_dgrad_he(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int bn, int rows, int Z, int H,
                         const float* h_e, float* da3, void* da3_hi, void* da3_lo, int ldm, const void* h_hi = nullptr,
                         const void* h_lo = nullptr);
-cudaError_t tc_wgrad45(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int rows, int H, int Z, float* gW4,
-                       float* gb4, float* gW5, float* gb5, float* scratch, TcReduceJobs* defer = nullptr);
 // scratch: device floats for the split-K slices of a weight gradient (tc_wgrad_scratch_elems), or nullptr
 size_t tc_wgrad_scratch_elems(int D, int H);
 cudaError_t tc_wgrad2(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int bn, int R, int H, int D,
-                      float* gW2, float* gb2, float* scratch, TcReduceJobs* defer = nullptr, float* gW6 = nullptr,
-                      float* gb6 = nullptr);
+                      float* gW2, float* gb2, float* scratch, float* gW6 = nullptr, float* gb6 = nullptr);
 cudaError_t tc_wgrad3(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int bn, int rows, int D, int H,
-                      int x_row_off, float* gW3, float* gb3, float* scratch, TcReduceJobs* defer = nullptr);
-
-// ---- the activation chain as one persistent launch (tc_chain.cu) -------------------------------------------------
-// enc1 -> enc2 -> dec1 -> dec2 -> dgrad h_d -> dz -> dgrad h_e for `rows` rows (L = 1, Bernoulli decoder) as items of ONE
-// launch; row blocks are handed from layer to layer through arrival counters in `ready` (tc_chain_ready_elems(rows)
-// unsigned ints, zeroed when the shapes change; `epoch` = launches since then, starting at 1).
-int tc_chain_ready_elems(int rows);
-cudaError_t tc_chain_step(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int bn, int rows, int D, int H,
-                          int Z, int la, int x_row_off, const float* b3, const float* b4, const float* b5, const float* b1,
-                          const float* b2, const EpsSource& src, float scale, float w, float* mu, float* ls, float* eps,
-                          float* z, float* dmu, float* dls, float* aux_part, int* n_aux, float* partial, int* n_tiles,
-                          const TcBuffers& b, const void* xm_hi, const void* xm_lo, unsigned int* ready,
-                          unsigned int epoch, int n_sm, int pair);   // pair: cta_group::2 form, bn = 256 over maps built for 128
+                      int x_row_off, float* gW3, float* gb3, float* scratch);
 
 // every weight-gradient GEMM of the step in ONE launch (W2, W1, [W4|W5], W3); the split-K slices stay in `scratch`
 // (four regions of `region` floats) and their reductions are appended to `jobs`
-bool tc_wgrad_merged_supported(int rows);
 cudaError_t tc_wgrad_all(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int bn, int R, int rows, int D, int H,
                          int Z, int x_row_off, float* gW2, float* gb2, float* gW1, float* gb1, float* gW4, float* gb4,
                          float* gW5, float* gb5, float* gW3, float* gb3, float* scratch, size_t region, TcReduceJobs* jobs,
