@@ -11,7 +11,6 @@
 #include "launchers.h"
 #include "philox.cuh"
 
-int dec2_col_tiles(int rows, int D);  // kernels_gemm.cu
 bool is_tc_supported(const vaeb_handle* h);   // is_tc.cu
 int is_tc_run(vaeb_handle* h, const float* d_x, const float* d_mu, const float* d_ls, int n, int L, const float* d_eps,
               int64_t row_offset, float* d_logp, float* d_logw);
@@ -254,7 +253,6 @@ struct BoundOut {
   float* base_out; float mult; const float* tprior; int n_tprior; float div; float* scalar_out;
 };
 
-// Forward (+ backward into `grads`) of the graph of VAEB.getGradient for x[rows,D] on device.
 // Hidden layers of the encoder (VAEB.py:246; deeper encoders: replic.tex:46-57) for x[rows, D] on the fp32 per-layer kernels:
 // the activations of layers 1 .. depth-1 go to ws.h_x[], the last one -- what the heads read -- to ws.h_e.
 int encoder_hidden(vaeb_handle* h, const float* theta, const float* x, int rows) {
@@ -273,10 +271,68 @@ int encoder_hidden(vaeb_handle* h, const float* theta, const float* x, int rows)
   return VAEB_OK;
 }
 
-// `tail` != nullptr (training update whose tail is one launch, tc_tail.cu): on the large-batch tensor-core path the bound
-// and the split-K reductions are NOT launched here; what they need is recorded in *tail (tail->rows > 0 says so).
+// UMMA N of the weight-gradient layers, of the activation layers and of dec2 (D wide: more column tiles per row block than
+// the H-wide layers), and the x mirror the maps read, for the tcgen05 layers of one step (tc_setup)
+struct TcStep {
+  int bn = 64, bna = 64, bnd = 64;
+  int x_row_off = 0; const void *x_hi = nullptr, *x_lo = nullptr;
+};
+
+// What both tensor-core paths set up before their first layer: the bf16 mirrors for this shape, the mirror of an x staged
+// from the host, the tile widths, programmatic dependent launch and the tensor maps.
+int tc_setup(vaeb_handle* h, const float* x, int rows, int R, TcStep& ts) {
+  TcState& t = h->tc;
+  const int D = h->D, H = h->H;
+  VAEB_TRY(tc_ensure(h, rows, R));
+  ts.bn = R >= 1024 ? 128 : 64;
+  ts.bna = tc_act_bn(rows, std::min(H, D));
+  ts.bnd = ts.bna;
+  // few row blocks (the data-parallel split): one tile per CTA, and a layer should fill most of the SMs in ONE wave --
+  // 64-wide tiles for the H-wide layers when 128-wide ones give fewer than 96 CTAs (2048 rows: 64 -> 128 CTAs, enc1
+  // 14.5 -> 12.2 us, dgrad 15.6 -> 13.1), dec2 keeps 128 (7 column tiles per row block: 112 CTAs)
+  if (ts.bna == 128) {
+    const int rb = (rows + 127) / 128;
+    if (rb * ((H + 127) / 128) < 96) ts.bna = 64;
+    if (rb * (((h->cont ? 2 * D : D) + 127) / 128) < 96) ts.bnd = 64;
+  }
+  // Programmatic dependent launch for the one-tile-per-CTA kernels: bf16x3 (one CTA per SM: an early dependent grid
+  // never takes slots from the running one; 16384 rows: 523 -> 499 us per update) and, in plain bf16, whenever the
+  // activation layers are NOT in the persistent form (8192 rows: 215 -> 196 us); next to the persistent kernels the
+  // early two-per-SM grids cost more than they hide (16384 rows: 241 -> 247 us).  Persistent launches always use it.
+  tc_set_pdl(ts.bna != 256 || t.ns == 2);
+  TcBuffers b = t.data;
+  int64_t rows_data;
+  const bool resident = h->d_x && x >= h->d_x && x < h->d_x + (size_t)h->n_data * D;
+  if (resident) {
+    ts.x_row_off = (int)((x - h->d_x) / D);
+    rows_data = h->n_data;
+  } else {
+    // x was staged from the host for this call: mirror it now
+    if (rows > t.cap_stage) {
+      VAEB_CUDA(cudaStreamSynchronize(h->stream));
+      VAEB_TRY(grow_bytes(&t.xsh, (size_t)rows * b.ldx * 2));
+      if (t.ns == 2) VAEB_TRY(grow_bytes(&t.xsl, (size_t)rows * b.ldx * 2));
+      t.cap_stage = rows;
+      t.key_rows = -1;
+    }
+    PH("mirror staged x", 0, 4.0 * rows * D,
+       tc_split_matrix(h->stream, &h->launches, x, rows, D, D, t.xsh, t.xsl, b.ldx, D));
+    b.xh = t.xsh; b.xl = t.xsl;
+    rows_data = rows;
+  }
+  ts.x_hi = b.xh; ts.x_lo = t.ns == 2 ? b.xl : nullptr;
+  const int key_bn = (ts.bna * 1024 + ts.bn) * 1024 + ts.bnd;
+  if (t.key_rows != rows || t.key_R != R || t.key_data != rows_data || t.key_bn != key_bn || t.key_x != b.xh) {
+    VAEB_TRY(tc_build_maps(&t.maps, b, (int)rows_data, R, rows, D, H, ts.bna, h->Z, ts.bn, ts.bnd, h->cont ? 2 * D : D));
+    t.key_rows = rows; t.key_R = R; t.key_data = rows_data; t.key_bn = key_bn; t.key_x = b.xh;
+  }
+  return VAEB_OK;
+}
+
+// Forward (+ backward into `grads`) of the graph of VAEB.getGradient for x[rows,D] on device, one launch per layer: the
+// fp32 kernels, or with tc.active the wide layers (enc1, dec2, dgrad h_d, the W2 and W3 gradients) on tcgen05.
 int forward_backward(vaeb_handle* h, const float* theta, const float* x, int rows, int L, bool want_grads, float w,
-                     EpsSource src, float* grads, const BoundOut& bo, TcTailArgs* tail = nullptr) {
+                     EpsSource src, float* grads, const BoundOut& bo) {
   const Layout& l = h->lay;
   Workspace& s = h->ws;
   const int D = h->D, H = h->H, Z = h->Z;
@@ -286,109 +342,34 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
   int64_t* lc = &h->launches;
   int tiles = 0;
   const double dR = R, dr = rows, dD = D, dH = H, dZ = Z, c = h->cont ? 2.0 : 1.0;
-  // ---- tensor-core path: mirrors, descriptors -------------------------------------------------
   const bool tcp = h->tc.active;
   TcState& t = h->tc;
-  int x_row_off = 0, bn = 64, bna = 64;   // UMMA N of the weight-gradient / of the activation layers
-  int bnd = 64;                           // ... of dec2 (D wide: more column tiles per row block than the H-wide layers)
-  const void *x_mirror_hi = nullptr, *x_mirror_lo = nullptr;
-  if (tcp) {
-    VAEB_TRY(tc_ensure(h, rows, R));
-    bn = R >= 1024 ? 128 : 64;
-    bna = tc_act_bn(rows, std::min(H, D));
-    bnd = bna;
-    // few row blocks (the data-parallel split): one tile per CTA, and a layer should fill most of the SMs in ONE wave --
-    // 64-wide tiles for the H-wide layers when 128-wide ones give fewer than 96 CTAs (2048 rows: 64 -> 128 CTAs, enc1
-    // 14.5 -> 12.2 us, dgrad 15.6 -> 13.1), dec2 keeps 128 (7 column tiles per row block: 112 CTAs)
-    if (bna == 128) {
-      const int rb = (rows + 127) / 128;
-      if (rb * ((H + 127) / 128) < 96) bna = 64;
-      if (rb * (((h->cont ? 2 * D : D) + 127) / 128) < 96) bnd = 64;
-    }
-    // Programmatic dependent launch for the one-tile-per-CTA kernels: bf16x3 (one CTA per SM: an early dependent grid
-    // never takes slots from the running one; 16384 rows: 523 -> 499 us per update) and, in plain bf16, whenever the
-    // activation layers are NOT in the persistent form (8192 rows: 215 -> 196 us); next to the persistent kernels the
-    // early two-per-SM grids cost more than they hide (16384 rows: 241 -> 247 us).  Persistent launches always use it.
-    tc_set_pdl(bna != 256 || t.ns == 2);
-    TcBuffers b = t.data;
-    int64_t rows_data;
-    const bool resident = h->d_x && x >= h->d_x && x < h->d_x + (size_t)h->n_data * D;
-    if (resident) {
-      x_row_off = (int)((x - h->d_x) / D);
-      rows_data = h->n_data;
-    } else {
-      // x was staged from the host for this call: mirror it now
-      if (rows > t.cap_stage) {
-        VAEB_CUDA(cudaStreamSynchronize(st));
-        VAEB_TRY(grow_bytes(&t.xsh, (size_t)rows * b.ldx * 2));
-        if (t.ns == 2) VAEB_TRY(grow_bytes(&t.xsl, (size_t)rows * b.ldx * 2));
-        t.cap_stage = rows;
-        t.key_rows = -1;
-      }
-      PH("mirror staged x", 0, 4.0 * dr * dD,
-         tc_split_matrix(st, lc, x, rows, D, D, t.xsh, t.xsl, b.ldx, D));
-      b.xh = t.xsh; b.xl = t.xsl;
-      rows_data = rows;
-    }
-    x_mirror_hi = b.xh; x_mirror_lo = t.ns == 2 ? b.xl : nullptr;
-    if (t.key_rows != rows || t.key_R != R || t.key_data != rows_data || t.key_bn != (bna * 1024 + bn) * 1024 + bnd || t.key_x != b.xh) {
-      VAEB_TRY(tc_build_maps(&t.maps, b, (int)rows_data, R, rows, D, H, bna, Z, bn, bnd, h->cont ? 2 * D : D));
-      t.key_rows = rows; t.key_R = R; t.key_data = rows_data; t.key_bn = (bna * 1024 + bn) * 1024 + bnd; t.key_x = b.xh;
-    }
-    if (want_grads && b.heh && b.zh && b.d1h && b.ddh && latent_large_batch(rows, H, Z, L) && t.weights_ready &&
-        theta == h->d_params) {
-      // the tail of the previous update wrote the mirrors of these very parameters
-    } else if (want_grads && b.heh && b.zh && b.d1h && b.ddh && latent_large_batch(rows, H, Z, L))
-      PH("weight mirrors / transposes -> bf16 (one launch)", 0, 12.0 * dD * dH + 60.0 * dZ * dH,
-         tc_prepare_weights(st, lc, T_(h, theta, l.iW3), T_(h, theta, l.iW2), T_(h, theta, l.iW4), T_(h, theta, l.iW5),
-                            T_(h, theta, l.iW1), b, h->d_w45t, D, H, Z, h->cont ? T_(h, theta, l.iW6) : nullptr));
-    else
-      PH("mirror W3,W2 -> bf16", 0, 12.0 * dD * dH,
-         tc_mirror_weights(st, lc, T_(h, theta, l.iW3), b.w3h, b.w3l, D, H, b.ldh, T_(h, theta, l.iW2), b.w2h, b.w2l,
-                           b.ldd, h->cont ? T_(h, theta, l.iW6) : nullptr));
-  }
   const TcBuffers& tb = t.data;
-  // large-batch training on the tensor-core path: the thin weight gradients also run on tcgen05 (their operands'
-  // bf16 mirrors come from the kernels that produce h_e, z, da1 and [dmu|dls])
-  const bool tcl = tcp && want_grads && tb.heh && tb.zh && tb.d1h && tb.ddh && latent_large_batch(rows, H, Z, L);
-  // large batch: the four weight-gradient GEMMs are one launch after the last dgrad; their split-K slices stay in
-  // their scratch regions, and one launch after it (or the tail kernel) sums them all
-  TcReduceJobs reduce_jobs;
+  TcStep ts;
+  if (tcp) {
+    VAEB_TRY(tc_setup(h, x, rows, R, ts));
+    PH("mirror W3,W2 -> bf16", 0, 12.0 * dD * dH,
+       tc_mirror_weights(st, lc, T_(h, theta, l.iW3), tb.w3h, tb.w3l, D, H, tb.ldh, T_(h, theta, l.iW2), tb.w2h, tb.w2l,
+                         tb.ldd, h->cont ? T_(h, theta, l.iW6) : nullptr));
+  }
   // encoder hidden layer, VAEB.py:246
   if (tcp)
     PH("enc1 x.W3+tanh [tcgen05]", 2 * dr * dD * dH, 2.0 * t.ns * (dr * dD + dD * dH) + 4 * dr * dH,
-       tc_enc1(st, lc, t.maps, t.ns, bna, rows, D, H, x_row_off, T_(h, theta, l.ib3), tcl ? nullptr : s.h_e,
-               tcl ? tb.heh : nullptr, tcl ? tb.hel : nullptr, tb.ldh));   // tcl: every consumer of h_e reads its mirror
-  else
-  if (l.depth > 1)
+       tc_enc1(st, lc, t.maps, t.ns, ts.bna, rows, D, H, ts.x_row_off, T_(h, theta, l.ib3), s.h_e, nullptr, nullptr,
+               tb.ldh));
+  else if (l.depth > 1)
     VAEB_TRY(encoder_hidden(h, theta, x, rows));      // deeper encoders: replic.tex:46-57
   else
     PH("enc1 x.W3+tanh", 2 * dr * dD * dH, 4 * (dr * dD + dD * dH + dr * dH),
        launch_dense_act(st, lc, x, rows, D, T_(h, theta, l.iW3), T_(h, theta, l.ib3), H, h->hidden_act, s.h_e));
   // latent heads + reparameterisation + row terms + decoder hidden layer, VAEB.py:248-254,41-47,343
-  if (!tcl)
-    PH("transpose W4,W5", 0, 16 * dH * dZ,
-       launch_transpose_heads(st, lc, T_(h, theta, l.iW4), T_(h, theta, l.iW5), H, Z, h->d_w45t));
-  // the KL / L^A row partials of enc2: when the tail kernel ends the update it sums them itself (they are parked in the
-  // dz workspace, idle on this path: s.partial is overwritten by dec2), else a small launch folds them into row_aux now
-  const bool aux_to_tail = tcl && tail && 4 * ((2 * Z + 63) / 64) <= Z;
-  int n_aux_tail = 0;
-  if (tcl) {
-    int n_aux = 0;
-    PH("enc2 h_e.[W4|W5] + reparam + KL [tcgen05]", 4 * dr * dH * dZ, 2.0 * t.ns * (dr * dH + 2 * dH * dZ) + 20 * dr * dZ,
-       tc_enc2_heads(st, lc, t.maps, t.ns, rows, H, Z, la, T_(h, theta, l.ib4), T_(h, theta, l.ib5), src, s.mu, s.ls,
-                     s.eps, s.z, tb.zh, tb.zl, tb.ldz, aux_to_tail ? s.dz : s.partial, &n_aux));
-    if (aux_to_tail) n_aux_tail = n_aux;
-    else VAEB_LAUNCH(launch_row_partials_sum(st, lc, s.partial, n_aux, rows, s.row_aux));
-    PH("dec1 tanh(z.W1+b1) [tcgen05]", 2 * dR * dZ * dH, 2.0 * t.ns * (dR * 32 + dZ * dH) + 4 * dR * dH + 2.0 * t.ns * dR * dH,
-       tc_dec1(st, lc, t.maps, t.ns, bna, R, Z, H, T_(h, theta, l.ib1), nullptr, tb.hdh, tb.hdl, tb.ldh));
-  } else
+  PH("transpose W4,W5", 0, 16 * dH * dZ,
+     launch_transpose_heads(st, lc, T_(h, theta, l.iW4), T_(h, theta, l.iW5), H, Z, h->d_w45t));
   PH("latent fwd (enc2,reparam,KL,dec1)", 4 * dr * dH * dZ + 2 * dR * dZ * dH,
      4 * (dr * dH + 3 * dH * dZ + 2 * dr * dZ + 2 * dR * dZ + dR * dH),
-     launch_latent_fwd(st, lc, s.h_e, rows, H, h->d_w45t, T_(h, theta, l.ib4),
-                       T_(h, theta, l.ib5), T_(h, theta, l.iW1), T_(h, theta, l.ib1), Z, L, la, src, s.mu, s.ls,
-                       s.eps, s.z, s.row_aux, s.h_d, tcp ? tb.hdh : nullptr, tcp ? tb.hdl : nullptr, tb.ldh,
-                       tcl ? tb.zh : nullptr, tcl ? tb.zl : nullptr, tb.ldz, h->hidden_act));
+     launch_latent_fwd(st, lc, s.h_e, rows, H, h->d_w45t, T_(h, theta, l.ib4), T_(h, theta, l.ib5), T_(h, theta, l.iW1),
+                       T_(h, theta, l.ib1), Z, L, la, src, s.mu, s.ls, s.eps, s.z, s.row_aux, s.h_d,
+                       tcp ? tb.hdh : nullptr, tcp ? tb.hdl : nullptr, tb.ldh, h->hidden_act));
   // decoder output layer + log-likelihood, VAEB.py:257-263,302-313
   const float scale = w / (float)L;
   const float* W6 = h->cont ? T_(h, theta, l.iW6) : nullptr;
@@ -396,15 +377,15 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
   if (tcp && h->cont)
     PH("dec2 h.[W2|W6]+Gaussian loglik [tcgen05]", 4 * dR * dH * dD,
        2.0 * t.ns * (dR * dH + 2 * dH * dD) + 4 * dr * dD + (want_grads ? 4.0 * t.ns * dR * dD : 0.0),
-       tc_dec2_gaussian(st, lc, t.maps, t.ns, bnd, R, H, D, T_(h, theta, l.ib2), b6, tcl ? nullptr : x, 1, rows, scale,
+       tc_dec2_gaussian(st, lc, t.maps, t.ns, ts.bnd, R, H, D, T_(h, theta, l.ib2), b6, x, 1, rows, scale,
                         want_grads ? tb.da2h : nullptr, want_grads ? tb.da2l : nullptr, tb.ldd, s.partial, &tiles,
-                        x_mirror_hi, x_mirror_lo, tb.ldx, x_row_off));
+                        ts.x_hi, ts.x_lo, tb.ldx, ts.x_row_off));
   else if (tcp)
     PH("dec2 h.W2+loglik [tcgen05]", 2 * dR * dH * dD,
        2.0 * t.ns * (dR * dH + dH * dD) + 4 * dr * dD + (want_grads ? 2.0 * t.ns * dR * dD : 0.0),
-       tc_dec2_bernoulli(st, lc, t.maps, t.ns, bnd, R, H, D, T_(h, theta, l.ib2), tcl ? nullptr : x, 1, rows, scale,
+       tc_dec2_bernoulli(st, lc, t.maps, t.ns, ts.bnd, R, H, D, T_(h, theta, l.ib2), x, 1, rows, scale,
                          want_grads ? tb.da2h : nullptr, want_grads ? tb.da2l : nullptr, tb.ldd, s.partial, &tiles,
-                         x_mirror_hi, x_mirror_lo, tb.ldx, x_row_off));   // tcl: x from the mirror enc1 reads
+                         ts.x_hi, ts.x_lo, tb.ldx, ts.x_row_off));
   else
     PH("dec2 h.W2+loglik", 2 * dR * dH * dD * c,
        4 * (dR * dH + c * dH * dD + dr * dD + (want_grads ? c * dR * dD : 0.0)),
@@ -419,13 +400,12 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
   }
   // backward (T.grad, VAEB.py:397); formulas in SURVEY.md 8a
   if (tcp) {
-    if (!tcl)
-      PH("wgrad W2,b2 [tcgen05]", 2 * dR * dH * dD, 2.0 * t.ns * (dR * dH + dR * dD) + 4 * dH * dD,
-         tc_wgrad2(st, lc, t.maps, t.ns, bn, R, H, h->cont ? 2 * D : D, T_(h, grads, l.iW2), T_(h, grads, l.ib2), tb.wg_scratch,
-                   h->cont ? T_(h, grads, l.iW6) : nullptr, h->cont ? T_(h, grads, l.ib6) : nullptr));
+    PH("wgrad W2,b2 [tcgen05]", 2 * dR * dH * dD, 2.0 * t.ns * (dR * dH + dR * dD) + 4 * dH * dD,
+       tc_wgrad2(st, lc, t.maps, t.ns, ts.bn, R, H, h->cont ? 2 * D : D, T_(h, grads, l.iW2), T_(h, grads, l.ib2),
+                 tb.wg_scratch, h->cont ? T_(h, grads, l.iW6) : nullptr, h->cont ? T_(h, grads, l.ib6) : nullptr));
     PH("dgrad h_d (.W2^T)*(1-h^2) [tcgen05]", 2 * dR * dH * dD * c, 2.0 * t.ns * c * (dR * dD + dH * dD) + 8 * dR * dH,
-       tc_dgrad_hd(st, lc, t.maps, t.ns, bna, R, h->cont ? 2 * D : D, H, tcl ? nullptr : s.h_d, tcl ? nullptr : s.da1,
-                   tcl ? tb.d1h : nullptr, tcl ? tb.d1l : nullptr, tb.ldh, tb.hdh, tb.hdl));
+       tc_dgrad_hd(st, lc, t.maps, t.ns, ts.bna, R, h->cont ? 2 * D : D, H, s.h_d, s.da1, nullptr, nullptr, tb.ldh,
+                   tb.hdh, tb.hdl));
   } else {
     PH("wgrad W2,b2", 2 * dR * dH * dD, 4 * (dR * dH + dR * dD + dH * dD),
        launch_wgrad(st, lc, s.h_d, R, H, s.da2, D, T_(h, grads, l.iW2), T_(h, grads, l.ib2)));
@@ -435,45 +415,22 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
     PH("dgrad h_d (.W2^T)*(1-h^2)", 2 * dR * dH * dD * c, 4 * (c * dR * dD + c * dH * dD + 2 * dR * dH),
        launch_dgrad_tanh(st, lc, s.da2, T_(h, theta, l.iW2), h->cont ? s.dlv : nullptr, W6, R, D, H, s.h_d, s.da1, h->hidden_act));
   }
-  if (tcl) {
-    PH("dz da1.W1^T + dmu,dls [tcgen05]", 2 * dR * dZ * dH, 2.0 * t.ns * (dR * dH + dZ * dH) + 28 * dR * dZ,
-       tc_dz_dprep(st, lc, t.maps, t.ns, R, H, Z, la, w, s.z, s.eps, s.mu, s.ls, s.dmu, s.dls, tb.ddh, tb.ddl, tb.ldq));
-    if (tail) {
-      tail->partial = s.partial; tail->n_tiles = tiles; tail->rows = rows;
-      tail->aux_part = aux_to_tail ? s.dz : nullptr; tail->n_aux = n_aux_tail; tail->row_aux = aux_to_tail ? nullptr : s.row_aux;
-    } else
-    PH("bound (per row + total)", 0, 4 * (dR * tiles + 2 * dr),
-       launch_finalize(st, lc, s.partial, tiles, s.row_aux, rows, L, s.per_row, bo.base_out, bo.mult, bo.tprior,
-                       bo.n_tprior, bo.div, bo.scalar_out, h->d_counter, s.dec_aux));   // dec_aux: idle outside the IS path
-  } else
   PH("latent bwd (dz,dmu,dls,da3,bound)", 2 * dR * dZ * dH + 4 * dr * dH * dZ,
      4 * (dR * dH + 3 * dZ * dH + 2 * dr * dH + 3 * dR * dZ + dR * tiles),
-     launch_latent_bwd(st, lc, s.da1, T_(h, theta, l.iW1), h->d_w45t, s.h_e, s.z, s.eps,
-                       s.mu, s.ls, rows, H, Z, L, la, w, s.dmu, s.dls, s.da3, tcp ? tb.da3h : nullptr,
-                       tcp ? tb.da3l : nullptr, tb.ldh, s.partial, tiles,
+     launch_latent_bwd(st, lc, s.da1, T_(h, theta, l.iW1), h->d_w45t, s.h_e, s.z, s.eps, s.mu, s.ls, rows, H, Z, L, la, w,
+                       s.dmu, s.dls, s.da3, tcp ? tb.da3h : nullptr, tcp ? tb.da3l : nullptr, tb.ldh, s.partial, tiles,
                        s.row_aux, s.per_row, h->d_counter, bo.base_out, bo.mult, bo.tprior, bo.n_tprior, bo.div,
-                       bo.scalar_out, tcl ? tb.ddh : nullptr, tcl ? tb.ddl : nullptr, tb.ldq, h->hidden_act));
-  if (tcl) {
-    PH("dgrad h_e ([dmu|dls].W45^T)*(1-h^2) [tcgen05]", 4 * dr * dH * dZ, 2.0 * t.ns * (dr * 64 + 2 * dZ * dH) + 8 * dr * dH,
-       tc_dgrad_he(st, lc, t.maps, t.ns, bna, rows, Z, H, nullptr, nullptr, tb.da3h, tb.da3l, tb.ldh, tb.heh, tb.hel));
-    if (t.n_sm == 0) VAEB_CUDA(cudaDeviceGetAttribute(&t.n_sm, cudaDevAttrMultiProcessorCount, h->cfg.device));
-    PH("wgrad W2,W1,W4|W5,W3 (+ biases) [tcgen05, one launch]", 4 * dR * dH * dD + 2 * dR * dZ * dH + 4 * dr * dH * dZ,
-       2.0 * t.ns * (2 * dR * dH + 2 * dR * dD) + 8 * dH * dD,
-       tc_wgrad_all(st, lc, t.maps, t.ns, bn, R, rows, D, H, Z, x_row_off, T_(h, grads, l.iW2), T_(h, grads, l.ib2),
-                    T_(h, grads, l.iW1), T_(h, grads, l.ib1), T_(h, grads, l.iW4), T_(h, grads, l.ib4), T_(h, grads, l.iW5),
-                    T_(h, grads, l.ib5), T_(h, grads, l.iW3), T_(h, grads, l.ib3), tb.wg_scratch,
-                    tc_wgrad_scratch_elems(D, H), &reduce_jobs, t.n_sm, h->cont ? T_(h, grads, l.iW6) : nullptr,
-                    h->cont ? T_(h, grads, l.ib6) : nullptr));
-  } else
+                       bo.scalar_out, h->hidden_act));
   PH("wgrad W1,b1,W4,b4,W5,b5", 2 * dR * dZ * dH + 4 * dr * dH * dZ,
      4 * (dR * dZ + dR * dH + dr * dH + 2 * dr * dZ + 3 * dH * dZ),
      launch_small_wgrad(st, lc, s.z, s.da1, R, s.h_e, s.dmu, s.dls, rows, H, Z, T_(h, grads, l.iW1),
                         T_(h, grads, l.ib1), T_(h, grads, l.iW4), T_(h, grads, l.ib4), T_(h, grads, l.iW5),
                         T_(h, grads, l.ib5), s.wg_scratch));
-  if (tcp && !tcl)
+  if (tcp)
     PH("wgrad W3,b3 [tcgen05]", 2 * dr * dD * dH, 2.0 * t.ns * (dr * dD + dr * dH) + 4 * dD * dH,
-       tc_wgrad3(st, lc, t.maps, t.ns, bn, rows, D, H, x_row_off, T_(h, grads, l.iW3), T_(h, grads, l.ib3), tb.wg_scratch));
-  else if (!tcp) {
+       tc_wgrad3(st, lc, t.maps, t.ns, ts.bn, rows, D, H, ts.x_row_off, T_(h, grads, l.iW3), T_(h, grads, l.ib3),
+                 tb.wg_scratch));
+  else {
     // deeper encoders: da3 is the gradient at the pre-activation of the LAST hidden layer; for k = depth .. 2 the layer's
     // weight gradient is h_{k-1}^T . da_k and da_{k-1} = (da_k . W3_k^T) * f'(h_{k-1})
     float* dcur = s.da3;
@@ -488,9 +445,129 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
     PH("wgrad W3,b3", 2 * dr * dD * dH, 4 * (dr * dD + dr * dH + dD * dH),
        launch_wgrad(st, lc, x, rows, D, dcur, H, T_(h, grads, l.iW3), T_(h, grads, l.ib3)));
   }
-  if (tail && tail->rows > 0) tail->jobs = reduce_jobs;
-  else if (reduce_jobs.n > 0)
-    PH("sum of the split-K weight-gradient slices (one launch)", 0, 0, tc_wgrad_reduce_all(st, lc, reduce_jobs));
+  return VAEB_OK;
+}
+
+// Training gradients of a large batch on the tensor-core path (latent_large_batch: L = 1): every layer runs on tcgen05,
+// the thin latent ones too (their operands' bf16 mirrors come from the kernels that produce h_e, z, da1 and [dmu|dls]),
+// and the four weight-gradient GEMMs are one launch after the last dgrad, their split-K slices left in scratch.  With
+// `tail` the update ends in ONE launch that also applies prior + Adagrad; else the bound and the sum of the slices are
+// launched here and the caller applies the update.
+int large_batch_step(vaeb_handle* h, const float* theta, const float* x, int rows, float w, EpsSource src, float* grads,
+                     const BoundOut& bo, bool tail) {
+  const Layout& l = h->lay;
+  Workspace& s = h->ws;
+  const int D = h->D, H = h->H, Z = h->Z;
+  const int R = rows;                     // L = 1
+  const int la = h->cfg.estimator == VAEB_EST_LA ? 1 : 0;
+  cudaStream_t st = h->stream;
+  int64_t* lc = &h->launches;
+  int tiles = 0;
+  const double dR = R, dr = rows, dD = D, dH = H, dZ = Z, c = h->cont ? 2.0 : 1.0;
+  TcState& t = h->tc;
+  const TcBuffers& tb = t.data;
+  TcStep ts;
+  VAEB_TRY(tc_setup(h, x, rows, R, ts));
+  if (!t.weights_ready || theta != h->d_params)   // (else the tail of the previous update wrote the mirrors of theta)
+    PH("weight mirrors / transposes -> bf16 (one launch)", 0, 12.0 * dD * dH + 60.0 * dZ * dH,
+       tc_prepare_weights(st, lc, T_(h, theta, l.iW3), T_(h, theta, l.iW2), T_(h, theta, l.iW4), T_(h, theta, l.iW5),
+                          T_(h, theta, l.iW1), tb, h->d_w45t, D, H, Z, h->cont ? T_(h, theta, l.iW6) : nullptr));
+  // encoder hidden layer, VAEB.py:246: every consumer of h_e reads its mirror
+  PH("enc1 x.W3+tanh [tcgen05]", 2 * dr * dD * dH, 2.0 * t.ns * (dr * dD + dD * dH) + 4 * dr * dH,
+     tc_enc1(st, lc, t.maps, t.ns, ts.bna, rows, D, H, ts.x_row_off, T_(h, theta, l.ib3), nullptr, tb.heh, tb.hel, tb.ldh));
+  // latent heads + reparameterisation + row terms, VAEB.py:248-249,41-47,343.  The KL / L^A row partials: when the tail
+  // kernel ends the update it sums them itself (they are parked in the dz workspace, idle on this path: s.partial is
+  // overwritten by dec2), else a small launch folds them into row_aux now
+  const bool aux_to_tail = tail && 4 * ((2 * Z + 63) / 64) <= Z;
+  int n_aux = 0;
+  PH("enc2 h_e.[W4|W5] + reparam + KL [tcgen05]", 4 * dr * dH * dZ, 2.0 * t.ns * (dr * dH + 2 * dH * dZ) + 20 * dr * dZ,
+     tc_enc2_heads(st, lc, t.maps, t.ns, rows, H, Z, la, T_(h, theta, l.ib4), T_(h, theta, l.ib5), src, s.mu, s.ls,
+                   s.eps, s.z, tb.zh, tb.zl, tb.ldz, aux_to_tail ? s.dz : s.partial, &n_aux));
+  if (!aux_to_tail) VAEB_LAUNCH(launch_row_partials_sum(st, lc, s.partial, n_aux, rows, s.row_aux));
+  // decoder hidden layer, VAEB.py:254
+  PH("dec1 tanh(z.W1+b1) [tcgen05]", 2 * dR * dZ * dH, 2.0 * t.ns * (dR * 32 + dZ * dH) + 4 * dR * dH + 2.0 * t.ns * dR * dH,
+     tc_dec1(st, lc, t.maps, t.ns, ts.bna, R, Z, H, T_(h, theta, l.ib1), nullptr, tb.hdh, tb.hdl, tb.ldh));
+  // decoder output layer + log-likelihood, VAEB.py:257-263,302-313; x from the mirror enc1 reads
+  if (h->cont)
+    PH("dec2 h.[W2|W6]+Gaussian loglik [tcgen05]", 4 * dR * dH * dD,
+       2.0 * t.ns * (dR * dH + 2 * dH * dD) + 4 * dr * dD + 4.0 * t.ns * dR * dD,
+       tc_dec2_gaussian(st, lc, t.maps, t.ns, ts.bnd, R, H, D, T_(h, theta, l.ib2), T_(h, theta, l.ib6), nullptr, 1, rows,
+                        w, tb.da2h, tb.da2l, tb.ldd, s.partial, &tiles, ts.x_hi, ts.x_lo, tb.ldx, ts.x_row_off));
+  else
+    PH("dec2 h.W2+loglik [tcgen05]", 2 * dR * dH * dD,
+       2.0 * t.ns * (dR * dH + dH * dD) + 4 * dr * dD + 2.0 * t.ns * dR * dD,
+       tc_dec2_bernoulli(st, lc, t.maps, t.ns, ts.bnd, R, H, D, T_(h, theta, l.ib2), nullptr, 1, rows, w, tb.da2h,
+                         tb.da2l, tb.ldd, s.partial, &tiles, ts.x_hi, ts.x_lo, tb.ldx, ts.x_row_off));
+  // backward (T.grad, VAEB.py:397); formulas in SURVEY.md 8a
+  PH("dgrad h_d (.W2^T)*(1-h^2) [tcgen05]", 2 * dR * dH * dD * c, 2.0 * t.ns * c * (dR * dD + dH * dD) + 8 * dR * dH,
+     tc_dgrad_hd(st, lc, t.maps, t.ns, ts.bna, R, h->cont ? 2 * D : D, H, nullptr, nullptr, tb.d1h, tb.d1l, tb.ldh,
+                 tb.hdh, tb.hdl));
+  PH("dz da1.W1^T + dmu,dls [tcgen05]", 2 * dR * dZ * dH, 2.0 * t.ns * (dR * dH + dZ * dH) + 28 * dR * dZ,
+     tc_dz_dprep(st, lc, t.maps, t.ns, R, H, Z, la, w, s.z, s.eps, s.mu, s.ls, s.dmu, s.dls, tb.ddh, tb.ddl, tb.ldq));
+  if (!tail)
+    PH("bound (per row + total)", 0, 4 * (dR * tiles + 2 * dr),
+       launch_finalize(st, lc, s.partial, tiles, s.row_aux, rows, 1, s.per_row, bo.base_out, bo.mult, bo.tprior,
+                       bo.n_tprior, bo.div, bo.scalar_out, h->d_counter, s.dec_aux));   // dec_aux: idle outside the IS path
+  PH("dgrad h_e ([dmu|dls].W45^T)*(1-h^2) [tcgen05]", 4 * dr * dH * dZ, 2.0 * t.ns * (dr * 64 + 2 * dZ * dH) + 8 * dr * dH,
+     tc_dgrad_he(st, lc, t.maps, t.ns, ts.bna, rows, Z, H, nullptr, nullptr, tb.da3h, tb.da3l, tb.ldh, tb.heh, tb.hel));
+  if (t.n_sm == 0) VAEB_CUDA(cudaDeviceGetAttribute(&t.n_sm, cudaDevAttrMultiProcessorCount, h->cfg.device));
+  TcReduceJobs jobs;
+  PH("wgrad W2,W1,W4|W5,W3 (+ biases) [tcgen05, one launch]", 4 * dR * dH * dD + 2 * dR * dZ * dH + 4 * dr * dH * dZ,
+     2.0 * t.ns * (2 * dR * dH + 2 * dR * dD) + 8 * dH * dD,
+     tc_wgrad_all(st, lc, t.maps, t.ns, ts.bn, R, rows, D, H, Z, ts.x_row_off, T_(h, grads, l.iW2), T_(h, grads, l.ib2),
+                  T_(h, grads, l.iW1), T_(h, grads, l.ib1), T_(h, grads, l.iW4), T_(h, grads, l.ib4), T_(h, grads, l.iW5),
+                  T_(h, grads, l.ib5), T_(h, grads, l.iW3), T_(h, grads, l.ib3), tb.wg_scratch,
+                  tc_wgrad_scratch_elems(D, H), &jobs, t.n_sm, h->cont ? T_(h, grads, l.iW6) : nullptr,
+                  h->cont ? T_(h, grads, l.ib6) : nullptr));
+  if (!tail) {
+    if (jobs.n > 0) PH("sum of the split-K weight-gradient slices (one launch)", 0, 0, tc_wgrad_reduce_all(st, lc, jobs));
+    return VAEB_OK;
+  }
+  // the tail as one launch (tc_tail.cu): slices -> gradient, bound, (data parallel over peer memory: the gradient sum,)
+  // prior + Adagrad and the bf16 weight mirrors of the new parameters
+  const bool fb = h->cfg.variant == VAEB_VARIANT_FULLBAYES, dp = h->world > 1;
+  if (!t.tail_bar) {
+    VAEB_CUDA(cudaMalloc((void**)&t.tail_bar, sizeof(unsigned int)));
+    VAEB_CUDA(cudaMemsetAsync(t.tail_bar, 0, sizeof(unsigned int), st));
+    t.tail_bar_count = 0;
+  }
+  TcTailArgs ta{};
+  ta.jobs = jobs;
+  ta.params = h->d_params; ta.ada = h->d_ada; ta.grads = h->d_grads; ta.padded = l.padded;
+  ta.lr = h->cfg.learning_rate; ta.eps = h->cfg.adagrad_eps; ta.prior = fb ? 0.f : h->cfg.prior_scale;
+  ta.p2 = fb ? h->cfg.learning_rate * 1e-6f : 0.f;
+  ta.partial = s.partial; ta.n_tiles = tiles; ta.rows = rows;
+  ta.aux_part = aux_to_tail ? s.dz : nullptr; ta.n_aux = aux_to_tail ? n_aux : 0; ta.row_aux = aux_to_tail ? nullptr : s.row_aux;
+  ta.per_row = s.per_row; ta.block_part = s.dec_aux; ta.base_out = bo.base_out;
+  ta.mult = bo.mult; ta.div = bo.div; ta.scalar_out = bo.scalar_out;
+  ta.w3h = tb.w3h; ta.w3l = tb.w3l; ta.w2h = tb.w2h; ta.w2l = tb.w2l; ta.w45h = tb.w45h; ta.w45l = tb.w45l;
+  ta.whh = tb.whh; ta.whl = tb.whl; ta.w1h = tb.w1h; ta.w1l = tb.w1l; ta.w45t = h->d_w45t;
+  ta.D = D; ta.H = H; ta.Z = Z; ta.ldh = tb.ldh; ta.ldd = tb.ldd; ta.ldq = tb.ldq;
+  ta.oW3 = l.off[l.iW3]; ta.oW4 = l.off[l.iW4]; ta.oW5 = l.off[l.iW5]; ta.oW1 = l.off[l.iW1]; ta.oW2 = l.off[l.iW2];
+  ta.oW6 = h->cont ? l.off[l.iW6] : -1;
+  ta.bar = t.tail_bar;
+  ta.world = h->world; ta.rank = h->rank;
+  for (int r = 0; r < h->world && dp; ++r) {
+    ta.gsum[r] = t.p2p_gsum[r]; ta.flags[r] = t.p2p_flags[r];
+    ta.peer_params[r] = t.p2p_params[r]; ta.peer_ada[r] = t.p2p_ada[r];
+  }
+  const int grid = tc_tail_grid(t.n_sm);
+  static const char* stamp_path = getenv("VAEB_TAIL_STAMPS");      // debug: time stamps of the last 2048 tail launches
+  static long long* d_stamps = nullptr;
+  if (stamp_path && !d_stamps) {
+    VAEB_CUDA(cudaMalloc((void**)&d_stamps, 2048 * 8 * sizeof(long long)));
+    VAEB_CUDA(cudaMemset(d_stamps, 0, 2048 * 8 * sizeof(long long)));
+    g_tail_stamps = d_stamps;
+  }
+  auto launch_tail = [&]() -> cudaError_t {
+    ta.stamps = d_stamps ? d_stamps + 8 * (size_t)(t.p2p_epoch % 2048) : nullptr;
+    ta.bar_base = t.tail_bar_count;
+    ta.epoch = ++t.p2p_epoch;
+    t.tail_bar_count += (unsigned int)grid * (dp ? 2u : 1u);
+    return tc_tail_launch(st, lc, ta, grid);
+  };
+  PH("tail: slices -> gradient, bound, (all-reduce over peer memory,) prior + Adagrad, weight mirrors (one launch)", 0,
+     28.0 * (double)l.total, launch_tail());
   return VAEB_OK;
 }
 
@@ -525,9 +602,6 @@ int all_reduce_grads(vaeb_handle* h) {
 // One update on device-resident rows; the scalar lands in d_scalars[slot].
 int enqueue_update(vaeb_handle* h, const float* d_xrows, int rows, const float* d_eps, const float* d_zeta,
                    int slot, bool apply) {
-  if (apply) h->steptc.mirrors_valid = false;       // the parameters change behind the step kernel's bf16 mirrors
-  // (h->tc.weights_ready -- the large-batch path's weight mirrors -- is cleared below by every update that does not
-  // end in the tail kernel, which rewrites them)
   const Layout& l = h->lay;
   const int L = h->L;
   VAEB_TRY(ensure_ws(h, rows, (int64_t)rows * L, true));
@@ -537,90 +611,41 @@ int enqueue_update(vaeb_handle* h, const float* d_xrows, int rows, const float* 
   float* base = h->d_grads + l.padded;
   const int64_t n4 = l.padded / 4;
   const float Mg = (float)rows * (float)h->world;
+  const bool large = h->tc.active && latent_large_batch(rows, h->H, h->Z, L);
+  bool tail = false;
   if (!is_fvb(h)) {
     const bool fb = h->cfg.variant == VAEB_VARIANT_FULLBAYES;
     const float w = fb ? 1.0f / Mg : 1.0f;
     const bool dp = h->world > 1;
-    BoundOut bo{base, 1.0f, nullptr, 0, Mg, dp ? nullptr : h->d_scalars + slot};
     const float prior = fb ? 0.f : h->cfg.prior_scale;
     // Large-batch tensor-core path: everything after the last GEMM is ONE launch (tc_tail.cu) -- and in data-parallel
     // runs whose ranks mapped each other's buffers (vaeb_comm_p2p_attach) that launch is also the gradient all-reduce.
     // With the single weight-gradient launch in front of it, it measures equal to the five separate launches at 16384 rows
     // and 1-3 % faster below on one GPU; VAEB_TC_TAIL=0 switches it off (then: slice sum, row sums, bound, Adagrad, mirrors).
     static const int env_tail = getenv("VAEB_TC_TAIL") ? atoi(getenv("VAEB_TC_TAIL")) : -1;      // measurement switch
-    TcTailArgs tail{};
-    const bool want_tail = apply && h->optimizer != VAEB_OPT_ADADELTA && h->tc.active && L == 1 &&
-                           env_tail != 0 && (!dp || h->tc.p2p_ready);
-    VAEB_TRY(forward_backward(h, h->d_params, d_xrows, rows, L, true, w, src, h->d_grads, bo, want_tail ? &tail : nullptr));
-    if (tail.rows > 0) {
-      TcState& t = h->tc;
-      const TcBuffers& b = t.data;
-      if (!t.tail_bar) {
-        VAEB_CUDA(cudaMalloc((void**)&t.tail_bar, sizeof(unsigned int)));
-        VAEB_CUDA(cudaMemsetAsync(t.tail_bar, 0, sizeof(unsigned int), st));
-        t.tail_bar_count = 0;
-      }
-      if (t.n_sm == 0) VAEB_CUDA(cudaDeviceGetAttribute(&t.n_sm, cudaDevAttrMultiProcessorCount, h->cfg.device));
-      tail.params = h->d_params; tail.ada = h->d_ada; tail.grads = h->d_grads; tail.padded = l.padded;
-      tail.lr = h->cfg.learning_rate; tail.eps = h->cfg.adagrad_eps; tail.prior = prior;
-      tail.p2 = fb ? h->cfg.learning_rate * 1e-6f : 0.f;
-      tail.per_row = h->ws.per_row; tail.block_part = h->ws.dec_aux; tail.base_out = base;
-      tail.mult = 1.0f; tail.div = Mg; tail.scalar_out = h->d_scalars + slot;
-      tail.w3h = b.w3h; tail.w3l = b.w3l; tail.w2h = b.w2h; tail.w2l = b.w2l; tail.w45h = b.w45h; tail.w45l = b.w45l;
-      tail.whh = b.whh; tail.whl = b.whl; tail.w1h = b.w1h; tail.w1l = b.w1l; tail.w45t = h->d_w45t;
-      tail.D = h->D; tail.H = h->H; tail.Z = h->Z; tail.ldh = b.ldh; tail.ldd = b.ldd; tail.ldq = b.ldq;
-      tail.oW3 = l.off[l.iW3]; tail.oW4 = l.off[l.iW4]; tail.oW5 = l.off[l.iW5]; tail.oW1 = l.off[l.iW1];
-      tail.oW2 = l.off[l.iW2];
-      tail.oW6 = h->cont ? l.off[l.iW6] : -1;
-      tail.bar = t.tail_bar;
-      tail.world = h->world; tail.rank = h->rank;
-      for (int r = 0; r < h->world && dp; ++r) {
-        tail.gsum[r] = t.p2p_gsum[r]; tail.flags[r] = t.p2p_flags[r];
-        tail.peer_params[r] = t.p2p_params[r]; tail.peer_ada[r] = t.p2p_ada[r];
-      }
-      const int grid = tc_tail_grid(t.n_sm);
-      static const char* stamp_path = getenv("VAEB_TAIL_STAMPS");      // debug: time stamps of the last 2048 tail launches
-      static long long* d_stamps = nullptr;
-      if (stamp_path && !d_stamps) {
-        VAEB_CUDA(cudaMalloc((void**)&d_stamps, 2048 * 8 * sizeof(long long)));
-        VAEB_CUDA(cudaMemset(d_stamps, 0, 2048 * 8 * sizeof(long long)));
-        g_tail_stamps = d_stamps;
-      }
-      auto launch_tail = [&]() -> cudaError_t {
-        tail.stamps = d_stamps ? d_stamps + 8 * (size_t)(t.p2p_epoch % 2048) : nullptr;
-        tail.bar_base = t.tail_bar_count;
-        tail.epoch = ++t.p2p_epoch;
-        t.tail_bar_count += (unsigned int)grid * (dp ? 2u : 1u);
-        return tc_tail_launch(st, lc, tail, grid);
-      };
-      PH("tail: slices -> gradient, bound, (all-reduce over peer memory,) prior + Adagrad, weight mirrors (one launch)", 0,
-         28.0 * (double)l.total, launch_tail());
-      h->tc.weights_ready = true;
-      h->grads_have_prior = false;
-      ++h->step;
-      return VAEB_OK;
+    tail = large && apply && h->optimizer != VAEB_OPT_ADADELTA && env_tail != 0 && (!dp || h->tc.p2p_ready);
+    // data parallel without the tail: the optimizer launch writes the scalar, after the all-reduce
+    BoundOut bo{base, 1.0f, nullptr, 0, Mg, dp && !tail ? nullptr : h->d_scalars + slot};
+    if (large) VAEB_TRY(large_batch_step(h, h->d_params, d_xrows, rows, w, src, h->d_grads, bo, tail));
+    else VAEB_TRY(forward_backward(h, h->d_params, d_xrows, rows, L, true, w, src, h->d_grads, bo));
+    if (!tail) {                          // (the tail applied prior + Adagrad)
+      VAEB_TRY(all_reduce_grads(h));
+      if (apply && h->optimizer == VAEB_OPT_ADADELTA)
+        PH("adadelta+prior (flat)", 0, 28.0 * (double)l.total,
+           launch_adadelta(st, lc, h->d_params, h->d_ada, h->d_ada2, h->d_grads, n4, h->rho, h->cfg.adagrad_eps, prior,
+                           base, 1.0f, Mg, dp ? h->d_scalars + slot : nullptr));
+      else if (apply)
+        PH("adagrad+prior (flat)", 0, 20.0 * (double)l.total,
+           launch_adagrad(st, lc, h->d_params, h->d_ada, h->d_grads, n4, h->cfg.learning_rate, h->cfg.adagrad_eps,
+                          prior, fb ? h->cfg.learning_rate * 1e-6f : 0.f, base, 1.0f, Mg,
+                          dp ? h->d_scalars + slot : nullptr));
+      else
+        VAEB_LAUNCH(launch_add_prior(st, lc, h->d_grads, h->d_params, n4, prior, base, 1.0f, Mg,
+                                     dp ? h->d_scalars + slot : nullptr));
     }
-    if (apply) h->tc.weights_ready = false;
-    VAEB_TRY(all_reduce_grads(h));
-    if (apply && h->optimizer == VAEB_OPT_ADADELTA) {
-      PH("adadelta+prior (flat)", 0, 28.0 * (double)l.total,
-         launch_adadelta(st, lc, h->d_params, h->d_ada, h->d_ada2, h->d_grads, n4, h->rho, h->cfg.adagrad_eps, prior,
-                         base, 1.0f, Mg, dp ? h->d_scalars + slot : nullptr));
-      h->grads_have_prior = false;
-    } else if (apply) {
-      PH("adagrad+prior (flat)", 0, 20.0 * (double)l.total,
-         launch_adagrad(st, lc, h->d_params, h->d_ada, h->d_grads, n4, h->cfg.learning_rate, h->cfg.adagrad_eps,
-                        prior, fb ? h->cfg.learning_rate * 1e-6f : 0.f, base, 1.0f, Mg,
-                        dp ? h->d_scalars + slot : nullptr));
-      h->grads_have_prior = false;
-    } else {
-      VAEB_LAUNCH(launch_add_prior(st, lc, h->d_grads, h->d_params, n4, prior, base, 1.0f, Mg,
-                                   dp ? h->d_scalars + slot : nullptr));
-      h->grads_have_prior = true;
-    }
+    h->grads_have_prior = !apply;
   } else {
     VAEB_REQUIRE(h->world == 1, "full-VB estimators are single-GPU (replicas only)");
-    if (apply) h->tc.weights_ready = false;
     const bool sampled = h->cfg.estimator == VAEB_EST_FVB_SAMPLED;
     const float* theta = h->d_params;  // VAEB.py:119,352: frozen MAP parameters, weights never sampled
     if (sampled) {
@@ -631,11 +656,14 @@ int enqueue_update(vaeb_handle* h, const float* d_xrows, int rows, const float* 
     VAEB_LAUNCH(launch_theta_prior(st, lc, h->d_vmu, h->d_vsig, l.total, h->d_tprior));
     // SGVB = x.shape[0]*(sum logp + sum KL) + thetaPrior (VAEB.py:364); update returns SGVB/M
     BoundOut bo{base, (float)rows, h->d_tprior, VAEB_TP_BLOCKS, apply ? (float)rows : 1.0f, h->d_scalars + slot};
-    VAEB_TRY(forward_backward(h, theta, d_xrows, rows, L, sampled, (float)rows, src, h->d_grads, bo));
+    if (large && sampled) VAEB_TRY(large_batch_step(h, theta, d_xrows, rows, (float)rows, src, h->d_grads, bo, false));
+    else VAEB_TRY(forward_backward(h, theta, d_xrows, rows, L, sampled, (float)rows, src, h->d_grads, bo));
     VAEB_LAUNCH(launch_fvb_adagrad(st, lc, h->d_vmu, h->d_vsig, h->d_ada_mu, h->d_ada_sig, h->d_grads, h->d_zeta,
                                    sampled ? 1 : 0, l.total, h->cfg.learning_rate, h->cfg.adagrad_eps,
                                    h->cfg.prior_scale, h->d_gmu, h->d_gsig, apply ? 1 : 0));
   }
+  if (apply) invalidate_weight_mirrors(h);
+  if (tail) h->tc.weights_ready = true;         // the tail wrote the large-batch path's mirrors of the new parameters
   ++h->step;
   return VAEB_OK;
 }
@@ -723,7 +751,7 @@ struct StateBackup {
     return e;
   }
   ~StateBackup() {
-    h->steptc.mirrors_valid = false; h->tc.weights_ready = false;
+    invalidate_weight_mirrors(h);
     h->step = step0;
     h->launches = launches0;
     if (bp && ba) {
@@ -842,7 +870,6 @@ int vaeb_destroy(vaeb_handle* h) {
     if (q.partial) cudaFree(q.partial);
   }
   if (h->h_scalars) cudaFreeHost(h->h_scalars);
-  if (h->h_pinned) cudaFreeHost(h->h_pinned);
   if (h->copy_stream) {
     cudaStreamSynchronize(h->copy_stream);
     for (int i = 0; i < vaeb_handle::ASYNC_BUFS; ++i) {
@@ -893,7 +920,7 @@ int vaeb_set_tensors(vaeb_handle* h, int32_t which, const float* const* tensors)
   float* flat = flat_by_which(h, which);
   VAEB_REQUIRE(flat, "buffer not available for this estimator");
   VAEB_CUDA(cudaSetDevice(h->cfg.device));
-  h->steptc.mirrors_valid = false; h->tc.weights_ready = false;
+  invalidate_weight_mirrors(h);
   for (int t = 0; t < h->lay.n; ++t) {
     const size_t n = (size_t)h->lay.rows[t] * h->lay.cols[t];
     VAEB_CUDA(cudaMemcpyAsync(flat + h->lay.off[t], tensors[t], n * sizeof(float), cudaMemcpyHostToDevice, h->stream));
@@ -991,7 +1018,7 @@ int vaeb_ae_train(vaeb_handle* h, int32_t kind, const int32_t* idx, int32_t n, f
   VAEB_REQUIRE(h->L == 1 && !is_fvb(h) && h->world == 1, "AE baselines: L = 1, single GPU");
   VAEB_REQUIRE(h->lay.depth <= 1, "AE baselines have one hidden layer per side (degenerate-vae/ae.py:41-117)");
   if (!h->d_x) { vaeb_set_error("vaeb_ae_train before vaeb_upload_data"); return VAEB_ESTATE; }
-  h->steptc.mirrors_valid = false; h->tc.weights_ready = false;
+  invalidate_weight_mirrors(h);
   for (int i = 0; i < n; ++i) VAEB_REQUIRE(idx[i] >= 0 && idx[i] < h->n_data, "row index outside the resident data");
   VAEB_CUDA(cudaSetDevice(h->cfg.device));
   const Layout& l = h->lay;
@@ -1089,7 +1116,7 @@ int vaeb_set_hidden_activation(vaeb_handle* h, int32_t act) {
   h->hidden_act = act;
   // the single-launch step kernels and the tensor-core estimators are tanh-only
   h->fused_off = (act != VAEB_ACT_TANH || h->optimizer != VAEB_OPT_ADAGRAD) ? true : h->fused_off_user;
-  h->steptc.mirrors_valid = false; h->tc.weights_ready = false;
+  invalidate_weight_mirrors(h);
   return VAEB_OK;
 }
 
@@ -1207,7 +1234,6 @@ static int host_async_submit(vaeb_handle* h, const float* x, const uint8_t* x_u8
   }
   h->a_rows = rows;
   ++h->a_pending;
-  ++h->a_submitted;
   ++h->a_outstanding;
   if (h->a_pending == GROUP) VAEB_TRY(async_flush(h));
   return VAEB_OK;
@@ -1302,7 +1328,7 @@ int vaeb_apply_update(vaeb_handle* h) {
   VAEB_CUDA(cudaSetDevice(h->cfg.device));
   const bool fb = h->cfg.variant == VAEB_VARIANT_FULLBAYES;
   const float prior = (fb || h->grads_have_prior) ? 0.f : h->cfg.prior_scale;
-  h->steptc.mirrors_valid = false; h->tc.weights_ready = false;
+  invalidate_weight_mirrors(h);
   VAEB_LAUNCH(launch_adagrad(h->stream, &h->launches, h->d_params, h->d_ada, h->d_grads, h->lay.padded / 4,
                              h->cfg.learning_rate, h->cfg.adagrad_eps, prior,
                              fb ? h->cfg.learning_rate * 1e-6f : 0.f, h->d_grads + h->lay.padded, 1.f, 1.f, nullptr));

@@ -69,7 +69,7 @@ struct Workspace {
   float* wg_scratch = nullptr;        // row-chunk partials of the thin weight gradients (large batches)
   // deeper encoders: activations of hidden layers 1 .. depth-1 (h_e holds the LAST one, which the heads read) and a second
   // buffer for the gradient walking back through them
-  float* h_x[3] = {nullptr, nullptr, nullptr}; float* da3b = nullptr; int depth_alloc = 1;
+  float* h_x[3] = {nullptr, nullptr, nullptr}; float* da3b = nullptr;
 };
 
 // Tensor-core path state: bf16 (hi/lo) mirrors and their TMA descriptors.
@@ -78,7 +78,7 @@ struct TcState {
   int ns = 1;                              // 1: bf16, 2: bf16 hi+lo (three MMAs per k-step)
   TcBuffers data;                          // mirrors with the resident dataset as x
   void *xsh = nullptr, *xsl = nullptr;     // mirror of a staged (host-supplied) batch
-  int64_t cap_data = 0, cap_stage = 0, cap_R = 0, cap_rows = 0;
+  int64_t cap_stage = 0, cap_R = 0, cap_rows = 0;
   TcMaps maps;
   int64_t key_rows = -1, key_R = -1, key_data = -1; int key_bn = 0; const void* key_x = nullptr;
   int n_sm = 0;
@@ -149,12 +149,11 @@ struct vaeb_handle {
   static constexpr int ASYNC_GROUP = 4;                   // updates per launch of the fused kernel
   int a_pending = 0, a_group = 0; int64_t a_rows = 0;     // minibatches copied but not yet launched; current group buffer
   int* d_iota = nullptr;                                  // {0, 1, .., ASYNC_GROUP-1}: slot order inside a group buffer
-  int64_t a_submitted = 0; int a_outstanding = 0;
+  int a_outstanding = 0;
   float* h_async = nullptr; int h_async_cap = 0;          // pinned host landing zone of the bounds
   float* d_stage2 = nullptr; int64_t stage2_cap = 0;     // eps staging
   float* d_out = nullptr; int64_t out_cap = 0;           // device staging for outputs
   float* d_scalars = nullptr; float* h_scalars = nullptr; int scalars_cap = 0;
-  float* h_pinned = nullptr; int64_t pinned_cap = 0;     // pinned bounce buffer for H2D of inputs
   uint32_t step = 0;
   int64_t launches = 0;
   bool grads_have_prior = false;
@@ -168,5 +167,9 @@ struct vaeb_handle {
   // data parallel
   NcclApi nccl; void* comm = nullptr; int rank = 0, world = 1;
 };
+
+// The parameters changed behind the cached bf16 weight mirrors: those of the tensor-core step kernel (step_tc.cu) and
+// those of the large-batch path (written by tc_prepare_weights or the tail kernel).
+inline void invalidate_weight_mirrors(vaeb_handle* h) { h->steptc.mirrors_valid = false; h->tc.weights_ready = false; }
 
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }

@@ -1012,7 +1012,7 @@ int fused_step_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, 
   h->step += (uint32_t)n_steps;
   if ((n_steps & 1) && !fvb && !faithful) std::swap(h->d_params, f.params_alt);   // theta now lives in the other buffer
   h->grads_have_prior = false;
-  h->steptc.mirrors_valid = false; h->tc.weights_ready = false;
+  invalidate_weight_mirrors(h);
   return VAEB_OK;
 }
 

@@ -30,8 +30,6 @@ cudaError_t run_gemm(cudaStream_t st, int64_t* launches, const GemmOperands& g, 
 
 }  // namespace
 
-int dec2_col_tiles(int rows, int D) { return use_big_tiles(rows, D) ? (D + 63) / 64 : (D + 31) / 32; }
-
 cudaError_t launch_dense_act(cudaStream_t st, int64_t* launches, const float* in, int rows, int K, const float* W,
                              const float* b, int N, int act, float* out) {
   GemmOperands g{in, W, nullptr, nullptr, K, N, rows, N, K};

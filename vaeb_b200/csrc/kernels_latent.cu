@@ -422,14 +422,14 @@ constexpr int LB_ROWS = 64, LB_T = 256, LB_KC = 32, LB_WS = 52, LB_NC = 48, LB_Z
 __device__ __forceinline__ float4 lds4(const float* p) { return *reinterpret_cast<const float4*>(p); }
 
 // mu|ls = h_e.[W4|W5] + b ; eps, z, row terms ; h_d = tanh(z.W1 + b1)        (VAEB.py:248-254, 41-47, 343)
-__global__ void __launch_bounds__(LB_T)
+// Three blocks per SM (80 registers): left to itself ptxas takes 99 and fits two.
+__global__ void __launch_bounds__(LB_T, 3)
 lb_latent_fwd_kernel(const float* __restrict__ h_e, int rows, int H, const float* __restrict__ w45t,
                      const float* __restrict__ b4, const float* __restrict__ b5, const float* __restrict__ W1,
                      const float* __restrict__ b1, int Z, int la, EpsSource src, float* __restrict__ mu,
                      float* __restrict__ ls, float* __restrict__ eps, float* __restrict__ z,
                      float* __restrict__ row_aux, float* __restrict__ h_d, __nv_bfloat16* __restrict__ hd_hi,
-                     __nv_bfloat16* __restrict__ hd_lo, int ld_mirror, __nv_bfloat16* __restrict__ z_hi,
-                     __nv_bfloat16* __restrict__ z_lo, int ldz, int act) {
+                     __nv_bfloat16* __restrict__ hd_lo, int ld_mirror, int act) {
   __shared__ __align__(16) float hs[LB_ROWS][LB_KC + 1];
   __shared__ __align__(16) float ws[LB_KC][LB_WS];
   __shared__ __align__(16) float outs[LB_ROWS][LB_NC];
@@ -502,7 +502,6 @@ lb_latent_fwd_kernel(const float* __restrict__ h_e, int rows, int H, const float
           const float zv = am + expf(0.5f * al) * e;
           mu[o2] = am; ls[o2] = al; eps[o2] = e; z[o2] = zv;
           zs[rr][j] = zv;
-          if (z_hi) store_split(z_hi, z_lo, (size_t)m * ldz + j, zv);
           term += la ? (-0.5f * zv * zv + 0.5f * al + 0.5f * e * e) : 0.5f * (1.0f + al - am * am - expf(al));
         }
       }
@@ -545,12 +544,10 @@ lb_latent_bwd_kernel(const float* __restrict__ da1, const float* __restrict__ W1
                      const float* __restrict__ h_e, const float* __restrict__ z, const float* __restrict__ eps,
                      const float* __restrict__ mu, const float* __restrict__ ls, int rows, int H, int Z, int la,
                      float w, float* __restrict__ dmu, float* __restrict__ dls, float* __restrict__ da3,
-                     __nv_bfloat16* __restrict__ da3_hi, __nv_bfloat16* __restrict__ da3_lo, int ld_mirror,
                      const float* __restrict__ partial, int n_tiles, const float* __restrict__ row_aux,
                      float* __restrict__ per_row, unsigned int* __restrict__ counter, float* __restrict__ base_out,
                      float mult, const float* __restrict__ tprior, int n_tprior, float div,
-                     float* __restrict__ scalar_out, __nv_bfloat16* __restrict__ dd_hi, __nv_bfloat16* __restrict__ dd_lo,
-                     int ldq, int act) {
+                     float* __restrict__ scalar_out, int act) {
   __shared__ __align__(16) float ds[LB_ROWS][LB_KC + 1];
   __shared__ __align__(16) float ws[LB_KC][28];
   __shared__ __align__(16) float psum[2][LB_ROWS][LB_ZP];
@@ -615,15 +612,10 @@ lb_latent_bwd_kernel(const float* __restrict__ da1, const float* __restrict__ W1
       }
       dmu[o2] = a; dls[o2] = b;
       dd[rr][j] = a; dd[rr][Z + j] = b;
-      if (dd_hi) {
-        store_split(dd_hi, dd_lo, (size_t)m * ldq + j, a);
-        store_split(dd_hi, dd_lo, (size_t)m * ldq + Z + j, b);
-      }
     }
   }
   __syncthreads();
-  // da3: skipped when the [dmu|dls] mirrors feed a tcgen05 GEMM that computes it (tc_dgrad_he)
-  for (int n = t; n < (dd_hi ? 0 : H); n += LB_T) {
+  for (int n = t; n < H; n += LB_T) {
     float wr[LB_NC];
 #pragma unroll
     for (int c = 0; c < LB_NC; ++c) wr[c] = c < 2 * Z ? w45t[(size_t)c * H + n] : 0.f;
@@ -641,7 +633,6 @@ lb_latent_bwd_kernel(const float* __restrict__ da1, const float* __restrict__ W1
       const float hv = h_e[(size_t)m * H + n];
       const float v = a * act_bwd(hv, act);
       da3[(size_t)m * H + n] = v;
-      if (da3_hi) store_split(da3_hi, da3_lo, (size_t)m * ld_mirror + n, v);
     }
   }
   // per-datapoint bound: sum of the log-likelihood tile partials + the KL / LA row term
@@ -768,15 +759,14 @@ cudaError_t launch_transpose_heads(cudaStream_t st, int64_t* launches, const flo
 cudaError_t launch_latent_fwd(cudaStream_t st, int64_t* launches, const float* h_e, int rows, int H,
                               const float* w45t, const float* b4, const float* b5, const float* W1, const float* b1,
                               int Z, int L, int la, EpsSource src, float* mu, float* ls, float* eps, float* z,
-                              float* row_aux, float* h_d, void* hd_hi, void* hd_lo, int ld_mirror, void* z_hi,
-                              void* z_lo, int ldz, int act) {
+                              float* row_aux, float* h_d, void* hd_hi, void* hd_lo, int ld_mirror, int act) {
   const int nchunks = (2 * Z + 7) / 8;
   const int KS = max(1, NWARPS / nchunks);
   ++*launches;
   if (latent_lb_supported(rows, H, Z, L)) {
     lb_latent_fwd_kernel<<<(rows + LB_ROWS - 1) / LB_ROWS, LB_T, 0, st>>>(
         h_e, rows, H, w45t, b4, b5, W1, b1, Z, la, src, mu, ls, eps, z, row_aux, h_d, (__nv_bfloat16*)hd_hi,
-        (__nv_bfloat16*)hd_lo, ld_mirror, (__nv_bfloat16*)z_hi, (__nv_bfloat16*)z_lo, ldz, act);
+        (__nv_bfloat16*)hd_lo, ld_mirror, act);
   } else if (rows <= 512) {
     const size_t smem = (size_t)((KS + 1) * 2 * Z + 2 * Z) * sizeof(float);
     latent_fwd_kernel<1><<<rows, NTHREADS, smem, st>>>(h_e, rows, H, w45t, b4, b5, W1, b1, Z, L, la, src, mu, ls, eps,
@@ -798,15 +788,14 @@ cudaError_t launch_latent_bwd(cudaStream_t st, int64_t* launches, const float* d
                               float* da3, void* da3_hi, void* da3_lo, int ld_mirror, const float* partial,
                               int n_tiles, const float* row_aux, float* per_row, unsigned int* counter,
                               float* base_out, float mult, const float* tprior, int n_tprior, float div,
-                              float* scalar_out, void* dd_hi, void* dd_lo, int ldq, int act) {
+                              float* scalar_out, int act) {
   const int nchunks = (Z + 7) / 8;
   const int NSL = max(1, (NWARPS - 2) / nchunks);
   ++*launches;
   if (latent_lb_supported(rows, H, Z, L)) {
     lb_latent_bwd_kernel<<<(rows + LB_ROWS - 1) / LB_ROWS, LB_T, 0, st>>>(
-        da1, W1, w45t, h_e, z, eps, mu, ls, rows, H, Z, la, w, dmu, dls, da3, (__nv_bfloat16*)da3_hi,
-        (__nv_bfloat16*)da3_lo, ld_mirror, partial, n_tiles, row_aux, per_row, counter, base_out, mult, tprior,
-        n_tprior, div, scalar_out, (__nv_bfloat16*)dd_hi, (__nv_bfloat16*)dd_lo, ldq, act);
+        da1, W1, w45t, h_e, z, eps, mu, ls, rows, H, Z, la, w, dmu, dls, da3, partial, n_tiles, row_aux, per_row,
+        counter, base_out, mult, tprior, n_tprior, div, scalar_out, act);
   } else if (rows <= 512) {
     const size_t smem = (size_t)(NSL + 2) * Z * sizeof(float);
     latent_bwd_kernel<1><<<rows, NTHREADS, smem, st>>>(

@@ -108,18 +108,19 @@ cudaError_t launch_transpose_heads(cudaStream_t st, int64_t* launches, const flo
 cudaError_t launch_latent_fwd(cudaStream_t st, int64_t* launches, const float* h_e, int rows, int H,
                               const float* w45t, const float* b4, const float* b5, const float* W1, const float* b1,
                               int Z, int L, int la, EpsSource src, float* mu, float* ls, float* eps, float* z,
-                              float* row_aux, float* h_d, void* hd_hi, void* hd_lo, int ld_mirror,
-                              void* z_hi = nullptr, void* z_lo = nullptr, int ldz = 0, int act = 1);
-// true when the 64-row large-batch kernels serve this shape (they also emit the z / [dmu|dls] mirrors)
+                              float* row_aux, float* h_d, void* hd_hi, void* hd_lo, int ld_mirror, int act = 1);
+// true when the 64-row large-batch kernels serve this shape
 bool latent_large_batch(int rows, int H, int Z, int L);
 // dz, dmu/dls, da3 and the bound (per row + deterministic total by the last block to finish).
+// da3_hi/da3_lo: optional bf16 mirrors of da3, written only below latent_large_batch (the tensor-core path of the
+// large-batch shapes computes da3 on tcgen05).
 cudaError_t launch_latent_bwd(cudaStream_t st, int64_t* launches, const float* da1, const float* W1,
                               const float* w45t, const float* h_e, const float* z, const float* eps, const float* mu,
                               const float* ls, int rows, int H, int Z, int L, int la, float w, float* dmu, float* dls,
                               float* da3, void* da3_hi, void* da3_lo, int ld_mirror, const float* partial,
                               int n_tiles, const float* row_aux, float* per_row, unsigned int* counter,
                               float* base_out, float mult, const float* tprior, int n_tprior, float div,
-                              float* scalar_out, void* dd_hi = nullptr, void* dd_lo = nullptr, int ldq = 0, int act = 1);
+                              float* scalar_out, int act = 1);
 size_t small_wgrad_scratch_elems(int rows, int H, int Z);
 // gW1,gb1,gW4,gb4,gW5,gb5 in one launch (two for large batches: row chunks + deterministic reduce)
 cudaError_t launch_small_wgrad(cudaStream_t st, int64_t* launches, const float* z, const float* da1, int R,

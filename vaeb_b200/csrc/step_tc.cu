@@ -1714,7 +1714,6 @@ int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, int
   StepTcState& s = h->steptc;
   const Layout& l = h->lay;
   const int D = h->D, H = h->H, Z = h->Z;
-  h->tc.weights_ready = false;        // this kernel updates the parameters behind the large-batch path's mirrors
   if (!s.ready) {
     VAEB_TRY(step_tc_init(h));
     if (s.unavailable) { vaeb_set_error("step_tc: thread-block clusters of 4 are not available on this device"); return VAEB_ESTATE; }
@@ -1760,7 +1759,7 @@ int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, int
     if (!s.mirrors_valid || s.theta_step != (long long)h->step) {
       VAEB_CUDA(launch_sample_theta(h->stream, &h->launches, h->d_vmu, h->d_vsig, nullptr, h->cfg.seed, h->step, l.total,
                                     h->d_theta, h->d_zeta));
-      s.mirrors_valid = false;
+      invalidate_weight_mirrors(h);
     }
   }
   if (p.fvb) {
@@ -1807,6 +1806,8 @@ int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, int
   else VAEB_CUDA(cudaLaunchKernelEx(&cfg, step_tc_kernel<false>, p));
   ++h->launches;
   h->grads_have_prior = false;
+  invalidate_weight_mirrors(h);
+  s.mirrors_valid = true;             // the kernel keeps its own mirrors current with the parameters it updates
   int done = n_steps;
   if (can_abort) {
     // the Gaussian decoder's deltas are unbounded: did a step leave the range of the fp16 operand pairs?

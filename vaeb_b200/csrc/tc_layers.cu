@@ -195,7 +195,7 @@ tc_wgrad_all_kernel(const __grid_constant__ WgradAllArgs args) {
                                              J.tiles_n, J.splits);
 }
 
-thread_local bool g_pdl = false;   // set and read within one forward_backward call of one thread
+thread_local bool g_pdl = false;   // set and read within one step of one thread (tc_setup)
 
 // ---- persistent form for large batches (A K-major: the activation layers) ---------------------------------
 // One CTA per SM walks the tile list (tile = blockIdx.x + i * gridDim.x; tiles of one row block are neighbours, so
@@ -874,24 +874,6 @@ cudaError_t tc_dgrad_hd(cudaStream_t st, int64_t* launches, const TcMaps& m, int
                    (const __nv_bfloat16*)h_hi, (const __nv_bfloat16*)h_lo};
   ++*launches;
   return dispatch_layer<false, false>(st, ns, bn, *reinterpret_cast<const LayerMaps*>(m.dgrad), epi, R, H, D, 0);
-}
-
-__global__ void __launch_bounds__(256)
-mirror_heads_kernel(const float* __restrict__ W4, const float* __restrict__ W5, int H, int Z, __nv_bfloat16* __restrict__ hi,
-                    __nv_bfloat16* __restrict__ lo, int ldq) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= H * ldq) return;
-  const int k = i / ldq, c = i - k * ldq, j = c >> 1;
-  float v = 0.f;
-  if (j < Z) v = (c & 1) ? W5[(size_t)k * Z + j] : W4[(size_t)k * Z + j];
-  put_split(hi, lo, (size_t)i, v);
-}
-
-cudaError_t tc_mirror_heads(cudaStream_t st, int64_t* launches, const float* W4, const float* W5, int H, int Z, void* hi,
-                            void* lo, int ldq) {
-  mirror_heads_kernel<<<(H * ldq + 255) / 256, 256, 0, st>>>(W4, W5, H, Z, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo, ldq);
-  ++*launches;
-  return cudaGetLastError();
 }
 
 cudaError_t tc_enc2_heads(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int rows, int H, int Z, int la,

@@ -82,9 +82,6 @@ cudaError_t tc_wgrad_reduce_all(cudaStream_t st, int64_t* launches, const TcRedu
 cudaError_t tc_prepare_weights(cudaStream_t st, int64_t* launches, const float* W3, const float* W2, const float* W4,
                                const float* W5, const float* W1, const TcBuffers& b, float* w45t, int D, int H, int Z,
                                const float* W6 = nullptr);
-// interleaved bf16 mirror of the two head weight matrices (so that one epilogue thread holds mu_j and ls_j together)
-cudaError_t tc_mirror_heads(cudaStream_t st, int64_t* launches, const float* W4, const float* W5, int H, int Z, void* hi,
-                            void* lo, int ldq);
 // (mu, ls) = h_e.[W4|W5] + b fused with eps, z = mu + exp(.5 ls) eps, the KL / LA row terms (4 partials per row in
 // aux_part) and the z mirror (VAEB.py:248-249, 41-47, 343, 322-325)
 struct EpsSource;
