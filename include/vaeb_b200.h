@@ -86,7 +86,8 @@ typedef struct vaeb_config {
 #define VAEB_ACT_RELU 3
 
 const char* vaeb_last_error(void);
-int vaeb_version(void);      /* 101: vaeb_config ends with encoder_hidden_layers, reserved0 (100: it ended with seed) */
+int vaeb_version(void);      /* 102: adds the encode, sample and validate_terms entry points (vaeb_config unchanged);
+                                101: vaeb_config ends with encoder_hidden_layers, reserved0 (100: it ended with seed) */
 /* sizeof(vaeb_config) as this library was compiled: a binding that declares the struct itself (ctypes, cgo) compares it
  * with its own size before the first vaeb_create -- a shorter struct would be read past its end. */
 int vaeb_config_size(void);
@@ -217,6 +218,36 @@ int vaeb_reconstruct(vaeb_handle* h, const float* x, int64_t n, int32_t n_sample
  * of freyFace.py:237-244 that the manifold renderer :350-369 calls): y_out[n,D] = sigmoid(tanh(z.W1+b1).W2+b2),
  * and for the Gaussian decoder lv_out[n,D] = tanh(z.W1+b1).W6+b6 (else may be NULL). */
 int vaeb_decode(vaeb_handle* h, const float* z, int64_t n, float* y_out, float* lv_out);
+
+/* The encoder alone (VAEB.py:245-251): the parameters of q(z|x) for host x[n,D].  mu_out[n,Z] is the mean and
+ * logvar_out[n,Z] the second head, a log-VARIANCE although the reference names it log_sigma (VAEB.py:45,343).  Every
+ * encoder depth and hidden activation; the fp32 per-layer kernels for every precision, in chunks of 32768 rows. */
+int vaeb_encode(vaeb_handle* h, const float* x, int64_t n, float* mu_out, float* logvar_out);
+
+/* Samples from the generative model (AEVB Fig. 5): for rows i < n, z_i ~ N(0, I), the decoder outputs of z_i and a draw
+ * x_i ~ p(x|z_i).  z_out[n,Z]; mean_out[n,D] = y (sigmoid outputs, as vaeb_decode); lv_out[n,D] the Gaussian decoder's
+ * log-variance output (the Bernoulli decoder: must be NULL); x_out[n,D].  Any output may be NULL.
+ * Noise: Philox stream 5 (VAEB_STREAM_SAMPLE), key = cfg.seed, counter step = `step`, global row r = row_offset + i:
+ *   z[i,j]   = normal   element r*Z + j of (stream 5, step, sample 0)
+ *   x[i,d]:  u / eps  = element r*D + d of (stream 5, step, sample 1)
+ *     Bernoulli: x = 1 if u < y else 0, u the uniform ((bits >> 8) + 0.5) * 2^-24 of that element's 32-bit output
+ *     Gaussian:  x = y + exp(lv / 2) * eps, eps the normal of that element -- the likelihood's own variance exp(lv)
+ *                (VAEB.py:302-313), not the exp(lv)^2 of the reference's reconstruct (VAEB.py:295-297)
+ * "normal" / "uniform element e" as in vaeb_philox_normal: group e / 4, output e % 4, Box-Muller pairs (0,1), (2,3).
+ * Results do not depend on how rows are split over calls or GPUs.  The step counter of the handle is not used or
+ * advanced. */
+int vaeb_sample(vaeb_handle* h, int64_t n, uint32_t step, int64_t row_offset, float* z_out, float* mean_out,
+                float* lv_out, float* x_out);
+
+/* The two terms of getLB / getLA (VAEB.py:332-346, :315-330) per row of x[n,D], with the inputs, noise and step counter
+ * of vaeb_validate: loglik_out[n] = mean over the L samples of log p(x|z); aux_out[n] = the term the estimator adds to
+ * it, the analytic -KL for L^B and the Monte-Carlo mean of log p(z) - log q(z|x) for L^A.  Their sum is vaeb_validate's
+ * per-row bound, bit for bit when L is a power of two; otherwise the bound is formed with one fused multiply-add and
+ * the float sum loglik + aux can differ from it in the last bit.  Full-VB handles return the same two terms under the
+ * parameters they evaluate with; the weight-prior term of their bound (VAEB.py:359-363) is not per row and is in
+ * neither. */
+int vaeb_validate_terms(vaeb_handle* h, const float* x, int64_t n, const float* eps, float* loglik_out,
+                        float* aux_out);
 
 /* Dense tanh layers of the AE-side builders (degenerate-vae/mlp.py:66-74 ConstructMLP):
  * out = f(...f(x.W0+b0)...Wk+bk), f = tanh on every layer (act=1) or identity on the last

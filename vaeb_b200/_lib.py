@@ -60,6 +60,10 @@ EXPORTS = {
                                 C.c_void_p, C.c_void_p]),
     "vaeb_reconstruct": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "vaeb_decode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
+    "vaeb_encode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
+    "vaeb_sample": (C.c_int, [C.c_void_p, C.c_int64, C.c_uint32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                              C.c_void_p]),
+    "vaeb_validate_terms": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "vaeb_mlp_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.POINTER(C.c_int32),
                                    C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int32, C.c_void_p]),
     "vaeb_philox_normal": (C.c_int, [C.c_void_p, C.c_int32, C.c_uint32, C.c_uint32, C.c_int64, C.c_int64, C.c_void_p]),

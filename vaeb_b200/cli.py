@@ -28,7 +28,10 @@ command_line_args = {'seed': (15485863, int),
                      'device': (0, int),
                      'precision': ('fp32', str),      # fp32 | bf16
                      'eps_mode': ('philox', str),     # philox | theano
-                     'manifold_file': ('', str)}      # PGM of the learned 2-d manifold (freyFace.py:346-369)
+                     'manifold_file': ('', str),      # PGM of the learned 2-d manifold (freyFace.py:346-369)
+                     # PGM of 10 x 10 random samples (AEVB Fig. 5); a Bernoulli model shows its decoder means,
+                     # since binary draws make a poor image
+                     'sample_file': ('', str)}
 command_line_flags = ['continuous', 'generic_estimator', 'full_varational',
                       # --- extensions ---
                       'synthetic',        # synthetic data of the dataset's shape if the files are absent
@@ -140,6 +143,10 @@ def train_model(args, data=None):
         from . import manifold
         _, tiled = manifold.render(model)
         manifold.save_pgm(tiled, args['manifold_file'])
+    if len(args.get('sample_file', '')) > 0:
+        from . import manifold
+        _, tiled = manifold.render_samples(model)
+        manifold.save_pgm(tiled, args['sample_file'])
 
     return model, data
 

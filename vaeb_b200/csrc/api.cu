@@ -248,9 +248,11 @@ inline float* T_(vaeb_handle* h, float* base, int idx) { return base + h->lay.of
 inline const float* T_(vaeb_handle* h, const float* base, int idx) { return base + h->lay.off[idx]; }
 
 // Where the bound of a step goes: base (sum of per-row bounds) always; the scalar
-// (mult*base + sum(tprior))/div if scalar_out != nullptr.
+// (mult*base + sum(tprior))/div if scalar_out != nullptr; with loglik_rows / aux_rows (evaluation only) the two terms
+// of every per-row bound.
 struct BoundOut {
   float* base_out; float mult; const float* tprior; int n_tprior; float div; float* scalar_out;
+  float* loglik_rows = nullptr; float* aux_rows = nullptr;
 };
 
 // Hidden layers of the encoder (VAEB.py:246; deeper encoders: replic.tex:46-57) for x[rows, D] on the fp32 per-layer kernels:
@@ -395,7 +397,7 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
   if (!want_grads) {
     PH("finalize bound", 0, 4.0 * R * tiles,
        launch_finalize(st, lc, s.partial, tiles, s.row_aux, rows, L, s.per_row, bo.base_out, bo.mult, bo.tprior,
-                       bo.n_tprior, bo.div, bo.scalar_out));
+                       bo.n_tprior, bo.div, bo.scalar_out, nullptr, nullptr, bo.loglik_rows, bo.aux_rows));
     return VAEB_OK;
   }
   // backward (T.grad, VAEB.py:397); formulas in SURVEY.md 8a
@@ -768,7 +770,7 @@ static int async_flush(vaeb_handle* h);
 static void p2p_release(vaeb_handle* h);   // unmaps the peers' buffers (data parallel over peer memory)   // launches streaming updates that were copied but not yet started
 
 const char* vaeb_last_error(void) { return g_last_error.c_str(); }
-int vaeb_version(void) { return 101; }
+int vaeb_version(void) { return 102; }   // 102: vaeb_encode, vaeb_sample, vaeb_validate_terms (101: encoder_hidden_layers)
 int vaeb_config_size(void) { return (int)sizeof(vaeb_config); }
 
 int vaeb_create(const vaeb_config* cfg, vaeb_handle** out) {
@@ -1336,7 +1338,10 @@ int vaeb_apply_update(vaeb_handle* h) {
   return VAEB_OK;
 }
 
-int vaeb_validate(vaeb_handle* h, const float* x, int64_t n, const float* eps, float* sgvb_out, float* per_row_out) {
+// vaeb_validate / vaeb_validate_terms: the bound of x[n,D] with the current parameters; loglik_out / aux_out (both or
+// neither, host float[n]) receive the two terms of every per-row bound.
+static int validate_rows(vaeb_handle* h, const float* x, int64_t n, const float* eps, float* sgvb_out, float* per_row_out,
+                         float* loglik_out, float* aux_out) {
   if (h && h->a_pending) VAEB_TRY(async_flush(h));
   VAEB_REQUIRE(h && x && sgvb_out && n > 0, "null argument");
   VAEB_REQUIRE(n * (int64_t)h->L < (int64_t)1 << 31, "too many rows for one validate call");
@@ -1365,12 +1370,31 @@ int vaeb_validate(vaeb_handle* h, const float* x, int64_t n, const float* eps, f
     div = (float)n;                      // T.mean, VAEBfullbayes.py:142
   }
   BoundOut bo{h->d_grads + h->lay.padded, mult, tp, VAEB_TP_BLOCKS, div, h->d_scalars};
+  if (loglik_out) {
+    VAEB_TRY(grow(&h->d_out, &h->out_cap, 2 * n));
+    bo.loglik_rows = h->d_out;
+    bo.aux_rows = h->d_out + n;
+  }
   VAEB_TRY(forward_backward(h, theta, h->d_stage, (int)n, L, false, 1.f, src, nullptr, bo));
   ++h->step;
   VAEB_TRY(read_scalars(h, 1, sgvb_out));
   if (per_row_out)
     VAEB_CUDA(cudaMemcpy(per_row_out, h->ws.per_row, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost));
+  if (loglik_out) {
+    VAEB_CUDA(cudaMemcpy(loglik_out, bo.loglik_rows, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost));
+    VAEB_CUDA(cudaMemcpy(aux_out, bo.aux_rows, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost));
+  }
   return VAEB_OK;
+}
+
+int vaeb_validate(vaeb_handle* h, const float* x, int64_t n, const float* eps, float* sgvb_out, float* per_row_out) {
+  return validate_rows(h, x, n, eps, sgvb_out, per_row_out, nullptr, nullptr);
+}
+
+int vaeb_validate_terms(vaeb_handle* h, const float* x, int64_t n, const float* eps, float* loglik_out, float* aux_out) {
+  VAEB_REQUIRE(loglik_out && aux_out, "null argument");
+  float sgvb = 0.f;
+  return validate_rows(h, x, n, eps, &sgvb, nullptr, loglik_out, aux_out);
 }
 
 int vaeb_is_logpx(vaeb_handle* h, const float* x, int64_t n, int32_t L, const float* eps, int64_t row_offset,
@@ -1555,6 +1579,71 @@ int vaeb_decode(vaeb_handle* h, const float* z, int64_t n, float* y_out, float* 
   VAEB_CUDA(cudaMemcpyAsync(y_out, d_y, (size_t)n * D * sizeof(float), cudaMemcpyDeviceToHost, st));
   if (h->cont)
     VAEB_CUDA(cudaMemcpyAsync(lv_out, d_lv, (size_t)n * D * sizeof(float), cudaMemcpyDeviceToHost, st));
+  VAEB_CUDA(cudaStreamSynchronize(st));
+  return VAEB_OK;
+}
+
+int vaeb_encode(vaeb_handle* h, const float* x, int64_t n, float* mu_out, float* logvar_out) {
+  if (h && h->a_pending) VAEB_TRY(async_flush(h));
+  VAEB_REQUIRE(h && x && mu_out && logvar_out && n > 0, "null argument");
+  VAEB_CUDA(cudaSetDevice(h->cfg.device));
+  const Layout& l = h->lay;
+  const int D = h->D, H = h->H, Z = h->Z;
+  // rows per chunk: the encoder's workspace is [rows, H] per hidden layer
+  const int pc = (int)std::min<int64_t>(n, (int64_t)1 << 15);
+  VAEB_TRY(ensure_ws(h, pc, 1, false));
+  cudaStream_t st = h->stream;
+  const float* th = h->d_params;
+  Workspace& s = h->ws;
+  const EpsSource no_eps{nullptr, 0, 0, 0, 0};
+  for (int64_t i0 = 0; i0 < n; i0 += pc) {
+    const int c = (int)std::min<int64_t>(pc, n - i0);
+    VAEB_TRY(stage_in(h, &h->d_stage, &h->stage_cap, x + i0 * D, (int64_t)c * D));
+    VAEB_TRY(encoder_hidden(h, th, h->d_stage, c));
+    // L = 0 and no row terms: the heads alone
+    VAEB_LAUNCH(launch_enc2(st, &h->launches, s.h_e, c, H, T_(h, th, l.iW4), T_(h, th, l.ib4), T_(h, th, l.iW5),
+                            T_(h, th, l.ib5), Z, 0, 0, no_eps, s.mu, s.ls, nullptr, nullptr, nullptr));
+    VAEB_CUDA(cudaMemcpyAsync(mu_out + i0 * Z, s.mu, (size_t)c * Z * sizeof(float), cudaMemcpyDeviceToHost, st));
+    VAEB_CUDA(cudaMemcpyAsync(logvar_out + i0 * Z, s.ls, (size_t)c * Z * sizeof(float), cudaMemcpyDeviceToHost, st));
+  }
+  VAEB_CUDA(cudaStreamSynchronize(st));
+  return VAEB_OK;
+}
+
+int vaeb_sample(vaeb_handle* h, int64_t n, uint32_t step, int64_t row_offset, float* z_out, float* mean_out,
+                float* lv_out, float* x_out) {
+  if (h && h->a_pending) VAEB_TRY(async_flush(h));
+  VAEB_REQUIRE(h && n > 0 && row_offset >= 0, "null argument or negative row_offset");
+  VAEB_REQUIRE(h->cont || !lv_out, "lv_out: the Bernoulli decoder has no log-variance output");
+  VAEB_CUDA(cudaSetDevice(h->cfg.device));
+  const Layout& l = h->lay;
+  const int D = h->D, H = h->H, Z = h->Z;
+  VAEB_REQUIRE(row_offset + n <= ((int64_t)1 << 58) / std::max(D, Z), "rows beyond the 2^58 elements of a Philox stream");
+  const int pc = (int)std::min<int64_t>(n, (int64_t)1 << 16);   // rows per chunk
+  VAEB_TRY(ensure_ws(h, 1, pc, false));
+  VAEB_TRY(grow(&h->d_out, &h->out_cap, 3 * (int64_t)pc * D));
+  float* d_y = h->d_out;
+  float* d_lv = h->d_out + (int64_t)pc * D;
+  float* d_x = h->d_out + 2 * (int64_t)pc * D;
+  cudaStream_t st = h->stream;
+  int64_t* lc = &h->launches;
+  const float* th = h->d_params;
+  Workspace& s = h->ws;
+  for (int64_t i0 = 0; i0 < n; i0 += pc) {
+    const int c = (int)std::min<int64_t>(pc, n - i0);
+    const int64_t r0 = row_offset + i0;                       // global row of the chunk's first sample
+    VAEB_LAUNCH(launch_philox_fill(st, lc, h->cfg.seed, VAEB_STREAM_SAMPLE, step, 0u, r0 * Z, (int64_t)c * Z, s.z));
+    VAEB_LAUNCH(launch_dense_act(st, lc, s.z, c, Z, T_(h, th, l.iW1), T_(h, th, l.ib1), H, h->hidden_act, s.h_d));
+    VAEB_LAUNCH(launch_dec2_recon(st, lc, h->cont, s.h_d, c, H, T_(h, th, l.iW2), T_(h, th, l.ib2),
+                                  h->cont ? T_(h, th, l.iW6) : nullptr, h->cont ? T_(h, th, l.ib6) : nullptr, D, d_y, d_lv,
+                                  1.0f, true));
+    if (x_out) VAEB_LAUNCH(launch_sample_x(st, lc, d_y, h->cont ? d_lv : nullptr, c, D, h->cfg.seed, step, r0, d_x));
+    const size_t bz = (size_t)c * Z * sizeof(float), bd = (size_t)c * D * sizeof(float);
+    if (z_out) VAEB_CUDA(cudaMemcpyAsync(z_out + i0 * Z, s.z, bz, cudaMemcpyDeviceToHost, st));
+    if (mean_out) VAEB_CUDA(cudaMemcpyAsync(mean_out + i0 * D, d_y, bd, cudaMemcpyDeviceToHost, st));
+    if (lv_out) VAEB_CUDA(cudaMemcpyAsync(lv_out + i0 * D, d_lv, bd, cudaMemcpyDeviceToHost, st));
+    if (x_out) VAEB_CUDA(cudaMemcpyAsync(x_out + i0 * D, d_x, bd, cudaMemcpyDeviceToHost, st));
+  }
   VAEB_CUDA(cudaStreamSynchronize(st));
   return VAEB_OK;
 }

@@ -66,7 +66,7 @@ enc2_kernel(const float* __restrict__ h_e, int rows, int H, const float* __restr
     st[o] = term;
   }
   __syncthreads();
-  if (threadIdx.x < ENC2_ROWS && m0 + threadIdx.x < rows) {
+  if (row_aux && threadIdx.x < ENC2_ROWS && m0 + threadIdx.x < rows) {
     float s = 0.f;
     for (int j = 0; j < Z; ++j) s += st[threadIdx.x * Z + j];
     row_aux[m0 + threadIdx.x] = s;
@@ -159,7 +159,8 @@ __device__ float block_sum_1024(float v, float* red) {
 __global__ void __launch_bounds__(1024)
 finalize_kernel(const float* __restrict__ partial, int n_tiles, const float* __restrict__ row_aux, int rows, int L,
                 float* __restrict__ per_row, float* __restrict__ base_out, float mult,
-                const float* __restrict__ tprior, int n_tprior, float div, float* __restrict__ scalar_out) {
+                const float* __restrict__ tprior, int n_tprior, float div, float* __restrict__ scalar_out,
+                float* __restrict__ loglik, float* __restrict__ aux) {
   __shared__ float red[32];
   float acc = 0.f;
   const float invL = 1.0f / (float)L;
@@ -173,6 +174,7 @@ finalize_kernel(const float* __restrict__ partial, int n_tiles, const float* __r
     }
     const float v = s * invL + row_aux[m];
     per_row[m] = v;
+    if (loglik) { loglik[m] = __fmul_rn(s, invL); aux[m] = row_aux[m]; }
     acc += v;
   }
   const float base = block_sum_1024(acc, red);
@@ -203,7 +205,7 @@ __global__ void __launch_bounds__(256)
 finalize_rows_kernel(const float* __restrict__ partial, int n_tiles, const float* __restrict__ row_aux, int rows, int L,
                      float* __restrict__ per_row, unsigned int* __restrict__ counter, float* __restrict__ block_part,
                      float* __restrict__ base_out, float mult, const float* __restrict__ tprior, int n_tprior, float div,
-                     float* __restrict__ scalar_out) {
+                     float* __restrict__ scalar_out, float* __restrict__ loglik, float* __restrict__ aux) {
   const int m = blockIdx.x * blockDim.x + threadIdx.x;
   float v = 0.f;
   if (m < rows) {
@@ -216,6 +218,7 @@ finalize_rows_kernel(const float* __restrict__ partial, int n_tiles, const float
     }
     v = s * (1.0f / (float)L) + row_aux[m];
     per_row[m] = v;
+    if (loglik) { loglik[m] = __fmul_rn(s, 1.0f / (float)L); aux[m] = row_aux[m]; }
   }
   if (!counter) return;
   __shared__ unsigned int is_last;
@@ -426,6 +429,21 @@ __global__ void philox_fill_kernel(uint64_t seed, uint32_t stream, uint32_t step
   out[i] = philox_normal1(seed, stream, step, sample, (uint64_t)(first + i));
 }
 
+// x[i, d] ~ p(x|z) of decoder outputs mean / lv [rows, D]; noise of element (row_offset + i) * D + d of
+// (VAEB_STREAM_SAMPLE, step, sample 1).  Bernoulli: x = 1 if u < mean else 0.  Gaussian: x = mean + exp(lv / 2) * eps,
+// the likelihood's own variance exp(lv) (VAEB.py:302-313).
+__global__ void __launch_bounds__(256)
+sample_x_kernel(const float* __restrict__ mean, const float* __restrict__ lv, int64_t n, int D, uint64_t seed,
+                uint32_t step, int64_t row_offset, float* __restrict__ x) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint64_t e = (uint64_t)(row_offset * D + i);
+  if (lv)
+    x[i] = mean[i] + expf(0.5f * lv[i]) * philox_normal_only(seed, VAEB_STREAM_SAMPLE, step, 1u, e);
+  else
+    x[i] = philox_uniform1(seed, VAEB_STREAM_SAMPLE, step, 1u, e) < mean[i] ? 1.0f : 0.0f;
+}
+
 // out[i, :] = src[idx[i], :]   (ae.py:83 `givens = { X : Xtr[idx] }`: minibatches are gathered, not sliced)
 __global__ void __launch_bounds__(256)
 gather_rows_kernel(const float* __restrict__ src, const int* __restrict__ idx, int n, int D, float* __restrict__ out) {
@@ -482,19 +500,26 @@ cudaError_t launch_dprep(cudaStream_t st, int64_t* launches, const float* dz, co
 cudaError_t launch_finalize(cudaStream_t st, int64_t* launches, const float* partial, int n_tiles,
                             const float* row_aux, int rows, int L, float* per_row, float* base_out, float mult,
                             const float* tprior, int n_tprior, float div, float* scalar_out, unsigned int* counter,
-                            float* block_part) {
+                            float* block_part, float* loglik, float* aux) {
   if (rows >= 2048) {
     if (!block_part) counter = nullptr;
     finalize_rows_kernel<<<blocks_for(rows, 256), 256, 0, st>>>(partial, n_tiles, row_aux, rows, L, per_row, counter,
                                                                 block_part, base_out, mult, tprior, n_tprior, div,
-                                                                scalar_out);
+                                                                scalar_out, loglik, aux);
     if (counter) return LAUNCHED();
     ++*launches;
     finalize_total_kernel<<<1, 1024, 0, st>>>(per_row, rows, base_out, mult, tprior, n_tprior, div, scalar_out);
     return LAUNCHED();
   }
   finalize_kernel<<<1, 1024, 0, st>>>(partial, n_tiles, row_aux, rows, L, per_row, base_out, mult, tprior, n_tprior,
-                                      div, scalar_out);
+                                      div, scalar_out, loglik, aux);
+  return LAUNCHED();
+}
+
+cudaError_t launch_sample_x(cudaStream_t st, int64_t* launches, const float* mean, const float* lv, int rows, int D,
+                            uint64_t seed, uint32_t step, int64_t row_offset, float* x) {
+  const int64_t n = (int64_t)rows * D;
+  sample_x_kernel<<<blocks_for(n, 256), 256, 0, st>>>(mean, lv, n, D, seed, step, row_offset, x);
   return LAUNCHED();
 }
 

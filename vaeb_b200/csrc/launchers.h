@@ -42,7 +42,8 @@ struct EpsSource {
 };
 // mu, ls = h_e.W4+b4, h_e.W5+b5 (VAEB.py:248-249); if L>0 also eps, z = mu+exp(.5 ls) eps
 // (VAEB.py:41-47) for l<L with rows laid out [L,rows,Z]; row_aux[rows] = KL row (VAEB.py:343)
-// for LB or (1/L) sum_l (log p(z) - log q(z|x)) (VAEB.py:322-325) for LA.
+// for LB or (1/L) sum_l (log p(z) - log q(z|x)) (VAEB.py:322-325) for LA.  row_aux == nullptr: no row terms (encoding
+// only, with L = 0).
 cudaError_t launch_enc2(cudaStream_t st, int64_t* launches, const float* h_e, int rows, int H, const float* W4,
                         const float* b4, const float* W5, const float* b5, int Z, int L, int la, EpsSource src,
                         float* mu, float* ls, float* eps, float* z, float* row_aux);
@@ -57,12 +58,17 @@ cudaError_t launch_dprep(cudaStream_t st, int64_t* launches, const float* dz, co
                          const float* mu, const float* ls, int rows, int Z, int L, int la, float w,
                          float* dmu, float* dls);
 // per_row[m] = (1/L) sum_l sum_t partial[(l*rows+m), t] + row_aux[m]; base = sum_m per_row;
-// scalar_out (nullable) = (mult*base + sum(tprior[0..n_tprior)))/div
+// scalar_out (nullable) = (mult*base + sum(tprior[0..n_tprior)))/div.  loglik / aux (both or neither): the two terms
+// of per_row, loglik[m] = (1/L) sum_l sum_t partial (one rounding) and aux[m] = row_aux[m]
 cudaError_t launch_finalize(cudaStream_t st, int64_t* launches, const float* partial, int n_tiles,
                             const float* row_aux, int rows, int L, float* per_row, float* base_out,
                             float mult, const float* tprior, int n_tprior, float div, float* scalar_out,
                             unsigned int* counter = nullptr,   // rows >= 2048 with a ticket counter and room for
-                            float* block_part = nullptr);      // rows/256 block sums: one launch
+                            float* block_part = nullptr,       // rows/256 block sums: one launch
+                            float* loglik = nullptr, float* aux = nullptr);
+// vaeb_sample: x[rows, D] drawn from p(x|z) given the decoder outputs (lv == nullptr: Bernoulli with means `mean`)
+cudaError_t launch_sample_x(cudaStream_t st, int64_t* launches, const float* mean, const float* lv, int rows, int D,
+                            uint64_t seed, uint32_t step, int64_t row_offset, float* x);
 // logw[r] = sum_t partial[r,t] + aux[r];  logp[i] = logsumexp_l logw[i*L+l] - log L
 cudaError_t launch_is_reduce(cudaStream_t st, int64_t* launches, const float* partial, int n_tiles,
                              const float* aux, int n, int L, float* logw, float* logp);

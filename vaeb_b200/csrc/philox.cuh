@@ -9,6 +9,7 @@
 #define VAEB_STREAM_IS 2u
 #define VAEB_STREAM_ZETA 3u
 #define VAEB_STREAM_RECON 4u
+#define VAEB_STREAM_SAMPLE 5u   // vaeb_sample: z ~ N(0, I) (sample 0) and the draw of x from p(x|z) (sample 1)
 
 __host__ __device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
                                                        uint32_t k0, uint32_t k1, uint32_t out[4]) {
@@ -43,6 +44,19 @@ __device__ __forceinline__ void philox_normal4(uint64_t seed, uint32_t stream, u
   sincospif(2.0f * u1, &s0, &c0);   // exact argument reduction: no slow path, small code
   sincospif(2.0f * u3, &s1, &c1);
   n[0] = rad0 * c0; n[1] = rad0 * s0; n[2] = rad1 * c1; n[3] = rad1 * s1;
+}
+
+// One U(0,1) draw, flat element e: the uniform philox_normal4 makes of output e % 4 of group e / 4, the same 24-bit
+// mapping ((r >> 8) + 0.5) * 2^-24, so never 0 or 1.  Restated on the CPU in tests/sample_oracle.py.
+__device__ __forceinline__ float philox_uniform1(uint64_t seed, uint32_t stream, uint32_t step, uint32_t sample,
+                                                 uint64_t e) {
+  uint32_t r[4];
+  const uint64_t g = e >> 2;
+  philox4x32_10((uint32_t)g, ((uint32_t)(g >> 32) & 0x00FFFFFFu) | ((stream & 0xFFu) << 24), sample, step,
+                (uint32_t)seed, (uint32_t)(seed >> 32), r);
+  const uint32_t q = (uint32_t)e & 3u;
+  const uint32_t rv = q == 0 ? r[0] : (q == 1 ? r[1] : (q == 2 ? r[2] : r[3]));
+  return ((float)(rv >> 8) + 0.5f) * 5.9604644775390625e-8f;  // 2^-24
 }
 
 // One draw: flat element e.

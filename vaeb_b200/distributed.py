@@ -77,3 +77,16 @@ def sharded_log_px(model, x, L, rank, world, gather=True):
     outs = [None] * world
     dist.all_gather_object(outs, local)
     return np.concatenate(outs)
+
+
+def sharded_sample(model, n, rank, world, step=0, gather=True):
+    """This rank's share of `n` samples from the generative model.  The Philox counters are keyed by the GLOBAL
+    sample row, so the concatenated samples are identical for any world size."""
+    lo, hi = shard_rows(n, rank, world)
+    local = model.sample(hi - lo, step=step, row_offset=lo) if hi > lo else np.empty((0, model.input_size), np.float32)
+    if not gather or world == 1:
+        return local
+    import torch.distributed as dist
+    outs = [None] * world
+    dist.all_gather_object(outs, local)
+    return np.concatenate(outs)

@@ -42,9 +42,21 @@ def render(model, n=10, offset=0.9, sample=False, rng=None):
             faces = mu + np.exp(ls) * rng.standard_normal(mu.shape).astype(np.float32)
     else:
         faces = out
+    return faces, tile(faces, n)
+
+
+def tile(faces, n):
+    """n x n data rows -> one 2-D image, row-major (VAEBImage.py:25-41)."""
     tiles = [to_image(f) for f in faces]
-    tiled = np.vstack([np.hstack(tiles[ii * n:(ii + 1) * n]) for ii in range(n)])   # VAEBImage.py:25-41
-    return faces, tiled
+    return np.vstack([np.hstack(tiles[ii * n:(ii + 1) * n]) for ii in range(n)])
+
+
+def render_samples(model, n=10, step=0):
+    """(faces[n*n, D], tiled) of n*n random samples from the generative model (AEVB Fig. 5).  A Bernoulli model shows
+    its decoder means, as the paper's figure does: the binary draws themselves make a poor image."""
+    z, mean, lv, x = model.sample(n * n, step=step, return_all=True)
+    faces = x if model.continuous else mean
+    return faces, tile(faces, n)
 
 
 def save_pgm(img, path):

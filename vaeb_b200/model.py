@@ -340,6 +340,36 @@ class VAEB(object):
 
     freyFace = decode       # freyFace.py:137 names the compiled decoder function after its first use
 
+    def encode(self, x):
+        """The encoder alone (VAEB.py:245-251): (mu, log_var) of q(z|x) for every row of x.  The second head is a
+        log-variance although the reference calls it log_sigma."""
+        xa = _f32(x).reshape(-1, self.input_size)
+        mu = np.empty((xa.shape[0], self.n_latent), np.float32)
+        lv = np.empty_like(mu)
+        _lib.check(self._lib.vaeb_encode(self._h, _ptr(xa), xa.shape[0], _ptr(mu), _ptr(lv)))
+        return mu, lv
+
+    def sample(self, n, step=0, row_offset=0, return_all=False):
+        """n samples x ~ p(x|z), z ~ N(0, I) from the generative model (AEVB Fig. 5), drawn on the device from the
+        Philox stream of (seed, step, row_offset + i).  return_all: (z, mean, lv, x), lv None for Bernoulli."""
+        n = int(n)
+        x = np.empty((n, self.input_size), np.float32)
+        z = np.empty((n, self.n_latent), np.float32) if return_all else None
+        mean = np.empty_like(x) if return_all else None
+        lv = np.empty_like(x) if return_all and self.continuous else None
+        _lib.check(self._lib.vaeb_sample(self._h, n, int(step), int(row_offset), _ptr(z), _ptr(mean), _ptr(lv), _ptr(x)))
+        return (z, mean, lv, x) if return_all else x
+
+    def validate_terms(self, x, eps=None):
+        """The two terms of validate's per-row bound: (mean over L of log p(x|z), the term the estimator adds --
+        -KL for L^B, the MC mean of log p(z) - log q(z|x) for L^A).  Same noise and step counter as validate."""
+        xa = _f32(x)
+        ea = _f32(eps) if eps is not None else self._draw_eps(xa.shape[0])
+        loglik = np.empty(xa.shape[0], np.float32)
+        aux = np.empty_like(loglik)
+        _lib.check(self._lib.vaeb_validate_terms(self._h, _ptr(xa), xa.shape[0], _ptr(ea), _ptr(loglik), _ptr(aux)))
+        return loglik, aux
+
     # ---- persistence ---------------------------------------------------------------------
     def save(self, file_name):
         """VAEB.py:189-203 (plus the `genericEstimator` entry `load` expects, VAEB.py:218)."""
