@@ -80,13 +80,15 @@ typedef struct vaeb_config {
 
 #define VAEB_OPT_ADAGRAD 0   /* getUpdates          VAEB.py:426-444 (the path the reference runs) */
 #define VAEB_OPT_ADADELTA 1  /* getAdaDeltaUpdates  VAEB.py:449-469 (the alternative commented out at :404) */
+#define VAEB_OPT_ADAM 2      /* Adam (Kingma & Ba 2015), selected with vaeb_set_adam */
 
 #define VAEB_ACT_TANH 1      /* the reference's hidden layers (VAEB.py:246,254) */
 #define VAEB_ACT_SIGMOID 2   /* alternatives compared in Report/replication/replic.tex:73-82 */
 #define VAEB_ACT_RELU 3
 
 const char* vaeb_last_error(void);
-int vaeb_version(void);      /* 102: adds the encode, sample and validate_terms entry points (vaeb_config unchanged);
+int vaeb_version(void);      /* 103: adds Adam (vaeb_set_adam, vaeb_adam_step, vaeb_set_adam_step; vaeb_config unchanged);
+                                102: adds the encode, sample and validate_terms entry points (vaeb_config unchanged);
                                 101: vaeb_config ends with encoder_hidden_layers, reserved0 (100: it ended with seed) */
 /* sizeof(vaeb_config) as this library was compiled: a binding that declares the struct itself (ctypes, cgo) compares it
  * with its own size before the first vaeb_create -- a shorter struct would be read past its end. */
@@ -103,9 +105,10 @@ int vaeb_set_stream(vaeb_handle* h, void* cuda_stream);
 int vaeb_synchronize(vaeb_handle* h);
 
 /* self.params / self.ADA / self.full_variational_params access (VAEB.py:111-125,178-182).
- * `which`: 0 params, 1 ADA accumulators, 2 gradients of the last step (criterion incl. prior),
- *          3 variational means, 4 variational sigmas, 5 ADA of means, 6 ADA of sigmas,
- *          7 gradients w.r.t. means, 8 gradients w.r.t. sigmas  (3..8: FVB estimators only).
+ * `which`: 0 params, 1 ADA accumulators (AdaDelta: g_ac; Adam: the first moment m), 2 gradients of the last step
+ *          (criterion incl. prior), 3 variational means, 4 variational sigmas, 5 ADA of means, 6 ADA of sigmas,
+ *          7 gradients w.r.t. means, 8 gradients w.r.t. sigmas  (3..8: FVB estimators only),
+ *          9 AdaDelta's dx_ac or Adam's second moment v (whichever optimizer is selected).
  * `tensors[i]` points at host storage of tensor i in reference order. */
 int vaeb_num_tensors(vaeb_handle* h, int32_t* n_tensors, int64_t* n_elements);
 int vaeb_tensor_shape(vaeb_handle* h, int32_t i, int32_t* rows, int32_t* cols);
@@ -143,6 +146,20 @@ int vaeb_ae_forward(vaeb_handle* h, int32_t kind, int32_t what, const float* in,
  * (Report/replication/replic.tex:73-82) run on the fp32 per-layer kernels (L^A / L^B estimators, one GPU). */
 int vaeb_set_hidden_activation(vaeb_handle* h, int32_t act);
 int vaeb_set_optimizer(vaeb_handle* h, int32_t optimizer, float rho);
+/* Selects Adam (Kingma & Ba 2015) for the next vaeb_update* calls, in the ascent convention and with the weight prior of
+ * getUpdates (VAEB.py:389-390), per element at Adam step t (t = 1 for the first update applied after this call):
+ *   g = grad - prior_scale p   (no prior term for the VAEBfullbayes variant);  m = b1 m + (1-b1) g;  v = b2 v + (1-b2) g^2;
+ *   p += alpha_t m / (sqrt(v) / s2_t + eps),  alpha_t = learning_rate / (1 - b1^t),  s2_t = sqrt(1 - b2^t)
+ * (alpha_t, s2_t computed in double and rounded to float once per update): torch.optim.Adam(maximize=True).  m, v and
+ * t restart at zero; vaeb_set_optimizer switches back to Adagrad or AdaDelta.  t advances once per applied update, when
+ * the update is enqueued.  The single-launch step kernels apply Adagrad only: Adam updates of M <= 128 rows run the
+ * per-layer kernels.  VAEB_EINVAL: beta1 or beta2 outside [0, 1), eps not positive and finite, or a full-VB estimator;
+ * VAEB_ESTATE after vaeb_comm_p2p_export (select the optimizer on every rank before exporting). */
+int vaeb_set_adam(vaeb_handle* h, float beta1, float beta2, float eps);
+/* Adam step counter t (updates applied since vaeb_set_adam): with m and v (which = 1, 9) it is the optimizer state to
+ * save and restore. */
+int vaeb_adam_step(vaeb_handle* h, int64_t* t);
+int vaeb_set_adam_step(vaeb_handle* h, int64_t t);
 
 /* `x_train = th.shared(...)` (VAEB.py:184): copies x[N,D] to the device once. */
 int vaeb_upload_data(vaeb_handle* h, const float* x, int64_t n_rows);
@@ -198,7 +215,7 @@ int vaeb_validate(vaeb_handle* h, const float* x, int64_t n, const float* eps,
  * resident data starting at index*M. */
 int vaeb_gradients(vaeb_handle* h, const float* x, int64_t rows, int64_t index, const float* eps,
                    const float* zeta, float* sgvb_out, float* per_row_out);
-/* The Adagrad update alone (VAEB.py:426-444) on the current gradient buffer. */
+/* The Adagrad update alone (VAEB.py:426-444) on the current gradient buffer.  VAEB_EINVAL for Adam handles. */
 int vaeb_apply_update(vaeb_handle* h);
 
 /* Importance-sampled marginal likelihood (new capability named by the north star; the
@@ -272,11 +289,13 @@ int vaeb_comm_attach(vaeb_handle* h, const char* nccl_library, const uint8_t id[
                      int32_t rank, int32_t world_size);
 int vaeb_comm_detach(vaeb_handle* h);
 /* Data parallel over PEER MEMORY (NVLink / NVSwitch, ranks = processes of one box): after vaeb_comm_attach every rank
- * exports three CUDA IPC handles (its gradient staging buffer + flags, its parameters, its Adagrad accumulators), the
+ * exports three CUDA IPC handles (its gradient staging buffer + flags, its parameters, its accumulators: Adam's m with v
+ * right after it in the same allocation, so every rank must have selected the same optimizer before exporting;
+ * vaeb_b200.distributed.attach_data_parallel compares the ranks' optimizers and refuses a mix), the
  * host plumbing all-gathers the 192 bytes per rank, every rank attaches all of them.  From then on the tail of a
  * large-batch tensor-core update (tc_tail.cu) IS the collective: each rank sums ITS slice of the flat gradient from
- * every rank's staging buffer with peer loads, applies prior + Adagrad, and stores the new parameters into every rank's
- * buffers -- one launch, no NCCL kernel.  Other update paths keep using ncclAllReduce.  vaeb_comm_detach unmaps. */
+ * every rank's staging buffer with peer loads, applies prior + Adagrad (or Adam), and stores the new parameters (and
+ * Adam's m and v) into every rank's buffers -- one launch, no NCCL kernel.  Other update paths keep using ncclAllReduce.  vaeb_comm_detach unmaps. */
 int vaeb_comm_p2p_export(vaeb_handle* h, uint8_t handles_out[192]);
 int vaeb_comm_p2p_attach(vaeb_handle* h, const uint8_t* all_handles, int32_t world_size);
 

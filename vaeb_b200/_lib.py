@@ -14,7 +14,8 @@ PREC_FP32, PREC_BF16, PREC_BF16X3 = 0, 1, 2
 
 # buffers addressable through vaeb_{get,set}_tensors
 BUF_PARAMS, BUF_ADA, BUF_GRADS, BUF_VMU, BUF_VSIG, BUF_ADA_MU, BUF_ADA_SIG, BUF_GMU, BUF_GSIG, BUF_ADA2 = range(10)
-OPT_ADAGRAD, OPT_ADADELTA = 0, 1
+OPT_ADAGRAD, OPT_ADADELTA, OPT_ADAM = 0, 1, 2
+BUF_ADAM_V = 9          # Adam's second moment (BUF_ADA is its first moment)
 AE_DEGENERATE, AE_VANILLA = 0, 1
 
 
@@ -49,6 +50,9 @@ EXPORTS = {
     "vaeb_update_host_async_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_float]),
     "vaeb_diag_tile_schedule": (C.c_int, [C.c_int32] * 6 + [C.c_void_p] * 3),
     "vaeb_set_optimizer": (C.c_int, [C.c_void_p, C.c_int32, C.c_float]),
+    "vaeb_set_adam": (C.c_int, [C.c_void_p, C.c_float, C.c_float, C.c_float]),
+    "vaeb_adam_step": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
+    "vaeb_set_adam_step": (C.c_int, [C.c_void_p, C.c_int64]),
     "vaeb_ae_train": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.POINTER(C.c_float)]),
     "vaeb_ae_forward": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
     "vaeb_collect": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.c_void_p]),

@@ -31,7 +31,8 @@ command_line_args = {'seed': (15485863, int),
                      'manifold_file': ('', str),      # PGM of the learned 2-d manifold (freyFace.py:346-369)
                      # PGM of 10 x 10 random samples (AEVB Fig. 5); a Bernoulli model shows its decoder means,
                      # since binary draws make a poor image
-                     'sample_file': ('', str)}
+                     'sample_file': ('', str),
+                     'optimizer': ('adagrad', str)}  # adagrad (VAEB.py:426-444) | adadelta (VAEB.py:449-469) | adam
 command_line_flags = ['continuous', 'generic_estimator', 'full_varational',
                       # --- extensions ---
                       'synthetic',        # synthetic data of the dataset's shape if the files are absent
@@ -112,7 +113,8 @@ def train_model(args, data=None):
         seed_model.close()
     model = VAEB(x_train, continuous, _default_hidden(continuous, args['hidden_unit']), args['n_latent'],
                  args['batch_size'], args['L'], args['learning_rate'], args['generic_estimator'],
-                 args['full_varational'], params, sample_weights=args.get('sample_weights', False), **ext)
+                 args['full_varational'], params, sample_weights=args.get('sample_weights', False),
+                 optimizer=args.get('optimizer', 'adagrad'), **ext)
 
     print("learning")
     tracing = len(trace_file) > 0

@@ -453,7 +453,7 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
 // Training gradients of a large batch on the tensor-core path (latent_large_batch: L = 1): every layer runs on tcgen05,
 // the thin latent ones too (their operands' bf16 mirrors come from the kernels that produce h_e, z, da1 and [dmu|dls]),
 // and the four weight-gradient GEMMs are one launch after the last dgrad, their split-K slices left in scratch.  With
-// `tail` the update ends in ONE launch that also applies prior + Adagrad; else the bound and the sum of the slices are
+// `tail` the update ends in ONE launch that also applies prior + Adagrad or Adam; else the bound and the sum of the slices are
 // launched here and the caller applies the update.
 int large_batch_step(vaeb_handle* h, const float* theta, const float* x, int rows, float w, EpsSource src, float* grads,
                      const BoundOut& bo, bool tail) {
@@ -526,7 +526,7 @@ int large_batch_step(vaeb_handle* h, const float* theta, const float* x, int row
     return VAEB_OK;
   }
   // the tail as one launch (tc_tail.cu): slices -> gradient, bound, (data parallel over peer memory: the gradient sum,)
-  // prior + Adagrad and the bf16 weight mirrors of the new parameters
+  // prior + Adagrad or Adam and the bf16 weight mirrors of the new parameters
   const bool fb = h->cfg.variant == VAEB_VARIANT_FULLBAYES, dp = h->world > 1;
   if (!t.tail_bar) {
     VAEB_CUDA(cudaMalloc((void**)&t.tail_bar, sizeof(unsigned int)));
@@ -549,11 +549,17 @@ int large_batch_step(vaeb_handle* h, const float* theta, const float* x, int row
   ta.oW6 = h->cont ? l.off[l.iW6] : -1;
   ta.bar = t.tail_bar;
   ta.world = h->world; ta.rank = h->rank;
+  const bool adam = h->optimizer == VAEB_OPT_ADAM;
+  if (adam) {
+    ta.alpha_t = h->adam_alpha_t; ta.s2_t = h->adam_s2_t; ta.b1 = h->adam_b1; ta.b2 = h->adam_b2; ta.adam_eps = h->adam_eps;
+    ta.v = h->d_adam_v;
+  }
   for (int r = 0; r < h->world && dp; ++r) {
     ta.gsum[r] = t.p2p_gsum[r]; ta.flags[r] = t.p2p_flags[r];
     ta.peer_params[r] = t.p2p_params[r]; ta.peer_ada[r] = t.p2p_ada[r];
+    if (adam) ta.peer_v[r] = t.p2p_ada[r] + (l.padded + 4);      // every rank keeps v right after m (vaeb_set_adam)
   }
-  const int grid = tc_tail_grid(t.n_sm);
+  const int grid = tc_tail_grid(t.n_sm, adam);
   static const char* stamp_path = getenv("VAEB_TAIL_STAMPS");      // debug: time stamps of the last 2048 tail launches
   static long long* d_stamps = nullptr;
   if (stamp_path && !d_stamps) {
@@ -566,10 +572,14 @@ int large_batch_step(vaeb_handle* h, const float* theta, const float* x, int row
     ta.bar_base = t.tail_bar_count;
     ta.epoch = ++t.p2p_epoch;
     t.tail_bar_count += (unsigned int)grid * (dp ? 2u : 1u);
-    return tc_tail_launch(st, lc, ta, grid);
+    return tc_tail_launch(st, lc, ta, grid, adam);
   };
-  PH("tail: slices -> gradient, bound, (all-reduce over peer memory,) prior + Adagrad, weight mirrors (one launch)", 0,
-     28.0 * (double)l.total, launch_tail());
+  if (adam)
+    PH("tail: slices -> gradient, bound, (all-reduce over peer memory,) prior + Adam, weight mirrors (one launch)", 0,
+       36.0 * (double)l.total, launch_tail());
+  else
+    PH("tail: slices -> gradient, bound, (all-reduce over peer memory,) prior + Adagrad, weight mirrors (one launch)", 0,
+       28.0 * (double)l.total, launch_tail());
   return VAEB_OK;
 }
 
@@ -615,6 +625,12 @@ int enqueue_update(vaeb_handle* h, const float* d_xrows, int rows, const float* 
   const float Mg = (float)rows * (float)h->world;
   const bool large = h->tc.active && latent_large_batch(rows, h->H, h->Z, L);
   bool tail = false;
+  const bool adam = h->optimizer == VAEB_OPT_ADAM;
+  if (apply && adam) {            // Adam step t of this update: bias corrections in double, rounded to float once
+    const double t = (double)(h->adam_t + 1);          // (h->adam_t advances below, once the update is enqueued)
+    h->adam_alpha_t = (float)((double)h->cfg.learning_rate / (1.0 - std::pow((double)h->adam_b1, t)));
+    h->adam_s2_t = (float)std::sqrt(1.0 - std::pow((double)h->adam_b2, t));
+  }
   if (!is_fvb(h)) {
     const bool fb = h->cfg.variant == VAEB_VARIANT_FULLBAYES;
     const float w = fb ? 1.0f / Mg : 1.0f;
@@ -625,14 +641,18 @@ int enqueue_update(vaeb_handle* h, const float* d_xrows, int rows, const float* 
     // With the single weight-gradient launch in front of it, it measures equal to the five separate launches at 16384 rows
     // and 1-3 % faster below on one GPU; VAEB_TC_TAIL=0 switches it off (then: slice sum, row sums, bound, Adagrad, mirrors).
     static const int env_tail = getenv("VAEB_TC_TAIL") ? atoi(getenv("VAEB_TC_TAIL")) : -1;      // measurement switch
-    tail = large && apply && h->optimizer != VAEB_OPT_ADADELTA && env_tail != 0 && (!dp || h->tc.p2p_ready);
+    tail = large && apply && (h->optimizer == VAEB_OPT_ADAGRAD || adam) && env_tail != 0 && (!dp || h->tc.p2p_ready);
     // data parallel without the tail: the optimizer launch writes the scalar, after the all-reduce
     BoundOut bo{base, 1.0f, nullptr, 0, Mg, dp && !tail ? nullptr : h->d_scalars + slot};
     if (large) VAEB_TRY(large_batch_step(h, h->d_params, d_xrows, rows, w, src, h->d_grads, bo, tail));
     else VAEB_TRY(forward_backward(h, h->d_params, d_xrows, rows, L, true, w, src, h->d_grads, bo));
-    if (!tail) {                          // (the tail applied prior + Adagrad)
+    if (!tail) {                          // (the tail applied prior + Adagrad / Adam)
       VAEB_TRY(all_reduce_grads(h));
-      if (apply && h->optimizer == VAEB_OPT_ADADELTA)
+      if (apply && adam)
+        PH("adam+prior (flat)", 0, 28.0 * (double)l.total,
+           launch_adam(st, lc, h->d_params, h->d_ada, h->d_adam_v, h->d_grads, n4, h->adam_alpha_t, h->adam_s2_t,
+                       h->adam_b1, h->adam_b2, h->adam_eps, prior, base, 1.0f, Mg, dp ? h->d_scalars + slot : nullptr));
+      else if (apply && h->optimizer == VAEB_OPT_ADADELTA)
         PH("adadelta+prior (flat)", 0, 28.0 * (double)l.total,
            launch_adadelta(st, lc, h->d_params, h->d_ada, h->d_ada2, h->d_grads, n4, h->rho, h->cfg.adagrad_eps, prior,
                            base, 1.0f, Mg, dp ? h->d_scalars + slot : nullptr));
@@ -666,6 +686,7 @@ int enqueue_update(vaeb_handle* h, const float* d_xrows, int rows, const float* 
   }
   if (apply) invalidate_weight_mirrors(h);
   if (tail) h->tc.weights_ready = true;         // the tail wrote the large-batch path's mirrors of the new parameters
+  if (apply && adam) ++h->adam_t;
   ++h->step;
   return VAEB_OK;
 }
@@ -714,7 +735,7 @@ float* flat_by_which(vaeb_handle* h, int which) {
     case 6: return h->d_ada_sig;
     case 7: return h->d_gmu;
     case 8: return h->d_gsig;
-    case 9: return h->d_ada2;
+    case 9: return h->optimizer == VAEB_OPT_ADAM ? h->d_adam_v : h->d_ada2;
     case 10: return h->d_theta;     // sampled full VB: theta of the next step (debug / tests)
     case 11: return h->d_zeta;
     default: return nullptr;
@@ -741,24 +762,27 @@ int load_nccl(NcclApi& api, const char* path) {
 
 extern "C" {
 
-// Backup of params + accumulators around the profiling entry points: restored and freed on EVERY exit path
+// Backup of params + accumulators (Adam: m, v and the Adam step) around the profiling entry points: restored and freed
+// on EVERY exit path
 struct StateBackup {
-  vaeb_handle* h; size_t nb; float* bp = nullptr; float* ba = nullptr; uint32_t step0; int64_t launches0;
-  StateBackup(vaeb_handle* hh, size_t n) : h(hh), nb(n), step0(hh->step), launches0(hh->launches) {}
+  vaeb_handle* h; size_t nb, nba; float* bp = nullptr; float* ba = nullptr; uint32_t step0; int64_t launches0, adam_t0;
+  StateBackup(vaeb_handle* hh, size_t n)
+      : h(hh), nb(n), nba(hh->d_adam_v ? 2 * n : n), step0(hh->step), launches0(hh->launches), adam_t0(hh->adam_t) {}
   cudaError_t take() {
     cudaError_t e = cudaMalloc((void**)&bp, nb);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&ba, nb);
+    if (e == cudaSuccess) e = cudaMalloc((void**)&ba, nba);
     if (e == cudaSuccess) e = cudaMemcpyAsync(bp, h->d_params, nb, cudaMemcpyDeviceToDevice, h->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(ba, h->d_ada, nb, cudaMemcpyDeviceToDevice, h->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(ba, h->d_ada, nba, cudaMemcpyDeviceToDevice, h->stream);   // m and v
     return e;
   }
   ~StateBackup() {
     invalidate_weight_mirrors(h);
     h->step = step0;
     h->launches = launches0;
+    h->adam_t = adam_t0;
     if (bp && ba) {
       cudaMemcpyAsync(h->d_params, bp, nb, cudaMemcpyDeviceToDevice, h->stream);
-      cudaMemcpyAsync(h->d_ada, ba, nb, cudaMemcpyDeviceToDevice, h->stream);
+      cudaMemcpyAsync(h->d_ada, ba, nba, cudaMemcpyDeviceToDevice, h->stream);
       cudaStreamSynchronize(h->stream);
     }
     if (bp) cudaFree(bp);
@@ -770,7 +794,7 @@ static int async_flush(vaeb_handle* h);
 static void p2p_release(vaeb_handle* h);   // unmaps the peers' buffers (data parallel over peer memory)   // launches streaming updates that were copied but not yet started
 
 const char* vaeb_last_error(void) { return g_last_error.c_str(); }
-int vaeb_version(void) { return 102; }   // 102: vaeb_encode, vaeb_sample, vaeb_validate_terms (101: encoder_hidden_layers)
+int vaeb_version(void) { return 103; }   // 103: Adam; 102: vaeb_encode, vaeb_sample, vaeb_validate_terms (101: encoder_hidden_layers)
 int vaeb_config_size(void) { return (int)sizeof(vaeb_config); }
 
 int vaeb_create(const vaeb_config* cfg, vaeb_handle** out) {
@@ -1140,6 +1164,49 @@ int vaeb_set_optimizer(vaeb_handle* h, int32_t optimizer, float rho) {
   return VAEB_OK;
 }
 
+int vaeb_set_adam(vaeb_handle* h, float beta1, float beta2, float eps) {
+  if (h && h->a_pending) VAEB_TRY(async_flush(h));
+  VAEB_REQUIRE(h, "null handle");
+  VAEB_REQUIRE(beta1 >= 0.f && beta1 < 1.f && beta2 >= 0.f && beta2 < 1.f, "beta1 and beta2 must lie in [0, 1)");
+  VAEB_REQUIRE(eps > 0.f && std::isfinite(eps), "eps must be positive and finite");
+  VAEB_REQUIRE(!is_fvb(h), "Adam is not wired to the full-VB estimators");
+  if (h->tc.p2p_buf) {
+    vaeb_set_error("vaeb_set_adam after vaeb_comm_p2p_export: the peers mapped an accumulator buffer without room for v");
+    return VAEB_ESTATE;
+  }
+  VAEB_CUDA(cudaSetDevice(h->cfg.device));
+  const int64_t n = h->lay.padded + 4;
+  VAEB_CUDA(cudaStreamSynchronize(h->stream));
+  if (!h->d_adam_v) {               // m and v in one allocation: the accumulator's IPC handle maps both
+    float* mv = nullptr;
+    VAEB_CUDA(cudaMalloc((void**)&mv, (size_t)2 * n * sizeof(float)));
+    VAEB_CUDA(cudaFree(h->d_ada));
+    h->d_ada = mv;
+    h->d_adam_v = mv + n;
+  }
+  VAEB_CUDA(cudaMemsetAsync(h->d_ada, 0, (size_t)2 * n * sizeof(float), h->stream));
+  VAEB_CUDA(cudaStreamSynchronize(h->stream));
+  h->optimizer = VAEB_OPT_ADAM;
+  h->adam_b1 = beta1; h->adam_b2 = beta2; h->adam_eps = eps;
+  h->adam_t = 0;
+  h->fused_off = true;              // the single-launch step kernels apply Adagrad only
+  return VAEB_OK;
+}
+
+int vaeb_adam_step(vaeb_handle* h, int64_t* t) {
+  if (h && h->a_pending) VAEB_TRY(async_flush(h));       // the copied-but-unlaunched updates count
+  VAEB_REQUIRE(h && t, "null argument");
+  *t = h->adam_t;
+  return VAEB_OK;
+}
+
+int vaeb_set_adam_step(vaeb_handle* h, int64_t t) {
+  if (h && h->a_pending) VAEB_TRY(async_flush(h));
+  VAEB_REQUIRE(h && t >= 0, "the Adam step must be non-negative");
+  h->adam_t = t;
+  return VAEB_OK;
+}
+
 // Launches the minibatches copied into the current group buffer: ONE fused-kernel launch for up to ASYNC_GROUP
 // updates (per-layer kernels otherwise), then the readback of their bounds.
 static int async_flush(vaeb_handle* h) {
@@ -1327,6 +1394,7 @@ int vaeb_apply_update(vaeb_handle* h) {
   if (h && h->a_pending) VAEB_TRY(async_flush(h));
   VAEB_REQUIRE(h, "null handle");
   VAEB_REQUIRE(!is_fvb(h), "vaeb_apply_update: use vaeb_update for the full-VB estimators");
+  VAEB_REQUIRE(h->optimizer != VAEB_OPT_ADAM, "vaeb_apply_update applies the Adagrad rule: Adam handles use vaeb_update*");
   VAEB_CUDA(cudaSetDevice(h->cfg.device));
   const bool fb = h->cfg.variant == VAEB_VARIANT_FULLBAYES;
   const float prior = (fb || h->grads_have_prior) ? 0.f : h->cfg.prior_scale;

@@ -138,6 +138,10 @@ struct vaeb_handle {
   float* d_x = nullptr; int64_t n_data = 0;
   Workspace ws;
   int optimizer = 0; float rho = 0.95f; float* d_ada2 = nullptr;   // AdaDelta: d_ada = g_ac, d_ada2 = dx_ac
+  // Adam: d_ada = m and d_adam_v = v, in ONE allocation (v right after m, so that the accumulator's IPC handle maps both);
+  // adam_t = updates applied since Adam was selected; alpha_t / s2_t of the update being enqueued
+  float adam_b1 = 0.9f, adam_b2 = 0.999f, adam_eps = 1e-8f; float* d_adam_v = nullptr; int64_t adam_t = 0;
+  float adam_alpha_t = 0.f, adam_s2_t = 0.f;
   float* d_stage = nullptr; int64_t stage_cap = 0;       // device staging for host inputs
   // streaming host-input updates (vaeb_update_host_async): copy stream + ring of staging buffers
   static constexpr int ASYNC_BUFS = 4;

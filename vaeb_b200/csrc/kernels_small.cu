@@ -3,6 +3,7 @@
 // importance-sampling reductions.
 #include <cfloat>
 
+#include "adam.cuh"
 #include "launchers.h"
 #include "philox.cuh"
 
@@ -373,6 +374,23 @@ adadelta_kernel(float4* __restrict__ p, float4* __restrict__ gac, float4* __rest
   p[i] = pv; gac[i] = av; dxac[i] = dv;
 }
 
+// Adam (adam.cuh) over the flat buffer, 28 B/parameter (read p, m, v, g; write p, m, v)
+__global__ void __launch_bounds__(256)
+adam_kernel(float4* __restrict__ p, float4* __restrict__ m, float4* __restrict__ v, const float4* __restrict__ g,
+            int64_t n4, float alpha_t, float s2_t, float b1, float b2, float eps, float prior,
+            const float* __restrict__ base, float mult, float div, float* __restrict__ scalar_out) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i == 0 && scalar_out) *scalar_out = (mult * *base) / div;
+  if (i >= n4) return;
+  float4 pv = p[i], mv = m[i], vv = v[i];
+  const float4 gv = g[i];
+  adam1(pv.x, mv.x, vv.x, gv.x, alpha_t, s2_t, b1, b2, eps, prior);
+  adam1(pv.y, mv.y, vv.y, gv.y, alpha_t, s2_t, b1, b2, eps, prior);
+  adam1(pv.z, mv.z, vv.z, gv.z, alpha_t, s2_t, b1, b2, eps, prior);
+  adam1(pv.w, mv.w, vv.w, gv.w, alpha_t, s2_t, b1, b2, eps, prior);
+  p[i] = pv; m[i] = mv; v[i] = vv;
+}
+
 __global__ void __launch_bounds__(256)
 theta_prior_kernel(const float* __restrict__ vmu, const float* __restrict__ vsig, int64_t n,
                    float* __restrict__ partials) {
@@ -560,6 +578,14 @@ cudaError_t launch_adadelta(cudaStream_t st, int64_t* launches, float* p, float*
                             float* scalar_out) {
   adadelta_kernel<<<blocks_for(n4, 256), 256, 0, st>>>((float4*)p, (float4*)gac, (float4*)dxac, (const float4*)g, n4, rho,
                                                        eps, prior, base, mult, div, scalar_out);
+  return LAUNCHED();
+}
+
+cudaError_t launch_adam(cudaStream_t st, int64_t* launches, float* p, float* m, float* v, const float* g, int64_t n4,
+                        float alpha_t, float s2_t, float b1, float b2, float eps, float prior, const float* base,
+                        float mult, float div, float* scalar_out) {
+  adam_kernel<<<blocks_for(n4, 256), 256, 0, st>>>((float4*)p, (float4*)m, (float4*)v, (const float4*)g, n4, alpha_t,
+                                                   s2_t, b1, b2, eps, prior, base, mult, div, scalar_out);
   return LAUNCHED();
 }
 

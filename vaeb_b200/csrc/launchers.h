@@ -86,6 +86,11 @@ cudaError_t launch_add_prior(cudaStream_t st, int64_t* launches, float* g, const
 cudaError_t launch_adadelta(cudaStream_t st, int64_t* launches, float* p, float* gac, float* dxac, const float* g,
                             int64_t n4, float rho, float eps, float prior, const float* base, float mult, float div,
                             float* scalar_out);
+// Adam (adam.cuh; alpha_t = lr / (1 - b1^t), s2_t = sqrt(1 - b2^t)) over the flat buffer.
+// If scalar_out != nullptr thread 0 also writes (mult*base)/div.
+cudaError_t launch_adam(cudaStream_t st, int64_t* launches, float* p, float* m, float* v, const float* g, int64_t n4,
+                        float alpha_t, float s2_t, float b1, float b2, float eps, float prior, const float* base,
+                        float mult, float div, float* scalar_out);
 cudaError_t launch_adagrad(cudaStream_t st, int64_t* launches, float* p, float* acc, const float* g, int64_t n4,
                            float lr, float eps, float prior, float p2, const float* base, float mult, float div,
                            float* scalar_out);

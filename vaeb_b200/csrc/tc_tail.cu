@@ -12,9 +12,12 @@
 //               kernel, no host)                                         -- grid barrier, "done" flag to every peer --
 //            P3 after every peer's slice has landed: mirrors of the new weights.
 // Flags are monotonic launch numbers written with st.release.sys into the PEER's flag array and polled locally.
+// The rule is a template parameter: prior + Adagrad, or Adam (adam.cuh), whose owner of a slice also stores the two
+// moments into every rank's buffers, so that they stay replicated and identical on all ranks.
 #include <cuda_bf16.h>
 #include <cstdlib>
 
+#include "adam.cuh"
 #include "common.cuh"
 #include "launchers.h"
 #include "tc_layers.h"
@@ -103,6 +106,7 @@ __device__ __forceinline__ void stamp(const TcTailArgs& a, int k) {
   }
 }
 
+template <bool ADAM>
 __global__ void __launch_bounds__(TAIL_THREADS)
 tc_tail_kernel(const TcTailArgs a) {
   __shared__ float red[32];
@@ -142,6 +146,17 @@ tc_tail_kernel(const TcTailArgs a) {
       const size_t f4 = (size_t)(j.gW - a.grads) / 4 + i4;
       if (dp) {
         reinterpret_cast<float4*>(a.gsum[a.rank])[f4] = g;
+      } else if constexpr (ADAM) {
+        reinterpret_cast<float4*>(a.grads)[f4] = g;
+        float4 p = reinterpret_cast<const float4*>(a.params)[f4], m = reinterpret_cast<const float4*>(a.ada)[f4],
+               v = reinterpret_cast<const float4*>(a.v)[f4];
+        adam1(p.x, m.x, v.x, g.x, a.alpha_t, a.s2_t, a.b1, a.b2, a.adam_eps, a.prior);
+        adam1(p.y, m.y, v.y, g.y, a.alpha_t, a.s2_t, a.b1, a.b2, a.adam_eps, a.prior);
+        adam1(p.z, m.z, v.z, g.z, a.alpha_t, a.s2_t, a.b1, a.b2, a.adam_eps, a.prior);
+        adam1(p.w, m.w, v.w, g.w, a.alpha_t, a.s2_t, a.b1, a.b2, a.adam_eps, a.prior);
+        reinterpret_cast<float4*>(a.params)[f4] = p;
+        reinterpret_cast<float4*>(a.ada)[f4] = m;
+        reinterpret_cast<float4*>(a.v)[f4] = v;
       } else {
         reinterpret_cast<float4*>(a.grads)[f4] = g;
         float4 p = reinterpret_cast<const float4*>(a.params)[f4], ac = reinterpret_cast<const float4*>(a.ada)[f4];
@@ -180,6 +195,13 @@ tc_tail_kernel(const TcTailArgs a) {
       const size_t f = (size_t)(dst - a.grads);
       if (dp) {
         a.gsum[a.rank][f] = g;
+      } else if constexpr (ADAM) {
+        *dst = g;
+        float p = a.params[f], m = a.ada[f], v = a.v[f];
+        adam1(p, m, v, g, a.alpha_t, a.s2_t, a.b1, a.b2, a.adam_eps, a.prior);
+        a.params[f] = p;
+        a.ada[f] = m;
+        a.v[f] = v;
       } else {
         *dst = g;
         float p = a.params[f], ac = a.ada[f];
@@ -260,14 +282,28 @@ tc_tail_kernel(const TcTailArgs a) {
 #pragma unroll
       for (int r = 0; r < TC_MAX_PEERS; ++r)
         if (r < a.world) { g.x += t[r].x; g.y += t[r].y; g.z += t[r].z; g.w += t[r].w; }
-      float4 p = reinterpret_cast<const float4*>(a.params)[i], ac = reinterpret_cast<const float4*>(a.ada)[i];
-      adagrad_one(p.x, ac.x, g.x, a.lr, a.eps, a.prior, a.p2);
-      adagrad_one(p.y, ac.y, g.y, a.lr, a.eps, a.prior, a.p2);
-      adagrad_one(p.z, ac.z, g.z, a.lr, a.eps, a.prior, a.p2);
-      adagrad_one(p.w, ac.w, g.w, a.lr, a.eps, a.prior, a.p2);
-      for (int r = 0; r < a.world; ++r) {
-        reinterpret_cast<float4*>(a.peer_params[r])[i] = p;
-        reinterpret_cast<float4*>(a.peer_ada[r])[i] = ac;
+      if constexpr (ADAM) {
+        float4 p = reinterpret_cast<const float4*>(a.params)[i], m = reinterpret_cast<const float4*>(a.ada)[i],
+               v = reinterpret_cast<const float4*>(a.v)[i];
+        adam1(p.x, m.x, v.x, g.x, a.alpha_t, a.s2_t, a.b1, a.b2, a.adam_eps, a.prior);
+        adam1(p.y, m.y, v.y, g.y, a.alpha_t, a.s2_t, a.b1, a.b2, a.adam_eps, a.prior);
+        adam1(p.z, m.z, v.z, g.z, a.alpha_t, a.s2_t, a.b1, a.b2, a.adam_eps, a.prior);
+        adam1(p.w, m.w, v.w, g.w, a.alpha_t, a.s2_t, a.b1, a.b2, a.adam_eps, a.prior);
+        for (int r = 0; r < a.world; ++r) {
+          reinterpret_cast<float4*>(a.peer_params[r])[i] = p;
+          reinterpret_cast<float4*>(a.peer_ada[r])[i] = m;
+          reinterpret_cast<float4*>(a.peer_v[r])[i] = v;
+        }
+      } else {
+        float4 p = reinterpret_cast<const float4*>(a.params)[i], ac = reinterpret_cast<const float4*>(a.ada)[i];
+        adagrad_one(p.x, ac.x, g.x, a.lr, a.eps, a.prior, a.p2);
+        adagrad_one(p.y, ac.y, g.y, a.lr, a.eps, a.prior, a.p2);
+        adagrad_one(p.z, ac.z, g.z, a.lr, a.eps, a.prior, a.p2);
+        adagrad_one(p.w, ac.w, g.w, a.lr, a.eps, a.prior, a.p2);
+        for (int r = 0; r < a.world; ++r) {
+          reinterpret_cast<float4*>(a.peer_params[r])[i] = p;
+          reinterpret_cast<float4*>(a.peer_ada[r])[i] = ac;
+        }
       }
     }
     if (tid == 0 && a.scalar_out) {       // the bound of the global minibatch (every rank sums the same values in rank order)
@@ -357,7 +393,7 @@ tc_tail_kernel(const TcTailArgs a) {
 
 }  // namespace
 
-cudaError_t tc_tail_launch(cudaStream_t st, int64_t* launches, const TcTailArgs& a, int grid) {
+cudaError_t tc_tail_launch(cudaStream_t st, int64_t* launches, const TcTailArgs& a, int grid, bool adam) {
   static const bool pdl = [] { const char* e = getenv("VAEB_TAIL_PDL"); return !(e && e[0] == '0') && !getenv("VAEB_NO_PDL"); }();
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(grid);
@@ -370,15 +406,17 @@ cudaError_t tc_tail_launch(cudaStream_t st, int64_t* launches, const TcTailArgs&
   cfg.attrs = &attr;
   cfg.numAttrs = pdl ? 1 : 0;
   ++*launches;
-  return cudaLaunchKernelEx(&cfg, tc_tail_kernel, a);
+  return adam ? cudaLaunchKernelEx(&cfg, tc_tail_kernel<true>, a) : cudaLaunchKernelEx(&cfg, tc_tail_kernel<false>, a);
 }
 
 // the grid must be co-resident (grid barriers): as many CTAs per SM as the kernel's registers allow
-int tc_tail_grid(int n_sm) {
-  static int per_sm = 0;
+int tc_tail_grid(int n_sm, bool adam) {
+  static int per_sm_of[2] = {0, 0};
+  int& per_sm = per_sm_of[adam ? 1 : 0];
   if (per_sm == 0) {
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tc_tail_kernel, TAIL_THREADS, 0) != cudaSuccess || per_sm < 1)
-      per_sm = 1;
+    const cudaError_t oe = adam ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tc_tail_kernel<true>, TAIL_THREADS, 0)
+                               : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tc_tail_kernel<false>, TAIL_THREADS, 0);
+    if (oe != cudaSuccess || per_sm < 1) per_sm = 1;
     if (per_sm > 6) per_sm = 6;
     const char* e = getenv("VAEB_TAIL_PER_SM");       // measurement switch
     if (e && atoi(e) >= 1 && atoi(e) < per_sm) per_sm = atoi(e);

@@ -32,12 +32,23 @@ def attach_data_parallel(model):
     # ranks of one box map each other's buffers (CUDA IPC over NVLink): the tail kernel of a large-batch tensor-core
     # update then IS the gradient all-reduce (vaeb_comm_p2p_attach); VAEB_DP_P2P=0 keeps ncclAllReduce
     if 1 < world <= 8 and os.environ.get("VAEB_DP_P2P", "1") != "0" and getattr(model, "precision", "fp32") != "fp32":
+        optimizers = [None] * world
+        dist.all_gather_object(optimizers, getattr(model, "optimizer", "adagrad"))
+        check_same_optimizer(optimizers)
         mine = model.p2p_export()
         handles = [None] * world
         dist.all_gather_object(handles, mine)
         model.p2p_attach(handles)
         dist.barrier()
     return rank, world
+
+
+def check_same_optimizer(optimizers):
+    """`optimizers`: every rank's update rule, in rank order.  Over peer memory the owner of a slice stores the updated
+    parameters and accumulators into every rank's buffers, Adam's v right after m in the accumulator allocation: a rank
+    whose allocation has no room for v (another rule) would be written past its end, so a mix is refused up front."""
+    if len(set(optimizers)) > 1:
+        raise ValueError("data parallel over peer memory needs the same optimizer on every rank, got %s" % (optimizers,))
 
 
 def close_data_parallel(model):

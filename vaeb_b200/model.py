@@ -71,7 +71,9 @@ class VAEB(object):
     #   sample_weights full-VB with sample_variational_params live (VAEB.py:127-129)
     #   variant        'vaeb' | 'fullbayes' (VAEBfullbayes.py objective/update scalars)
     #   optimizer      'adagrad' (getUpdates, VAEB.py:426-444) | 'adadelta' (getAdaDeltaUpdates, VAEB.py:449-469,
-    #                  the alternative the reference keeps commented out at VAEB.py:404; rho = self.rho = 0.95)
+    #                  the alternative the reference keeps commented out at VAEB.py:404; rho = self.rho = 0.95) |
+    #                  'adam' (Kingma & Ba 2015 with the weight prior, ascent; adam_betas, adam_eps; moments in
+    #                  self.ADA (m) and self.ADAM_V (v), step counter in self.adam_step; L^A / L^B estimators)
     #   encoder_layers 1 (VAEB.py:245-251) | 2..4: the deeper encoders of Report/replication/replic.tex:46-57 -- extra H x H
     #                  hidden layers between the first one and the heads; their parameters W3_k, b3_k (k = 2..) follow the
     #                  reference's list, weights first; fp32 per-layer kernels, L^A / L^B estimators
@@ -80,7 +82,7 @@ class VAEB(object):
     def __init__(self, x_train, continuous, hidden_units, latent_size, batch_size,
                  L, learning_rate, genericEstimator, fullVariational, params=None, prng=None, sigmaInit=None,
                  *, device=0, precision="fp32", eps_mode="philox", sample_weights=False, variant="vaeb", seed=10,
-                 optimizer="adagrad", activation="tanh", encoder_layers=1):
+                 optimizer="adagrad", activation="tanh", encoder_layers=1, adam_betas=(0.9, 0.999), adam_eps=1e-8):
         x_train = np.asarray(x_train)
         [self.N, self.input_size] = x_train.shape       # VAEB.py:135
         self.n_hidden_units = hidden_units
@@ -162,11 +164,16 @@ class VAEB(object):
                 self.full_variational_params += [SharedParam(self, _lib.BUF_VMU, i, nm + "_mu_vb", s),
                                                  SharedParam(self, _lib.BUF_VSIG, i, nm + "_sigma_vb", s)]
 
-        if optimizer not in ("adagrad", "adadelta"):
-            raise ValueError("optimizer must be 'adagrad' or 'adadelta'")
+        if optimizer not in ("adagrad", "adadelta", "adam"):
+            raise ValueError("optimizer must be 'adagrad', 'adadelta' or 'adam'")
         self.optimizer = optimizer
         if optimizer == "adadelta":
             _lib.check(self._lib.vaeb_set_optimizer(self._h, _lib.OPT_ADADELTA, self.rho))
+        if optimizer == "adam":
+            b1, b2 = adam_betas
+            _lib.check(self._lib.vaeb_set_adam(self._h, float(b1), float(b2), float(adam_eps)))
+            self.ADAM_V = [SharedParam(self, _lib.BUF_ADAM_V, i, "adam_v_" + nm, s)
+                           for i, (nm, s) in enumerate(zip(self._names, self._shapes))]
         if activation not in ("tanh", "sigmoid", "relu"):
             raise ValueError("activation must be 'tanh', 'sigmoid' or 'relu'")
         self.activation = activation
@@ -417,6 +424,18 @@ class VAEB(object):
         """Adagrad step (VAEB.py:426-444) with the gradients left in the buffer by `gradients()` (or written
         there by the caller): the second half of `update()` on its own."""
         _lib.check(self._lib.vaeb_apply_update(self._h))
+
+    @property
+    def adam_step(self):
+        """Adam's step counter t: updates applied since Adam was selected.  With the moments (self.ADA and
+        self.ADAM_V) it is the optimizer state a checkpoint saves and restores."""
+        t = C.c_int64()
+        _lib.check(self._lib.vaeb_adam_step(self._h, C.byref(t)))
+        return t.value
+
+    @adam_step.setter
+    def adam_step(self, t):
+        _lib.check(self._lib.vaeb_set_adam_step(self._h, int(t)))
 
     def profile_optimizer(self, iters=20, variant=0):
         """(ms per launch, algorithmic bytes per launch) of the flat Adagrad pass over this model's buffers."""
