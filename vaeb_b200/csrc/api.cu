@@ -698,32 +698,6 @@ int read_scalars(vaeb_handle* h, int n, float* out) {
   return VAEB_OK;
 }
 
-// n updates through the fused single-launch kernel (fused_step.cu); scalars land in d_scalars[0..n)
-int fused_updates(vaeb_handle* h, const int32_t* batch_order, const float* d_xrows, int rows, int n,
-                  const float* d_eps, int slot0 = 0) {
-  VAEB_TRY(ensure_ws(h, rows, rows, true));
-  const int* d_order = nullptr;
-  if (batch_order) {
-    FusedState& f = h->fused;
-    if (n > f.order_cap) {
-      VAEB_CUDA(cudaStreamSynchronize(h->stream));
-      if (f.d_order) VAEB_CUDA(cudaFree(f.d_order));
-      f.d_order = nullptr;
-      VAEB_CUDA(cudaMalloc((void**)&f.d_order, (size_t)n * sizeof(int)));
-      f.order_cap = n;
-    }
-    VAEB_CUDA(cudaMemcpyAsync(f.d_order, batch_order, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, h->stream));
-    d_order = f.d_order;
-  }
-  if (step_tc_supported(h, rows)) return step_tc_launch(h, d_order, d_xrows, rows, n, d_eps, slot0, nullptr);
-  return fused_step_launch(h, d_order, d_xrows, rows, n, d_eps, slot0, nullptr);
-}
-
-// an update of `rows` rows is ONE launch: the tensor-core step kernel (step_tc.cu) or the FFMA one (fused_step.cu)
-inline bool single_launch_supported(const vaeb_handle* h, int rows) {
-  return step_tc_supported(h, rows) || fused_step_supported(h, rows);
-}
-
 float* flat_by_which(vaeb_handle* h, int which) {
   switch (which) {
     case 0: return h->d_params;
@@ -759,6 +733,57 @@ int load_nccl(NcclApi& api, const char* path) {
 }
 
 }  // namespace
+
+// How an update of `rows` rows runs: ONE launch of the tensor-core step kernel (step_tc.cu) or of the fp32 FFMA one
+// (fused_step.cu), or the per-layer kernels of enqueue_update.  The values are those of vaeb_step_kernel.
+enum StepPath { PER_LAYER = 0, FUSED = 1, STEP_TC = 2 };
+
+// What both single-launch kernels implement: the four estimators, L = 1, one GPU, one encoder hidden layer, tanh hidden
+// layers and Adagrad applied in their weight-gradient epilogues.
+static bool single_launch_model(const vaeb_handle* h) {
+  const int e = h->cfg.estimator;
+  return (e == VAEB_EST_LB || e == VAEB_EST_LA || e == VAEB_EST_FVB || e == VAEB_EST_FVB_SAMPLED) && h->L == 1 &&
+         h->world == 1 && h->lay.depth == 1 && h->hidden_act == VAEB_ACT_TANH && h->optimizer == VAEB_OPT_ADAGRAD;
+}
+
+bool fused_step_supported(const vaeb_handle* h, int rows) {
+  return !h->env_no_fused && single_launch_model(h) && h->cfg.precision == VAEB_PREC_FP32 && rows >= 1 && rows <= 4096;
+}
+
+static bool step_tc_supported(const vaeb_handle* h, int rows) {
+  return !h->steptc.unavailable && !h->env_no_step_tc && single_launch_model(h) && h->cfg.precision != VAEB_PREC_BF16 &&
+         rows >= 1 && rows <= st2::MP && (h->D % 8) == 0 && (h->H % 4) == 0 && h->D >= 64 && h->H >= 64 && h->D <= 1024 &&
+         h->H <= 512 && h->Z >= 1 && h->Z <= 20 &&
+         (!h->cont || fused_step_supported(h, rows));   // Gaussian decoder: the fp32 kernel takes over a step whose deltas
+}                                                       // leave the fp16 range
+
+static StepPath step_path(const vaeb_handle* h, int rows) {
+  if (step_tc_supported(h, rows)) return STEP_TC;
+  return fused_step_supported(h, rows) ? FUSED : PER_LAYER;
+}
+
+// n updates of `rows` rows in ONE launch of the kernel of `path` (STEP_TC or FUSED); their bounds land in
+// d_scalars[slot0 ..].  The minibatch indices of the updates come from the host (host_order) or are on the device
+// already (d_order); see fused_step_launch for how they and d_xrows address the rows.
+static int run_single_launch(vaeb_handle* h, StepPath path, const int32_t* host_order, const int* d_order,
+                             const float* d_xrows, int rows, int n, const float* d_eps, int slot0, long long* d_timing) {
+  // the fp32 kernel's workspace, for step_tc_launch too: it hands a Gaussian step whose deltas overflow to that kernel
+  VAEB_TRY(ensure_ws(h, rows, rows, true));
+  VAEB_TRY(ensure_scalars(h, slot0 + n));
+  if (host_order) {
+    if (n > h->order_cap) {
+      VAEB_CUDA(cudaStreamSynchronize(h->stream));
+      if (h->d_order) VAEB_CUDA(cudaFree(h->d_order));
+      h->d_order = nullptr;
+      VAEB_CUDA(cudaMalloc((void**)&h->d_order, (size_t)n * sizeof(int)));
+      h->order_cap = n;
+    }
+    VAEB_CUDA(cudaMemcpyAsync(h->d_order, host_order, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    d_order = h->d_order;
+  }
+  if (path == STEP_TC) return step_tc_launch(h, d_order, d_xrows, rows, n, d_eps, slot0, d_timing);
+  return fused_step_launch(h, d_order, d_xrows, rows, n, d_eps, slot0, d_timing);
+}
 
 extern "C" {
 
@@ -824,12 +849,8 @@ int vaeb_create(const vaeb_config* cfg, vaeb_handle** out) {
   h->D = cfg->input_dim; h->H = cfg->hidden_units; h->Z = cfg->latent_size; h->M = cfg->batch_size; h->L = cfg->L;
   h->cont = cfg->continuous != 0;
   build_layout(h->lay, h->D, h->H, h->Z, h->cont, cfg->encoder_hidden_layers);
-  { const char* e = getenv("VAEB_B200_FUSED"); h->fused_off = e && e[0] == '0'; h->fused_off_user = h->fused_off; }
-  { const char* e = getenv("VAEB_B200_STEP_TC"); h->steptc_off = e && e[0] == '0'; }
-  if (h->lay.depth > 1) {      // deeper encoders run on the per-layer kernels only
-    h->fused_off = h->fused_off_user = true;
-    h->steptc_off = true;
-  }
+  { const char* e = getenv("VAEB_B200_FUSED"); h->env_no_fused = e && e[0] == '0'; }
+  { const char* e = getenv("VAEB_B200_STEP_TC"); h->env_no_step_tc = e && e[0] == '0'; }
   h->tc.active = cfg->precision != VAEB_PREC_FP32;
   h->tc.ns = cfg->precision == VAEB_PREC_BF16X3 ? 2 : 1;
   VAEB_CUDA(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
@@ -869,12 +890,13 @@ int vaeb_destroy(vaeb_handle* h) {
                    h->d_gsig, h->d_theta, h->d_zeta, h->d_tprior, h->d_x, h->d_stage, h->d_stage2, h->d_out,
                    h->d_scalars, h->d_ada2};
   for (float* p : bufs) if (p) cudaFree(p);
+  if (h->d_order) cudaFree(h->d_order);
   if (h->d_counter) cudaFree(h->d_counter);
   if (h->d_w45t) cudaFree(h->d_w45t);
   step_tc_free(h->steptc);
   {
     FusedState& f = h->fused;
-    void* fb[] = {f.bar, f.params_alt, f.partial, f.aux_part, f.tprior_part, f.d_order, f.d_timing};
+    void* fb[] = {f.bar, f.params_alt, f.partial, f.aux_part, f.tprior_part, f.d_timing};
     for (void* q : fb) if (q) cudaFree(q);
   }
   {
@@ -1015,10 +1037,12 @@ int vaeb_update(vaeb_handle* h, int64_t index, const float* eps, float* elbo_out
   VAEB_CUDA(cudaSetDevice(h->cfg.device));
   const float* d_eps;
   VAEB_TRY(stage_eps_zeta(h, eps, (int64_t)h->L * h->M * h->Z, &d_eps));
-  if (single_launch_supported(h, h->M))
-    VAEB_TRY(fused_updates(h, nullptr, h->d_x + (size_t)index * h->M * h->D, h->M, 1, d_eps));
+  const float* x = h->d_x + (size_t)index * h->M * h->D;
+  const StepPath path = step_path(h, h->M);
+  if (path != PER_LAYER)
+    VAEB_TRY(run_single_launch(h, path, nullptr, nullptr, x, h->M, 1, d_eps, 0, nullptr));
   else
-    VAEB_TRY(enqueue_update(h, h->d_x + (size_t)index * h->M * h->D, h->M, d_eps, nullptr, 0, true));
+    VAEB_TRY(enqueue_update(h, x, h->M, d_eps, nullptr, 0, true));
   return read_scalars(h, 1, elbo_out);
 }
 
@@ -1029,8 +1053,9 @@ int vaeb_update_host(vaeb_handle* h, const float* x, int64_t rows, const float* 
   VAEB_TRY(stage_in(h, &h->d_stage, &h->stage_cap, x, rows * h->D));
   const float* d_eps;
   VAEB_TRY(stage_eps_zeta(h, eps, (int64_t)h->L * rows * h->Z, &d_eps));
-  if (single_launch_supported(h, (int)rows))
-    VAEB_TRY(fused_updates(h, nullptr, h->d_stage, (int)rows, 1, d_eps));
+  const StepPath path = step_path(h, (int)rows);
+  if (path != PER_LAYER)
+    VAEB_TRY(run_single_launch(h, path, nullptr, nullptr, h->d_stage, (int)rows, 1, d_eps, 0, nullptr));
   else
     VAEB_TRY(enqueue_update(h, h->d_stage, (int)rows, d_eps, nullptr, 0, true));
   return read_scalars(h, 1, elbo_out);
@@ -1140,8 +1165,6 @@ int vaeb_set_hidden_activation(vaeb_handle* h, int32_t act) {
   VAEB_REQUIRE(act == VAEB_ACT_TANH || (h->cfg.precision == VAEB_PREC_FP32 && !is_fvb(h) && h->world == 1),
                "sigmoid / ReLU hidden layers: fp32 per-layer kernels, L^A / L^B estimators, one GPU");
   h->hidden_act = act;
-  // the single-launch step kernels and the tensor-core estimators are tanh-only
-  h->fused_off = (act != VAEB_ACT_TANH || h->optimizer != VAEB_OPT_ADAGRAD) ? true : h->fused_off_user;
   invalidate_weight_mirrors(h);
   return VAEB_OK;
 }
@@ -1160,7 +1183,6 @@ int vaeb_set_optimizer(vaeb_handle* h, int32_t optimizer, float rho) {
   VAEB_CUDA(cudaMemsetAsync(h->d_ada, 0, nb, h->stream));
   h->optimizer = optimizer;
   h->rho = rho;
-  h->fused_off = (optimizer != VAEB_OPT_ADAGRAD || h->hidden_act != VAEB_ACT_TANH) ? true : h->fused_off_user;
   return VAEB_OK;
 }
 
@@ -1189,7 +1211,6 @@ int vaeb_set_adam(vaeb_handle* h, float beta1, float beta2, float eps) {
   h->optimizer = VAEB_OPT_ADAM;
   h->adam_b1 = beta1; h->adam_b2 = beta2; h->adam_eps = eps;
   h->adam_t = 0;
-  h->fused_off = true;              // the single-launch step kernels apply Adagrad only
   return VAEB_OK;
 }
 
@@ -1207,8 +1228,8 @@ int vaeb_set_adam_step(vaeb_handle* h, int64_t t) {
   return VAEB_OK;
 }
 
-// Launches the minibatches copied into the current group buffer: ONE fused-kernel launch for up to ASYNC_GROUP
-// updates (per-layer kernels otherwise), then the readback of their bounds.
+// Launches the minibatches copied into the current group buffer: ONE launch of a single-launch step kernel for up to
+// ASYNC_GROUP updates (per-layer kernels otherwise), then the readback of their bounds.
 static int async_flush(vaeb_handle* h) {
   if (h->a_pending == 0) return VAEB_OK;
   const int g = h->a_group, n = h->a_pending;
@@ -1216,11 +1237,9 @@ static int async_flush(vaeb_handle* h) {
   const int slot0 = h->a_outstanding - n;
   VAEB_CUDA(cudaEventRecord(h->a_copied[g], h->copy_stream));
   VAEB_CUDA(cudaStreamWaitEvent(h->stream, h->a_copied[g], 0));
-  if (step_tc_supported(h, rows)) {
-    VAEB_TRY(step_tc_launch(h, h->d_iota, h->a_stage[g], rows, n, nullptr, slot0, nullptr));
-  } else if (fused_step_supported(h, rows)) {
-    VAEB_TRY(ensure_ws(h, rows, rows, true));
-    VAEB_TRY(fused_step_launch(h, h->d_iota, h->a_stage[g], rows, n, nullptr, slot0, nullptr));
+  const StepPath path = step_path(h, rows);
+  if (path != PER_LAYER) {
+    VAEB_TRY(run_single_launch(h, path, nullptr, h->d_iota, h->a_stage[g], rows, n, nullptr, slot0, nullptr));
   } else {
     for (int i = 0; i < n; ++i)
       VAEB_TRY(enqueue_update(h, h->a_stage[g] + (size_t)i * rows * h->D, rows, nullptr, nullptr, slot0 + i, true));
@@ -1341,8 +1360,9 @@ int vaeb_update_many(vaeb_handle* h, const int32_t* batch_order, int32_t n, floa
     const int64_t index = batch_order[i];
     VAEB_REQUIRE(index >= 0 && (index + 1) * (int64_t)h->M <= h->n_data, "batch index outside the resident data");
   }
-  if (single_launch_supported(h, h->M)) {
-    VAEB_TRY(fused_updates(h, batch_order, nullptr, h->M, n, nullptr));
+  const StepPath path = step_path(h, h->M);
+  if (path != PER_LAYER) {
+    VAEB_TRY(run_single_launch(h, path, batch_order, nullptr, nullptr, h->M, n, nullptr, 0, nullptr));
     return read_scalars(h, n, elbo_out);
   }
   for (int i = 0; i < n; ++i) {
@@ -1890,77 +1910,72 @@ int vaeb_profile_update(vaeb_handle* h, int64_t index, int32_t iters, int32_t ma
   const size_t nb = (size_t)(h->lay.padded + 4) * sizeof(float);
   StateBackup backup(h, nb);              // restores params / ADA / step / launch count on every exit path
   VAEB_CUDA(backup.take());
-  int rc = VAEB_OK;
-  int n = 0;
-  if (step_tc_supported(h, h->M)) {
-    // the tensor-core step kernel stamps %globaltimer after every grid barrier (CTA 0): ns per phase, averaged over
-    // `iters` consecutive updates of one launch (the first two are warm-up)
+  const StepPath path = step_path(h, h->M);
+  // The single-launch kernels stamp %globaltimer at every phase boundary (CTA 0) into d_timing: ONE launch of `steps`
+  // updates of minibatch `index`, its stamps read back into tm, ns per phase averaged over the last `iters` updates (the
+  // first two are warm-up); kn / fl / by: the kernel's phase names, algorithmic flops and bytes.
+  const int steps = iters + 2;
+  auto stamped = [&](int np, long long* d_timing, std::vector<long long>& tm, const char* const* kn, const double* fl,
+                     const double* by) -> int {
+    const std::vector<int32_t> order((size_t)steps, (int32_t)index);
+    VAEB_TRY(run_single_launch(h, path, order.data(), nullptr, nullptr, h->M, steps, nullptr, 0, d_timing));
+    VAEB_CUDA(cudaMemcpyAsync(tm.data(), d_timing, tm.size() * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+    VAEB_CUDA(cudaStreamSynchronize(h->stream));
+    const int n = std::min(np, (int)max_phases);
+    for (int i = 0; i < n; ++i) {
+      double acc = 0;
+      for (int s = 2; s < steps; ++s) acc += (double)(tm[(size_t)s * (np + 1) + i + 1] - tm[(size_t)s * (np + 1) + i]);
+      ms[i] = (float)(acc / iters * 1e-6);
+      flops[i] = fl[i]; bytes[i] = by[i];
+      std::strncpy(names + 48 * i, kn[i], 47);
+      names[48 * i + 47] = 0;
+    }
+    *n_phases = n;
+    return VAEB_OK;
+  };
+  if (path == STEP_TC) {
     constexpr int NP = st2::N_PHASES;
     static const char* const kNames[NP] = {
         "P1 enc1 x.W3+tanh | W4,W5 update", "P2 heads+reparam+KL", "P3 dec1+dec2 h.W2+loglik+delta",
         "P4 dgrad (da.W2^T)*(1-h^2)", "P5 dz | W2 update | bound", "P6 W3 update | W1 update"};
-    const int steps = iters + 2;
     StepTcState& f = h->steptc;
+    const size_t n_stamps = (size_t)steps * (NP + 1) + 128 + 256 * NP;      // + sub-phase trace + per-CTA arrivals
     if (steps * (NP + 1) > f.timing_cap) {
       if (f.d_timing) cudaFree(f.d_timing);
       f.d_timing = nullptr;
-      VAEB_CUDA(cudaMalloc((void**)&f.d_timing, ((size_t)steps * (NP + 1) + 128 + 256 * NP) * sizeof(long long)));   // + sub-phase trace + per-CTA arrivals
+      VAEB_CUDA(cudaMalloc((void**)&f.d_timing, n_stamps * sizeof(long long)));
       f.timing_cap = steps * (NP + 1);
     }
-    VAEB_CUDA(cudaMemsetAsync(f.d_timing, 0, ((size_t)steps * (NP + 1) + 128 + 256 * NP) * sizeof(long long), h->stream));
-    if (steps > f.order_cap) {
-      if (f.d_order) cudaFree(f.d_order);
-      f.d_order = nullptr;
-      VAEB_CUDA(cudaMalloc((void**)&f.d_order, (size_t)steps * sizeof(int)));
-      f.order_cap = steps;
-    }
-    std::vector<int32_t> order((size_t)steps, (int32_t)index);
-    VAEB_CUDA(cudaMemcpyAsync(f.d_order, order.data(), (size_t)steps * sizeof(int), cudaMemcpyHostToDevice, h->stream));
-    VAEB_CUDA(cudaStreamSynchronize(h->stream));
-    VAEB_TRY(ensure_scalars(h, steps));
-    rc = step_tc_launch(h, f.d_order, nullptr, h->M, steps, nullptr, 0, f.d_timing);
-    std::vector<long long> tm((size_t)steps * (NP + 1) + 128 + 256 * NP);
-    if (rc == VAEB_OK) {
-      VAEB_CUDA(cudaMemcpyAsync(tm.data(), f.d_timing, tm.size() * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
-      VAEB_CUDA(cudaStreamSynchronize(h->stream));
-      if (getenv("VAEB_STEPTC_TRACE")) {               // sub-phase stamps of CTA 0 in the last step (ns since the first)
-        const long long* tr = tm.data() + (size_t)steps * (NP + 1);
-        for (int q = 0; q < 60 && tr[2 * q] != 0; ++q)
-          fprintf(stderr, "st2 trace %3lld  +%8.3f us\n", tr[2 * q], 1e-3 * (double)(tr[2 * q + 1] - tr[1]));
-        // arrival of every CTA at the barrier that ends each phase of the last step (us after the phase opened for CTA 0)
-        const long long* ar = tr + 128;
-        const long long* last = tm.data() + (size_t)(steps - 1) * (NP + 1);
-        for (int ph = 0; ph < NP; ++ph) {
-          fprintf(stderr, "st2 arrive P%d:", ph + 1);
-          for (int b = 0; b < f.n_cta && b < 256; ++b) fprintf(stderr, " %.1f", 1e-3 * (double)(ar[(size_t)b * NP + ph] - last[ph]));
-          fprintf(stderr, "\n");
-        }
-      }
-      const double dM = h->M, dD = h->D, dH = h->H, dZ = h->Z;
-      const double fl[NP] = {2 * dM * dD * dH + 4 * dM * dH * dZ, 4 * dM * dH * dZ, 2 * dM * dZ * dH + 2 * dM * dH * dD,
-                             2 * dM * dH * dD, 2 * dM * dZ * dH + 2 * dM * dH * dD, 2 * dM * dD * dH + 4 * dM * dH * dZ + 2 * dM * dZ * dH};
-      const double by[NP] = {4 * (dM * dD + dD * dH + dM * dH) + 40 * dH * dZ, 4 * (dM * dH + 2 * dH * dZ + 4 * dM * dZ),
-                             4 * (dM * dZ + dZ * dH + dH * dD + 2 * dM * dD), 4 * (dM * dD + dH * dD + 2 * dM * dH),
-                             4 * (dM * dH + dM * dD) + 24 * dH * dD, 4 * (dM * dD + dM * dH) + 20 * dD * dH + 20 * dZ * dH};
-      n = std::min(NP, (int)max_phases);
-      for (int i = 0; i < n; ++i) {
-        double acc = 0;
-        for (int q = 2; q < steps; ++q) acc += (double)(tm[(size_t)q * (NP + 1) + i + 1] - tm[(size_t)q * (NP + 1) + i]);
-        ms[i] = (float)(acc / iters * 1e-6);
-        flops[i] = fl[i]; bytes[i] = by[i];
-        std::strncpy(names + 48 * i, kNames[i], 47);
-        names[48 * i + 47] = 0;
+    VAEB_CUDA(cudaMemsetAsync(f.d_timing, 0, n_stamps * sizeof(long long), h->stream));
+    const double dM = h->M, dD = h->D, dH = h->H, dZ = h->Z;
+    const double fl[NP] = {2 * dM * dD * dH + 4 * dM * dH * dZ, 4 * dM * dH * dZ, 2 * dM * dZ * dH + 2 * dM * dH * dD,
+                           2 * dM * dH * dD, 2 * dM * dZ * dH + 2 * dM * dH * dD, 2 * dM * dD * dH + 4 * dM * dH * dZ + 2 * dM * dZ * dH};
+    const double by[NP] = {4 * (dM * dD + dD * dH + dM * dH) + 40 * dH * dZ, 4 * (dM * dH + 2 * dH * dZ + 4 * dM * dZ),
+                           4 * (dM * dZ + dZ * dH + dH * dD + 2 * dM * dD), 4 * (dM * dD + dH * dD + 2 * dM * dH),
+                           4 * (dM * dH + dM * dD) + 24 * dH * dD, 4 * (dM * dD + dM * dH) + 20 * dD * dH + 20 * dZ * dH};
+    std::vector<long long> tm(n_stamps);
+    VAEB_TRY(stamped(NP, f.d_timing, tm, kNames, fl, by));
+    if (getenv("VAEB_STEPTC_TRACE")) {               // sub-phase stamps of CTA 0 in the last step (ns since the first)
+      const long long* tr = tm.data() + (size_t)steps * (NP + 1);
+      for (int q = 0; q < 60 && tr[2 * q] != 0; ++q)
+        fprintf(stderr, "st2 trace %3lld  +%8.3f us\n", tr[2 * q], 1e-3 * (double)(tr[2 * q + 1] - tr[1]));
+      // arrival of every CTA at the barrier that ends each phase of the last step (us after the phase opened for CTA 0)
+      const long long* ar = tr + 128;
+      const long long* last = tm.data() + (size_t)(steps - 1) * (NP + 1);
+      for (int ph = 0; ph < NP; ++ph) {
+        fprintf(stderr, "st2 arrive P%d:", ph + 1);
+        for (int b = 0; b < f.n_cta && b < 256; ++b) fprintf(stderr, " %.1f", 1e-3 * (double)(ar[(size_t)b * NP + ph] - last[ph]));
+        fprintf(stderr, "\n");
       }
     }
-  } else if (fused_step_supported(h, h->M)) {
-    // the fused kernel stamps %globaltimer at every phase boundary (CTA 0): ns per phase, averaged
-    // over `iters` consecutive updates of one launch (the first two are warm-up)
+    return VAEB_OK;
+  }
+  if (path == FUSED) {
     constexpr int NP = fs::N_PHASES;
     static const char* const kNames[NP] = {
         "P1 enc1 x.W3+tanh", "P2 heads+reparam+KL", "P3 dec1 z.W1+tanh", "P4 dec2 h.W2+loglik+delta",
         "P5 dgrad (da.W2^T)*(1-h^2)", "P6 W2,W1 wgrad+Adagrad | dz | bound", "P7 dh_e | W4,W5 wgrad+Adagrad",
         "P8 W3 wgrad+Adagrad"};
-    const int steps = iters + 2;
     FusedState& f = h->fused;
     if (steps * (NP + 1) > f.timing_cap) {
       if (f.d_timing) cudaFree(f.d_timing);
@@ -1968,63 +1983,33 @@ int vaeb_profile_update(vaeb_handle* h, int64_t index, int32_t iters, int32_t ma
       VAEB_CUDA(cudaMalloc((void**)&f.d_timing, (size_t)steps * (NP + 1) * sizeof(long long)));
       f.timing_cap = steps * (NP + 1);
     }
-    std::vector<int32_t> order((size_t)steps, (int32_t)index);
-    rc = ensure_ws(h, h->M, h->M, true);
-    const int* d_order = nullptr;
-    if (rc == VAEB_OK) {
-      if (steps > f.order_cap) {
-        if (f.d_order) cudaFree(f.d_order);
-        f.d_order = nullptr;
-        VAEB_CUDA(cudaMalloc((void**)&f.d_order, (size_t)steps * sizeof(int)));
-        f.order_cap = steps;
-      }
-      VAEB_CUDA(cudaMemcpyAsync(f.d_order, order.data(), (size_t)steps * sizeof(int), cudaMemcpyHostToDevice, h->stream));
-      VAEB_CUDA(cudaStreamSynchronize(h->stream));
-      d_order = f.d_order;
-      VAEB_TRY(ensure_scalars(h, steps));
-      rc = fused_step_launch(h, d_order, nullptr, h->M, steps, nullptr, 0, f.d_timing);
-    }
+    const double dM = h->M, dD = h->D, dH = h->H, dZ = h->Z, c = h->cont ? 2.0 : 1.0;
+    const double fl[NP] = {2 * dM * dD * dH, 4 * dM * dH * dZ, 2 * dM * dZ * dH, 2 * dM * dH * dD * c, 2 * dM * dH * dD * c,
+                           2 * dM * dH * dD * c + 4 * dM * dZ * dH, 8 * dM * dH * dZ, 2 * dM * dD * dH};
+    const double by[NP] = {4 * (dM * dD + dD * dH + dM * dH), 4 * (dM * dH + 2 * dH * dZ + 4 * dM * dZ),
+                           4 * (dM * dZ + dZ * dH + dM * dH), 4 * (dM * dH + c * dH * dD + dM * dD + c * dM * dD),
+                           4 * (c * dM * dD + c * dH * dD + 2 * dM * dH),
+                           4 * (dM * dH + c * dM * dD + dM * dH + dM * dZ) + 16 * (c * dH * dD + dZ * dH),
+                           4 * (2 * dM * dZ + 2 * dH * dZ + 2 * dM * dH) + 16 * 2 * dH * dZ,
+                           4 * (dM * dD + dM * dH) + 16 * dD * dH};
     std::vector<long long> tm((size_t)steps * (NP + 1));
-    if (rc == VAEB_OK) {
-      VAEB_CUDA(cudaMemcpyAsync(tm.data(), f.d_timing, tm.size() * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
-      VAEB_CUDA(cudaStreamSynchronize(h->stream));
-      const double dM = h->M, dD = h->D, dH = h->H, dZ = h->Z, c = h->cont ? 2.0 : 1.0, P = (double)h->lay.total;
-      const double fl[NP] = {2 * dM * dD * dH, 4 * dM * dH * dZ, 2 * dM * dZ * dH, 2 * dM * dH * dD * c, 2 * dM * dH * dD * c,
-                             2 * dM * dH * dD * c + 4 * dM * dZ * dH, 8 * dM * dH * dZ, 2 * dM * dD * dH};
-      const double by[NP] = {4 * (dM * dD + dD * dH + dM * dH), 4 * (dM * dH + 2 * dH * dZ + 4 * dM * dZ),
-                             4 * (dM * dZ + dZ * dH + dM * dH), 4 * (dM * dH + c * dH * dD + dM * dD + c * dM * dD),
-                             4 * (c * dM * dD + c * dH * dD + 2 * dM * dH),
-                             4 * (dM * dH + c * dM * dD + dM * dH + dM * dZ) + 16 * (c * dH * dD + dZ * dH),
-                             4 * (2 * dM * dZ + 2 * dH * dZ + 2 * dM * dH) + 16 * 2 * dH * dZ,
-                             4 * (dM * dD + dM * dH) + 16 * dD * dH};
-      (void)P;
-      n = std::min(NP, (int)max_phases);
-      for (int i = 0; i < n; ++i) {
-        double acc = 0;
-        for (int s = 2; s < steps; ++s) acc += (double)(tm[(size_t)s * (NP + 1) + i + 1] - tm[(size_t)s * (NP + 1) + i]);
-        ms[i] = (float)(acc / iters * 1e-6);
-        flops[i] = fl[i]; bytes[i] = by[i];
-        std::strncpy(names + 48 * i, kNames[i], 47);
-        names[48 * i + 47] = 0;
-      }
-    }
-  } else {
-    PhaseProf prof;
-    prof.iters = iters;
-    VAEB_CUDA(cudaEventCreate(&prof.e0));
-    VAEB_CUDA(cudaEventCreate(&prof.e1));
-    g_prof = &prof;
-    rc = enqueue_update(h, h->d_x + (size_t)index * h->M * h->D, h->M, nullptr, nullptr, 0, true);
-    g_prof = nullptr;
-    cudaEventDestroy(prof.e0); cudaEventDestroy(prof.e1);
-    n = std::min<int>((int)prof.ms.size(), max_phases);
-    for (int i = 0; i < n && rc == VAEB_OK; ++i) {
-      ms[i] = prof.ms[i]; flops[i] = prof.flops[i]; bytes[i] = prof.bytes[i];
-      std::strncpy(names + 48 * i, prof.names[i].c_str(), 47);
-      names[48 * i + 47] = 0;
-    }
+    return stamped(NP, f.d_timing, tm, kNames, fl, by);
   }
+  PhaseProf prof;
+  prof.iters = iters;
+  VAEB_CUDA(cudaEventCreate(&prof.e0));
+  VAEB_CUDA(cudaEventCreate(&prof.e1));
+  g_prof = &prof;
+  const int rc = enqueue_update(h, h->d_x + (size_t)index * h->M * h->D, h->M, nullptr, nullptr, 0, true);
+  g_prof = nullptr;
+  cudaEventDestroy(prof.e0); cudaEventDestroy(prof.e1);
   if (rc != VAEB_OK) return rc;
+  const int n = std::min<int>((int)prof.ms.size(), max_phases);
+  for (int i = 0; i < n; ++i) {
+    ms[i] = prof.ms[i]; flops[i] = prof.flops[i]; bytes[i] = prof.bytes[i];
+    std::strncpy(names + 48 * i, prof.names[i].c_str(), 47);
+    names[48 * i + 47] = 0;
+  }
   *n_phases = n;
   return VAEB_OK;
 }
@@ -2082,7 +2067,7 @@ int vaeb_launch_count(vaeb_handle* h, int64_t* n_launches) {
 
 int vaeb_step_kernel(vaeb_handle* h, int64_t rows, int32_t* which) {
   VAEB_REQUIRE(h && which && rows > 0, "null argument");
-  *which = step_tc_supported(h, (int)rows) ? 2 : (fused_step_supported(h, (int)rows) ? 1 : 0);
+  *which = step_path(h, (int)rows);
   return VAEB_OK;
 }
 

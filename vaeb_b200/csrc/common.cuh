@@ -100,7 +100,6 @@ struct FusedState {
   float* params_alt = nullptr;             // the other half of the parameter double buffer
   float* partial = nullptr; float* aux_part = nullptr;
   float* tprior_part = nullptr;            // per-CTA thetaPrior partial sums (sampled full VB)
-  int* d_order = nullptr; int order_cap = 0;
   long long* d_timing = nullptr; int timing_cap = 0;
   int rows = -1;
   fs::JobCfg job[fs::J_COUNT];
@@ -158,15 +157,15 @@ struct vaeb_handle {
   float* d_stage2 = nullptr; int64_t stage2_cap = 0;     // eps staging
   float* d_out = nullptr; int64_t out_cap = 0;           // device staging for outputs
   float* d_scalars = nullptr; float* h_scalars = nullptr; int scalars_cap = 0;
+  int* d_order = nullptr; int order_cap = 0;             // minibatch indices of a single-launch update (device)
   uint32_t step = 0;
   int64_t launches = 0;
   bool grads_have_prior = false;
   FusedState fused;
   IsTcState istc;
   StepTcState steptc;                 // tensor-core single-launch step (step_tc.cu)
-  bool steptc_off = false;            // VAEB_B200_STEP_TC=0: the FFMA kernel of fused_step.cu serves M <= 128 too
-  bool fused_off = false;             // VAEB_B200_FUSED=0: always use the per-layer kernels
-  bool fused_off_user = false;        // what the environment asked for (AdaDelta also turns the fused kernel off)
+  bool env_no_step_tc = false;        // VAEB_B200_STEP_TC=0: the FFMA kernel of fused_step.cu serves M <= 128 too
+  bool env_no_fused = false;          // VAEB_B200_FUSED=0: the FFMA single-launch kernel is off
   int hidden_act = 1;                 // VAEB_ACT_*: activation of both hidden layers (tanh in the reference's VAEB.py:246,254)
   // data parallel
   NcclApi nccl; void* comm = nullptr; int rank = 0, world = 1;

@@ -906,13 +906,6 @@ static JobCfg plan_job(int job, int M, int N, int K, int n_cta, bool dual_n) {
 
 }  // namespace fs
 
-bool fused_step_supported(const vaeb_handle* h, int rows) {
-  const int e = h->cfg.estimator;
-  return (e == VAEB_EST_LB || e == VAEB_EST_LA || e == VAEB_EST_FVB_SAMPLED || e == VAEB_EST_FVB) && h->L == 1 &&
-         h->world == 1 &&
-         h->cfg.precision == VAEB_PREC_FP32 && rows >= 1 && rows <= 4096 && !h->fused_off;
-}
-
 int fused_step_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, int rows, int n_steps,
                       const float* d_eps, int slot0, long long* d_timing) {
   using namespace fs;

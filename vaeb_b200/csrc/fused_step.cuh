@@ -85,8 +85,9 @@ struct StepParams {
 }  // namespace fs
 
 struct vaeb_handle;
-// true if the configuration is served by the fused kernel
+// true if the fused kernel can run this configuration (api.cu, next to step_path, which chooses the update kernel)
 bool fused_step_supported(const vaeb_handle* h, int rows);
-// n_steps updates in one launch.  Exactly one of (d_order, d_xrows) is non-null.
+// n_steps updates in one launch.  Rows of step s: minibatch d_order[s] (of `rows` rows) of the resident data -- or of
+// d_xrows when both are given (the staging ring of the streaming host-input updates) -- else d_xrows itself every step.
 int fused_step_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, int rows, int n_steps,
                       const float* d_eps, int slot0, long long* d_timing);

@@ -1625,18 +1625,9 @@ __global__ void __launch_bounds__(128) init_ones_kernel(OnesArgs a) {
 // =====================================================================================================================
 // host side
 // =====================================================================================================================
-bool step_tc_supported(const vaeb_handle* h, int rows) {
-  const int e = h->cfg.estimator;
-  if (h->steptc.unavailable || h->steptc_off || h->hidden_act != 1) return false;   // tanh hidden layers only
-  return (e == VAEB_EST_LB || e == VAEB_EST_LA || e == VAEB_EST_FVB || e == VAEB_EST_FVB_SAMPLED) && h->L == 1 && h->world == 1 &&
-         h->cfg.precision != VAEB_PREC_BF16 && h->optimizer == VAEB_OPT_ADAGRAD && rows >= 1 && rows <= st2::MP &&
-         (h->D % 8) == 0 && (h->H % 4) == 0 && h->D >= 64 && h->H >= 64 && h->D <= 1024 && h->H <= 512 && h->Z >= 1 &&
-         h->Z <= 20 && (!h->cont || fused_step_supported(h, rows));   // Gaussian decoder: the fp32 kernel takes over a step
-}                                                                      // whose deltas leave the fp16 range
-
 void step_tc_free(StepTcState& s) {
   void* ptrs[] = {s.bar, s.m_enc1, s.m_heads, s.m_dec2, s.m_dgrad, s.m_dz, s.m_dec1, s.act, s.he, s.hd, s.mu, s.ls,
-                  s.eps, s.z, s.m_w45k, s.partial, s.aux, s.d_order, s.d_timing, s.d_status, s.tprior_part};
+                  s.eps, s.z, s.m_w45k, s.partial, s.aux, s.d_timing, s.d_status, s.tprior_part};
   for (void* q : ptrs)
     if (q) cudaFree(q);
   s = StepTcState();
@@ -1748,7 +1739,6 @@ int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, int
   p.partial = s.partial; p.aux = s.aux;
   p.scalars = h->d_scalars + slot0; p.Mg = (float)rows; p.bmult = 1.0f;
   p.n_steps = n_steps;
-  { const char* e = getenv("VAEB_ST2_DBG"); p.dbg = e ? atoi(e) : 0; }
   p.bar = s.bar; p.bar_base = s.bar_count;
   p.timing = d_timing;
   p.status = s.d_status;

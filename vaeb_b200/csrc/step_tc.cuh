@@ -63,7 +63,6 @@ struct Params {
   int n_tiles3;                         // n tiles of dec2 (partial's leading dimension)
   float* scalars; float Mg; float bmult;
   int n_steps;
-  int dbg;                              // experiment switches (VAEB_ST2_DBG): timing studies only
   // Gaussian decoder only: its deltas scale with exp(-log variance) and can leave the range of the fp16 operand
   // pairs.  A step whose da2 / da1 exceed DLIMIT writes its index here (-1 otherwise) and the launch stops BEFORE
   // that step's first parameter update; the host finishes the remaining steps with the fp32 FFMA kernel.
@@ -99,15 +98,12 @@ struct StepTcState {
   bool mirrors_valid = false;
   float *he = nullptr, *hd = nullptr, *mu = nullptr, *ls = nullptr, *eps = nullptr, *z = nullptr,
         *partial = nullptr, *aux = nullptr;
-  int* d_order = nullptr; int order_cap = 0;
   long long* d_timing = nullptr; int timing_cap = 0;
   int* d_status = nullptr;
   float* tprior_part = nullptr;
   long long theta_step = -1;            // sampled full VB: the step the theta buffer / mirrors were drawn for
 };
 
-// true if this configuration / minibatch is served by the tensor-core step kernel
-bool step_tc_supported(const vaeb_handle* h, int rows);
 // n_steps updates in one launch (same contract as fused_step_launch)
 int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, int rows, int n_steps, const float* d_eps,
                    int slot0, long long* d_timing);
