@@ -45,9 +45,11 @@ def _check_step(x, continuous, H, Z, M, L, est, params, seed):
     for a, b, n in zip(g, g_ref, O.param_names(continuous)):
         worst = max(worst, assert_close_tensor(a, b, RTOL, name="grad " + n))
     # update(): pre-update value returned, Adagrad applied.  Two checks:
-    #  (a) the Adagrad rule itself (VAEB.py:438-442).  update() runs the fused single-launch kernel,
-    #      whose gradient is summed in a different order than gradients()'s, so the rule is checked on
-    #      the gradient the update itself used: after the first step ADA = g^2 exactly, hence
+    #  (a) the Adagrad rule itself (VAEB.py:438-442).  update() runs a single-launch step kernel (the
+    #      tensor-core one at C1/C2, M = 100; the fp32 FFMA one at the small ragged shapes, whose D is
+    #      below the tensor-core kernel's minimum), whose gradient is summed in a different order than
+    #      gradients()'s, so the rule is checked on the gradient the update itself used: after the first
+    #      step ADA = g^2 exactly, hence
     #      |dp| = lr*sqrt(ADA)/(sqrt(ADA)+1e-6) must hold everywhere to fp32 rounding, sqrt(ADA) must
     #      agree with |g| of gradients() at the gradient tolerance, and dp carries the sign of g;
     #  (b) end-to-end against the oracle's own update where the step is well conditioned: the

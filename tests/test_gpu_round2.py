@@ -130,8 +130,9 @@ def test_c3_parameters_after_tensor_core_updates(precision):
 
 # ---- vaeb_device_buffer lifetime (ADVICE r1) -----------------------------------------------------------------------
 def test_device_buffer_tracks_updates():
-    """The parameter buffer is double-buffered by the single-launch step kernel: vaeb_device_buffer(which=0) must be
-    re-queried after every update, and the re-queried address must hold exactly what vaeb_get_tensors returns."""
+    """vaeb_device_buffer(which=0) must be re-queried after every update, and the re-queried address must hold exactly
+    what vaeb_get_tensors returns.  At M = 100 update() runs the tensor-core step kernel, which updates the parameters
+    in place; the double buffer of the fp32 step kernel is held by tests/test_gpu_fused_step.py."""
     import vaeb_b200
     from vaeb_b200 import _lib
     from cuda.bindings import runtime as rt
