@@ -87,7 +87,9 @@ typedef struct vaeb_config {
 #define VAEB_ACT_RELU 3
 
 const char* vaeb_last_error(void);
-int vaeb_version(void);      /* 103: adds Adam (vaeb_set_adam, vaeb_adam_step, vaeb_set_adam_step; vaeb_config unchanged);
+int vaeb_version(void);      /* 104: adds the KL weight (vaeb_set_kl_weight, vaeb_kl_step, vaeb_set_kl_step; vaeb_config
+                                unchanged);
+                                103: adds Adam (vaeb_set_adam, vaeb_adam_step, vaeb_set_adam_step; vaeb_config unchanged);
                                 102: adds the encode, sample and validate_terms entry points (vaeb_config unchanged);
                                 101: vaeb_config ends with encoder_hidden_layers, reserved0 (100: it ended with seed) */
 /* sizeof(vaeb_config) as this library was compiled: a binding that declares the struct itself (ctypes, cgo) compares it
@@ -160,6 +162,27 @@ int vaeb_set_adam(vaeb_handle* h, float beta1, float beta2, float eps);
  * save and restore. */
 int vaeb_adam_step(vaeb_handle* h, int64_t* t);
 int vaeb_set_adam_step(vaeb_handle* h, int64_t t);
+
+/* Weight of the latent term while training: KL warm-up (Bowman et al. 2016; Sonderby et al. 2016) and beta-VAE (Higgins
+ * et al. 2017).  Sets the weight and resets the KL step counter t to 0.  The n-th update applied after this call
+ * (n = 1, 2, ...) ascends
+ *   loglik + beta_n aux,   beta_n = beta * min(1, n / warmup_updates)   (warmup_updates = 0: beta_n = beta)
+ * where aux is the term vaeb_validate_terms returns: the analytic -KL for L^B, the Monte-Carlo log p(z) - log q(z|x)
+ * for L^A.  beta_n is computed in double and rounded to float once per update.  t advances once per applied update,
+ * when the update is enqueued, on every update path (vaeb_update_many advances it by n, each of its updates with its
+ * own beta_n); vaeb_apply_update does not advance it.  Only the gradient is weighted: the values vaeb_update,
+ * vaeb_update_host, vaeb_update_many and vaeb_collect return stay the unweighted bound SGVB/M.  vaeb_gradients uses
+ * beta_{t+1}, the weight the next applied update would use, and does not advance t.  vaeb_validate, vaeb_validate_terms,
+ * vaeb_is_logpx, vaeb_encode, vaeb_sample, vaeb_reconstruct and the AE entry points ignore the weight;
+ * vaeb_profile_update restores t.  A handle that never calls this, or calls it with (1, 0), computes exactly what it
+ * computed before the weight existed.  Any optimizer, variant, L, activation and encoder depth; data-parallel ranks
+ * must agree on (beta, warmup_updates, t).  VAEB_EINVAL: beta negative, NaN or infinite, warmup_updates < 0, or a
+ * full-VB estimator (its bound has its own weight-prior term). */
+int vaeb_set_kl_weight(vaeb_handle* h, float beta, int64_t warmup_updates);
+/* The KL step counter t (updates applied since vaeb_set_kl_weight): save and restore it so that a resumed run continues
+ * its warm-up. */
+int vaeb_kl_step(vaeb_handle* h, int64_t* t);
+int vaeb_set_kl_step(vaeb_handle* h, int64_t t);
 
 /* `x_train = th.shared(...)` (VAEB.py:184): copies x[N,D] to the device once. */
 int vaeb_upload_data(vaeb_handle* h, const float* x, int64_t n_rows);

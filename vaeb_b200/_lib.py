@@ -53,6 +53,9 @@ EXPORTS = {
     "vaeb_set_adam": (C.c_int, [C.c_void_p, C.c_float, C.c_float, C.c_float]),
     "vaeb_adam_step": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
     "vaeb_set_adam_step": (C.c_int, [C.c_void_p, C.c_int64]),
+    "vaeb_set_kl_weight": (C.c_int, [C.c_void_p, C.c_float, C.c_int64]),
+    "vaeb_kl_step": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
+    "vaeb_set_kl_step": (C.c_int, [C.c_void_p, C.c_int64]),
     "vaeb_ae_train": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.POINTER(C.c_float)]),
     "vaeb_ae_forward": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
     "vaeb_collect": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.c_void_p]),

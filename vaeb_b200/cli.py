@@ -32,7 +32,11 @@ command_line_args = {'seed': (15485863, int),
                      # PGM of 10 x 10 random samples (AEVB Fig. 5); a Bernoulli model shows its decoder means,
                      # since binary draws make a poor image
                      'sample_file': ('', str),
-                     'optimizer': ('adagrad', str)}  # adagrad (VAEB.py:426-444) | adadelta (VAEB.py:449-469) | adam
+                     'optimizer': ('adagrad', str),  # adagrad (VAEB.py:426-444) | adadelta (VAEB.py:449-469) | adam
+                     # weight of the latent term (-KL / log p(z) - log q(z|x)) in the gradient, and the epochs over
+                     # which it ramps up linearly (KL warm-up); 1.0 and 0 train on the reference's bound
+                     'kl_weight': (1.0, float),
+                     'kl_warmup': (0, int)}
 command_line_flags = ['continuous', 'generic_estimator', 'full_varational',
                       # --- extensions ---
                       'synthetic',        # synthetic data of the dataset's shape if the files are absent
@@ -88,6 +92,12 @@ def _default_hidden(continuous, hidden_unit):
     return hidden_unit if hidden_unit >= 0 else (200 if continuous else 500)
 
 
+def kl_warmup_updates(epochs, n_rows, batch_size):
+    """--kl_warmup is given in epochs; the model counts updates, N // batch_size of them per epoch (VAEB.py:571), so
+    the weight grows with every update inside an epoch's update_many."""
+    return int(epochs) * (int(n_rows) // int(batch_size))
+
+
 def train_model(args, data=None):
     """The training driver of VAEB.py:524-598: seed numpy's global RNG (it only drives the shuffle), load the
     dataset of the chosen mode, build the model (on top of --vb_param_file for full VB), then per epoch: shuffle
@@ -114,7 +124,8 @@ def train_model(args, data=None):
     model = VAEB(x_train, continuous, _default_hidden(continuous, args['hidden_unit']), args['n_latent'],
                  args['batch_size'], args['L'], args['learning_rate'], args['generic_estimator'],
                  args['full_varational'], params, sample_weights=args.get('sample_weights', False),
-                 optimizer=args.get('optimizer', 'adagrad'), **ext)
+                 optimizer=args.get('optimizer', 'adagrad'), kl_weight=args.get('kl_weight', 1.0),
+                 kl_warmup=kl_warmup_updates(args.get('kl_warmup', 0), len(x_train), args['batch_size']), **ext)
 
     print("learning")
     tracing = len(trace_file) > 0

@@ -334,7 +334,7 @@ int tc_setup(vaeb_handle* h, const float* x, int rows, int R, TcStep& ts) {
 // Forward (+ backward into `grads`) of the graph of VAEB.getGradient for x[rows,D] on device, one launch per layer: the
 // fp32 kernels, or with tc.active the wide layers (enc1, dec2, dgrad h_d, the W2 and W3 gradients) on tcgen05.
 int forward_backward(vaeb_handle* h, const float* theta, const float* x, int rows, int L, bool want_grads, float w,
-                     EpsSource src, float* grads, const BoundOut& bo) {
+                     float w_aux, EpsSource src, float* grads, const BoundOut& bo) {
   const Layout& l = h->lay;
   Workspace& s = h->ws;
   const int D = h->D, H = h->H, Z = h->Z;
@@ -419,7 +419,7 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
   }
   PH("latent bwd (dz,dmu,dls,da3,bound)", 2 * dR * dZ * dH + 4 * dr * dH * dZ,
      4 * (dR * dH + 3 * dZ * dH + 2 * dr * dH + 3 * dR * dZ + dR * tiles),
-     launch_latent_bwd(st, lc, s.da1, T_(h, theta, l.iW1), h->d_w45t, s.h_e, s.z, s.eps, s.mu, s.ls, rows, H, Z, L, la, w,
+     launch_latent_bwd(st, lc, s.da1, T_(h, theta, l.iW1), h->d_w45t, s.h_e, s.z, s.eps, s.mu, s.ls, rows, H, Z, L, la, w_aux,
                        s.dmu, s.dls, s.da3, tcp ? tb.da3h : nullptr, tcp ? tb.da3l : nullptr, tb.ldh, s.partial, tiles,
                        s.row_aux, s.per_row, h->d_counter, bo.base_out, bo.mult, bo.tprior, bo.n_tprior, bo.div,
                        bo.scalar_out, h->hidden_act));
@@ -455,8 +455,8 @@ int forward_backward(vaeb_handle* h, const float* theta, const float* x, int row
 // and the four weight-gradient GEMMs are one launch after the last dgrad, their split-K slices left in scratch.  With
 // `tail` the update ends in ONE launch that also applies prior + Adagrad or Adam; else the bound and the sum of the slices are
 // launched here and the caller applies the update.
-int large_batch_step(vaeb_handle* h, const float* theta, const float* x, int rows, float w, EpsSource src, float* grads,
-                     const BoundOut& bo, bool tail) {
+int large_batch_step(vaeb_handle* h, const float* theta, const float* x, int rows, float w, float w_aux, EpsSource src,
+                     float* grads, const BoundOut& bo, bool tail) {
   const Layout& l = h->lay;
   Workspace& s = h->ws;
   const int D = h->D, H = h->H, Z = h->Z;
@@ -505,7 +505,7 @@ int large_batch_step(vaeb_handle* h, const float* theta, const float* x, int row
      tc_dgrad_hd(st, lc, t.maps, t.ns, ts.bna, R, h->cont ? 2 * D : D, H, nullptr, nullptr, tb.d1h, tb.d1l, tb.ldh,
                  tb.hdh, tb.hdl));
   PH("dz da1.W1^T + dmu,dls [tcgen05]", 2 * dR * dZ * dH, 2.0 * t.ns * (dR * dH + dZ * dH) + 28 * dR * dZ,
-     tc_dz_dprep(st, lc, t.maps, t.ns, R, H, Z, la, w, s.z, s.eps, s.mu, s.ls, s.dmu, s.dls, tb.ddh, tb.ddl, tb.ldq));
+     tc_dz_dprep(st, lc, t.maps, t.ns, R, H, Z, la, w_aux, s.z, s.eps, s.mu, s.ls, s.dmu, s.dls, tb.ddh, tb.ddl, tb.ldq));
   if (!tail)
     PH("bound (per row + total)", 0, 4 * (dR * tiles + 2 * dr),
        launch_finalize(st, lc, s.partial, tiles, s.row_aux, rows, 1, s.per_row, bo.base_out, bo.mult, bo.tprior,
@@ -594,6 +594,12 @@ int ensure_scalars(vaeb_handle* h, int n) {
   return VAEB_OK;
 }
 
+// beta_n of vaeb_set_kl_weight for the n-th update applied since the call (n >= 1): in double, rounded to float once
+float kl_weight_at(const vaeb_handle* h, int64_t n) {
+  if (h->kl_warmup == 0 || n >= h->kl_warmup) return h->kl_beta;
+  return (float)((double)h->kl_beta * ((double)n / (double)h->kl_warmup));
+}
+
 int stage_in(vaeb_handle* h, float** dbuf, int64_t* cap, const float* host, int64_t n) {
   VAEB_TRY(grow(dbuf, cap, n));
   VAEB_CUDA(cudaMemcpyAsync(*dbuf, host, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, h->stream));
@@ -634,6 +640,8 @@ int enqueue_update(vaeb_handle* h, const float* d_xrows, int rows, const float* 
   if (!is_fvb(h)) {
     const bool fb = h->cfg.variant == VAEB_VARIANT_FULLBAYES;
     const float w = fb ? 1.0f / Mg : 1.0f;
+    // the latent term's weight: beta_n of the update this one would be if applied (h->kl_t advances below)
+    const float w_aux = w * kl_weight_at(h, h->kl_t + 1);
     const bool dp = h->world > 1;
     const float prior = fb ? 0.f : h->cfg.prior_scale;
     // Large-batch tensor-core path: everything after the last GEMM is ONE launch (tc_tail.cu) -- and in data-parallel
@@ -644,8 +652,8 @@ int enqueue_update(vaeb_handle* h, const float* d_xrows, int rows, const float* 
     tail = large && apply && (h->optimizer == VAEB_OPT_ADAGRAD || adam) && env_tail != 0 && (!dp || h->tc.p2p_ready);
     // data parallel without the tail: the optimizer launch writes the scalar, after the all-reduce
     BoundOut bo{base, 1.0f, nullptr, 0, Mg, dp && !tail ? nullptr : h->d_scalars + slot};
-    if (large) VAEB_TRY(large_batch_step(h, h->d_params, d_xrows, rows, w, src, h->d_grads, bo, tail));
-    else VAEB_TRY(forward_backward(h, h->d_params, d_xrows, rows, L, true, w, src, h->d_grads, bo));
+    if (large) VAEB_TRY(large_batch_step(h, h->d_params, d_xrows, rows, w, w_aux, src, h->d_grads, bo, tail));
+    else VAEB_TRY(forward_backward(h, h->d_params, d_xrows, rows, L, true, w, w_aux, src, h->d_grads, bo));
     if (!tail) {                          // (the tail applied prior + Adagrad / Adam)
       VAEB_TRY(all_reduce_grads(h));
       if (apply && adam)
@@ -678,8 +686,8 @@ int enqueue_update(vaeb_handle* h, const float* d_xrows, int rows, const float* 
     VAEB_LAUNCH(launch_theta_prior(st, lc, h->d_vmu, h->d_vsig, l.total, h->d_tprior));
     // SGVB = x.shape[0]*(sum logp + sum KL) + thetaPrior (VAEB.py:364); update returns SGVB/M
     BoundOut bo{base, (float)rows, h->d_tprior, VAEB_TP_BLOCKS, apply ? (float)rows : 1.0f, h->d_scalars + slot};
-    if (large && sampled) VAEB_TRY(large_batch_step(h, theta, d_xrows, rows, (float)rows, src, h->d_grads, bo, false));
-    else VAEB_TRY(forward_backward(h, theta, d_xrows, rows, L, sampled, (float)rows, src, h->d_grads, bo));
+    if (large && sampled) VAEB_TRY(large_batch_step(h, theta, d_xrows, rows, (float)rows, (float)rows, src, h->d_grads, bo, false));
+    else VAEB_TRY(forward_backward(h, theta, d_xrows, rows, L, sampled, (float)rows, (float)rows, src, h->d_grads, bo));
     VAEB_LAUNCH(launch_fvb_adagrad(st, lc, h->d_vmu, h->d_vsig, h->d_ada_mu, h->d_ada_sig, h->d_grads, h->d_zeta,
                                    sampled ? 1 : 0, l.total, h->cfg.learning_rate, h->cfg.adagrad_eps,
                                    h->cfg.prior_scale, h->d_gmu, h->d_gsig, apply ? 1 : 0));
@@ -687,6 +695,7 @@ int enqueue_update(vaeb_handle* h, const float* d_xrows, int rows, const float* 
   if (apply) invalidate_weight_mirrors(h);
   if (tail) h->tc.weights_ready = true;         // the tail wrote the large-batch path's mirrors of the new parameters
   if (apply && adam) ++h->adam_t;
+  if (apply) ++h->kl_t;
   ++h->step;
   return VAEB_OK;
 }
@@ -781,18 +790,37 @@ static int run_single_launch(vaeb_handle* h, StepPath path, const int32_t* host_
     VAEB_CUDA(cudaMemcpyAsync(h->d_order, host_order, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, h->stream));
     d_order = h->d_order;
   }
-  if (path == STEP_TC) return step_tc_launch(h, d_order, d_xrows, rows, n, d_eps, slot0, d_timing);
-  return fused_step_launch(h, d_order, d_xrows, rows, n, d_eps, slot0, d_timing);
+  // the KL weight of every update of the launch (none while it is 1 throughout: the kernels then read no weights)
+  const float* d_kl = nullptr;
+  if (h->kl_beta != 1.f || h->kl_warmup != 0) {
+    if (n > h->kl_cap) {
+      VAEB_CUDA(cudaStreamSynchronize(h->stream));
+      if (h->d_kl) VAEB_CUDA(cudaFree(h->d_kl));
+      h->d_kl = nullptr;
+      VAEB_CUDA(cudaMalloc((void**)&h->d_kl, (size_t)n * sizeof(float)));
+      h->kl_cap = n;
+    }
+    std::vector<float> kl((size_t)n);
+    for (int i = 0; i < n; ++i) kl[(size_t)i] = kl_weight_at(h, h->kl_t + 1 + i);
+    // (pageable source: the call returns once the values are staged, so `kl` may go out of scope)
+    VAEB_CUDA(cudaMemcpyAsync(h->d_kl, kl.data(), (size_t)n * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    d_kl = h->d_kl;
+  }
+  const int rc = path == STEP_TC ? step_tc_launch(h, d_order, d_kl, d_xrows, rows, n, d_eps, slot0, d_timing)
+                                 : fused_step_launch(h, d_order, d_kl, d_xrows, rows, n, d_eps, slot0, d_timing);
+  if (rc == VAEB_OK) h->kl_t += n;
+  return rc;
 }
 
 extern "C" {
 
-// Backup of params + accumulators (Adam: m, v and the Adam step) around the profiling entry points: restored and freed
+// Backup of params + accumulators (Adam: m, v and the Adam step; the KL step) around the profiling entry points: restored and freed
 // on EVERY exit path
 struct StateBackup {
-  vaeb_handle* h; size_t nb, nba; float* bp = nullptr; float* ba = nullptr; uint32_t step0; int64_t launches0, adam_t0;
+  vaeb_handle* h; size_t nb, nba; float* bp = nullptr; float* ba = nullptr; uint32_t step0; int64_t launches0, adam_t0, kl_t0;
   StateBackup(vaeb_handle* hh, size_t n)
-      : h(hh), nb(n), nba(hh->d_adam_v ? 2 * n : n), step0(hh->step), launches0(hh->launches), adam_t0(hh->adam_t) {}
+      : h(hh), nb(n), nba(hh->d_adam_v ? 2 * n : n), step0(hh->step), launches0(hh->launches), adam_t0(hh->adam_t),
+        kl_t0(hh->kl_t) {}
   cudaError_t take() {
     cudaError_t e = cudaMalloc((void**)&bp, nb);
     if (e == cudaSuccess) e = cudaMalloc((void**)&ba, nba);
@@ -805,6 +833,7 @@ struct StateBackup {
     h->step = step0;
     h->launches = launches0;
     h->adam_t = adam_t0;
+    h->kl_t = kl_t0;
     if (bp && ba) {
       cudaMemcpyAsync(h->d_params, bp, nb, cudaMemcpyDeviceToDevice, h->stream);
       cudaMemcpyAsync(h->d_ada, ba, nba, cudaMemcpyDeviceToDevice, h->stream);
@@ -819,7 +848,7 @@ static int async_flush(vaeb_handle* h);
 static void p2p_release(vaeb_handle* h);   // unmaps the peers' buffers (data parallel over peer memory)   // launches streaming updates that were copied but not yet started
 
 const char* vaeb_last_error(void) { return g_last_error.c_str(); }
-int vaeb_version(void) { return 103; }   // 103: Adam; 102: vaeb_encode, vaeb_sample, vaeb_validate_terms (101: encoder_hidden_layers)
+int vaeb_version(void) { return 104; }   // 104: KL weight; 103: Adam; 102: vaeb_encode, vaeb_sample, vaeb_validate_terms (101: encoder_hidden_layers)
 int vaeb_config_size(void) { return (int)sizeof(vaeb_config); }
 
 int vaeb_create(const vaeb_config* cfg, vaeb_handle** out) {
@@ -891,6 +920,7 @@ int vaeb_destroy(vaeb_handle* h) {
                    h->d_scalars, h->d_ada2};
   for (float* p : bufs) if (p) cudaFree(p);
   if (h->d_order) cudaFree(h->d_order);
+  if (h->d_kl) cudaFree(h->d_kl);
   if (h->d_counter) cudaFree(h->d_counter);
   if (h->d_w45t) cudaFree(h->d_w45t);
   step_tc_free(h->steptc);
@@ -1228,6 +1258,32 @@ int vaeb_set_adam_step(vaeb_handle* h, int64_t t) {
   return VAEB_OK;
 }
 
+int vaeb_set_kl_weight(vaeb_handle* h, float beta, int64_t warmup_updates) {
+  if (h && h->a_pending) VAEB_TRY(async_flush(h));      // updates enqueued before the call keep the old weights
+  VAEB_REQUIRE(h, "null handle");
+  VAEB_REQUIRE(std::isfinite(beta) && beta >= 0.f, "the KL weight must be finite and non-negative");
+  VAEB_REQUIRE(warmup_updates >= 0, "the KL warm-up must be non-negative");
+  VAEB_REQUIRE(!is_fvb(h), "the KL weight is not wired to the full-VB estimators");
+  h->kl_beta = beta;
+  h->kl_warmup = warmup_updates;
+  h->kl_t = 0;
+  return VAEB_OK;
+}
+
+int vaeb_kl_step(vaeb_handle* h, int64_t* t) {
+  if (h && h->a_pending) VAEB_TRY(async_flush(h));       // the copied-but-unlaunched updates count
+  VAEB_REQUIRE(h && t, "null argument");
+  *t = h->kl_t;
+  return VAEB_OK;
+}
+
+int vaeb_set_kl_step(vaeb_handle* h, int64_t t) {
+  if (h && h->a_pending) VAEB_TRY(async_flush(h));
+  VAEB_REQUIRE(h && t >= 0, "the KL step must be non-negative");
+  h->kl_t = t;
+  return VAEB_OK;
+}
+
 // Launches the minibatches copied into the current group buffer: ONE launch of a single-launch step kernel for up to
 // ASYNC_GROUP updates (per-layer kernels otherwise), then the readback of their bounds.
 static int async_flush(vaeb_handle* h) {
@@ -1463,7 +1519,7 @@ static int validate_rows(vaeb_handle* h, const float* x, int64_t n, const float*
     bo.loglik_rows = h->d_out;
     bo.aux_rows = h->d_out + n;
   }
-  VAEB_TRY(forward_backward(h, theta, h->d_stage, (int)n, L, false, 1.f, src, nullptr, bo));
+  VAEB_TRY(forward_backward(h, theta, h->d_stage, (int)n, L, false, 1.f, 1.f, src, nullptr, bo));
   ++h->step;
   VAEB_TRY(read_scalars(h, 1, sgvb_out));
   if (per_row_out)

@@ -141,6 +141,11 @@ struct vaeb_handle {
   // adam_t = updates applied since Adam was selected; alpha_t / s2_t of the update being enqueued
   float adam_b1 = 0.9f, adam_b2 = 0.999f, adam_eps = 1e-8f; float* d_adam_v = nullptr; int64_t adam_t = 0;
   float adam_alpha_t = 0.f, adam_s2_t = 0.f;
+  // KL weight (vaeb_set_kl_weight): the n-th update applied since the call, n = kl_t + 1, ascends
+  // loglik + beta_n aux with beta_n = kl_beta * min(1, n / kl_warmup); d_kl holds beta_n of each update of one
+  // single-launch call (grown as d_order)
+  float kl_beta = 1.f; int64_t kl_warmup = 0, kl_t = 0;
+  float* d_kl = nullptr; int kl_cap = 0;
   float* d_stage = nullptr; int64_t stage_cap = 0;       // device staging for host inputs
   // streaming host-input updates (vaeb_update_host_async): copy stream + ring of staging buffers
   static constexpr int ASYNC_BUFS = 4;

@@ -691,7 +691,7 @@ __device__ __forceinline__ void update_phases(const StepParams& p, float* smem, 
       const Gemm g6 = make_gemm(p.h_d, nullptr, H, p.dlv, nullptr, D, H + 1, D, M, 0, H, p.job[J_WG6]);
       const EpiAdagrad<FVB> e6{Pu, Pn, p.ada, p.oW6, p.ob6, H, D, hy, fv};
       const Gemm gz = make_gemm(p.da1, nullptr, H, P + p.oW1, nullptr, H, M, Z, H, 0, -1, p.job[J_DZ]);
-      const EpiDz ez{p.z, p.eps, p.mu, p.ls, Z, p.la, p.w, p.dmu, p.dls};
+      const EpiDz ez{p.z, p.eps, p.mu, p.ls, Z, p.la, p.kl_beta ? p.w * __ldg(p.kl_beta + s) : p.w, p.dmu, p.dls};
       const Gemm g1 = make_gemm(p.z, nullptr, Z, p.da1, nullptr, H, Z + 1, H, M, 0, Z, p.job[J_WG1]);
       const EpiAdagrad<FVB> e1{Pu, Pn, p.ada, p.oW1, p.ob1, Z, H, hy, fv};
       const int n2 = g2.c.n_items, n6 = p.cont ? g6.c.n_items : 0, nz = gz.c.n_items, n1 = g1.c.n_items;
@@ -906,7 +906,7 @@ static JobCfg plan_job(int job, int M, int N, int K, int n_cta, bool dual_n) {
 
 }  // namespace fs
 
-int fused_step_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, int rows, int n_steps,
+int fused_step_launch(vaeb_handle* h, const int* d_order, const float* d_kl, const float* d_xrows, int rows, int n_steps,
                       const float* d_eps, int slot0, long long* d_timing) {
   using namespace fs;
   FusedState& f = h->fused;
@@ -961,6 +961,7 @@ int fused_step_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, 
   p.la = h->cfg.estimator == VAEB_EST_LA ? 1 : 0;
   const bool fb = h->cfg.variant == VAEB_VARIANT_FULLBAYES;
   p.w = fb ? 1.0f / (float)rows : 1.0f;
+  p.kl_beta = d_kl;
   p.lr = h->cfg.learning_rate; p.ada_eps = h->cfg.adagrad_eps;
   p.prior = fb ? 0.f : h->cfg.prior_scale;
   p.p2 = fb ? h->cfg.learning_rate * 1e-6f : 0.f;

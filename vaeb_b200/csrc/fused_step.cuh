@@ -54,6 +54,7 @@ struct StepParams {
   int D, H, Z, M;                 // M = rows of the minibatch (L == 1)
   int cont, la;
   float w;                        // weight of the data term in the criterion (1, or 1/M: VAEBfullbayes)
+  const float* kl_beta;           // device [n_steps]: weight of the latent term of each update (nullptr: 1)
   float lr, ada_eps, prior, p2;
   float* params[2];               // ping-pong flat parameter buffers (reference tensor order)
   float* ada;
@@ -89,5 +90,6 @@ struct vaeb_handle;
 bool fused_step_supported(const vaeb_handle* h, int rows);
 // n_steps updates in one launch.  Rows of step s: minibatch d_order[s] (of `rows` rows) of the resident data -- or of
 // d_xrows when both are given (the staging ring of the streaming host-input updates) -- else d_xrows itself every step.
-int fused_step_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, int rows, int n_steps,
+// d_kl: nullptr, or device [n_steps] with the KL weight beta_n of each step (vaeb_set_kl_weight).
+int fused_step_launch(vaeb_handle* h, const int* d_order, const float* d_kl, const float* d_xrows, int rows, int n_steps,
                       const float* d_eps, int slot0, long long* d_timing);

@@ -185,7 +185,7 @@ __global__ void __launch_bounds__(NTHREADS)
 latent_bwd_kernel(const float* __restrict__ da1, const float* __restrict__ W1, const float* __restrict__ w45t,
                   const float* __restrict__ h_e, const float* __restrict__ z, const float* __restrict__ eps,
                   const float* __restrict__ mu, const float* __restrict__ ls, int rows, int H, int Z, int L, int la,
-                  float w, float* __restrict__ dmu, float* __restrict__ dls, float* __restrict__ da3,
+                  float w_aux, float* __restrict__ dmu, float* __restrict__ dls, float* __restrict__ da3,
                   __nv_bfloat16* __restrict__ da3_hi, __nv_bfloat16* __restrict__ da3_lo, int ld_mirror,
                   const float* __restrict__ partial, int n_tiles, const float* __restrict__ row_aux,
                   float* __restrict__ per_row, unsigned int* __restrict__ counter, float* __restrict__ base_out,
@@ -199,7 +199,7 @@ latent_bwd_kernel(const float* __restrict__ da1, const float* __restrict__ W1, c
   float* dl = dm + RB * Z;             // [RB][Z] dls
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int m0 = blockIdx.x * RB;
-  const float s = w / (float)L;
+  const float s = w_aux / (float)L;
   const int nchunks = (Z + 7) / 8;
   for (int i = threadIdx.x; i < RB * Z; i += NTHREADS) { dm[i] = 0.f; dl[i] = 0.f; }
   for (int l = 0; l < L; ++l) {
@@ -253,10 +253,10 @@ latent_bwd_kernel(const float* __restrict__ da1, const float* __restrict__ W1, c
       const float lsv = ls[(size_t)m * Z + j], muv = mu[(size_t)m * Z + j];
       float a = dm[i], b = dl[i];
       if (la) {
-        b += w * 0.5f;
+        b += w_aux * 0.5f;
       } else {
-        a -= w * muv;
-        b += w * 0.5f * (1.0f - expf(lsv));
+        a -= w_aux * muv;
+        b += w_aux * 0.5f * (1.0f - expf(lsv));
       }
       dm[i] = a;
       dl[i] = b;
@@ -543,7 +543,7 @@ __global__ void __launch_bounds__(LB_T)
 lb_latent_bwd_kernel(const float* __restrict__ da1, const float* __restrict__ W1, const float* __restrict__ w45t,
                      const float* __restrict__ h_e, const float* __restrict__ z, const float* __restrict__ eps,
                      const float* __restrict__ mu, const float* __restrict__ ls, int rows, int H, int Z, int la,
-                     float w, float* __restrict__ dmu, float* __restrict__ dls, float* __restrict__ da3,
+                     float w_aux, float* __restrict__ dmu, float* __restrict__ dls, float* __restrict__ da3,
                      const float* __restrict__ partial, int n_tiles, const float* __restrict__ row_aux,
                      float* __restrict__ per_row, unsigned int* __restrict__ counter, float* __restrict__ base_out,
                      float mult, const float* __restrict__ tprior, int n_tprior, float div,
@@ -602,13 +602,13 @@ lb_latent_bwd_kernel(const float* __restrict__ da1, const float* __restrict__ W1
       const size_t o2 = (size_t)m * Z + j;
       const float lsv = ls[o2], muv = mu[o2];
       float d = psum[0][rr][j] + psum[1][rr][j];
-      if (la) d -= w * z[o2];
+      if (la) d -= w_aux * z[o2];
       float a = d, b = d * (0.5f * expf(0.5f * lsv) * eps[o2]);
       if (la) {
-        b += w * 0.5f;
+        b += w_aux * 0.5f;
       } else {
-        a -= w * muv;
-        b += w * 0.5f * (1.0f - expf(lsv));
+        a -= w_aux * muv;
+        b += w_aux * 0.5f * (1.0f - expf(lsv));
       }
       dmu[o2] = a; dls[o2] = b;
       dd[rr][j] = a; dd[rr][Z + j] = b;
@@ -784,7 +784,7 @@ cudaError_t launch_latent_fwd(cudaStream_t st, int64_t* launches, const float* h
 
 cudaError_t launch_latent_bwd(cudaStream_t st, int64_t* launches, const float* da1, const float* W1,
                               const float* w45t, const float* h_e, const float* z, const float* eps, const float* mu,
-                              const float* ls, int rows, int H, int Z, int L, int la, float w, float* dmu, float* dls,
+                              const float* ls, int rows, int H, int Z, int L, int la, float w_aux, float* dmu, float* dls,
                               float* da3, void* da3_hi, void* da3_lo, int ld_mirror, const float* partial,
                               int n_tiles, const float* row_aux, float* per_row, unsigned int* counter,
                               float* base_out, float mult, const float* tprior, int n_tprior, float div,
@@ -794,19 +794,19 @@ cudaError_t launch_latent_bwd(cudaStream_t st, int64_t* launches, const float* d
   ++*launches;
   if (latent_lb_supported(rows, H, Z, L)) {
     lb_latent_bwd_kernel<<<(rows + LB_ROWS - 1) / LB_ROWS, LB_T, 0, st>>>(
-        da1, W1, w45t, h_e, z, eps, mu, ls, rows, H, Z, la, w, dmu, dls, da3, partial, n_tiles, row_aux, per_row,
+        da1, W1, w45t, h_e, z, eps, mu, ls, rows, H, Z, la, w_aux, dmu, dls, da3, partial, n_tiles, row_aux, per_row,
         counter, base_out, mult, tprior, n_tprior, div, scalar_out, act);
   } else if (rows <= 512) {
     const size_t smem = (size_t)(NSL + 2) * Z * sizeof(float);
     latent_bwd_kernel<1><<<rows, NTHREADS, smem, st>>>(
-        da1, W1, w45t, h_e, z, eps, mu, ls, rows, H, Z, L, la, w, dmu, dls, da3, (__nv_bfloat16*)da3_hi,
+        da1, W1, w45t, h_e, z, eps, mu, ls, rows, H, Z, L, la, w_aux, dmu, dls, da3, (__nv_bfloat16*)da3_hi,
         (__nv_bfloat16*)da3_lo, ld_mirror, partial, n_tiles, row_aux, per_row, counter, base_out, mult, tprior,
         n_tprior, div, scalar_out, NSL, act);
   } else {
     constexpr int RB = 8;
     const size_t smem = (size_t)RB * (NSL + 2) * Z * sizeof(float);
     latent_bwd_kernel<RB><<<(rows + RB - 1) / RB, NTHREADS, smem, st>>>(
-        da1, W1, w45t, h_e, z, eps, mu, ls, rows, H, Z, L, la, w, dmu, dls, da3, (__nv_bfloat16*)da3_hi,
+        da1, W1, w45t, h_e, z, eps, mu, ls, rows, H, Z, L, la, w_aux, dmu, dls, da3, (__nv_bfloat16*)da3_hi,
         (__nv_bfloat16*)da3_lo, ld_mirror, partial, n_tiles, row_aux, per_row, counter, base_out, mult, tprior,
         n_tprior, div, scalar_out, NSL, act);
   }

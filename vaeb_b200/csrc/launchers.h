@@ -124,10 +124,11 @@ cudaError_t launch_latent_fwd(cudaStream_t st, int64_t* launches, const float* h
 bool latent_large_batch(int rows, int H, int Z, int L);
 // dz, dmu/dls, da3 and the bound (per row + deterministic total by the last block to finish).
 // da3_hi/da3_lo: optional bf16 mirrors of da3, written only below latent_large_batch (the tensor-core path of the
-// large-batch shapes computes da3 on tcgen05).
+// large-batch shapes computes da3 on tcgen05).  w_aux: weight of the latent term's gradient (the data weight times the
+// KL weight of vaeb_set_kl_weight); the data term arrives in da1 already weighted.
 cudaError_t launch_latent_bwd(cudaStream_t st, int64_t* launches, const float* da1, const float* W1,
                               const float* w45t, const float* h_e, const float* z, const float* eps, const float* mu,
-                              const float* ls, int rows, int H, int Z, int L, int la, float w, float* dmu, float* dls,
+                              const float* ls, int rows, int H, int Z, int L, int la, float w_aux, float* dmu, float* dls,
                               float* da3, void* da3_hi, void* da3_lo, int ld_mirror, const float* partial,
                               int n_tiles, const float* row_aux, float* per_row, unsigned int* counter,
                               float* base_out, float mult, const float* tprior, int n_tprior, float div,

@@ -787,8 +787,9 @@ __device__ __forceinline__ void item_dgrad(Ctx& c, const Params& p, int t, bool 
   ST2_TRACE(c, 45);
 }
 
-// P5: dz = da1.W1^T -> dmu, dls (SURVEY.md 8a backward formulas)
-__device__ __forceinline__ void item_dz(Ctx& c, const Params& p, bool more) {
+// P5: dz = da1.W1^T -> dmu, dls (SURVEY.md 8a backward formulas).  kb = the step's KL weight: its three terms carry it,
+// and the weight-gradient epilogues scale the whole gradient by w, so the update ascends w (grad loglik + kb grad aux)
+__device__ __forceinline__ void item_dz(Ctx& c, const Params& p, bool more, float kb) {
   ST2_TRACE(c, 50);
   const int c0 = c.rank * p.KH / CL, c1 = (c.rank + 1) * p.KH / CL, nch = c1 - c0;
   const int TB = p.NZ * 128, Z = p.Z, N = p.NZ;
@@ -824,13 +825,13 @@ __device__ __forceinline__ void item_dz(Ctx& c, const Params& p, bool more) {
     const int gr = c.rank * 32 + row;
     if (gr < p.M) {
       float d = recv_sum(recv, N, row, j) * WUNSCALE;
-      if (p.la) d -= zm_[i];
+      if (p.la) d -= kb * zm_[i];
       float a = d, b = d * (0.5f * expf(0.5f * ls_[i]) * ev_[i]);
       if (p.la) {
-        b += 0.5f;
+        b += kb * 0.5f;
       } else {
-        a -= zm_[i];
-        b += 0.5f * (1.0f - expf(ls_[i]));
+        a -= kb * zm_[i];
+        b += kb * 0.5f * (1.0f - expf(ls_[i]));
       }
       put_dl(km_addr(p.dd_km, gr, j), TBA, a);                                   // A operand of the dh_e GEMMs (P6)
       put_dl(km_addr(p.dd_km, gr, Z + j), TBA, b);
@@ -1495,7 +1496,7 @@ __global__ void __launch_bounds__(NT, 1) step_tc_kernel(const __grid_constant__ 
       const int n2 = m_h1 * n3 * nw;
       const int g2 = n_groups(n2 + 1);
       for (int it = c.cid; it < 1 + g2; it += c.ncl) {
-        if (it == 0) { item_dz(c, p, false); continue; }
+        if (it == 0) { item_dz(c, p, false, p.kl_beta ? __ldg(p.kl_beta + s) : 1.f); continue; }
         const int i = (it - 1) * CL + c.rank;
         if (i < n2) item_wg2<SV>(c, p, hy, i / (n3 * nw), (i / nw) % n3, i % nw);
         else if (i == n2 && !SV) item_bound(c, p, s);
@@ -1699,8 +1700,8 @@ static int step_tc_init(vaeb_handle* h) {
   return VAEB_OK;
 }
 
-int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, int rows, int n_steps, const float* d_eps,
-                   int slot0, long long* d_timing) {
+int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_kl, const float* d_xrows, int rows, int n_steps,
+                   const float* d_eps, int slot0, long long* d_timing) {
   using namespace st2;
   StepTcState& s = h->steptc;
   const Layout& l = h->lay;
@@ -1719,6 +1720,7 @@ int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, int
   p.la = h->cfg.estimator == VAEB_EST_LA ? 1 : 0;
   const bool fb = h->cfg.variant == VAEB_VARIANT_FULLBAYES;
   p.w = fb ? 1.0f / (float)rows : 1.0f;
+  p.kl_beta = d_kl;
   p.lr = h->cfg.learning_rate; p.ada_eps = h->cfg.adagrad_eps;
   p.prior = fb ? 0.f : h->cfg.prior_scale;
   p.p2 = fb ? h->cfg.learning_rate * 1e-6f : 0.f;
@@ -1813,7 +1815,7 @@ int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, int
   if (done < n_steps) {
     // steps done .. n_steps-1 through the fp32 FFMA kernel (same contract; it invalidates the operand mirrors)
     VAEB_REQUIRE(fused_step_supported(h, rows), "step_tc: delta overflow and no fp32 single-launch kernel for this configuration");
-    return fused_step_launch(h, d_order ? d_order + done : nullptr, d_xrows, rows, n_steps - done, d_eps, slot0 + done, nullptr);
+    return fused_step_launch(h, d_order ? d_order + done : nullptr, d_kl ? d_kl + done : nullptr, d_xrows, rows, n_steps - done, d_eps, slot0 + done, nullptr);
   }
   return VAEB_OK;
 }

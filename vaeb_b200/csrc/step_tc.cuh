@@ -36,6 +36,7 @@ struct Params {
   int TR3;                              // rows of a dec2 B tile (UMMA N of the output layer): 32, or 64 (Gaussian)
   int KV;                               // 64-wide k chunks over the virtual output columns (Bernoulli: KD)
   float w, lr, ada_eps, prior, p2;
+  const float* kl_beta;                 // device [n_steps]: weight of the latent term of each update (nullptr: 1)
   float* P;                             // flat fp32 parameters (reference tensor order), updated in place
   float* ada;
   int64_t oW3, oW4, oW5, oW1, oW2, ob3, ob4, ob5, ob1, ob2, oW6, ob6;
@@ -105,6 +106,6 @@ struct StepTcState {
 };
 
 // n_steps updates in one launch (same contract as fused_step_launch)
-int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_xrows, int rows, int n_steps, const float* d_eps,
-                   int slot0, long long* d_timing);
+int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_kl, const float* d_xrows, int rows, int n_steps,
+                   const float* d_eps, int slot0, long long* d_timing);
 void step_tc_free(StepTcState& s);

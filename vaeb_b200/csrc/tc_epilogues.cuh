@@ -436,10 +436,11 @@ struct EpiHeads {
   }
 };
 
-// dz = da1.W1^T -> dmu, dls (L = 1; formulas of SURVEY.md 8a, as launch_dprep / lb_latent_bwd) + bf16 mirror [dmu|dls]
+// dz = da1.W1^T -> dmu, dls (L = 1; formulas of SURVEY.md 8a, as launch_dprep / lb_latent_bwd) + bf16 mirror [dmu|dls];
+// w_aux weights the latent term (the data weight times the KL weight of vaeb_set_kl_weight)
 struct EpiDzPrep {
   static constexpr bool PREFETCH = false;   // persistent kernel: unrolled epilogue with the next chunk's operand in flight
-  const float* z; const float* eps; const float* mu; const float* ls; int Z; int la; float w;
+  const float* z; const float* eps; const float* mu; const float* ls; int Z; int la; float w_aux;
   float* dmu; float* dls; __nv_bfloat16* dd_hi; __nv_bfloat16* dd_lo; int ldq;
   __device__ __forceinline__ void begin() {}
   __device__ __forceinline__ void split(int) {}
@@ -473,13 +474,13 @@ struct EpiDzPrep {
 #pragma unroll
       for (int q = 0; q < 4; ++q) {
         float d = v[4 * g + q];
-        if (la) d -= w * zv[q];
+        if (la) d -= w_aux * zv[q];
         a[q] = d; b[q] = d * (0.5f * expf(0.5f * lsv[q]) * ev[q]);
         if (la) {
-          b[q] += w * 0.5f;
+          b[q] += w_aux * 0.5f;
         } else {
-          a[q] -= w * mv[q];
-          b[q] += w * 0.5f * (1.0f - expf(lsv[q]));
+          a[q] -= w_aux * mv[q];
+          b[q] += w_aux * 0.5f * (1.0f - expf(lsv[q]));
         }
       }
       if (vec) {

@@ -892,10 +892,10 @@ cudaError_t tc_dec1(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns,
   return dispatch_layer<false, true>(st, ns, bn, *reinterpret_cast<const LayerMaps*>(m.dec1), epi, R, H, Z, 0);
 }
 
-cudaError_t tc_dz_dprep(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int R, int H, int Z, int la, float w,
+cudaError_t tc_dz_dprep(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int R, int H, int Z, int la, float w_aux,
                         const float* z, const float* eps, const float* mu, const float* ls, float* dmu, float* dls,
                         void* dd_hi, void* dd_lo, int ldq) {
-  EpiDzPrep epi{z, eps, mu, ls, Z, la, w, dmu, dls, (__nv_bfloat16*)dd_hi, (__nv_bfloat16*)dd_lo, ldq};
+  EpiDzPrep epi{z, eps, mu, ls, Z, la, w_aux, dmu, dls, (__nv_bfloat16*)dd_hi, (__nv_bfloat16*)dd_lo, ldq};
   ++*launches;
   return dispatch_layer<false, false>(st, ns, 64, *reinterpret_cast<const LayerMaps*>(m.dz), epi, R, Z, H, 0);
 }

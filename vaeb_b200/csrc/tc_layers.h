@@ -91,8 +91,9 @@ cudaError_t tc_enc2_heads(cudaStream_t st, int64_t* launches, const TcMaps& m, i
 // h_d = tanh(z.W1 + b1) with its bf16 mirror (VAEB.py:254)
 cudaError_t tc_dec1(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int bn, int R, int Z, int H,
                     const float* b1, float* h_d, void* hd_hi, void* hd_lo, int ldm);
-// dz = da1.W1^T fused with the encoder-side gradient assembly (SURVEY.md 8a: dmu, dls) and the [dmu|dls] mirror
-cudaError_t tc_dz_dprep(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int R, int H, int Z, int la, float w,
+// dz = da1.W1^T fused with the encoder-side gradient assembly (SURVEY.md 8a: dmu, dls) and the [dmu|dls] mirror;
+// w_aux weights the latent term's gradient
+cudaError_t tc_dz_dprep(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int R, int H, int Z, int la, float w_aux,
                         const float* z, const float* eps, const float* mu, const float* ls, float* dmu, float* dls,
                         void* dd_hi, void* dd_lo, int ldq);
 cudaError_t tc_dgrad_he(cudaStream_t st, int64_t* launches, const TcMaps& m, int ns, int bn, int rows, int Z, int H,

@@ -22,10 +22,15 @@ def broadcast_bytes(payload, src=0):
 
 def attach_data_parallel(model):
     """Give `model` (one per rank, built on this rank's GPU with batch_size = per-rank share)
-    an NCCL communicator: afterwards every update all-reduces gradients and the bound."""
+    an NCCL communicator: afterwards every update all-reduces gradients and the bound.  The ranks must weight the
+    latent term alike (set_kl_weight, kl_step)."""
     import torch.distributed as dist
     from .model import comm_unique_id
     rank, world = dist.get_rank(), dist.get_world_size()
+    if world > 1:
+        schedules = [None] * world
+        dist.all_gather_object(schedules, (model.kl_weight, model.kl_warmup, model.kl_step))
+        check_same_kl_weight(schedules)
     uid = comm_unique_id() if rank == 0 else None
     uid = broadcast_bytes(uid, 0)
     model.attach_comm(uid, rank, world)
@@ -49,6 +54,13 @@ def check_same_optimizer(optimizers):
     whose allocation has no room for v (another rule) would be written past its end, so a mix is refused up front."""
     if len(set(optimizers)) > 1:
         raise ValueError("data parallel over peer memory needs the same optimizer on every rank, got %s" % (optimizers,))
+
+
+def check_same_kl_weight(schedules):
+    """`schedules`: every rank's (KL weight, warm-up, KL step), in rank order.  The summed gradient is the gradient of
+    one objective only when every rank weights the latent term alike, so a mix is refused."""
+    if len(set(schedules)) > 1:
+        raise ValueError("data parallel needs the same KL weight, warm-up and KL step on every rank, got %s" % (schedules,))
 
 
 def close_data_parallel(model):

@@ -79,10 +79,14 @@ class VAEB(object):
     #                  reference's list, weights first; fp32 per-layer kernels, L^A / L^B estimators
     #   activation     'tanh' (the reference's hidden layers, VAEB.py:246,254) | 'sigmoid' | 'relu' (the alternatives of
     #                  Report/replication/replic.tex:73-82; fp32 per-layer kernels, L^A / L^B estimators)
+    #   kl_weight      beta: weight of the latent term (-KL for L^B, log p(z) - log q(z|x) for L^A) in the gradient
+    #   kl_warmup      updates over which that weight ramps linearly from beta/kl_warmup to beta (0: constant beta);
+    #                  see set_kl_weight.  The defaults (1.0, 0) train on the reference's bound
     def __init__(self, x_train, continuous, hidden_units, latent_size, batch_size,
                  L, learning_rate, genericEstimator, fullVariational, params=None, prng=None, sigmaInit=None,
                  *, device=0, precision="fp32", eps_mode="philox", sample_weights=False, variant="vaeb", seed=10,
-                 optimizer="adagrad", activation="tanh", encoder_layers=1, adam_betas=(0.9, 0.999), adam_eps=1e-8):
+                 optimizer="adagrad", activation="tanh", encoder_layers=1, adam_betas=(0.9, 0.999), adam_eps=1e-8,
+                 kl_weight=1.0, kl_warmup=0):
         x_train = np.asarray(x_train)
         [self.N, self.input_size] = x_train.shape       # VAEB.py:135
         self.n_hidden_units = hidden_units
@@ -179,6 +183,9 @@ class VAEB(object):
         self.activation = activation
         if activation != "tanh":
             _lib.check(self._lib.vaeb_set_hidden_activation(self._h, {"sigmoid": 2, "relu": 3}[activation]))
+        self.kl_weight, self.kl_warmup = 1.0, 0
+        if kl_weight != 1.0 or kl_warmup != 0:
+            self.set_kl_weight(kl_weight, kl_warmup)
         _lib.check(self._lib.vaeb_upload_data(self._h, _ptr(_f32(x_train)), self.N))   # VAEB.py:184
 
     # ---- parameters -------------------------------------------------------------------
@@ -437,6 +444,25 @@ class VAEB(object):
     def adam_step(self, t):
         _lib.check(self._lib.vaeb_set_adam_step(self._h, int(t)))
 
+    def set_kl_weight(self, beta, warmup=0):
+        """Weight the latent term of the bound in the gradient: the n-th update applied after this call ascends
+        loglik + beta_n * aux with beta_n = kl_weight_at(beta, warmup, n) -- a linear KL warm-up over `warmup` updates,
+        or beta-VAE's constant beta when warmup = 0.  Resets kl_step to 0.  The bounds update() and friends return stay
+        the unweighted SGVB / batch_size.  Not available for the full-VB estimators."""
+        _lib.check(self._lib.vaeb_set_kl_weight(self._h, float(beta), int(warmup)))
+        self.kl_weight, self.kl_warmup = float(beta), int(warmup)
+
+    @property
+    def kl_step(self):
+        """Updates applied since set_kl_weight (the position in the warm-up): save and restore it to resume a run."""
+        t = C.c_int64()
+        _lib.check(self._lib.vaeb_kl_step(self._h, C.byref(t)))
+        return t.value
+
+    @kl_step.setter
+    def kl_step(self, t):
+        _lib.check(self._lib.vaeb_set_kl_step(self._h, int(t)))
+
     def profile_optimizer(self, iters=20, variant=0):
         """(ms per launch, algorithmic bytes per launch) of the flat Adagrad pass over this model's buffers."""
         ms, by = C.c_float(), C.c_double()
@@ -511,6 +537,15 @@ def pinned_empty(shape, dtype=np.float32):
     blk.buf = None
     buf._owner = blk      # arr.base chain -> buf -> blk: the block is freed when the last view of it goes away
     return np.frombuffer(buf, dtype=dt, count=int(np.prod(shape))).reshape(shape)
+
+
+def kl_weight_at(beta, warmup, n):
+    """beta_n of set_kl_weight(beta, warmup) for the n-th update applied after the call (n >= 1), as the library
+    computes it: beta * min(1, n / warmup) in double from the float32 beta, rounded to float32 once."""
+    beta = float(np.float32(beta))
+    if warmup == 0 or n >= warmup:
+        return np.float32(beta)
+    return np.float32(beta * (float(n) / float(warmup)))
 
 
 def comm_unique_id(nccl_library=None):
