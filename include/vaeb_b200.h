@@ -87,7 +87,8 @@ typedef struct vaeb_config {
 #define VAEB_ACT_RELU 3
 
 const char* vaeb_last_error(void);
-int vaeb_version(void);      /* 104: adds the KL weight (vaeb_set_kl_weight, vaeb_kl_step, vaeb_set_kl_step; vaeb_config
+int vaeb_version(void);      /* 105: vaeb_profile_optimizer loses its variant argument (vaeb_config unchanged);
+                                104: adds the KL weight (vaeb_set_kl_weight, vaeb_kl_step, vaeb_set_kl_step; vaeb_config
                                 unchanged);
                                 103: adds Adam (vaeb_set_adam, vaeb_adam_step, vaeb_set_adam_step; vaeb_config unchanged);
                                 102: adds the encode, sample and validate_terms entry points (vaeb_config unchanged);
@@ -331,11 +332,9 @@ int vaeb_profile_update(vaeb_handle* h, int64_t index, int32_t iters, int32_t ma
 
 /* Measurement aid for bench.py: the flat Adagrad pass of getUpdates (VAEB.py:426-444) over this handle's parameter,
  * accumulator and gradient buffers, `iters` launches back to back between two CUDA events on the handle's stream.
- * bytes_per_launch = 20 B x the number of parameters (SURVEY.md 8d).  variant: 0 / 1 = the production kernel,
- * 2 = with streaming cache hints, 4 = also two float4 per thread (measured alternatives).  A handle with a large hidden layer gives the stream-sized buffer the HBM roofline needs;
- * parameters and accumulators are restored afterwards. */
-int vaeb_profile_optimizer(vaeb_handle* h, int32_t iters, int32_t variant, float* ms_per_launch,
-                           double* bytes_per_launch);
+ * bytes_per_launch = 20 B x the number of parameters (SURVEY.md 8d).  A handle with a large hidden layer gives the
+ * stream-sized buffer the HBM roofline needs; parameters and accumulators are restored afterwards. */
+int vaeb_profile_optimizer(vaeb_handle* h, int32_t iters, float* ms_per_launch, double* bytes_per_launch);
 
 /* Self-test of the tcgen05/TMA GEMM building block: C[M,N] = bf16(A[M,K]) . bf16(B[K,N]) with fp32
  * TMEM accumulation.  a_mn_major / b_mn_major choose the memory layout handed to TMA (0: the

@@ -83,7 +83,7 @@ EXPORTS = {
     "vaeb_comm_p2p_attach": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32]),
     "vaeb_profile_update": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.c_void_p,
                                       C.c_void_p, C.c_void_p, C.c_void_p]),
-    "vaeb_profile_optimizer": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_double)]),
+    "vaeb_profile_optimizer": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_double)]),
     "vaeb_tc_gemm_test": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                     C.c_void_p, C.c_void_p, C.c_void_p]),
     "vaeb_launch_count": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),

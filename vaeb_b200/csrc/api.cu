@@ -37,7 +37,6 @@ struct PhaseProf {
   std::vector<double> flops, bytes;
 };
 static thread_local PhaseProf* g_prof = nullptr;
-static long long* g_tail_stamps = nullptr;   // debug (VAEB_TAIL_STAMPS)
 
 #define PH(NAME, FLOPS, BYTES, EXPR)                                                   \
   do {                                                                                 \
@@ -560,15 +559,7 @@ int large_batch_step(vaeb_handle* h, const float* theta, const float* x, int row
     if (adam) ta.peer_v[r] = t.p2p_ada[r] + (l.padded + 4);      // every rank keeps v right after m (vaeb_set_adam)
   }
   const int grid = tc_tail_grid(t.n_sm, adam);
-  static const char* stamp_path = getenv("VAEB_TAIL_STAMPS");      // debug: time stamps of the last 2048 tail launches
-  static long long* d_stamps = nullptr;
-  if (stamp_path && !d_stamps) {
-    VAEB_CUDA(cudaMalloc((void**)&d_stamps, 2048 * 8 * sizeof(long long)));
-    VAEB_CUDA(cudaMemset(d_stamps, 0, 2048 * 8 * sizeof(long long)));
-    g_tail_stamps = d_stamps;
-  }
   auto launch_tail = [&]() -> cudaError_t {
-    ta.stamps = d_stamps ? d_stamps + 8 * (size_t)(t.p2p_epoch % 2048) : nullptr;
     ta.bar_base = t.tail_bar_count;
     ta.epoch = ++t.p2p_epoch;
     t.tail_bar_count += (unsigned int)grid * (dp ? 2u : 1u);
@@ -848,7 +839,7 @@ static int async_flush(vaeb_handle* h);
 static void p2p_release(vaeb_handle* h);   // unmaps the peers' buffers (data parallel over peer memory)   // launches streaming updates that were copied but not yet started
 
 const char* vaeb_last_error(void) { return g_last_error.c_str(); }
-int vaeb_version(void) { return 104; }   // 104: KL weight; 103: Adam; 102: vaeb_encode, vaeb_sample, vaeb_validate_terms (101: encoder_hidden_layers)
+int vaeb_version(void) { return 105; }   // 105: vaeb_profile_optimizer without variant; 104: KL weight; 103: Adam; 102: vaeb_encode, vaeb_sample, vaeb_validate_terms (101: encoder_hidden_layers)
 int vaeb_config_size(void) { return (int)sizeof(vaeb_config); }
 
 int vaeb_create(const vaeb_config* cfg, vaeb_handle** out) {
@@ -1878,13 +1869,6 @@ int vaeb_comm_attach(vaeb_handle* h, const char* nccl_library, const uint8_t id[
 
 static void p2p_release(vaeb_handle* h) {
   TcState& t = h->tc;
-  if (g_tail_stamps && getenv("VAEB_TAIL_STAMPS")) {      // debug dump: <path>.<rank>
-    std::vector<long long> hs(2048 * 8);
-    cudaDeviceSynchronize();
-    cudaMemcpy(hs.data(), g_tail_stamps, hs.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-    const std::string fn = std::string(getenv("VAEB_TAIL_STAMPS")) + "." + std::to_string(h->rank);
-    if (FILE* f = fopen(fn.c_str(), "wb")) { fwrite(hs.data(), sizeof(long long), hs.size(), f); fclose(f); }
-  }
   for (int i = 0; i < t.p2p_n_opened; ++i) cudaIpcCloseMemHandle(t.p2p_opened[i]);
   t.p2p_n_opened = 0;
   if (t.p2p_buf) cudaFree(t.p2p_buf);
@@ -1971,8 +1955,16 @@ int vaeb_profile_update(vaeb_handle* h, int64_t index, int32_t iters, int32_t ma
   // updates of minibatch `index`, its stamps read back into tm, ns per phase averaged over the last `iters` updates (the
   // first two are warm-up); kn / fl / by: the kernel's phase names, algorithmic flops and bytes.
   const int steps = iters + 2;
-  auto stamped = [&](int np, long long* d_timing, std::vector<long long>& tm, const char* const* kn, const double* fl,
+  auto stamped = [&](int np, long long*& d_timing, int& timing_cap, const char* const* kn, const double* fl,
                      const double* by) -> int {
+    if (steps * (np + 1) > timing_cap) {
+      if (d_timing) cudaFree(d_timing);
+      d_timing = nullptr;
+      VAEB_CUDA(cudaMalloc((void**)&d_timing, (size_t)steps * (np + 1) * sizeof(long long)));
+      timing_cap = steps * (np + 1);
+    }
+    std::vector<long long> tm((size_t)steps * (np + 1));
+    VAEB_CUDA(cudaMemsetAsync(d_timing, 0, tm.size() * sizeof(long long), h->stream));
     const std::vector<int32_t> order((size_t)steps, (int32_t)index);
     VAEB_TRY(run_single_launch(h, path, order.data(), nullptr, nullptr, h->M, steps, nullptr, 0, d_timing));
     VAEB_CUDA(cudaMemcpyAsync(tm.data(), d_timing, tm.size() * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
@@ -1995,36 +1987,13 @@ int vaeb_profile_update(vaeb_handle* h, int64_t index, int32_t iters, int32_t ma
         "P1 enc1 x.W3+tanh | W4,W5 update", "P2 heads+reparam+KL", "P3 dec1+dec2 h.W2+loglik+delta",
         "P4 dgrad (da.W2^T)*(1-h^2)", "P5 dz | W2 update | bound", "P6 W3 update | W1 update"};
     StepTcState& f = h->steptc;
-    const size_t n_stamps = (size_t)steps * (NP + 1) + 128 + 256 * NP;      // + sub-phase trace + per-CTA arrivals
-    if (steps * (NP + 1) > f.timing_cap) {
-      if (f.d_timing) cudaFree(f.d_timing);
-      f.d_timing = nullptr;
-      VAEB_CUDA(cudaMalloc((void**)&f.d_timing, n_stamps * sizeof(long long)));
-      f.timing_cap = steps * (NP + 1);
-    }
-    VAEB_CUDA(cudaMemsetAsync(f.d_timing, 0, n_stamps * sizeof(long long), h->stream));
     const double dM = h->M, dD = h->D, dH = h->H, dZ = h->Z;
     const double fl[NP] = {2 * dM * dD * dH + 4 * dM * dH * dZ, 4 * dM * dH * dZ, 2 * dM * dZ * dH + 2 * dM * dH * dD,
                            2 * dM * dH * dD, 2 * dM * dZ * dH + 2 * dM * dH * dD, 2 * dM * dD * dH + 4 * dM * dH * dZ + 2 * dM * dZ * dH};
     const double by[NP] = {4 * (dM * dD + dD * dH + dM * dH) + 40 * dH * dZ, 4 * (dM * dH + 2 * dH * dZ + 4 * dM * dZ),
                            4 * (dM * dZ + dZ * dH + dH * dD + 2 * dM * dD), 4 * (dM * dD + dH * dD + 2 * dM * dH),
                            4 * (dM * dH + dM * dD) + 24 * dH * dD, 4 * (dM * dD + dM * dH) + 20 * dD * dH + 20 * dZ * dH};
-    std::vector<long long> tm(n_stamps);
-    VAEB_TRY(stamped(NP, f.d_timing, tm, kNames, fl, by));
-    if (getenv("VAEB_STEPTC_TRACE")) {               // sub-phase stamps of CTA 0 in the last step (ns since the first)
-      const long long* tr = tm.data() + (size_t)steps * (NP + 1);
-      for (int q = 0; q < 60 && tr[2 * q] != 0; ++q)
-        fprintf(stderr, "st2 trace %3lld  +%8.3f us\n", tr[2 * q], 1e-3 * (double)(tr[2 * q + 1] - tr[1]));
-      // arrival of every CTA at the barrier that ends each phase of the last step (us after the phase opened for CTA 0)
-      const long long* ar = tr + 128;
-      const long long* last = tm.data() + (size_t)(steps - 1) * (NP + 1);
-      for (int ph = 0; ph < NP; ++ph) {
-        fprintf(stderr, "st2 arrive P%d:", ph + 1);
-        for (int b = 0; b < f.n_cta && b < 256; ++b) fprintf(stderr, " %.1f", 1e-3 * (double)(ar[(size_t)b * NP + ph] - last[ph]));
-        fprintf(stderr, "\n");
-      }
-    }
-    return VAEB_OK;
+    return stamped(NP, f.d_timing, f.timing_cap, kNames, fl, by);
   }
   if (path == FUSED) {
     constexpr int NP = fs::N_PHASES;
@@ -2033,12 +2002,6 @@ int vaeb_profile_update(vaeb_handle* h, int64_t index, int32_t iters, int32_t ma
         "P5 dgrad (da.W2^T)*(1-h^2)", "P6 W2,W1 wgrad+Adagrad | dz | bound", "P7 dh_e | W4,W5 wgrad+Adagrad",
         "P8 W3 wgrad+Adagrad"};
     FusedState& f = h->fused;
-    if (steps * (NP + 1) > f.timing_cap) {
-      if (f.d_timing) cudaFree(f.d_timing);
-      f.d_timing = nullptr;
-      VAEB_CUDA(cudaMalloc((void**)&f.d_timing, (size_t)steps * (NP + 1) * sizeof(long long)));
-      f.timing_cap = steps * (NP + 1);
-    }
     const double dM = h->M, dD = h->D, dH = h->H, dZ = h->Z, c = h->cont ? 2.0 : 1.0;
     const double fl[NP] = {2 * dM * dD * dH, 4 * dM * dH * dZ, 2 * dM * dZ * dH, 2 * dM * dH * dD * c, 2 * dM * dH * dD * c,
                            2 * dM * dH * dD * c + 4 * dM * dZ * dH, 8 * dM * dH * dZ, 2 * dM * dD * dH};
@@ -2048,8 +2011,7 @@ int vaeb_profile_update(vaeb_handle* h, int64_t index, int32_t iters, int32_t ma
                            4 * (dM * dH + c * dM * dD + dM * dH + dM * dZ) + 16 * (c * dH * dD + dZ * dH),
                            4 * (2 * dM * dZ + 2 * dH * dZ + 2 * dM * dH) + 16 * 2 * dH * dZ,
                            4 * (dM * dD + dM * dH) + 16 * dD * dH};
-    std::vector<long long> tm((size_t)steps * (NP + 1));
-    return stamped(NP, f.d_timing, tm, kNames, fl, by);
+    return stamped(NP, f.d_timing, f.timing_cap, kNames, fl, by);
   }
   PhaseProf prof;
   prof.iters = iters;
@@ -2070,11 +2032,9 @@ int vaeb_profile_update(vaeb_handle* h, int64_t index, int32_t iters, int32_t ma
   return VAEB_OK;
 }
 
-int vaeb_profile_optimizer(vaeb_handle* h, int32_t iters, int32_t variant, float* ms_per_launch,
-                            double* bytes_per_launch) {
+int vaeb_profile_optimizer(vaeb_handle* h, int32_t iters, float* ms_per_launch, double* bytes_per_launch) {
   VAEB_REQUIRE(h && ms_per_launch && bytes_per_launch && iters > 0, "null argument");
   VAEB_REQUIRE(!is_fvb(h), "vaeb_profile_optimizer covers the flat Adagrad pass of the LB/LA estimators");
-  VAEB_REQUIRE(variant == 0 || variant == 1 || variant == 2 || variant == 4, "variant must be 0, 1, 2 or 4");
   VAEB_CUDA(cudaSetDevice(h->cfg.device));
   const size_t nb = (size_t)(h->lay.padded + 4) * sizeof(float);
   StateBackup backup(h, nb);
@@ -2083,7 +2043,6 @@ int vaeb_profile_optimizer(vaeb_handle* h, int32_t iters, int32_t variant, float
   VAEB_CUDA(cudaEventCreate(&e0));
   if (cudaEventCreate(&e1) != cudaSuccess) { cudaEventDestroy(e0); VAEB_CUDA(cudaErrorUnknown); }
   const bool fb = h->cfg.variant == VAEB_VARIANT_FULLBAYES;
-  g_adagrad_unroll = variant;          // thread_local: the switch belongs to this call
   cudaError_t ce = cudaSuccess;
   for (int i = -2; i < iters && ce == cudaSuccess; ++i) {          // two untimed launches first
     if (i == 0) ce = cudaEventRecord(e0, h->stream);
@@ -2092,7 +2051,6 @@ int vaeb_profile_optimizer(vaeb_handle* h, int32_t iters, int32_t variant, float
                           h->cfg.learning_rate, h->cfg.adagrad_eps, fb ? 0.f : h->cfg.prior_scale,
                           fb ? h->cfg.learning_rate * 1e-6f : 0.f, h->d_grads + h->lay.padded, 1.f, 1.f, nullptr);
   }
-  g_adagrad_unroll = 0;
   if (ce == cudaSuccess) ce = cudaEventRecord(e1, h->stream);
   if (ce == cudaSuccess) ce = cudaEventSynchronize(e1);
   float ms = 0.f;

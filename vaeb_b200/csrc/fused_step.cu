@@ -29,10 +29,6 @@ enum { PLAIN = 0, DUALK = 1, DUALN = 2 };
 // DUALK: k <  K0 -> (A0, B0), k >= K0 -> (A1, B1) at k - K0   (sum of two products)
 // DUALN: tile columns [0, TN/2) come from B0, [TN/2, TN) from B1 at the same n (two heads)
 
-__device__ long long* g_dbg = nullptr;   // optional clock64 trace of CTA 0 (tools/dbg_fused.py)
-__device__ int g_dbg_n = 0;
-#define FS_STAMP(sign) do { if (dbg) g_dbg[g_dbg_n++] = (sign) * clock64(); } while (0)
-
 struct Gemm {
   const float* A0; const float* A1; int lda;
   const float* B0; const float* B1; int ldb;
@@ -291,8 +287,6 @@ __device__ __forceinline__ void run_item(const Gemm& g, int item, const Epi& epi
   else { tm = tile % g.c.tiles_m; tn = tile / g.c.tiles_m; active = active && tile < g.c.tiles_m * g.c.tiles_n; }
   float* wbuf = smem + warp * WBUF;
   const int m0 = tm * TM, n0 = tn * TNE;
-  const bool dbg = g_dbg != nullptr && blockIdx.x == 0 && threadIdx.x == 0;
-  FS_STAMP(1);
   if (active) {
     const int K = g.K0 + g.K1;
     // k slices start at multiples of four (16-byte copies along k stay aligned)
@@ -317,7 +311,6 @@ __device__ __forceinline__ void run_item(const Gemm& g, int item, const Epi& epi
       }
       cp_commit();
     }
-    FS_STAMP(1);
     int st = 0;
 #pragma unroll 1
     for (int c = 0; c < nch; ++c) {
@@ -338,7 +331,6 @@ __device__ __forceinline__ void run_item(const Gemm& g, int item, const Epi& epi
       }
       cp_wait<NSTAGE - 1>();
       __syncwarp();
-      FS_STAMP(1);
       if (ones_here) {                     // bias-gradient row of [act | 1]^T
         if (lane < ((kv + 3) & ~3)) sA[lane * (TM + 4) + (g.ones_row - m0)] = lane < kv ? 1.f : 0.f;
         __syncwarp();
@@ -346,11 +338,9 @@ __device__ __forceinline__ void run_item(const Gemm& g, int item, const Epi& epi
 #pragma unroll 1
       for (int kk = 0; kk < kv; kk += 4) fma_quad<TMT, TNT, AL, BL>(sA, sB, kk, rg, cg, acc);
       __syncwarp();
-      FS_STAMP(1);
       if (++st == NSTAGE) st = 0;
     }
     cp_wait<0>();
-    FS_STAMP(1);
     // this warp's partial tile, row-major [TM][TN], over its own stage
 #pragma unroll
     for (int i = 0; i < TMT; ++i)
@@ -358,7 +348,6 @@ __device__ __forceinline__ void run_item(const Gemm& g, int item, const Epi& epi
       for (int j = 0; j < TNT; ++j) wbuf[row_of<TMT, AL>(i, rg) * TN + col_of<TNT, BL>(j, cg)] = acc[i][j];
   }
   __syncthreads();
-  FS_STAMP(1);
   const int gidx = ksi * 32 + lane, gsize = ks * 32;
   float* gbuf = smem + (tl * ks) * WBUF;
   if (active) {
@@ -406,9 +395,7 @@ __device__ __forceinline__ void run_item(const Gemm& g, int item, const Epi& epi
       epi.rowsum(m0 + gidx, tn, s);
     }
   }
-  FS_STAMP(1);
   __syncthreads();
-  FS_STAMP(1);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -609,8 +596,6 @@ struct EpiAdagrad2 {                  // two heads at once (W4|W5, b4|b5)
 // grid barrier + kernel
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ void grid_barrier(unsigned long long* bar, unsigned long long target) {
-  const bool dbg = g_dbg != nullptr && blockIdx.x == 0 && threadIdx.x == 0;
-  FS_STAMP(-1);
   __syncthreads();
   if (threadIdx.x == 0) {
     // release: orders every write this CTA made before the bar.sync (cumulativity) before the arrival
@@ -622,7 +607,6 @@ __device__ __forceinline__ void grid_barrier(unsigned long long* bar, unsigned l
     __threadfence();   // also drops this SM's L1 lines (4-byte cp.async.ca staging goes through L1)
   }
   __syncthreads();
-  FS_STAMP(-1);
 }
 
 __device__ __forceinline__ long long gtime() {
@@ -1008,11 +992,4 @@ int fused_step_launch(vaeb_handle* h, const int* d_order, const float* d_kl, con
   h->grads_have_prior = false;
   invalidate_weight_mirrors(h);
   return VAEB_OK;
-}
-
-extern "C" int vaeb_fused_debug(long long* d_buf) {
-  int zero = 0;
-  cudaMemcpyToSymbol(fs::g_dbg, &d_buf, sizeof(d_buf));
-  cudaMemcpyToSymbol(fs::g_dbg_n, &zero, sizeof(int));
-  return 0;
 }

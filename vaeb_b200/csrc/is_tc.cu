@@ -248,7 +248,7 @@ struct TmaIssuer {
   uint32_t stage = 0, parity = 0;
   // TWO issuing threads (lane 0 of warps 0 and 3) walk the same item sequence and issue alternate items: an item costs
   // its thread an mbarrier round trip (~0.3 us) whatever the bytes, and the fill rate scales with the number of
-  // issuing threads (tools/tma_fill_probe.py: 30 / 59 / 118 GB/s per SM for 1 / 2 / 4 threads).
+  // issuing threads (the TMA fill-rate probe, DESIGN.md 4.3: 30 / 59 / 118 GB/s per SM for 1 / 2 / 4 threads).
   uint32_t me = 0, turn = 0;
   __device__ __forceinline__ void load(const CUtensorMap* m, uint32_t bytes, int c0, int c1) {
     if (turn == me) {
@@ -733,8 +733,7 @@ int is_tc_run(vaeb_handle* h, const float* d_x, const float* d_mu, const float* 
   p.cont = h->cont ? 1 : 0; p.Dx = Dx;
   p.eps_inj = d_eps; p.seed = h->cfg.seed; p.row_offset = row_offset;
   p.partial = (float2*)s.partial; p.logw_out = d_logw;
-  int grid = (int)std::min<int64_t>(n_tiles, s.n_sm);
-  { const char* e = getenv("VAEB_IS_GRID"); if (e) grid = std::min(grid, atoi(e)); }
+  const int grid = (int)std::min<int64_t>(n_tiles, s.n_sm);
   is_tc_kernel<<<grid, THREADS, Smem::TOTAL, st>>>(*(const CUtensorMap*)s.map_full, *(const CUtensorMap*)s.map_w1, p);
   ++h->launches;
   VAEB_CUDA(cudaGetLastError());

@@ -315,39 +315,23 @@ __device__ __forceinline__ void adagrad1(float& p, float& a, float g, float lr, 
 }
 
 // One vectorised, coalesced pass over the flat parameter buffer: 20 B/parameter (read p, acc, g; write p, acc).
-// U float4 per thread, every load issued before the first use; g is read once (ld.global.cs: it is dead after this
-// kernel); p and acc are rewritten in place.  Production = U 1 without cache hints: more loads per thread, streaming
-// hints, a persistent grid-stride form and a cp.async.bulk shared-memory pipeline all measured slower on B200
-// (profiles/r1_adagrad_hbm.txt).
-template <int U, bool CS>
+// One float4 per thread; g is read once (ld.global.cs: it is dead after this kernel); p and acc are rewritten in
+// place.  More loads per thread, streaming hints on p and acc, a persistent grid-stride form and a cp.async.bulk
+// shared-memory pipeline all measured slower on B200 (profiles/r1_adagrad_hbm.txt).
 __global__ void __launch_bounds__(256)
 adagrad_kernel(float4* __restrict__ p, float4* __restrict__ acc, const float4* __restrict__ g, int64_t n4, float lr,
                float eps, float prior, float p2, const float* __restrict__ base, float mult, float div,
                float* __restrict__ scalar_out) {
-  const int64_t i0 = (int64_t)blockIdx.x * (blockDim.x * U) + threadIdx.x;
-  if (i0 == 0 && scalar_out) *scalar_out = (mult * *base) / div;
-  float4 pv[U], av[U], gv[U];
-#pragma unroll
-  for (int u = 0; u < U; ++u) {
-    const int64_t i = i0 + (int64_t)u * blockDim.x;
-    if (i < n4) {
-      pv[u] = CS ? __ldcs(p + i) : p[i];
-      av[u] = CS ? __ldcs(acc + i) : acc[i];
-      gv[u] = __ldcs(g + i);
-    }
-  }
-#pragma unroll
-  for (int u = 0; u < U; ++u) {
-    const int64_t i = i0 + (int64_t)u * blockDim.x;
-    if (i < n4) {
-      adagrad1(pv[u].x, av[u].x, gv[u].x, lr, eps, prior, p2);
-      adagrad1(pv[u].y, av[u].y, gv[u].y, lr, eps, prior, p2);
-      adagrad1(pv[u].z, av[u].z, gv[u].z, lr, eps, prior, p2);
-      adagrad1(pv[u].w, av[u].w, gv[u].w, lr, eps, prior, p2);
-      if (CS) { __stcs(p + i, pv[u]); __stcs(acc + i, av[u]); }
-      else { p[i] = pv[u]; acc[i] = av[u]; }
-    }
-  }
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i == 0 && scalar_out) *scalar_out = (mult * *base) / div;
+  if (i >= n4) return;
+  float4 pv = p[i], av = acc[i];
+  const float4 gv = __ldcs(g + i);
+  adagrad1(pv.x, av.x, gv.x, lr, eps, prior, p2);
+  adagrad1(pv.y, av.y, gv.y, lr, eps, prior, p2);
+  adagrad1(pv.z, av.z, gv.z, lr, eps, prior, p2);
+  adagrad1(pv.w, av.w, gv.w, lr, eps, prior, p2);
+  p[i] = pv; acc[i] = av;
 }
 
 // getAdaDeltaUpdates, VAEB.py:449-469 (g already carries the prior: VAEB.py:389-390), 28 B/parameter
@@ -589,21 +573,11 @@ cudaError_t launch_adam(cudaStream_t st, int64_t* launches, float* p, float* m, 
   return LAUNCHED();
 }
 
-thread_local int g_adagrad_unroll = 0;   // measurement switch (vaeb_profile_optimizer): 0/1 production, 2 = streaming cache hints, 4 = + two float4 per thread
-
 cudaError_t launch_adagrad(cudaStream_t st, int64_t* launches, float* p, float* acc, const float* g, int64_t n4,
                            float lr, float eps, float prior, float p2, const float* base, float mult, float div,
                            float* scalar_out) {
-  // one float4 per thread is the fastest form measured at both sizes (profiles/r1_adagrad_hbm.txt)
-  const int u = g_adagrad_unroll ? g_adagrad_unroll : 1;
-  float4 *p4 = (float4*)p, *a4 = (float4*)acc;
-  const float4* g4 = (const float4*)g;
-  if (u == 4)
-    adagrad_kernel<2, true><<<blocks_for(n4, 512), 256, 0, st>>>(p4, a4, g4, n4, lr, eps, prior, p2, base, mult, div, scalar_out);
-  else if (u == 2)
-    adagrad_kernel<1, true><<<blocks_for(n4, 256), 256, 0, st>>>(p4, a4, g4, n4, lr, eps, prior, p2, base, mult, div, scalar_out);
-  else
-    adagrad_kernel<1, false><<<blocks_for(n4, 256), 256, 0, st>>>(p4, a4, g4, n4, lr, eps, prior, p2, base, mult, div, scalar_out);
+  adagrad_kernel<<<blocks_for(n4, 256), 256, 0, st>>>((float4*)p, (float4*)acc, (const float4*)g, n4, lr, eps, prior, p2,
+                                                      base, mult, div, scalar_out);
   return LAUNCHED();
 }
 

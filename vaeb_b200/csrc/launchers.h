@@ -94,7 +94,6 @@ cudaError_t launch_adam(cudaStream_t st, int64_t* launches, float* p, float* m, 
 cudaError_t launch_adagrad(cudaStream_t st, int64_t* launches, float* p, float* acc, const float* g, int64_t n4,
                            float lr, float eps, float prior, float p2, const float* base, float mult, float div,
                            float* scalar_out);
-extern thread_local int g_adagrad_unroll;   // measurement switch of the flat Adagrad kernel (vaeb_profile_optimizer)
 #define VAEB_TP_BLOCKS 128
 // thetaPrior partials (VAEB.py:359-363) over n real elements
 cudaError_t launch_theta_prior(cudaStream_t st, int64_t* launches, const float* vmu, const float* vsig, int64_t n,

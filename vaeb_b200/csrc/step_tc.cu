@@ -60,7 +60,6 @@ struct Ctx {
   uint64_t *mma_bar, *op_bar, *x_bar, *rs_bar;
   uint32_t mma_phase, op_phase, x_phase, rs_phase;
   int rank, cid, ncl, warp, lane;
-  long long* trace; int tn;            // optional sub-phase stamps (CTA 0, thread 0, last step of a profiling launch)
   float tp;                            // sampled full VB: this thread's share of thetaPrior of the running step
   uint32_t step;                       // global index of the running step (Philox key of the weight noise)
 };
@@ -101,14 +100,6 @@ __device__ __forceinline__ long long gtime() {
   asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
   return t;
 }
-#define ST2_TRACE(c, id)                                               \
-  do {                                                                 \
-    if ((c).trace && threadIdx.x == 0 && (c).tn < 62) {                \
-      (c).trace[(c).tn * 2] = (id);                                    \
-      (c).trace[(c).tn * 2 + 1] = gtime();                             \
-      ++(c).tn;                                                        \
-    }                                                                  \
-  } while (0)
 // Operand format: every fp32 value v is carried as an fp16 pair hi = rn(v), lo = rn(v - hi): 22 mantissa bits
 // (|error| <= max(2^-23 |v|, 2^-25): the residual of a small value is an fp16 subnormal with absolute spacing 2^-24),
 // so hi*hi + hi*lo + lo*hi reproduces the fp32 product to ~2^-21 -- the fp32 parity tier.  Weights (|w| ~ 1e-2 at
@@ -434,7 +425,6 @@ enum { A_BULK = 0,       // one bulk copy from x_km (written in P2 of the previo
        A_STAGED = 2,     // already converted into shared memory by this CTA (first step of a launch)
        A_SOFTWARE = 3 }; // convert from the fp32 rows now (first step of a launch, second item of a cluster)
 __device__ __forceinline__ void item_enc1(Ctx& c, const Params& p, const float* x, float* he, uint8_t* he_t, int t, int a_mode, bool more) {
-  ST2_TRACE(c, 10);
   const int c0 = c.rank * p.KD / CL, c1 = (c.rank + 1) * p.KD / CL, nch = c1 - c0;
   constexpr int TB = TR_ENC1 * 128;
   if (threadIdx.x == 0 && nch > 0) {
@@ -447,11 +437,8 @@ __device__ __forceinline__ void item_enc1(Ctx& c, const Params& p, const float* 
   const int row = threadIdx.x >> 4, col = threadIdx.x & 15;
   const int gr = c.rank * 32 + row, j = t * 16 + col;
   const float bias = j < p.H ? __ldcg(p.P + p.ob3 + j) : 0.f;
-  ST2_TRACE(c, 11);
   mma_run(c, nch, min(nch * 4, (p.D - c0 * 64 + 15) / 16), TB, TR_ENC1, nch > 0);
-  ST2_TRACE(c, 12);
   reduce_scatter(c, TR_ENC1, nch > 0);
-  ST2_TRACE(c, 13);
   const float* recv = reinterpret_cast<const float*>(c.sm + SM_RECV);
   if (gr < p.M) {
     const float v = j < p.H ? tanh_fast(fmaf(recv_sum(recv, TR_ENC1, row, col), WUNSCALE, bias)) : 0.f;
@@ -459,15 +446,12 @@ __device__ __forceinline__ void item_enc1(Ctx& c, const Params& p, const float* 
     put_hl(km_addr(p.he_km, gr, j), TBA, v);
     if (j < p.H) put_hl(t_addr(he_t, j >> 7, TBA, j & 127, gr), TBA, v);
   }
-  ST2_TRACE(c, 14);
   if (more) cluster_sync();          // the receive buffer is reused by this cluster's next item of the phase
   else __syncthreads();
-  ST2_TRACE(c, 15);
 }
 
 // P2: (mu, ls) = h_e.[W4|W5] + b, eps, z = mu + exp(ls/2) eps, the KL / L^A row term        VAEB.py:248-249,41-47,343,322-325
 __device__ __forceinline__ void item_heads(Ctx& c, const Params& p, uint32_t step, bool more) {
-  ST2_TRACE(c, 20);
   const int c0 = c.rank * p.KH / CL, c1 = (c.rank + 1) * p.KH / CL, nch = c1 - c0;
   const int TB = p.NH * 128, Z = p.Z, N = p.NH;
   if (threadIdx.x == 0 && nch > 0) {
@@ -489,11 +473,8 @@ __device__ __forceinline__ void item_heads(Ctx& c, const Params& p, uint32_t ste
       b4_[i] = __ldcg(p.P + p.ob4 + j); b5_[i] = __ldcg(p.P + p.ob5 + j);
     }
   }
-  ST2_TRACE(c, 21);
   mma_run(c, nch, nch * 4, TB, N, nch > 0);
-  ST2_TRACE(c, 22);
   reduce_scatter(c, N, nch > 0);
-  ST2_TRACE(c, 23);
   const float* recv = reinterpret_cast<const float*>(c.sm + SM_RECV);
   float* term = reinterpret_cast<float*>(c.sm + SM_B);          // [32][Z] (the B tiles are dead)
   const int zt_half = p.NZ * 128;
@@ -527,10 +508,8 @@ __device__ __forceinline__ void item_heads(Ctx& c, const Params& p, uint32_t ste
       p.aux[gr] = s;
     }
   }
-  ST2_TRACE(c, 24);
   if (more) cluster_sync();          // the receive buffer is reused by this cluster's next item of the phase
   else __syncthreads();
-  ST2_TRACE(c, 25);
 }
 
 // P3: h_d = tanh(z.W1 + b1) recomputed into the A tile, a = h_d.W2 + b2, x a - softplus(a), da2 = x - sigmoid a
@@ -538,7 +517,6 @@ __device__ __forceinline__ void item_heads(Ctx& c, const Params& p, uint32_t ste
 // Gaussian decoder: the tile holds [W2 | W6] for 32 pixels; mu = sigmoid(a), lv = h_d.W6 + b6, the log-density of
 // VAEB.py:306-307 and its two deltas.
 __device__ __forceinline__ void item_dec2(Ctx& c, const Params& p, const float* x, int t, bool more, bool publish, int s) {
-  ST2_TRACE(c, 30);
   const int c0 = c.rank * p.KH / CL, c1 = (c.rank + 1) * p.KH / CL, nch = c1 - c0;
   const int TR = p.TR3, TB = TR * 128;
   const int H = p.H, M = p.M;
@@ -564,7 +542,6 @@ __device__ __forceinline__ void item_dec2(Ctx& c, const Params& p, const float* 
     b2_[i] = ok ? __ldcg(p.P + p.ob2 + n) : 0.f;
     b6_[i] = (ok && p.cont) ? __ldcg(p.P + p.ob6 + n) : 0.f;
   }
-  ST2_TRACE(c, 36);
   // ---- hidden layer on the tensor cores: D1[128 x 64 nch] = [z|1] . [W1^T|b1]^T (K = 32: latent code + bias) --------
   tc::tc_fence_before();
   __syncthreads();                                              // the previous item's TMEM reads are complete
@@ -594,7 +571,6 @@ __device__ __forceinline__ void item_dec2(Ctx& c, const Params& p, const float* 
     c.mma_phase ^= 1u;
     tc::tc_fence_after();
   }
-  ST2_TRACE(c, 38);
   {
     // h_d = tanh(D1) (the bias rode along as latent column Z) -> the A tile of the output layer; thread = batch row,
     // eight consecutive hidden units per TMEM read = one 16-byte unit of the tile
@@ -627,12 +603,8 @@ __device__ __forceinline__ void item_dec2(Ctx& c, const Params& p, const float* 
       }
     }
   }
-  ST2_TRACE(c, 39);
-  ST2_TRACE(c, 31);
   mma_run(c, nch, nch * 4, TB, TR, false);
-  ST2_TRACE(c, 32);
   reduce_scatter(c, TR, nch > 0);
-  ST2_TRACE(c, 33);
   const float* recv = reinterpret_cast<const float*>(c.sm + SM_RECV);
   float* term = reinterpret_cast<float*>(c.sm + SM_B);          // [32][32]
   float* dtile = term + 32 * 32;                                // [32][33] (+ a second one for the Gaussian lv deltas)
@@ -688,10 +660,8 @@ __device__ __forceinline__ void item_dec2(Ctx& c, const Params& p, const float* 
       p.partial[(size_t)gr * p.n_tiles3 + t] = s;
     }
   }
-  ST2_TRACE(c, 34);
   if (more) cluster_sync();          // the receive buffer is reused by this cluster's next item of the phase
   else __syncthreads();
-  ST2_TRACE(c, 35);
 }
 
 // P3, spare clusters: h_d = tanh([z|1].[W1^T|b1]^T) for 16 hidden units per CTA, published for P4 (fp32, the tanh'
@@ -754,7 +724,6 @@ __device__ __forceinline__ void item_hd(Ctx& c, const Params& p, int g) {
 // (Gaussian decoder: K runs over the virtual columns [da | dlv] against [W2 | W6]^T.)  A rank's share of K may exceed
 // the A region (Frey Face: 18 chunks over 4 ranks): further passes accumulate into the same TMEM columns.
 __device__ __forceinline__ void item_dgrad(Ctx& c, const Params& p, int t, bool more, int s) {
-  ST2_TRACE(c, 40);
   const int c0 = c.rank * p.KV / CL, c1 = (c.rank + 1) * p.KV / CL, nch = c1 - c0;
   constexpr int TB = TR_DGRAD * 128;
   const int row = threadIdx.x >> 4, col = threadIdx.x & 15;
@@ -767,13 +736,10 @@ __device__ __forceinline__ void item_dgrad(Ctx& c, const Params& p, int t, bool 
       bulk_g2s(c.sm + SM_A, p.da2_km + (size_t)(c0 + base) * 2 * TBA, (uint32_t)(n * 2 * TBA), c.op_bar);
       bulk_g2s(c.sm + SM_B, p.m_dgrad + ((size_t)t * p.KV + c0 + base) * 2 * TB, (uint32_t)(n * 2 * TB), c.op_bar);
     }
-    ST2_TRACE(c, 41);
     const int k16 = p.cont ? n * 4 : min(n * 4, (p.D - (c0 + base) * 64 + 15) / 16);
     mma_run(c, max(n, 0), k16, TB, TR_DGRAD, n > 0, base ? 1u : 0u, 1, 0);
   }
-  ST2_TRACE(c, 42);
   reduce_scatter(c, TR_DGRAD, nch > 0, true);
-  ST2_TRACE(c, 43);
   const float* recv = reinterpret_cast<const float*>(c.sm + SM_RECV);
   if (gr < p.M) {
     const float d = recv_sum(recv, TR_DGRAD, row, col) * WUNSCALE * (1.0f - hv * hv);
@@ -781,16 +747,13 @@ __device__ __forceinline__ void item_dgrad(Ctx& c, const Params& p, int t, bool 
     put_dl(km_addr(p.da1_km, gr, j), TBA, d);
     if (j < p.H) put_dl(t_addr(p.da1_t, j >> 7, TBA, j & 127, gr), TBA, d);
   }
-  ST2_TRACE(c, 44);
   if (more) cluster_sync();          // the receive buffer is reused by this cluster's next item of the phase
   else __syncthreads();
-  ST2_TRACE(c, 45);
 }
 
 // P5: dz = da1.W1^T -> dmu, dls (SURVEY.md 8a backward formulas).  kb = the step's KL weight: its three terms carry it,
 // and the weight-gradient epilogues scale the whole gradient by w, so the update ascends w (grad loglik + kb grad aux)
 __device__ __forceinline__ void item_dz(Ctx& c, const Params& p, bool more, float kb) {
-  ST2_TRACE(c, 50);
   const int c0 = c.rank * p.KH / CL, c1 = (c.rank + 1) * p.KH / CL, nch = c1 - c0;
   const int TB = p.NZ * 128, Z = p.Z, N = p.NZ;
   if (threadIdx.x == 0 && nch > 0) {
@@ -811,11 +774,8 @@ __device__ __forceinline__ void item_dz(Ctx& c, const Params& p, bool more, floa
       zm_[i] = p.la ? __ldcg(p.z + o) : __ldcg(p.mu + o);
     }
   }
-  ST2_TRACE(c, 51);
   mma_run(c, nch, nch * 4, TB, N, nch > 0, 0u, 1, 0);
-  ST2_TRACE(c, 52);
   reduce_scatter(c, N, nch > 0, true);
-  ST2_TRACE(c, 53);
   const float* recv = reinterpret_cast<const float*>(c.sm + SM_RECV);
 #pragma unroll
   for (int i = 0; i < 2; ++i) {
@@ -839,10 +799,8 @@ __device__ __forceinline__ void item_dz(Ctx& c, const Params& p, bool more, floa
       put_dl(t_addr(p.dd_t, (Z + j) >> 4, 2048, (Z + j) & 15, gr), 2048, b);
     }
   }
-  ST2_TRACE(c, 54);
   if (more) cluster_sync();          // the receive buffer is reused by this cluster's next item of the phase
   else __syncthreads();
-  ST2_TRACE(c, 55);
 }
 
 // =================================================================================================================
@@ -1047,7 +1005,6 @@ __device__ __forceinline__ void wgrad_epilogue_coalesced(Ctx& c, const Params& p
 // the W6 / b6 half of the tile (rows 32..63 of the transposed delta mirror, virtual columns 32..63 of the chunk).
 template <bool SV>
 __device__ __forceinline__ void item_wg2(Ctx& c, const Params& p, const Hyper& hy, int mt, int nt, int which) {
-  ST2_TRACE(c, 60);
   constexpr int TB = 32 * 128;                                  // the B tile of the item: 32 rows
   const int TBM = p.TR3 * 128;                                  // one half (hi or lo) of a delta-mirror tile
   if (threadIdx.x == 0) {
@@ -1068,7 +1025,6 @@ __device__ __forceinline__ void item_wg2(Ctx& c, const Params& p, const Hyper& h
     return i < H ? oW + (long long)i * D + n : ob + n;
   }, pre, vec4);
   mma_run(c, 2, (p.M + 15) / 16, TB, 32, true, 0u, 0, 1);
-  ST2_TRACE(c, 61);
   wgrad_epilogue_coalesced<32, SV>(
       c, p, hy, pre,
       [&](int row, int col0, float* nv) {
@@ -1086,14 +1042,12 @@ __device__ __forceinline__ void item_wg2(Ctx& c, const Params& p, const Hyper& h
         const int kv = p.cont ? nt * 64 + vr : n0;
         put_unit<true>(p.m_dgrad + ((size_t)(i >> 4) * p.KV + (kv >> 6)) * 2 * TG + unit_off(i & 15, (kv & 63) >> 3), TG, nv);
       }, vec4);
-  ST2_TRACE(c, 62);
 }
 
 // W3, b3 <- Adagrad([x | 1]^T . da3), da3 = ([dmu|dls].[W4|W5]^T) * (1 - h_e^2) recomputed on the tensor cores (K = one
 // chunk) and written, transposed, into the B tile; tile = 128 pixels x 32 hidden units
 template <bool SV>
 __device__ __forceinline__ void item_wg3(Ctx& c, const Params& p, const Hyper& hy, const float* he, int mt, int nt, int par) {
-  ST2_TRACE(c, 70);
   const int H = p.H, M = p.M, D = p.D;
   constexpr int TB = 32 * 128;                                  // one half (hi or lo) of a 32-row tile
   uint8_t* dd_sm = c.sm + SM_A + 2 * 2 * TBA;                   // [dmu|dls]: the chunk slot behind the two chunks of x^T
@@ -1144,7 +1098,6 @@ __device__ __forceinline__ void item_wg3(Ctx& c, const Params& p, const Hyper& h
   tc::mbar_wait(c.mma_bar, c.mma_phase);
   c.mma_phase ^= 1u;
   tc::tc_fence_after();
-  ST2_TRACE(c, 74);
   {
     float v[8], vh[8];
     tmem_ld8(c.tmem + ((uint32_t)(q * 32) << 16) + 64u + (uint32_t)(cg * 8), v);
@@ -1160,9 +1113,7 @@ __device__ __forceinline__ void item_wg3(Ctx& c, const Params& p, const Hyper& h
       put_dl(bt + tc::sw128_offset(cg * 8 + e, b & 63), TB, d);
     }
   }
-  ST2_TRACE(c, 71);
   mma_run(c, 2, (M + 15) / 16, TB, 32, false, 0u, 0, 1);
-  ST2_TRACE(c, 72);
   wgrad_epilogue_coalesced<32, SV>(
       c, p, hy, pre,
       [&](int row, int col0, float* nv) {
@@ -1172,7 +1123,6 @@ __device__ __forceinline__ void item_wg3(Ctx& c, const Params& p, const Hyper& h
         for (int e = 0; e < 8; ++e)
           if (j0_ + e < H) mirror_put(p.m_enc1, TR_ENC1, p.KD, (j0_ + e) >> 4, (j0_ + e) & 15, i, nv[e]);
       }, vec4);
-  ST2_TRACE(c, 73);
 }
 
 // W1, b1 <- Adagrad([z | 1]^T . da1), computed transposed: tile = 128 hidden units x (Z + 1) latent columns.  W1 is
@@ -1381,7 +1331,6 @@ __global__ void __launch_bounds__(NT, 1) step_tc_kernel(const __grid_constant__ 
   c.mma_phase = 0; c.op_phase = 0; c.x_phase = 0; c.rs_phase = 0;
   c.rank = (int)cluster_ctarank(); c.cid = (int)cluster_idx(); c.ncl = (int)cluster_count();
   c.warp = threadIdx.x >> 5; c.lane = threadIdx.x & 31;
-  c.trace = nullptr; c.tn = 0;
   if (threadIdx.x == 0) {
     tc::mbar_init(c.mma_bar, 1);
     tc::mbar_init(c.op_bar, 1);
@@ -1420,11 +1369,6 @@ __global__ void __launch_bounds__(NT, 1) step_tc_kernel(const __grid_constant__ 
   const int n_spare = c.ncl - n3;                   // clusters without a dec2 item: they publish h_d in P3
   int last_done = -1;                               // last step whose updates were applied (a Gaussian launch may stop early)
 
-#define ARRIVE(ph)                                                                                           \
-  do {                                                                                                       \
-    if (p.timing && threadIdx.x == 0 && s == p.n_steps - 1 && blockIdx.x < 256)                              \
-      p.timing[(size_t)p.n_steps * (N_PHASES + 1) + 128 + (size_t)blockIdx.x * N_PHASES + (ph)] = gtime();   \
-  } while (0)
   for (int s = 0; s < p.n_steps; ++s) {
     const float* x = x_of(s);
     const int par = (int)((p.step0 + (uint32_t)s) & 1u);        // which copy of the k-major [W4|W5] mirror this step reads
@@ -1434,7 +1378,6 @@ __global__ void __launch_bounds__(NT, 1) step_tc_kernel(const __grid_constant__ 
     if (SV && s > 0 && (int)blockIdx.x == G - 1) item_bound(c, p, s - 1);
     long long* tm = rec ? p.timing + (size_t)s * (N_PHASES + 1) : nullptr;
     if (tm) tm[0] = gtime();
-    if (p.timing && blockIdx.x == 0 && s == p.n_steps - 1) c.trace = p.timing + (size_t)p.n_steps * (N_PHASES + 1);
 
     // ---- P1: encoder hidden layer | this step's noise ----------------------------------------------------------
     {
@@ -1448,29 +1391,20 @@ __global__ void __launch_bounds__(NT, 1) step_tc_kernel(const __grid_constant__ 
         item_eps(p, p.step0 + (uint32_t)s, c.rank);
       }
     }
-    ST2_TRACE(c, 81);
-    ARRIVE(0);
     grid_barrier(p.bar, target += G);
     if (tm) tm[1] = gtime();
-    ST2_TRACE(c, 91);
     // ---- P2: latent heads | the minibatch operands of P6 and of the next step's P1 ---------------------------------
     if (c.cid == 0) item_heads(c, p, p.step0 + (uint32_t)s, false);
     else item_xmirrors(p, s + 1 < p.n_steps ? x_of(s + 1) : nullptr, x, (c.cid - 1) * CL + c.rank, (c.ncl - 1) * CL);
     if (p.fvb == 1) item_fvb_prior(c, p, hy, s, c.cid == 0 ? -1 : (c.cid - 1) * CL + c.rank, (c.ncl - 1) * CL);   // nothing downstream reads (mu, sigma)
-    ST2_TRACE(c, 82);
-    ARRIVE(1);
     grid_barrier(p.bar, target += G);
     if (tm) tm[2] = gtime();
-    ST2_TRACE(c, 92);
     // ---- P3: decoder + log-likelihood | h_d published by the spare clusters ------------------------------------------
     for (int it = c.cid; it < n3; it += c.ncl) item_dec2(c, p, x, it, it + c.ncl < n3, n_spare <= 0, s);
     if (c.cid >= n3)
       for (int g = (c.cid - n3) * CL + c.rank; g < p.HP / 16; g += n_spare * CL) item_hd(c, p, g);
-    ST2_TRACE(c, 83);
-    ARRIVE(2);
     grid_barrier(p.bar, target += G);
     if (tm) tm[3] = gtime();
-    ST2_TRACE(c, 93);
     if (p.fvb == 1) {
       // reference-faithful full VB: the bound is all the layers are needed for.  One CTA (rotating) sums it; the
       // partials it reads are overwritten two barriers into the next step at the earliest.
@@ -1483,11 +1417,8 @@ __global__ void __launch_bounds__(NT, 1) step_tc_kernel(const __grid_constant__ 
     }
     // ---- P4: back through the decoder output layer ---------------------------------------------------------------
     for (int it = c.cid; it < n1; it += c.ncl) item_dgrad(c, p, it, it + c.ncl < n1, s);
-    ST2_TRACE(c, 84);
-    ARRIVE(3);
     grid_barrier(p.bar, target += G);
     if (tm) tm[4] = gtime();
-    ST2_TRACE(c, 94);
     // Gaussian decoder: a delta left the operand range -> every CTA leaves before the first parameter update of step s
     if (p.cont && __syncthreads_or(threadIdx.x == 0 && __ldcg(p.status) >= 0)) break;
     // ---- P5: dz | W2 update | the bound ---------------------------------------------------------------------------
@@ -1502,11 +1433,8 @@ __global__ void __launch_bounds__(NT, 1) step_tc_kernel(const __grid_constant__ 
         else if (i == n2 && !SV) item_bound(c, p, s);
       }
     }
-    ST2_TRACE(c, 85);
-    ARRIVE(4);
     grid_barrier(p.bar, target += G);
     if (tm) tm[5] = gtime();
-    ST2_TRACE(c, 95);
     // ---- P6: W3 update | W1 update | W4, W5 update -----------------------------------------------------------------
     {
       const int n45 = m_h1 * n45t;
@@ -1523,11 +1451,8 @@ __global__ void __launch_bounds__(NT, 1) step_tc_kernel(const __grid_constant__ 
       tc::mbar_expect_tx(c.x_bar, (uint32_t)(kdn * 2 * TBA));
       bulk_g2s(c.sm + SM_A, p.x_km + (size_t)kd0 * 2 * TBA, (uint32_t)(kdn * 2 * TBA), c.x_bar);
     }
-    ST2_TRACE(c, 86);
-    ARRIVE(5);
     grid_barrier(p.bar, target += G);
     if (tm) tm[6] = gtime();
-    ST2_TRACE(c, 96);
     last_done = s;
   }
   if (SV && last_done >= 0 && (int)blockIdx.x == G - 1) item_bound(c, p, last_done);
@@ -1790,10 +1715,7 @@ int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_kl, const 
   at[0].id = cudaLaunchAttributeClusterDimension;
   at[0].val.clusterDim.x = CL; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
   at[1].id = cudaLaunchAttributeCooperative; at[1].val.cooperative = 1;
-  // (ncu cannot launch a cluster kernel with the cooperative attribute: VAEB_ST2_NOCOOP=1 drops it for profiling runs;
-  // the grid is sized to be co-resident either way)
-  static const bool no_coop = getenv("VAEB_ST2_NOCOOP") != nullptr;
-  cfg.attrs = at; cfg.numAttrs = no_coop ? 1 : 2;
+  cfg.attrs = at; cfg.numAttrs = 2;
   if (p.fvb == 2) VAEB_CUDA(cudaLaunchKernelEx(&cfg, step_tc_kernel<true>, p));
   else VAEB_CUDA(cudaLaunchKernelEx(&cfg, step_tc_kernel<false>, p));
   ++h->launches;

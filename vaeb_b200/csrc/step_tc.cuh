@@ -80,7 +80,7 @@ struct Params {
   float* zeta;                          // the draws of the current step (written by the previous step's epilogues)
   float* tprior_part;                   // [2][gridDim.x] per-CTA partial sums of thetaPrior (step parity)
   unsigned long long* bar; unsigned long long bar_base;
-  long long* timing;                    // nullptr or [n_steps * (N_PHASES + 1) + 128] globaltimer stamps of CTA 0
+  long long* timing;                    // nullptr or [n_steps * (N_PHASES + 1)] globaltimer stamps of CTA 0
 };
 
 }  // namespace st2

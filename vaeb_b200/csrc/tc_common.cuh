@@ -193,7 +193,7 @@ __device__ __forceinline__ uint32_t sw128_offset(int r, int c) {
 // MN-major operand [k_rows, cols] (cols contiguous, row stride a multiple of 64 elements) seen as
 // [cols/64 groups][k_rows][64]: ONE box of `groups` column groups x 64 contraction rows per tile and k block lands in
 // shared memory as `groups` consecutive [64 x 128 B] SWIZZLE_128B blocks -- a TMA box costs ~120 ns of issue time
-// whatever its size (tools/tma_fill_probe.py), so one 32 KB box instead of four 8 KB ones.
+// whatever its size (the TMA fill-rate probe, profiles/r1_c3_phases.txt), so one 32 KB box instead of four 8 KB ones.
 int vaeb_make_tmap_bf16_mn(CUtensorMap* out, const void* base, uint64_t k_rows, uint64_t cols, uint64_t row_stride_elems,
                            uint32_t groups, uint32_t k_box = 64);
 int vaeb_make_tmap_bf16(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols, uint64_t row_stride_elems,

@@ -29,9 +29,7 @@ struct GemmSmem {
 template <int BN, bool A_MN, bool B_MN>
 __global__ void __launch_bounds__(256, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, float* __restrict__ C,
-               int M, int N, int K, int ldc, long long* __restrict__ dbg) {
-  const bool rec = dbg != nullptr && blockIdx.x == 0 && blockIdx.y == 0;
-  if (rec && threadIdx.x == 0) dbg[0] = clock64();
+               int M, int N, int K, int ldc) {
   using S = GemmSmem<BN>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
@@ -57,7 +55,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   __syncthreads();
   tc::tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  if (rec && threadIdx.x == 0) dbg[1] = clock64();
 
   if (warp == 0 && lane == 0) {
     // ===== TMA producer =====
@@ -65,7 +62,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       const int s = kb % STAGES;
       const uint32_t ph = (kb / STAGES) & 1;
       tc::mbar_wait(&empty[s], ph ^ 1);
-      if (rec && kb < 16) dbg[8 + kb] = clock64();
       uint8_t* a = smem + s * S::STAGE_BYTES;
       uint8_t* b = a + S::A_BYTES;
       tc::mbar_expect_tx(&full[s], S::STAGE_BYTES);
@@ -88,7 +84,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       const uint32_t ph = (kb / STAGES) & 1;
       tc::mbar_wait(&full[s], ph);
       tc::tc_fence_after();
-      if (rec && kb < 16) dbg[24 + kb] = clock64();
       const uint32_t a = tc::smem_u32(smem + s * S::STAGE_BYTES);
       const uint32_t b = a + S::A_BYTES;
 #pragma unroll
@@ -100,12 +95,10 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       tc::umma_commit(&empty[s]);     // frees the smem slot once these MMAs have read it
     }
     tc::umma_commit(tmem_full);       // accumulator complete
-    if (rec) dbg[2] = clock64();
   } else if (warp >= 4) {
     // ===== epilogue: TMEM -> registers -> global =====
     tc::mbar_wait(tmem_full, 0);
     tc::tc_fence_after();
-    if (rec && threadIdx.x == 128) dbg[3] = clock64();
     const int q = warp & 3;                       // TMEM lane quarter of this warp
     const int row = m0 + q * 32 + lane;
 #pragma unroll 1
@@ -122,7 +115,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   }
   tc::tc_fence_before();
   __syncthreads();
-  if (rec && threadIdx.x == 0) dbg[4] = clock64();
   if (warp == 2) tc::tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
@@ -150,12 +142,12 @@ uint16_t f32_to_bf16(float f) {   // round to nearest even
 
 template <int BN, bool A_MN, bool B_MN>
 int launch_tc_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, float* C, int M, int N, int K, int ldc,
-                   cudaStream_t st, long long* dbg = nullptr) {
+                   cudaStream_t st) {
   using S = GemmSmem<BN>;
   auto kfn = tc_gemm_kernel<BN, A_MN, B_MN>;
   VAEB_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, S::TOTAL));
   dim3 grid((N + BN - 1) / BN, (M + BM - 1) / BM);
-  kfn<<<grid, 256, S::TOTAL, st>>>(tmA, tmB, C, M, N, K, ldc, dbg);
+  kfn<<<grid, 256, S::TOTAL, st>>>(tmA, tmB, C, M, N, K, ldc);
   VAEB_CUDA(cudaGetLastError());
   return VAEB_OK;
 }
@@ -262,131 +254,5 @@ extern "C" int vaeb_tc_gemm_test(int32_t device, int32_t M, int32_t N, int32_t K
     if (e != cudaSuccess) { vaeb_set_error(std::string("tc_gemm copy: ") + cudaGetErrorString(e)); rc = VAEB_ECUDA; }
   }
   cudaFree(dA); cudaFree(dB); cudaFree(dC);
-  return rc;
-}
-
-// Timeline probe of one GEMM launch (CTA 0): clock64 stamps written to dbg[40]
-//  [0] kernel start, [1] setup done, [2] last MMA issued, [3] accumulator ready, [4] epilogue done,
-//  [8+kb] producer got slot kb, [24+kb] consumer saw data of kb.  Returns also the event-timed duration of
-//  `iters` back-to-back launches.
-extern "C" int vaeb_tc_gemm_probe(int32_t device, int32_t M, int32_t N, int32_t K, int32_t a_mn_major,
-                                  int32_t b_mn_major, int32_t iters, int64_t* stamps, float* us_per_launch) {
-  VAEB_CUDA(cudaSetDevice(device));
-  void *dA = nullptr, *dB = nullptr; float* dC = nullptr; long long* dD = nullptr;
-  VAEB_CUDA(cudaMalloc(&dA, (size_t)M * K * 2)); VAEB_CUDA(cudaMalloc(&dB, (size_t)N * K * 2));
-  VAEB_CUDA(cudaMalloc((void**)&dC, (size_t)M * N * 4)); VAEB_CUDA(cudaMalloc((void**)&dD, 40 * 8));
-  VAEB_CUDA(cudaMemset(dA, 0, (size_t)M * K * 2)); VAEB_CUDA(cudaMemset(dB, 0, (size_t)N * K * 2));
-  VAEB_CUDA(cudaMemset(dD, 0, 40 * 8));
-  CUtensorMap tmA, tmB;
-  if (a_mn_major) VAEB_TRY(vaeb_make_tmap_bf16(&tmA, dA, K, M, M, 64));
-  else VAEB_TRY(vaeb_make_tmap_bf16(&tmA, dA, M, K, K, BM));
-  if (b_mn_major) VAEB_TRY(vaeb_make_tmap_bf16(&tmB, dB, K, N, N, 64));
-  else VAEB_TRY(vaeb_make_tmap_bf16(&tmB, dB, N, K, K, 64));
-  auto run = [&](long long* dbg) -> int {
-    if (a_mn_major && b_mn_major) return launch_tc_gemm<64, true, true>(tmA, tmB, dC, M, N, K, N, 0, dbg);
-    if (a_mn_major) return launch_tc_gemm<64, true, false>(tmA, tmB, dC, M, N, K, N, 0, dbg);
-    if (b_mn_major) return launch_tc_gemm<64, false, true>(tmA, tmB, dC, M, N, K, N, 0, dbg);
-    return launch_tc_gemm<64, false, false>(tmA, tmB, dC, M, N, K, N, 0, dbg);
-  };
-  for (int i = 0; i < 3; ++i) VAEB_TRY(run(nullptr));
-  VAEB_TRY(run(dD));
-  cudaEvent_t e0, e1;
-  VAEB_CUDA(cudaEventCreate(&e0)); VAEB_CUDA(cudaEventCreate(&e1));
-  VAEB_CUDA(cudaEventRecord(e0, 0));
-  for (int i = 0; i < iters; ++i) VAEB_TRY(run(nullptr));
-  VAEB_CUDA(cudaEventRecord(e1, 0));
-  VAEB_CUDA(cudaEventSynchronize(e1));
-  float ms = 0.f;
-  VAEB_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-  *us_per_launch = 1e3f * ms / iters;
-  VAEB_CUDA(cudaMemcpy(stamps, dD, 40 * 8, cudaMemcpyDeviceToHost));
-  cudaFree(dA); cudaFree(dB); cudaFree(dC); cudaFree(dD);
-  return VAEB_OK;
-}
-
-
-// ---- L2 -> shared-memory fill-rate probe ------------------------------------------------------------------
-// Every CTA (one per SM, or `ctas` of them) streams the SAME [rows x 64] bf16 matrix (rows*128 bytes, L2 resident
-// after the first pass) through a ring of `stages` stages with TMA boxes of `box_rows` rows, `batch` boxes per stage
-// (one mbarrier wait + one expect_tx per stage, like a GEMM producer loop), `passes` times, and does nothing else:
-// the rate at which ONE issuing thread can fill shared memory from L2 when all SMs read one hot weight matrix -- the
-// access pattern of the persistent layers and of the IS kernel.  Returns GB/s over all CTAs.
-namespace {
-__global__ void __launch_bounds__(128, 1)
-tma_fill_kernel(const __grid_constant__ CUtensorMap map, int rows, int box_rows, int batch, int stages, int passes,
-                int producers, unsigned long long* sink) {
-  extern __shared__ uint8_t fill_smem_raw[];
-  uint8_t* smem0 = (uint8_t*)(((uintptr_t)fill_smem_raw + 1023) & ~(uintptr_t)1023);
-  const int box_bytes = box_rows * 128, stage_bytes = batch * box_bytes;
-  // `producers` issuing threads (lane 0 of warps 0..producers-1), each with its own ring and barriers
-  const int w = threadIdx.x >> 5;
-  const size_t ring_bytes = ((size_t)stages * stage_bytes + stages * 8 + 1023) & ~(size_t)1023;
-  uint8_t* smem = smem0 + (size_t)w * ring_bytes;
-  uint64_t* full = (uint64_t*)(smem + (size_t)stages * stage_bytes);
-  const bool issuer = (threadIdx.x & 31) == 0 && w < producers;
-  if (issuer) {
-    tc::tma_prefetch_desc(&map);
-    for (int s = 0; s < stages; ++s) tc::mbar_init(&full[s], 1);
-    tc::fence_barrier_init();
-  }
-  __syncthreads();
-  if (issuer) {
-    const int boxes = rows / box_rows;
-    const long long total = (long long)(boxes / batch) * passes / producers;       // stages issued by this thread
-    long long issued = 0, done = 0;
-    const int start = (int)((blockIdx.x * 7 + w * 13) % boxes);                     // start at different rows
-    auto issue = [&](long long it) {
-      const int s = (int)(it % stages);
-      tc::mbar_expect_tx(&full[s], stage_bytes);
-      for (int b = 0; b < batch; ++b)
-        tc::tma_load_2d(smem + (size_t)s * stage_bytes + (size_t)b * box_bytes, &map, &full[s], 0,
-                        (int)((start + it * batch + b) % boxes) * box_rows);
-    };
-    for (; issued < total && issued < stages; ++issued) issue(issued);
-    for (; done < total; ++done) {
-      const int s = (int)(done % stages);
-      tc::mbar_wait(&full[s], (uint32_t)((done / stages) & 1));
-      if (issued < total) { issue(issued); ++issued; }
-    }
-    if (sink) atomicAdd(sink, (unsigned long long)done);
-  }
-}
-}  // namespace
-
-extern "C" int vaeb_tma_fill_probe(int32_t device, int32_t rows, int32_t box_rows, int32_t batch, int32_t stages,
-                                   int32_t passes, int32_t ctas, int32_t producers, float* gbytes_per_s) {
-  VAEB_REQUIRE(gbytes_per_s && rows > 0 && box_rows >= 8 && box_rows <= 256 && batch >= 1 &&
-               rows % (box_rows * batch) == 0 && stages >= 1 && passes >= 1 && ctas >= 1 && producers >= 1 && producers <= 4,
-               "bad argument");
-  passes = (passes + producers - 1) / producers * producers;
-  const size_t smem = (((size_t)stages * batch * box_rows * 128 + stages * 8 + 1023) & ~(size_t)1023) * producers + 2048;
-  VAEB_REQUIRE(smem <= 227 * 1024, "ring does not fit in shared memory");
-  VAEB_CUDA(cudaSetDevice(device));
-  void* d = nullptr;
-  unsigned long long* sink = nullptr;
-  VAEB_CUDA(cudaMalloc(&d, (size_t)rows * 128));
-  VAEB_CUDA(cudaMemset(d, 0, (size_t)rows * 128));
-  VAEB_CUDA(cudaMalloc((void**)&sink, 8));
-  VAEB_CUDA(cudaMemset(sink, 0, 8));
-  CUtensorMap tm;
-  int rc = vaeb_make_tmap_bf16(&tm, d, (uint64_t)rows, 64, 64, (uint32_t)box_rows);
-  if (rc == VAEB_OK) {
-    cudaError_t e = cudaFuncSetAttribute(tma_fill_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    cudaEvent_t e0, e1;
-    cudaEventCreate(&e0); cudaEventCreate(&e1);
-    if (e == cudaSuccess) {
-      tma_fill_kernel<<<ctas, 128, smem>>>(tm, rows, box_rows, batch, stages, producers, producers, sink);   // warm-up: into L2
-      cudaEventRecord(e0);
-      tma_fill_kernel<<<ctas, 128, smem>>>(tm, rows, box_rows, batch, stages, passes, producers, sink);
-      cudaEventRecord(e1);
-      e = cudaEventSynchronize(e1);
-    }
-    float ms = 0.f;
-    if (e == cudaSuccess) e = cudaEventElapsedTime(&ms, e0, e1);
-    cudaEventDestroy(e0); cudaEventDestroy(e1);
-    if (e != cudaSuccess) { vaeb_set_error(std::string("tma fill probe: ") + cudaGetErrorString(e)); rc = VAEB_ECUDA; }
-    else *gbytes_per_s = (float)((double)rows * 128.0 * passes * ctas / (ms * 1e-3) / 1e9);
-  }
-  cudaFree(d); cudaFree(sink);
   return rc;
 }

@@ -26,7 +26,7 @@ namespace {
 
 // contraction extent of one ring stage: the weight gradients in plain bf16 (both operands MN-major, one 3-D box each)
 // take 128 rows per stage -- two 32 KB boxes per mbarrier round trip instead of two 16 KB ones: their producer is bound
-// by issues (wait + expect_tx + ~120 ns per box, tools/tma_fill_probe.py), not by bytes
+// by issues (wait + expect_tx + ~120 ns per box, the TMA fill-rate probe, profiles/r1_c3_phases.txt), not by bytes
 template <bool A_MN, bool B_MN, int NS>
 constexpr int stage_k() { return (A_MN && B_MN && NS == 1) ? 2 * BK : BK; }
 
@@ -440,9 +440,8 @@ cudaError_t launch_layer_persistent(cudaStream_t st, const LayerMaps& maps, cons
   cfg.attrs = &attr;
   // always a programmatic dependent launch: one CTA per SM with ~200 KB of shared memory never shares an SM with the
   // kernel before it, so its prologue (barriers, TMEM, descriptors) simply hides behind that kernel's tail
-  // (16384 rows, bf16: 250 -> 239 us per update; VAEB_NO_PDL=1 switches it off)
-  static const bool no_pdl = getenv("VAEB_NO_PDL") != nullptr;
-  cfg.numAttrs = no_pdl ? 0 : 1;
+  // (16384 rows, bf16: 250 -> 239 us per update)
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kfn, maps, epi, M, N, K, a_row_off);
 }
 
@@ -471,12 +470,11 @@ cudaError_t launch_layer(cudaStream_t st, const LayerMaps& maps, const Epi& epi,
   cudaLaunchAttribute attr{};
   attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr.val.programmaticStreamSerializationAllowed = 1;
-  static const bool no_pdl = getenv("VAEB_NO_PDL") != nullptr;      // measurement switch
   cfg.attrs = &attr;
   // worth it when launch latency and prologue dominate, i.e. when every kernel of the step is at most about one
   // wave (tc_set_pdl): 2048 rows 195 -> 163 us per update.  With several waves the early CTAs of the dependent grid
   // only take SM slots from the tail of the previous kernel (16384 rows, bf16: 463 -> 494 us).
-  cfg.numAttrs = (no_pdl || !g_pdl) ? 0 : 1;
+  cfg.numAttrs = g_pdl ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kfn, maps, epi, M, N, K, a_row_off);
 }
 
@@ -974,9 +972,8 @@ cudaError_t tc_wgrad_all(cudaStream_t st, int64_t* launches, const TcMaps& m, in
   cudaLaunchAttribute attr{};
   attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr.val.programmaticStreamSerializationAllowed = 1;
-  static const bool no_pdl = getenv("VAEB_NO_PDL") != nullptr;
   cfg.attrs = &attr;
-  cfg.numAttrs = no_pdl ? 0 : 1;
+  cfg.numAttrs = 1;
   ++*launches;
   auto go = [&](auto kfn, int smem) -> cudaError_t {
     cudaError_t e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);

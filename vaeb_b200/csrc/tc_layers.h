@@ -131,7 +131,6 @@ struct TcTailArgs {
   // data parallel over peer memory (world == 1: unused)
   int world, rank; unsigned int epoch;
   float* gsum[TC_MAX_PEERS]; unsigned int* flags[TC_MAX_PEERS]; float* peer_params[TC_MAX_PEERS]; float* peer_ada[TC_MAX_PEERS];
-  long long* stamps;       // debug (VAEB_TAIL_STAMPS): 8 %globaltimer values of this launch, written by block 0
   // Adam (adam.cuh): `ada` holds m and v holds the second moment; peer_ada / peer_v are every rank's m / v
   float alpha_t, s2_t, b1, b2, adam_eps;
   float* v; float* peer_v[TC_MAX_PEERS];

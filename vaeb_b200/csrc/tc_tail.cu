@@ -98,22 +98,13 @@ __device__ __forceinline__ void put_pair(__nv_bfloat16* hi, __nv_bfloat16* lo, s
   if (lo) lo[o] = __float2bfloat16_rn(v - __bfloat162float(h));
 }
 
-__device__ __forceinline__ void stamp(const TcTailArgs& a, int k) {
-  if (a.stamps && blockIdx.x == 0 && threadIdx.x == 0) {
-    long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    a.stamps[k] = t;
-  }
-}
-
 template <bool ADAM>
 __global__ void __launch_bounds__(TAIL_THREADS)
 tc_tail_kernel(const TcTailArgs a) {
   __shared__ float red[32];
-  // programmatic dependent launch (VAEB_TAIL_PDL, default on): the grid is scheduled while the weight-gradient launch drains
+  // programmatic dependent launch: the grid is scheduled while the weight-gradient launch drains
   // (its CTAs fill the SMs: nothing of this grid becomes resident before they exit); nothing is read before this point
   asm volatile("griddepcontrol.wait;" ::: "memory");
-  stamp(a, 0);
   const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t nth = (int64_t)gridDim.x * blockDim.x;
   unsigned int bar_target = a.bar_base;
@@ -229,10 +220,8 @@ tc_tail_kernel(const TcTailArgs a) {
   }
   const float bs = block_sum(v, red);
   if (threadIdx.x == 0) a.block_part[blockIdx.x] = bs;
-  stamp(a, 1);
   bar_target += gridDim.x;
   grid_barrier(a.bar, bar_target);
-  stamp(a, 2);
 
   // total bound of this rank: block 0, fixed order
   float base = 0.f;
@@ -268,7 +257,6 @@ tc_tail_kernel(const TcTailArgs a) {
       }
     }
     __syncthreads();
-    stamp(a, 3);
     const int64_t n4 = a.padded / 4;
     const int64_t per = (n4 + a.world - 1) / a.world;
     const int64_t lo = per * a.rank, hi = lo + per < n4 ? lo + per : n4;
@@ -312,10 +300,8 @@ tc_tail_kernel(const TcTailArgs a) {
       *a.scalar_out = (a.mult * t) / a.div;
     }
     __threadfence_system();
-    stamp(a, 4);
     bar_target += gridDim.x;
     grid_barrier(a.bar, bar_target);
-    stamp(a, 5);
     if (blockIdx.x == 0 && threadIdx.x < a.world) {      // "my slice is everywhere": thread r tells peer r
       __threadfence_system();
       st_relaxed_sys(a.flags[threadIdx.x] + a.world + a.rank, a.epoch);
@@ -329,7 +315,6 @@ tc_tail_kernel(const TcTailArgs a) {
       }
     }
     __syncthreads();
-    stamp(a, 6);
   }
 
   // ---- P3: bf16 (hi, lo) operand mirrors of the new weights, in the layouts the TMA maps of the next step read --------
@@ -378,7 +363,6 @@ tc_tail_kernel(const TcTailArgs a) {
     mirror(W2, w2h, w2l, H, D, a.ldd);
   }
   mirror(W1, w1h, w1l, Z, H, a.ldh);
-  stamp(a, 7);
   for (int i = t32; i < H * Z; i += n32) {      // W4[k, j], W5[k, j]
     const int k = i / Z, j = i - k * Z;
     const float v4 = __ldcg(W4 + i), v5 = __ldcg(W5 + i);
@@ -394,7 +378,6 @@ tc_tail_kernel(const TcTailArgs a) {
 }  // namespace
 
 cudaError_t tc_tail_launch(cudaStream_t st, int64_t* launches, const TcTailArgs& a, int grid, bool adam) {
-  static const bool pdl = [] { const char* e = getenv("VAEB_TAIL_PDL"); return !(e && e[0] == '0') && !getenv("VAEB_NO_PDL"); }();
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(TAIL_THREADS);
@@ -404,7 +387,7 @@ cudaError_t tc_tail_launch(cudaStream_t st, int64_t* launches, const TcTailArgs&
   attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr.val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = &attr;
-  cfg.numAttrs = pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   ++*launches;
   return adam ? cudaLaunchKernelEx(&cfg, tc_tail_kernel<true>, a) : cudaLaunchKernelEx(&cfg, tc_tail_kernel<false>, a);
 }
@@ -418,8 +401,6 @@ int tc_tail_grid(int n_sm, bool adam) {
                                : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tc_tail_kernel<false>, TAIL_THREADS, 0);
     if (oe != cudaSuccess || per_sm < 1) per_sm = 1;
     if (per_sm > 6) per_sm = 6;
-    const char* e = getenv("VAEB_TAIL_PER_SM");       // measurement switch
-    if (e && atoi(e) >= 1 && atoi(e) < per_sm) per_sm = atoi(e);
   }
   return per_sm * n_sm;
 }

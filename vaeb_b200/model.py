@@ -463,10 +463,10 @@ class VAEB(object):
     def kl_step(self, t):
         _lib.check(self._lib.vaeb_set_kl_step(self._h, int(t)))
 
-    def profile_optimizer(self, iters=20, variant=0):
+    def profile_optimizer(self, iters=20):
         """(ms per launch, algorithmic bytes per launch) of the flat Adagrad pass over this model's buffers."""
         ms, by = C.c_float(), C.c_double()
-        _lib.check(self._lib.vaeb_profile_optimizer(self._h, int(iters), int(variant), C.byref(ms), C.byref(by)))
+        _lib.check(self._lib.vaeb_profile_optimizer(self._h, int(iters), C.byref(ms), C.byref(by)))
         return ms.value, by.value
 
     def step_kernel_name(self, rows=None):
