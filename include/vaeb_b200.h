@@ -87,7 +87,8 @@ typedef struct vaeb_config {
 #define VAEB_ACT_RELU 3
 
 const char* vaeb_last_error(void);
-int vaeb_version(void);      /* 105: vaeb_profile_optimizer loses its variant argument (vaeb_config unchanged);
+int vaeb_version(void);      /* 106: adds vaeb_step_counter, the getter of vaeb_set_step_counter (vaeb_config unchanged);
+                                105: vaeb_profile_optimizer loses its variant argument (vaeb_config unchanged);
                                 104: adds the KL weight (vaeb_set_kl_weight, vaeb_kl_step, vaeb_set_kl_step; vaeb_config
                                 unchanged);
                                 103: adds Adam (vaeb_set_adam, vaeb_adam_step, vaeb_set_adam_step; vaeb_config unchanged);
@@ -301,7 +302,36 @@ int vaeb_mlp_forward(vaeb_handle* h, const float* x, int64_t n, int32_t n_layers
  * out[n] = N(0,1) for flat elements first_elem.. of (stream, step, sample). */
 int vaeb_philox_normal(vaeb_handle* h, int32_t stream, uint32_t step, uint32_t sample,
                        int64_t first_elem, int64_t n, float* out);
+/* The Philox step counter: every update, validate and reconstruct draws its noise from (seed, stream, step) and advances
+ * it by one.  vaeb_step_counter first launches any streaming updates still pending (as vaeb_get_tensors does). */
 int vaeb_set_step_counter(vaeb_handle* h, uint32_t step);
+int vaeb_step_counter(vaeb_handle* h, uint32_t* step);
+
+/* ---- The training state of a handle ----------------------------------------------------------------------------
+ * What a binding saves between two updates, and restores into a fresh handle, so that the next update -- and every
+ * validate, reconstruct and update after it -- computes the same bits as a run that was never interrupted:
+ *   buffers (vaeb_get_tensors / vaeb_set_tensors, by `which`):
+ *     0             the parameters;
+ *     1             Adagrad's accumulators, AdaDelta's g_ac or Adam's m;
+ *     9             AdaDelta's dx_ac or Adam's v (those two optimizers only);
+ *     3, 4, 5, 6    the variational means and sigmas and their Adagrad accumulators (full-VB estimators only);
+ *     10, 11        VAEB_EST_FVB_SAMPLED only: theta and zeta of the next update.  The tensor-core step kernel draws
+ *                   them for step t + 1 in the epilogues of step t (MUFU forms), so they are not re-derivable with the
+ *                   same bits.  Reading them returns the draw for the current step counter (made then, with the
+ *                   accurate forms of the other paths, if nothing has drawn it yet); writing them declares them the
+ *                   draw for the current step counter;
+ *   counters:
+ *     vaeb_step_counter / vaeb_set_step_counter, vaeb_adam_step / vaeb_set_adam_step (Adam),
+ *     vaeb_kl_step / vaeb_set_kl_step.
+ * Restore in this order: vaeb_create with the same vaeb_config (seed included) and vaeb_upload_data; then the settings
+ * that reset counters or accumulators -- vaeb_set_optimizer or vaeb_set_adam, vaeb_set_hidden_activation,
+ * vaeb_set_kl_weight; then buffers 0-9; then the three counters; then buffers 10 and 11 (after the step counter, whose
+ * draw they are).
+ * Not state: the gradient buffers (2, 7, 8), which every update overwrites; buffers 10 and 11 of the other estimators;
+ * the operand mirrors of the tensor-core paths and the parameter double buffer of the single-launch kernels, which
+ * are rebuilt from the fp32 buffers with the bits the kernels themselves would have written.  Streaming updates
+ * (vaeb_update_host_async) must be collected before the state is read.  Data-parallel ranks hold the same state: one
+ * rank saves it, every rank restores it before attaching. */
 
 /* Data-parallel training (new; SURVEY 8e): one handle per rank/GPU.  Rank 0 makes an id,
  * the host plumbing broadcasts the 128 bytes, every rank attaches.  After attaching,

@@ -16,6 +16,7 @@ PREC_FP32, PREC_BF16, PREC_BF16X3 = 0, 1, 2
 BUF_PARAMS, BUF_ADA, BUF_GRADS, BUF_VMU, BUF_VSIG, BUF_ADA_MU, BUF_ADA_SIG, BUF_GMU, BUF_GSIG, BUF_ADA2 = range(10)
 OPT_ADAGRAD, OPT_ADADELTA, OPT_ADAM = 0, 1, 2
 BUF_ADAM_V = 9          # Adam's second moment (BUF_ADA is its first moment)
+BUF_THETA, BUF_ZETA = 10, 11    # sampled full VB: theta and zeta of the next update
 AE_DEGENERATE, AE_VANILLA = 0, 1
 
 
@@ -75,6 +76,7 @@ EXPORTS = {
                                    C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int32, C.c_void_p]),
     "vaeb_philox_normal": (C.c_int, [C.c_void_p, C.c_int32, C.c_uint32, C.c_uint32, C.c_int64, C.c_int64, C.c_void_p]),
     "vaeb_set_step_counter": (C.c_int, [C.c_void_p, C.c_uint32]),
+    "vaeb_step_counter": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint32)]),
     "vaeb_comm_unique_id": (C.c_int, [C.c_char_p, C.c_void_p]),
     "vaeb_comm_attach": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int32, C.c_int32]),
     "vaeb_comm_detach": (C.c_int, [C.c_void_p]),

@@ -710,7 +710,7 @@ float* flat_by_which(vaeb_handle* h, int which) {
     case 7: return h->d_gmu;
     case 8: return h->d_gsig;
     case 9: return h->optimizer == VAEB_OPT_ADAM ? h->d_adam_v : h->d_ada2;
-    case 10: return h->d_theta;     // sampled full VB: theta of the next step (debug / tests)
+    case 10: return h->d_theta;     // sampled full VB: theta and zeta of the next step (training state)
     case 11: return h->d_zeta;
     default: return nullptr;
   }
@@ -839,7 +839,7 @@ static int async_flush(vaeb_handle* h);
 static void p2p_release(vaeb_handle* h);   // unmaps the peers' buffers (data parallel over peer memory)   // launches streaming updates that were copied but not yet started
 
 const char* vaeb_last_error(void) { return g_last_error.c_str(); }
-int vaeb_version(void) { return 105; }   // 105: vaeb_profile_optimizer without variant; 104: KL weight; 103: Adam; 102: vaeb_encode, vaeb_sample, vaeb_validate_terms (101: encoder_hidden_layers)
+int vaeb_version(void) { return 106; }   // 106: vaeb_step_counter; 105: vaeb_profile_optimizer without variant; 104: KL weight; 103: Adam; 102: vaeb_encode, vaeb_sample, vaeb_validate_terms (101: encoder_hidden_layers)
 int vaeb_config_size(void) { return (int)sizeof(vaeb_config); }
 
 int vaeb_create(const vaeb_config* cfg, vaeb_handle** out) {
@@ -995,6 +995,8 @@ int vaeb_set_tensors(vaeb_handle* h, int32_t which, const float* const* tensors)
     VAEB_CUDA(cudaMemcpyAsync(flat + h->lay.off[t], tensors[t], n * sizeof(float), cudaMemcpyHostToDevice, h->stream));
   }
   VAEB_CUDA(cudaStreamSynchronize(h->stream));
+  // sampled full VB: a theta / zeta written here is the draw of the current step (the training state, see the header)
+  if ((which == 10 || which == 11) && h->cfg.estimator == VAEB_EST_FVB_SAMPLED) h->steptc.theta_step = (long long)h->step;
   return VAEB_OK;
 }
 
@@ -1004,6 +1006,14 @@ int vaeb_get_tensors(vaeb_handle* h, int32_t which, float* const* tensors) {
   float* flat = flat_by_which(h, which);
   VAEB_REQUIRE(flat, "buffer not available for this estimator");
   VAEB_CUDA(cudaSetDevice(h->cfg.device));
+  if ((which == 10 || which == 11) && h->cfg.estimator == VAEB_EST_FVB_SAMPLED && h->steptc.theta_step != (long long)h->step) {
+    // sampled full VB: return the theta / zeta the next update uses -- the draw the step kernel would make for the
+    // current step, made now and kept for it (an update through another path draws its own, the same bits)
+    VAEB_LAUNCH(launch_sample_theta(h->stream, &h->launches, h->d_vmu, h->d_vsig, nullptr, h->cfg.seed, h->step,
+                                    h->lay.total, h->d_theta, h->d_zeta));
+    invalidate_weight_mirrors(h);
+    h->steptc.theta_step = (long long)h->step;
+  }
   for (int t = 0; t < h->lay.n; ++t) {
     const size_t n = (size_t)h->lay.rows[t] * h->lay.cols[t];
     VAEB_CUDA(cudaMemcpyAsync(tensors[t], flat + h->lay.off[t], n * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
@@ -1833,6 +1843,13 @@ int vaeb_philox_normal(vaeb_handle* h, int32_t stream, uint32_t step, uint32_t s
 int vaeb_set_step_counter(vaeb_handle* h, uint32_t step) {
   VAEB_REQUIRE(h, "null handle");
   h->step = step;
+  return VAEB_OK;
+}
+
+int vaeb_step_counter(vaeb_handle* h, uint32_t* step) {
+  if (h && h->a_pending) VAEB_TRY(async_flush(h));     // streaming updates advance the counter when they are launched
+  VAEB_REQUIRE(h && step, "null argument");
+  *step = h->step;
   return VAEB_OK;
 }
 

@@ -178,6 +178,11 @@ struct vaeb_handle {
 
 // The parameters changed behind the cached bf16 weight mirrors: those of the tensor-core step kernel (step_tc.cu) and
 // those of the large-batch path (written by tc_prepare_weights or the tail kernel).
-inline void invalidate_weight_mirrors(vaeb_handle* h) { h->steptc.mirrors_valid = false; h->tc.weights_ready = false; }
+// the parameters may have changed: the operand mirrors and the sampled full-VB theta of the step kernel are stale
+inline void invalidate_weight_mirrors(vaeb_handle* h) {
+  h->steptc.mirrors_valid = false;
+  h->steptc.theta_step = -1;
+  h->tc.weights_ready = false;
+}
 
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }

@@ -1371,7 +1371,7 @@ __global__ void __launch_bounds__(NT, 1) step_tc_kernel(const __grid_constant__ 
 
   for (int s = 0; s < p.n_steps; ++s) {
     const float* x = x_of(s);
-    const int par = (int)((p.step0 + (uint32_t)s) & 1u);        // which copy of the k-major [W4|W5] mirror this step reads
+    const int par = (p.w45_par0 + s) & 1;                        // which copy of the k-major [W4|W5] mirror this step reads
     c.step = p.step0 + (uint32_t)s; c.tp = 0.f;
     // sampled full VB: the bound of the previous step needs the thetaPrior sums of ITS update epilogues (P5, P6): it is
     // summed here, by a CTA that has no enc1 item, before P2 / P3 overwrite the row partials
@@ -1660,6 +1660,7 @@ int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_kl, const 
   p.x_base = (d_order && d_xrows) ? d_xrows : h->d_x; p.batch_order = d_order; p.x_direct = d_xrows;
   p.eps_inj = d_eps;
   p.seed = h->cfg.seed; p.step0 = h->step; p.row_offset = 0;
+  p.w45_par0 = s.w45_par;
   p.he = s.he; p.hd = s.hd; p.mu = s.mu; p.ls = s.ls; p.eps = s.eps; p.z = s.z;
   p.dd_km = s.act + s.o_dd_km; p.x_km = s.act + s.o_x_km; p.x_t = s.act + s.o_x_t;
   p.m_w45k = s.m_w45k; p.w45k_bytes = p.HP * 64 * 4;
@@ -1673,7 +1674,9 @@ int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_kl, const 
   if (p.fvb == 2) {
     // the layers run on the sampled theta; the data term of the gradient carries the factor M of VAEB.py:364
     p.P = h->d_theta; p.zeta = h->d_zeta; p.w = (float)rows;
-    if (!s.mirrors_valid || s.theta_step != (long long)h->step) {
+    // theta and zeta of this step: drawn by the previous launch's epilogues (MUFU forms), restored with
+    // vaeb_set_tensors(10, 11), or drawn here; the operand mirrors are rebuilt from the fp32 theta below when stale
+    if (s.theta_step != (long long)h->step) {
       VAEB_CUDA(launch_sample_theta(h->stream, &h->launches, h->d_vmu, h->d_vsig, nullptr, h->cfg.seed, h->step, l.total,
                                     h->d_theta, h->d_zeta));
       invalidate_weight_mirrors(h);
@@ -1733,6 +1736,7 @@ int step_tc_launch(vaeb_handle* h, const int* d_order, const float* d_kl, const 
   // an aborted launch passed 4 of the grid barriers of step `done`
   s.bar_count += (unsigned long long)s.n_cta * ((unsigned long long)(p.fvb == 1 ? 3 : N_PHASES) * (unsigned long long)done + (done < n_steps ? 4ull : 0ull));
   h->step += (uint32_t)done;
+  s.w45_par ^= done & 1;              // each completed step wrote the other copy
   s.theta_step = (long long)h->step;
   if (done < n_steps) {
     // steps done .. n_steps-1 through the fp32 FFMA kernel (same contract; it invalidates the operand mirrors)

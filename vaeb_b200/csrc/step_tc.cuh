@@ -59,6 +59,7 @@ struct Params {
   const float* x_base; const int* batch_order; const float* x_direct;
   const float* eps_inj;
   uint64_t seed; uint32_t step0; int64_t row_offset;
+  int w45_par0;                         // the copy of the k-major [W4|W5] mirror that holds theta at the first step
   float *he, *hd, *mu, *ls, *eps, *z;   // fp32 copies the epilogues read: [MP, HP], [MP, HP], [MP, Z] x 4
   float *partial, *aux;                 // [MP, tiles of dec2] log-likelihood row partials; [MP] KL / LA row terms
   int n_tiles3;                         // n tiles of dec2 (partial's leading dimension)
@@ -102,7 +103,11 @@ struct StepTcState {
   long long* d_timing = nullptr; int timing_cap = 0;
   int* d_status = nullptr;
   float* tprior_part = nullptr;
-  long long theta_step = -1;            // sampled full VB: the step the theta buffer / mirrors were drawn for
+  long long theta_step = -1;            // sampled full VB: the step the theta / zeta buffers were drawn for (-1: stale)
+  // which of the two copies of the k-major [W4|W5] mirror holds the current parameters: a step reads one and its
+  // epilogue writes the next step's into the other.  Kept here rather than taken from the step counter's parity,
+  // which validate / reconstruct advance without touching the mirrors.
+  int w45_par = 0;
 };
 
 // n_steps updates in one launch (same contract as fused_step_launch)

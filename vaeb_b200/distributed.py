@@ -23,7 +23,8 @@ def broadcast_bytes(payload, src=0):
 def attach_data_parallel(model):
     """Give `model` (one per rank, built on this rank's GPU with batch_size = per-rank share)
     an NCCL communicator: afterwards every update all-reduces gradients and the bound.  The ranks must weight the
-    latent term alike (set_kl_weight, kl_step)."""
+    latent term alike (set_kl_weight, kl_step) and stand at the same Philox step (a run resumed on every rank from the
+    same checkpoint does)."""
     import torch.distributed as dist
     from .model import comm_unique_id
     rank, world = dist.get_rank(), dist.get_world_size()
@@ -31,6 +32,9 @@ def attach_data_parallel(model):
         schedules = [None] * world
         dist.all_gather_object(schedules, (model.kl_weight, model.kl_warmup, model.kl_step))
         check_same_kl_weight(schedules)
+        steps = [None] * world
+        dist.all_gather_object(steps, model.step_counter)
+        check_same_step_counter(steps)
     uid = comm_unique_id() if rank == 0 else None
     uid = broadcast_bytes(uid, 0)
     model.attach_comm(uid, rank, world)
@@ -61,6 +65,36 @@ def check_same_kl_weight(schedules):
     one objective only when every rank weights the latent term alike, so a mix is refused."""
     if len(set(schedules)) > 1:
         raise ValueError("data parallel needs the same KL weight, warm-up and KL step on every rank, got %s" % (schedules,))
+
+
+def check_same_step_counter(steps):
+    """`steps`: every rank's Philox step counter, in rank order.  Each rank draws its rows' noise from (seed, step,
+    global row); ranks at different steps -- resumed from different checkpoints, say -- would not train one model."""
+    if len(set(steps)) > 1:
+        raise ValueError("data parallel needs the same step counter on every rank, got %s" % (steps,))
+
+
+def save_checkpoint(model, path, driver_state=None):
+    """Collective: the training state of a data-parallel model, written by rank 0 (the state is replicated) with the
+    data fingerprint of every rank's shard.  Every rank returns once the file is in place."""
+    import torch.distributed as dist
+    from . import checkpoint
+    rank, world = dist.get_rank(), dist.get_world_size()
+    header, arrays = model.training_state()
+    fps = [None] * world
+    dist.all_gather_object(fps, model._data_fp)
+    if rank == 0:
+        header.update(world_size=world, data=fps)
+        checkpoint.write(path, header, arrays, driver_state)
+    dist.barrier()
+
+
+def resume(path, x_shard, device, return_driver_state=False):
+    """This rank's model from a checkpoint of save_checkpoint, on its own shard; attach_data_parallel afterwards."""
+    import torch.distributed as dist
+    from .model import VAEB
+    return VAEB.resume(path, x_shard, device=device, rank=dist.get_rank(), world_size=dist.get_world_size(),
+                       return_driver_state=return_driver_state)
 
 
 def close_data_parallel(model):

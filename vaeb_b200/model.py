@@ -12,7 +12,7 @@ import ctypes as C
 
 import numpy as np
 
-from . import _lib, io
+from . import _lib, checkpoint, io
 from .rng import RandomStreams
 
 _NAMES_D = ["W3", "W4", "W5", "W1", "W2", "b3", "b4", "b5", "b1", "b2"]
@@ -104,6 +104,11 @@ class VAEB(object):
         self.fullVariational = bool(fullVariational)
         self.variant = variant
         self.eps_mode = eps_mode
+        self.seed = int(seed)
+        self.sample_weights = bool(sample_weights)
+        self.adam_betas = (float(adam_betas[0]), float(adam_betas[1]))
+        self.adam_eps = float(adam_eps)
+        self._rank, self._world = 0, 1
         if eps_mode not in ("philox", "theano"):
             raise ValueError("eps_mode must be 'philox' or 'theano'")
         if self.fullVariational:
@@ -186,7 +191,9 @@ class VAEB(object):
         self.kl_weight, self.kl_warmup = 1.0, 0
         if kl_weight != 1.0 or kl_warmup != 0:
             self.set_kl_weight(kl_weight, kl_warmup)
-        _lib.check(self._lib.vaeb_upload_data(self._h, _ptr(_f32(x_train)), self.N))   # VAEB.py:184
+        xf = _f32(x_train)
+        _lib.check(self._lib.vaeb_upload_data(self._h, _ptr(xf), self.N))   # VAEB.py:184
+        self._data_fp = checkpoint.data_fingerprint(xf)          # what a checkpoint of this model was trained on
 
     # ---- parameters -------------------------------------------------------------------
     def initialize_params(self, params):
@@ -409,6 +416,116 @@ class VAEB(object):
                      **dict({"encoder_layers": header.get("encoder_layers", 1)}, **kwargs))
         return model, data
 
+    # ---- training state ------------------------------------------------------------------
+    def _ctor_args(self):
+        """The constructor arguments that shape the computation (everything but the data and the device)."""
+        return dict(continuous=self.continuous, hidden_units=self.n_hidden_units, latent_size=self.n_latent,
+                    batch_size=self.batch_size, L=self.L, learning_rate=self.learning_rate,
+                    genericEstimator=self.genericEstimator, fullVariational=self.fullVariational,
+                    precision=self.precision, eps_mode=self.eps_mode, sample_weights=self.sample_weights,
+                    variant=self.variant, seed=self.seed, optimizer=self.optimizer, activation=self.activation,
+                    encoder_layers=self.encoder_layers, adam_betas=list(self.adam_betas), adam_eps=self.adam_eps,
+                    kl_weight=self.kl_weight, kl_warmup=self.kl_warmup)
+
+    def _state_buffers(self):
+        """(file name, which) of the buffers of the training state (include/vaeb_b200.h), in restore order: theta and
+        zeta of sampled full VB (the draw of the current step) are restored after the counters."""
+        bufs = [("params", _lib.BUF_PARAMS), ("ada", _lib.BUF_ADA)]
+        if self.optimizer in ("adadelta", "adam"):
+            bufs.append(("ada2", _lib.BUF_ADA2))
+        if self._fvb:
+            bufs += [("vmu", _lib.BUF_VMU), ("vsig", _lib.BUF_VSIG), ("ada_mu", _lib.BUF_ADA_MU),
+                     ("ada_sig", _lib.BUF_ADA_SIG)]
+        if self._estimator == _lib.EST_FVB_SAMPLED:
+            bufs += [("theta", _lib.BUF_THETA), ("zeta", _lib.BUF_ZETA)]
+        return bufs
+
+    @property
+    def step_counter(self):
+        """The Philox step counter: every update, validate and reconstruct draws its noise from (seed, step)."""
+        t = C.c_uint32()
+        _lib.check(self._lib.vaeb_step_counter(self._h, C.byref(t)))
+        return t.value
+
+    @step_counter.setter
+    def step_counter(self, t):
+        _lib.check(self._lib.vaeb_set_step_counter(self._h, int(t)))
+
+    def training_state(self):
+        """(header, arrays) of a checkpoint: what `resume` needs to continue bit for bit."""
+        if self._async_keep:
+            raise ValueError("collect() the streaming updates before saving the training state")
+        arrays = {}
+        for name, which in self._state_buffers():
+            for nm, a in zip(self._names, self._get_buffer(which)):
+                arrays["%s.%s" % (name, nm)] = a
+        arrays["counter.step"] = np.array(self.step_counter, dtype=np.uint32)
+        arrays["counter.adam_step"] = np.array(self.adam_step, dtype=np.int64)
+        arrays["counter.kl_step"] = np.array(self.kl_step, dtype=np.int64)
+        if self.eps_mode == "theano":
+            checkpoint.pack_random_state(arrays, "seedgen", self.srng.gen_seedgen.get_state())
+            for k, node in enumerate(self.srng.nodes):
+                checkpoint.pack_random_state(arrays, "node%d" % k, node.get_state())
+        header = dict(vaeb_version=int(self._lib.vaeb_version()), args=self._ctor_args(),
+                      tensors=[[n, list(s)] for n, s in zip(self._names, self._shapes)],
+                      buffers=[name for name, _ in self._state_buffers()], world_size=self._world,
+                      data=[self._data_fp], theano_nodes=len(self.srng.nodes) if self.eps_mode == "theano" else 0)
+        return header, arrays
+
+    def save_checkpoint(self, path, driver_state=None):
+        """Write the complete training state to one .npz (vaeb_b200/checkpoint.py), atomically: parameters, optimizer
+        state, full-VB state, the step, Adam and KL counters, the host noise streams and `driver_state` (a dict of
+        arrays and scalars for the training loop).  `VAEB.resume` continues from it with the same bits as an
+        uninterrupted run.  Data parallel: vaeb_b200.distributed.save_checkpoint."""
+        if self._world > 1:
+            raise ValueError("a data-parallel model saves with vaeb_b200.distributed.save_checkpoint")
+        header, arrays = self.training_state()
+        checkpoint.write(path, header, arrays, driver_state)
+
+    @staticmethod
+    def resume(path, x_train, device=0, rank=0, world_size=1, return_driver_state=False):
+        """The model of a checkpoint, in exactly its saved state, on `device` with the rows `x_train` (this rank's
+        shard in data-parallel runs; attach_data_parallel afterwards).  Built with the constructor (which selects the
+        optimizer, the activation and the KL weight), then the buffers, then the counters.  ValueError naming the
+        field on an unknown format version, another data set, world size or tensor shape, or a missing array."""
+        header, arrays, driver = checkpoint.read(path)
+        a = dict(header["args"])
+        checkpoint.check_compatible(header, data=checkpoint.data_fingerprint(x_train), rank=rank, world_size=world_size)
+        need = lambda name: checkpoint.require(arrays, name)
+        params = [need("params.%s" % n) for n, _ in header["tensors"]]
+        model = VAEB(x_train, a["continuous"], a["hidden_units"], a["latent_size"], a["batch_size"], a["L"],
+                     a["learning_rate"], a["genericEstimator"], a["fullVariational"], params, device=device,
+                     precision=a["precision"], eps_mode=a["eps_mode"], sample_weights=a["sample_weights"],
+                     variant=a["variant"], seed=a["seed"], optimizer=a["optimizer"], activation=a["activation"],
+                     encoder_layers=a["encoder_layers"], adam_betas=tuple(a["adam_betas"]), adam_eps=a["adam_eps"],
+                     kl_weight=a["kl_weight"], kl_warmup=a["kl_warmup"])
+        try:
+            checkpoint.check_tensors(header, list(zip(model._names, model._shapes)))
+
+            def restore(buffers):
+                for name, which in buffers:
+                    model._set_buffer(which, [checkpoint.require(arrays, "%s.%s" % (name, n), shape)
+                                              for n, shape in zip(model._names, model._shapes)])
+
+            draws = (_lib.BUF_THETA, _lib.BUF_ZETA)
+            restore([b for b in model._state_buffers() if b[1] not in draws])
+            if model.optimizer == "adam":
+                model.adam_step = int(need("counter.adam_step"))
+            model.kl_step = int(need("counter.kl_step"))
+            model.step_counter = int(need("counter.step"))
+            restore([b for b in model._state_buffers() if b[1] in draws])     # the draw of the restored step
+            if model.eps_mode == "theano":
+                model.srng.gen_seedgen.set_state(checkpoint.unpack_random_state(arrays, "seedgen"))
+                model.srng.nodes = []
+                for k in range(int(header["theano_nodes"])):
+                    node = np.random.RandomState()
+                    node.set_state(checkpoint.unpack_random_state(arrays, "node%d" % k))
+                    model.srng.nodes.append(node)
+        except BaseException:
+            model.close()
+            raise
+        return (model, driver) if return_driver_state else model
+
     # ---- plumbing ------------------------------------------------------------------------
     def set_stream(self, cuda_stream):
         _lib.check(self._lib.vaeb_set_stream(self._h, C.c_void_p(cuda_stream)))
@@ -485,6 +602,7 @@ class VAEB(object):
         path = (nccl_library or _lib.nccl_library_path()).encode()
         buf = (C.c_uint8 * 128).from_buffer_copy(bytes(unique_id))
         _lib.check(self._lib.vaeb_comm_attach(self._h, path, buf, rank, world_size))
+        self._rank, self._world = int(rank), int(world_size)
 
     def p2p_export(self):
         """CUDA IPC handles (192 bytes) of this rank's gradient staging buffer, parameters and accumulators."""
